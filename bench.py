@@ -330,6 +330,25 @@ def oracle_agreement(gsmcal, raw, res, n_iq, tpl, coef, count, workers):
             "compared": "coarse_pos, fcch_pos, pos_info bit-exact; sampling/carrier ppm (both stages and totals) within 1e-3"}
 
 
+def dump_outputs(out_dir, res, record_type):
+    """What the timed path hands its caller: the per-stream result records (gsmcal_calibrate_batch_collect), in stream order, one
+    float64 array per record field (counts, flags and lengths are integers, exact in float64), so two builds can be compared field by
+    field on the same seeded inputs.
+
+    A stream that does not calibrate reports its ppm as inf (the reference's "no estimate", FCCH_fine_correction.m:8-15), so every
+    floating-point field is written finite: <field>.npy holds 0 where the value is not finite and <field>_nonfinite.npy says which
+    value it was (0 finite, 1 +inf, -1 -inf, 2 nan)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, ctype in record_type._fields_:
+        vals = [getattr(r, name) for r in res]
+        a = np.array([list(v) if isinstance(v, C.Array) else v for v in vals], dtype=np.float64)
+        if (ctype._type_ if issubclass(ctype, C.Array) else ctype) is C.c_double:
+            code = np.select([np.isposinf(a), np.isneginf(a), np.isnan(a)], [1.0, -1.0, 2.0], 0.0)
+            np.save(os.path.join(out_dir, name + "_nonfinite.npy"), code)
+            a = np.where(code == 0, a, 0.0)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ---------------------------------------------------------------------------------------------------
 def numa_pin(local_rank):
     """Pin this process (and the pinned host allocations it makes afterwards, first-touch) to the NUMA node of its GPU."""
@@ -539,7 +558,12 @@ def main():
     ap.add_argument("--debug", action="append", default=[], metavar="KEY=VALUE", help="gsmcal_debug_set(KEY, VALUE) before the run (A/B of kernel paths, see include/gsmcal.h)")
     ap.add_argument("--ingest", type=int, default=0, metavar="D",
                     help="instead of the benchmark: D loopback rtl_tcp replay servers -> gsmcal.ingest -> calibrate (SURVEY 8(f) row 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result records of the last timed step (rank 0's streams) as DIR/<field>.npy, float64 and finite "
+                         "(a non-finite value is stored as 0, with its kind in DIR/<field>_nonfinite.npy)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.weak and not args.streams:
         args.streams = 128
@@ -694,6 +718,8 @@ def main():
     clocks = sampler.stop()
     launches = gsmcal.launch_count()
     ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res, StreamResult)
     pipelined_phases = None
     if "13=1" in args.debug:                      # phase cycles of the last two batches of the timed run (the one before the last ran under the next front)
         cn = ["staging", "fir", "energies_k0", "chunk_sums", "prefix", "segment_starts", "diff_slide", "argmax", "certificate"]

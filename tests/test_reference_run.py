@@ -51,12 +51,14 @@ def test_run_reference_m_calls_the_reference_functions_in_script_order():
              "carrier_correct_post_SCH(", "total_ppm_calculation("]
     pos = [src.index(k) for k in order]
     assert pos == sorted(pos)                                   # gsm_sync_demod.m:107-124
-    ref = "/root/reference"
-    if os.path.isdir(ref):                                      # only in the build container
-        for fn in ("raw2iq", "FCCH_coarse_position", "move_fft_snr_runtime_avg", "FCCH_fine_correction", "SCH_corr_rate_correction",
-                   "carrier_correct_post_SCH", "total_ppm_calculation", "chn_filter_8x_4x", "chn_filter_4x"):
-            assert re.search(r"\b%s\(" % fn, src), fn          # the script calls it ...
-            assert os.path.exists(os.path.join(ref, fn + ".m")), fn   # ... and the reference defines it (nothing of ours shadows it)
+    with open(os.path.join(ROOT, "tests", "golden", "reference_functions.json")) as f:
+        defined = json.load(f)["functions"]                     # the reference's function files, with their defining lines
+    for fn in ("raw2iq", "FCCH_coarse_position", "move_fft_snr_runtime_avg", "FCCH_fine_correction", "SCH_corr_rate_correction",
+               "carrier_correct_post_SCH", "total_ppm_calculation", "chn_filter_8x_4x", "chn_filter_4x"):
+        assert re.search(r"\b%s\(" % fn, src), fn              # the script calls it ...
+        assert defined[fn].startswith(fn + ".m:"), fn           # ... and the reference defines it ...
+        assert not re.search(r"^\s*function\b.*\b%s\s*\(" % fn, src, re.M), fn                       # ... not the script itself
+        assert not any(os.path.exists(os.path.join(d, fn + ".m")) for d in (os.path.join(ROOT, "oracle"), RUN)), fn   # nor a .m of ours
 
 
 def _have_run():
