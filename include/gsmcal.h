@@ -216,6 +216,41 @@ int gsmcal_calibrate_batch_r(const uint8_t *raw, int raw_mem, int64_t n_iq, int6
                              double *coarse_pos, double *coarse_snr, double *fcch_pos, double *pos_info,
                              void *cuda_stream, double *r_correct, int r_mem, int64_t r_stride);
 
+/* The same call followed by the two demodulators gsm_sync_demod.m:144-145 hands r_correct to, for every stream, without materialising
+ * r_correct: SCH_demod(r_correct, pos_info, ...) (SCH_demod.m:65-110) and FCCH_demod (FCCH_demod.m:21-66) on the samples
+ * filter -> interp1(1+e1) -> .*exp(1i*n*dphi1) -> interp1(1+e2) -> .*exp(1i*n*dphi2) evaluated from the uint8 capture where each burst
+ * reads them.  results, coarse_*, fcch_pos and pos_info are those of gsmcal_calibrate_batch.
+ * Row i of stream d (B = gsmcal_max_bursts(...) as above) is the i-th row of that type in the stream's pos_info.  Per-row outputs may be
+ * NULL (not copied back):
+ *   sch_ok [n_streams][B]: 1 when the 194*osr-sample equaliser window x = r_correct(pos-8*osr : ...) lies inside r_correct (where the
+ *     reference would raise, SCH_demod.m:79-81, the row gets sch_ok = 0 and zero bits / correlations);
+ *   demod_bits, bits_to_decoder [n_streams][B][148] (SCH_demod.m:94-97); corr_val [n_streams][B][85] (:103-110);
+ *   fcch_freq, fcch_snr, fcch_max_idx [n_streams][B] (FCCH_demod.m:41,57-66; NaN for a window outside r_correct).
+ * The per-stream record tells which rows are valid and why a demodulator did not run. */
+typedef struct gsmcal_demod_result {
+    int32_t n_sch;            /* type-1 rows of pos_info, in pos_info order; -1: SCH_demod not run (flags say why) */
+    int32_t n_sch_ok;         /* of those, rows whose 194*osr-sample equaliser window lies inside r_correct */
+    int32_t n_fcch;           /* type-0 rows; -1 like n_sch */
+    int32_t flags;            /* GSMCAL_DEMOD_* */
+    double  fcch_mean_freq;   /* FCCH_demod.m:43; NaN unless every FCCH window lies inside r_correct */
+    double  fcch_carrier_ppm; /* FCCH_demod.m:46-47; NaN likewise */
+} gsmcal_demod_result;        /* 32 bytes */
+
+#define GSMCAL_DEMOD_NO_POS_INFO  1  /* pos_info == -1 in the all-elements sense (SCH_demod.m:8-11, FCCH_demod.m:7-10) */
+#define GSMCAL_DEMOD_NO_R_CORRECT 2  /* pos_info valid but r_correct = -1 (results.r_len[2] == -1): the reference would fail at SCH_demod.m:81 */
+#define GSMCAL_DEMOD_SCH_RANGE    4  /* some SCH window leaves r_correct (the reference raises at :79-81); those rows have sch_ok = 0 */
+#define GSMCAL_DEMOD_FCCH_RANGE   8  /* some FCCH window leaves r_correct; mean / ppm are NaN */
+
+int gsmcal_calibrate_demod_batch(const uint8_t *raw, int raw_mem, int64_t n_iq, int64_t n_streams,
+                                 double carrier_freq, const double *sch_training_sequence,
+                                 const double *coef, int n_taps, int oversampling_ratio, int coarse_decimation,
+                                 gsmcal_stream_result *results,
+                                 double *coarse_pos, double *coarse_snr, double *fcch_pos, double *pos_info,
+                                 void *cuda_stream,
+                                 gsmcal_demod_result *demod /* [n_streams], required */, uint8_t *sch_ok,
+                                 uint8_t *demod_bits, uint8_t *bits_to_decoder, double *corr_val,
+                                 double *fcch_freq, double *fcch_snr, double *fcch_max_idx);
+
 /* The same pipeline with several batches in flight (continuous captures): _submit enqueues batch `slot` (0..3) on the library's
  * own streams once the caller's `cuda_stream` has produced the DEVICE-resident capture, and returns; _collect waits for that batch
  * and fills the result pointers given to _submit (they must stay valid until then).  Batches are staggered on the device: the
@@ -236,8 +271,8 @@ int gsmcal_calibrate_batch_cancel(int slot);
 
 /* CUDA-event times (ms) of the stages of the last gsmcal_calibrate_batch call on this process:
  * [0] uint8 column sums (+ H2D when raw is on the host) [1] coarse FCCH [2] fine FCCH sliding-DFT peak search
- * [3] fine ppm + tone estimate + gate [4] SCH correlation + pos_info [5] post-SCH tone estimate + result records.
- * Returns the number of stages written. */
+ * [3] fine ppm + tone estimate + gate [4] SCH correlation + pos_info [5] post-SCH tone estimate + result records
+ * [6] (gsmcal_calibrate_demod_batch only) SCH_demod + FCCH_demod.  Returns the number of stages written. */
 int gsmcal_last_batch_stage_ms(double *ms, int cap);
 
 /* FCCH scanner per-channel processing, multi_rtl_sdr_gsm_FCCH_scanner.m:132-135,163-186, for n_chan

@@ -19,6 +19,9 @@
 #include "chn_filter_taps.inc"
 
 static_assert(sizeof(gsmcal_stream_result) == sizeof(StreamResultDev), "result record layout");
+static_assert(sizeof(gsmcal_demod_result) == sizeof(DemodResultDev) && sizeof(gsmcal_demod_result) == 32, "demod record layout");
+static_assert(GSMCAL_DEMOD_NO_POS_INFO == DM_NO_POS_INFO && GSMCAL_DEMOD_NO_R_CORRECT == DM_NO_R_CORRECT && GSMCAL_DEMOD_SCH_RANGE == DM_SCH_RANGE &&
+              GSMCAL_DEMOD_FCCH_RANGE == DM_FCCH_RANGE, "demod flags");
 
 namespace {
 
@@ -111,7 +114,7 @@ struct Ctx {
     cudaEvent_t stage_ev[kNumStageEvents];
     bool stage_ev_ok = false;
     Slot slots[kSlots];
-    DevBuf in, out, work, tplbuf, wc;
+    DevBuf in, out, work, tplbuf, wc, dem;     // dem: outputs and row lists of gsmcal_calibrate_demod_batch
     std::map<int, double2 *> tw;     // N -> exp(-2*pi*i*j/N)
     std::vector<cudaStream_t> side;  // extra streams: stream groups of a batch overlap their latency-bound stages
     std::vector<cudaStream_t> side_hi; // one high-priority stream per group for the latency-bound burst chain (see gsmcal_calibrate_batch)
@@ -198,6 +201,8 @@ int get_ctx(Ctx **out) {
         CU(cudaFuncSetAttribute(fcch_demod_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));      // (attributes are per device:
         CU(cudaFuncSetAttribute(fde_template_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 120 * 1024));    //  all of them live here, keyed by
         CU(cudaFuncSetAttribute(sch_demod_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 120 * 1024));       //  the device's Ctx)
+        CU(cudaFuncSetAttribute(sch_demod_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
+        CU(cudaFuncSetAttribute(fcch_demod_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
         c.attrs = true;
     }
     *out = &c;
@@ -488,6 +493,64 @@ int check_fir_args(const double *coef, int n_taps, const void *s, i64 n, i64 n_c
 }
 
 void gmsk_template(int osr, double *out);
+size_t fcch_demod_smem(int osr);
+size_t sch_demod_smem(int osr);
+void gmsk_branch_table(int osr, double *W);
+void sch_training_pm(signed char *data_pm);
+
+// ---- batched SCH_demod / FCCH_demod stage of gsmcal_calibrate_demod_batch -----------------------------------------------------
+struct DemodOut {                    // the caller's host outputs (any per-row pointer may be NULL)
+    gsmcal_demod_result *rec; uint8_t *sch_ok, *bits, *dec; double *corr, *freq, *snr, *idx;
+};
+struct DemodDev {                    // device buffers, [D][cap] rows unless noted
+    DemodResultDev *rec; double *sch_pos, *fcch_pos, *corr /* x85 */, *freq, *snr, *idx;
+    unsigned char *sch_ok, *fcch_ok, *bits /* x148 */, *dec /* x148 */; double2 *Ft /* N */, *Wtab /* 16*osr */; signed char *dpm /* 64 */;
+};
+DemodDev sub_demod(const DemodDev &a, i64 d0, int cap) {
+    DemodDev s = a;
+    const i64 r = d0 * cap;
+    s.rec += d0; s.sch_pos += r; s.fcch_pos += r; s.corr += r * 85; s.freq += r; s.snr += r; s.idx += r;
+    s.sch_ok += r; s.fcch_ok += r; s.bits += r * 148; s.dec += r * 148;
+    return s;
+}
+// workspace, branch table, training bits and fft(template) (SCH_demod.m:47-59), once per call on `st` before the stream groups fork
+int demod_setup(Ctx &c, i64 D, int cap, int osr, const double2 *tpl_dev, std::vector<double> &W, signed char *data_pm, cudaStream_t st, DemodDev *dd) {
+    const int N = SD_NSYM * osr;
+    size_t off = 0;
+    auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes); return o; };
+    const size_t rows = (size_t)D * cap;
+    const size_t o_rec = take(sizeof(DemodResultDev) * D), o_sp = take(8 * rows), o_fp = take(8 * rows), o_corr = take(8 * 85 * rows),
+                 o_fr = take(8 * rows), o_sn = take(8 * rows), o_ix = take(8 * rows), o_so = take(rows), o_fo = take(rows),
+                 o_b = take(148 * rows), o_d = take(148 * rows), o_ft = take(sizeof(double2) * N), o_w = take(sizeof(double2) * 16 * osr), o_pm = take(64);
+    void *base; TRY(c.dem.get(off, &base));
+    char *b = (char *)base;
+    dd->rec = (DemodResultDev *)(b + o_rec); dd->sch_pos = (double *)(b + o_sp); dd->fcch_pos = (double *)(b + o_fp); dd->corr = (double *)(b + o_corr);
+    dd->freq = (double *)(b + o_fr); dd->snr = (double *)(b + o_sn); dd->idx = (double *)(b + o_ix);
+    dd->sch_ok = (unsigned char *)(b + o_so); dd->fcch_ok = (unsigned char *)(b + o_fo); dd->bits = (unsigned char *)(b + o_b); dd->dec = (unsigned char *)(b + o_d);
+    dd->Ft = (double2 *)(b + o_ft); dd->Wtab = (double2 *)(b + o_w); dd->dpm = (signed char *)(b + o_pm);
+    W.assign(2 * 16 * (size_t)osr, 0.0);
+    gmsk_branch_table(osr, W.data());
+    sch_training_pm(data_pm);
+    CU(cudaMemcpyAsync(dd->Wtab, W.data(), sizeof(double) * W.size(), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(dd->dpm, data_pm, 64, cudaMemcpyHostToDevice, st));
+    const double2 *tw; TRY(get_twiddle(c, N, st, &tw));
+    LAUNCH(fde_template_kernel, 1, SD_THREADS, 3 * (size_t)N * sizeof(double2), st, tpl_dev, osr, tw, dd->Ft);
+    return GSMCAL_OK;
+}
+// one stream group: row lists + sentinels, SCH bursts, FCCH bursts, FCCH means
+int run_demod(Ctx &c, WinSrc src, const Work &ws, const DemodDev &dd, int osr, double carrier_freq, i64 nd, int cap, cudaStream_t st) {
+    const double2 *tw_s, *tw_f;
+    TRY(get_twiddle(c, SD_NSYM * osr, st, &tw_s));
+    TRY(get_twiddle(c, 148 * osr, st, &tw_f));
+    LAUNCH(demod_compact_kernel, (unsigned)nd, 32, 0, st, ws.ctl, ws.pos_info, cap, osr, dd.rec, dd.sch_pos, dd.sch_ok, dd.fcch_pos, dd.fcch_ok);
+    LAUNCH(sch_demod_batch_kernel, dim3((unsigned)cap, (unsigned)nd), SDB_THREADS, sch_demod_smem(osr), st, src, ws.ctl, dd.rec, dd.sch_pos, dd.sch_ok,
+           cap, osr, tw_s, dd.Ft, dd.Wtab, dd.dpm, dd.bits, dd.dec, dd.corr);
+    const size_t fs = fcch_demod_smem(osr), fs_load = sizeof(double2) * (3 * 148 * (size_t)osr + 144);      // + the loader's scratch behind u
+    LAUNCH(fcch_demod_batch_kernel, dim3((unsigned)cap, (unsigned)nd), FD_THREADS, fs > fs_load ? fs : fs_load, st, with_cache(src, ws, cap), ws.ctl, dd.rec,
+           dd.fcch_pos, dd.fcch_ok, cap, osr, tw_f, dd.freq, dd.snr, dd.idx);
+    LAUNCH(demod_fcch_mean_kernel, (unsigned)((nd + 127) / 128), 128, 0, st, dd.rec, (int)nd, dd.freq, cap, carrier_freq);
+    return GSMCAL_OK;
+}
 
 }  // namespace
 
@@ -512,7 +575,7 @@ void gsmcal_release(void) {
     g_last_need_full = nullptr; g_last_need_band = nullptr; g_last_need_full_n = 0; g_last_pass_hist = nullptr; g_prev_pass_hist = nullptr;   // they point into the workspaces freed below
     for (auto &kv : g_ctx) {
         cudaSetDevice(kv.first);
-        kv.second.ring.release(); kv.second.in.release(); kv.second.out.release(); kv.second.work.release(); kv.second.tplbuf.release(); kv.second.wc.release();
+        kv.second.ring.release(); kv.second.in.release(); kv.second.out.release(); kv.second.work.release(); kv.second.tplbuf.release(); kv.second.wc.release(); kv.second.dem.release();
         for (auto &t : kv.second.tw) cudaFree(t.second);
         kv.second.tw.clear();
         if (kv.second.stage_ev_ok) { for (cudaEvent_t e : kv.second.stage_ev) cudaEventDestroy(e); kv.second.stage_ev_ok = false; }
@@ -1004,7 +1067,7 @@ int gsmcal_total_ppm_calculation(const double *ppm_in, int64_t n, double *ppm_ou
 static int calibrate_batch_impl(const uint8_t *raw, int raw_mem, int64_t n_iq, int64_t D, double carrier_freq, const double *tpl,
                                 const double *coef, int n_taps, int osr, int coarse_dr, gsmcal_stream_result *results,
                                 double *coarse_pos, double *coarse_snr, double *fcch_pos, double *pos_info, void *cuda_stream,
-                                double *r_out, int r_mem, int64_t r_stride) {
+                                double *r_out, int r_mem, int64_t r_stride, const DemodOut *dm = nullptr) {
     std::lock_guard<std::mutex> lk(g_mu);
     if (r_out && r_stride < n_iq) return fail(GSMCAL_ERR_ARG, "calibrate_batch_r: r_stride must be >= n_iq");
     if (!raw || !tpl || !coef || !results || n_iq < 1 || D < 1 || osr < 1 || osr > 8) return fail(GSMCAL_ERR_ARG, "calibrate_batch: bad arguments (osr 1..8)");
@@ -1032,6 +1095,9 @@ static int calibrate_batch_impl(const uint8_t *raw, int raw_mem, int64_t n_iq, i
     g_last_need_full = w.need_full; g_last_need_band = w.need_band; g_last_need_full_n = (long long)D * cap;
     g_last_pass_hist = w.pass_hist;
     CU(cudaMemsetAsync(w.pass_hist, 0, sizeof(unsigned) * 16 + sizeof(unsigned long long) * 64, st));
+    DemodDev dd;
+    std::vector<double> dm_w; signed char dm_pm[64];                 // host sources of the uploads, alive until the final synchronise
+    if (dm) TRY(demod_setup(*c, D, cap, osr, w.tpl, dm_w, dm_pm, st, &dd));
     g_stage_n = 0;
     // Streams are independent, so the batch is cut into groups that run the stage sequence on their own CUDA
     // streams: the latency-bound stages of one group (burst chain, per-stream solves) overlap the FP64-bound
@@ -1105,6 +1171,10 @@ static int calibrate_batch_impl(const uint8_t *raw, int raw_mem, int64_t n_iq, i
         if (timing) TRY(stage_mark(*c, sg));
         TRY(run_post(*c, with_cache(lazy_src(graw, n_iq, n_taps, 3, 1), ws, cap), osr, carrier_freq, nd, cap, ws, true, sg));
         if (timing) TRY(stage_mark(*c, sg));
+        if (dm) {
+            TRY(run_demod(*c, lazy_src(graw, n_iq, n_taps, 3, 1), ws, sub_demod(dd, d0, cap), osr, carrier_freq, nd, cap, sg));
+            if (timing) TRY(stage_mark(*c, sg));
+        }
         if (sg != st) {
             cudaEvent_t ev; CU(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
             CU(cudaEventRecord(ev, sg));
@@ -1134,6 +1204,17 @@ static int calibrate_batch_impl(const uint8_t *raw, int raw_mem, int64_t n_iq, i
     if (coarse_snr) CU(cudaMemcpyAsync(coarse_snr, w.coarse_snr, sizeof(double) * D * cap, cudaMemcpyDeviceToHost, st));
     if (fcch_pos) CU(cudaMemcpyAsync(fcch_pos, w.fcch_pos, sizeof(double) * D * cap, cudaMemcpyDeviceToHost, st));
     if (pos_info) CU(cudaMemcpyAsync(pos_info, w.pos_info, sizeof(double) * D * cap * 12, cudaMemcpyDeviceToHost, st));
+    if (dm) {
+        const size_t rows = (size_t)D * cap;
+        CU(cudaMemcpyAsync(dm->rec, dd.rec, sizeof(DemodResultDev) * D, cudaMemcpyDeviceToHost, st));
+        if (dm->sch_ok) TRY(copy_d2h(c->ring, g_device, dm->sch_ok, dd.sch_ok, rows, st));
+        if (dm->bits) TRY(copy_d2h(c->ring, g_device, dm->bits, dd.bits, 148 * rows, st));
+        if (dm->dec) TRY(copy_d2h(c->ring, g_device, dm->dec, dd.dec, 148 * rows, st));
+        if (dm->corr) TRY(copy_d2h(c->ring, g_device, dm->corr, dd.corr, sizeof(double) * 85 * rows, st));
+        if (dm->freq) TRY(copy_d2h(c->ring, g_device, dm->freq, dd.freq, sizeof(double) * rows, st));
+        if (dm->snr) TRY(copy_d2h(c->ring, g_device, dm->snr, dd.snr, sizeof(double) * rows, st));
+        if (dm->idx) TRY(copy_d2h(c->ring, g_device, dm->idx, dd.idx, sizeof(double) * rows, st));
+    }
     CU(cudaStreamSynchronize(st));
     if (timing) for (int i = 0; i + 1 < g_stage_n; ++i) CU(cudaEventElapsedTime(&g_stage_ms[i], c->stage_ev[i], c->stage_ev[i + 1]));
     if (!timing) g_stage_n = 0;
@@ -1154,6 +1235,17 @@ int gsmcal_calibrate_batch_r(const uint8_t *raw, int raw_mem, int64_t n_iq, int6
     if (!r_correct) return fail(GSMCAL_ERR_ARG, "calibrate_batch_r: null r_correct");
     return calibrate_batch_impl(raw, raw_mem, n_iq, D, carrier_freq, tpl, coef, n_taps, osr, coarse_dr, results, coarse_pos, coarse_snr, fcch_pos, pos_info,
                                 cuda_stream, r_correct, r_mem, r_stride);
+}
+
+int gsmcal_calibrate_demod_batch(const uint8_t *raw, int raw_mem, int64_t n_iq, int64_t D, double carrier_freq, const double *tpl,
+                                 const double *coef, int n_taps, int osr, int coarse_dr, gsmcal_stream_result *results,
+                                 double *coarse_pos, double *coarse_snr, double *fcch_pos, double *pos_info, void *cuda_stream,
+                                 gsmcal_demod_result *demod, uint8_t *sch_ok, uint8_t *demod_bits, uint8_t *bits_to_decoder, double *corr_val,
+                                 double *fcch_freq, double *fcch_snr, double *fcch_max_idx) {
+    if (!demod) return fail(GSMCAL_ERR_ARG, "calibrate_demod_batch: null demod");
+    const DemodOut o = {demod, sch_ok, demod_bits, bits_to_decoder, corr_val, fcch_freq, fcch_snr, fcch_max_idx};
+    return calibrate_batch_impl(raw, raw_mem, n_iq, D, carrier_freq, tpl, coef, n_taps, osr, coarse_dr, results, coarse_pos, coarse_snr, fcch_pos, pos_info,
+                                cuda_stream, nullptr, GSMCAL_MEM_DEVICE, 0, &o);
 }
 
 // ---- submit / collect: the same pipeline, several batches in flight -----------------------------------------------------------
@@ -1347,7 +1439,7 @@ int gsmcal_calibrate_batch_cancel(int slot) {
 }
 
 int gsmcal_last_batch_stage_ms(double *ms, int cap_n) {
-    // colsum(+H2D), coarse, fine_peak, fine ppm+tone+carrier, SCH, post-SCH - of the last gsmcal_calibrate_batch call
+    // colsum(+H2D), coarse, fine_peak, fine ppm+tone+carrier, SCH, post-SCH (+ demod) - of the last gsmcal_calibrate_batch* call
     int n = g_stage_n > 0 ? g_stage_n - 1 : 0;
     for (int i = 0; i < n && i < cap_n; ++i) ms[i] = g_stage_ms[i];
     return n;

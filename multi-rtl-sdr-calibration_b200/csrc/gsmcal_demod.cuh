@@ -9,22 +9,16 @@
 // so the spectrum is evaluated once through the 37 x M row FFT.
 // ===================================================================================================
 #define FD_THREADS 256
-__global__ void __launch_bounds__(FD_THREADS) fcch_demod_kernel(const double2 *__restrict__ s, const double *__restrict__ pos, int osr,
-                                                               const double2 *__restrict__ tw, double *__restrict__ freq_out,
-                                                               double *__restrict__ snr_out, double *__restrict__ idx_out) {
-    extern __shared__ double2 sm[];
+// the arithmetic of one burst, its N = 148*osr samples in u (shared; A, F: N double2, P: N doubles of scratch); thread 0 writes output o
+__device__ __forceinline__ void fcch_demod_body(double2 *u, double2 *A, double2 *F, double *P, int osr, const double2 *__restrict__ tw,
+                                double *__restrict__ freq_out, double *__restrict__ snr_out, double *__restrict__ idx_out, i64 o) {
     __shared__ double red_v[8];
     __shared__ int red_i[8];
     __shared__ double red_n[32];
     __shared__ double sh_pr;
-    const int burst = blockIdx.x, tid = threadIdx.x;
+    const int tid = threadIdx.x;
     const int N = 148 * osr;
     const double sampling_rate = ((1625.0 / 6.0) * 1e3) * (double)osr;
-    double2 *u = sm, *A = u + N, *F = A + N;
-    double *P = (double *)(F + N);                             // fd_fcch column in fftshift order
-    const i64 sp = (i64)pos[burst];
-    for (int n = tid; n < N; n += FD_THREADS) u[n] = s[sp - 1 + n];
-    __syncthreads();
     const double2 *Tm = fft_rows(u, A, F, N, tw);
     double v = -1.0; int j_best = 0x7fffffff;
     for (int j = tid; j < N; j += FD_THREADS) {
@@ -42,8 +36,8 @@ __global__ void __launch_bounds__(FD_THREADS) fcch_demod_kernel(const double2 *_
     block_sum_n<2, false>(sn, red_n);
     if (tid == 0) {
         const double noise = sn[1] - sn[0];
-        snr_out[burst] = 10.0 * log10(sn[0] / noise);
-        idx_out[burst] = (double)(j_best + 1 - (N / 2 + 1));
+        snr_out[o] = 10.0 * log10(sn[0] / noise);
+        idx_out[o] = (double)(j_best + 1 - (N / 2 + 1));
     }
     // tone frequency (:35-41): integer-bin derotation, unit phasors, angle of the mean one-sample rotation
     const int jr = j_best + 1 - ((N / 2) + 1);
@@ -65,7 +59,20 @@ __global__ void __launch_bounds__(FD_THREADS) fcch_demod_kernel(const double2 *_
     block_sum_n<2, false>(rri, red_n);
     if (tid == 0) sh_pr = atan2(rri[1] / (double)(N - 1), rri[0] / (double)(N - 1));
     __syncthreads();
-    if (tid == 0) freq_out[burst] = sampling_rate * (int_phase_rotate + sh_pr) / (2 * GSMCAL_PI);
+    if (tid == 0) freq_out[o] = sampling_rate * (int_phase_rotate + sh_pr) / (2 * GSMCAL_PI);
+}
+__global__ void __launch_bounds__(FD_THREADS) fcch_demod_kernel(const double2 *__restrict__ s, const double *__restrict__ pos, int osr,
+                                                               const double2 *__restrict__ tw, double *__restrict__ freq_out,
+                                                               double *__restrict__ snr_out, double *__restrict__ idx_out) {
+    extern __shared__ double2 sm[];
+    const int burst = blockIdx.x, tid = threadIdx.x;
+    const int N = 148 * osr;
+    double2 *u = sm, *A = u + N, *F = A + N;
+    double *P = (double *)(F + N);                             // fd_fcch column in fftshift order
+    const i64 sp = (i64)pos[burst];
+    for (int n = tid; n < N; n += FD_THREADS) u[n] = s[sp - 1 + n];
+    __syncthreads();
+    fcch_demod_body(u, A, F, P, osr, tw, freq_out, snr_out, idx_out, burst);
 }
 
 // ===================================================================================================
@@ -189,6 +196,39 @@ __device__ void gmsk_viterbi_warp(const double2 *cb, int nsym, unsigned char *bi
     }
 }
 
+// SCH_demod.m:92-110 on the equalised burst x (shared, 194*osr samples): branch correlations of every symbol interval (the trellis
+// then only adds; cb: 194*16 double2 of scratch), MLSE, the 148 burst bits, their differential decoding and the 85-lag correlation
+__device__ __forceinline__ void sch_bits_body(const double2 *x, double2 *cb, int osr, const double2 *__restrict__ Wtab, const signed char *dpm /* shared */,
+                              unsigned char *bits /* shared, SD_NSYM + 2 */, unsigned char *__restrict__ demod_bits, unsigned char *__restrict__ dec_bits,
+                              double *__restrict__ corr_val) {
+    const int tid = threadIdx.x;
+    for (int i = tid; i < SD_NSYM * 16; i += blockDim.x) {
+        const int m = i >> 4, combo = i & 15;
+        double ar = 0.0, ai = 0.0;
+        for (int j = 0; j < osr; ++j) {
+            const double2 v = x[m * osr + j], w = Wtab[combo * osr + j];
+            ar += v.x * w.x + v.y * w.y;                         // v * conj(w)
+            ai += v.y * w.x - v.x * w.y;
+        }
+        cb[i] = make_double2(ar, ai);
+    }
+    __syncthreads();
+    if (tid < 32) gmsk_viterbi_warp(cb, SD_NSYM, bits);
+    __syncthreads();
+    // :94-110
+    const unsigned char *db = bits + SD_TB + SD_EX;
+    for (int i = tid; i < 148; i += blockDim.x) {
+        demod_bits[i] = db[i];
+        const int nb = 1 - db[i], pb = (i > 0) ? 1 - db[i - 1] : 0;
+        dec_bits[i] = (unsigned char)(nb != pb);
+    }
+    for (int k = tid; k < 148 - 64 + 1; k += blockDim.x) {
+        int acc = 0;
+        for (int i = 0; i < 64; ++i) acc += dpm[i] * (2 * (int)db[k + i] - 1);
+        corr_val[k] = (double)acc;
+    }
+}
+
 __global__ void __launch_bounds__(SD_THREADS) sch_demod_kernel(const double2 *__restrict__ s, const double *__restrict__ pos, int osr,
                                                               const double2 *__restrict__ tw, const double2 *__restrict__ Ft,
                                                               const double2 *__restrict__ Wtab /* 16 x osr */, const signed char *__restrict__ data_pm /* 64 */,
@@ -215,31 +255,243 @@ __global__ void __launch_bounds__(SD_THREADS) sch_demod_kernel(const double2 *__
     for (int n = tid; n < N; n += SD_THREADS) fb[n] = cdiv(fb[n], fa[n]);       // :89
     __syncthreads();
     dft_pxm<true>(fb, tmp, x, N, 97, tw);                      // x = ifft(fd_x) (:90)
-    // branch correlations of every symbol interval (the trellis then only adds)
-    double2 *cb = tmp;                                          // 194*16 <= 2*N entries for osr >= 8; sized by the host for smaller osr
-    for (int i = tid; i < SD_NSYM * 16; i += SD_THREADS) {
-        const int m = i >> 4, combo = i & 15;
-        double ar = 0.0, ai = 0.0;
-        for (int j = 0; j < osr; ++j) {
-            const double2 v = x[m * osr + j], w = Wtab[combo * osr + j];
-            ar += v.x * w.x + v.y * w.y;                         // v * conj(w)
-            ai += v.y * w.x - v.x * w.y;
+    sch_bits_body(x, tmp, osr, Wtab, dpm, bits, demod_bits + (i64)burst * 148, dec_bits + (i64)burst * 148, corr_val + (i64)burst * 85);
+}
+
+// ===================================================================================================
+// Batched SCH_demod / FCCH_demod (gsm_sync_demod.m:144-145) for every stream of gsmcal_calibrate_demod_batch, on the pipeline's own
+// r_correct evaluated where it is read: the level-3 loader (filter -> interp1(e1) -> derotation(dphi1) -> interp1(e2)) and then
+// r_correct(j) = r(j) * exp(1i*(j-1)*dphi2) (carrier_correct_post_SCH.m:81-83), phasors as materialise_r_kernel forms them.
+// ===================================================================================================
+struct DemodResultDev {              // mirrors gsmcal_demod_result (include/gsmcal.h)
+    int n_sch, n_sch_ok, n_fcch, flags;
+    double fcch_mean_freq, fcch_carrier_ppm;
+};
+#define DM_NO_POS_INFO  1
+#define DM_NO_R_CORRECT 2
+#define DM_SCH_RANGE    4
+#define DM_FCCH_RANGE   8
+
+// One warp per stream: the `pos_info == -1` rule (all elements, SCH_demod.m:8-11, FCCH_demod.m:7-10), r_correct = -1, the split of
+// pos_info into SCH (type 1) and FCCH (type 0) rows in pos_info order, and the window range checks against len3 = length(r_correct):
+// SCH x = r(sp:ep), sp = pos - 8*osr, 194*osr samples (SCH_demod.m:79-81); FCCH r(pos : pos + 148*osr - 1) (FCCH_demod.m:28).
+__global__ void __launch_bounds__(32) demod_compact_kernel(const StreamCtl *__restrict__ ctl, const double *__restrict__ pos_info /* [stream][6*cap][2] */,
+                                                           int cap, int osr, DemodResultDev *__restrict__ rec, double *__restrict__ sch_pos,
+                                                           unsigned char *__restrict__ sch_ok, double *__restrict__ fcch_pos,
+                                                           unsigned char *__restrict__ fcch_ok) {
+    const int stream = blockIdx.x, lane = threadIdx.x;
+    const StreamCtl c = ctl[stream];
+    const double *pi = pos_info + (i64)stream * 6 * cap * 2;
+    const int rows = c.n_pos_info;
+    bool other = false;
+    for (int i = lane; i < 2 * rows; i += 32) other |= (pi[i] != -1.0);
+    const bool all_m1 = rows < 0 || (rows > 0 && !__any_sync(0xffffffffu, other));
+    DemodResultDev r;
+    r.n_sch = r.n_sch_ok = r.n_fcch = -1; r.flags = 0;
+    r.fcch_mean_freq = NAN; r.fcch_carrier_ppm = NAN;           // filled by demod_fcch_mean_kernel
+    if (all_m1) r.flags = DM_NO_POS_INFO;
+    else if (c.len3 < 0) r.flags = DM_NO_R_CORRECT;
+    else {
+        const double len = (double)c.len3, ns_win = (double)(SD_NSYM * osr), nf_win = (double)(148 * osr);
+        const unsigned below = (1u << lane) - 1u;
+        int ns = 0, nok = 0, nf = 0; bool f_bad = false;
+        for (int i0 = 0; i0 < rows; i0 += 32) {
+            const int i = i0 + lane;
+            double p = 0.0, t = -1.0;
+            if (i < rows) { p = pi[2 * i]; t = pi[2 * i + 1]; }
+            const bool is_s = (t == 1.0), is_f = (t == 0.0);
+            const double sp = p - SD_EX * osr;
+            const bool s_ok = is_s && p == floor(p) && sp >= 1.0 && sp + ns_win - 1.0 <= len;
+            const bool f_ok = is_f && p == floor(p) && p >= 1.0 && p + nf_win - 1.0 <= len;
+            const unsigned ms = __ballot_sync(0xffffffffu, is_s), mf = __ballot_sync(0xffffffffu, is_f);
+            const int ks = ns + __popc(ms & below), kf = nf + __popc(mf & below);
+            if (is_s && ks < cap) { sch_pos[(i64)stream * cap + ks] = p; sch_ok[(i64)stream * cap + ks] = s_ok; }
+            if (is_f && kf < cap) { fcch_pos[(i64)stream * cap + kf] = p; fcch_ok[(i64)stream * cap + kf] = f_ok; }
+            nok += __popc(__ballot_sync(0xffffffffu, s_ok));
+            f_bad |= __any_sync(0xffffffffu, is_f && !f_ok);
+            ns += __popc(ms); nf += __popc(mf);
         }
-        cb[i] = make_double2(ar, ai);
+        r.n_sch = ns < cap ? ns : cap; r.n_sch_ok = nok; r.n_fcch = nf < cap ? nf : cap;
+        r.flags = (nok < ns ? DM_SCH_RANGE : 0) | (f_bad ? DM_FCCH_RANGE : 0);
+    }
+    if (lane == 0) rec[stream] = r;
+}
+
+// N = 97*M point DFT, N = 194*osr, M = 2*osr (n = M*n1 + n2, k = k1 + 97*k2), the same factorisation as dft_pxm:
+//   stage 1: the 97-point DFT of every column n2 through its conjugate-pair form: with a_n = v_n + v_(97-n), b_n = v_n - v_(97-n),
+//            X(k) = v_0 + A_k + i*B_k and X(97-k) = v_0 + A_k - i*B_k (inverse: i*B_k negated), A_k = sum_n a_n cos, B_k = sum_n b_n Im(W^nk),
+//            n = n_lo..48 - real-by-complex products, a quarter of the direct stage's DFMA.  Inputs with v_n = 0 for n < n_lo and
+//            48 < 97 - n < n_lo pass n_lo > 1 (the received training sequence occupies outer indices 25..56 only).
+//   twiddle W_N^(n2*k1), then stage 2: 97 row DFTs of M points (radix-2 Stockham in shared memory when M is a power of two).
+// in and out may alias; t0, t1: N double2 of scratch each; w97[j] = W_97^j, wm[j] = W_M^j (j < M/2), both in shared memory.
+#define D97_R 3                        // k values per thread: 16 groups of 3 cover the 48 conjugate pairs
+template <bool INV>
+__device__ void dft97(const double2 *in, double2 *t0, double2 *t1, double2 *out, int M, int n_lo, const double2 *__restrict__ tw,
+                      const double2 *w97, const double2 *wm) {
+    const int N = 97 * M, tid = threadIdx.x, nt = blockDim.x;
+    for (int task = tid; task < 16 * M; task += nt) {
+        const int n2 = task % M, g = task / M, k0 = 1 + D97_R * g;
+        double ar[D97_R], ai[D97_R], br[D97_R], bi[D97_R];
+        int t[D97_R];
+#pragma unroll
+        for (int r = 0; r < D97_R; ++r) { ar[r] = ai[r] = br[r] = bi[r] = 0.0; t[r] = (n_lo * (k0 + r)) % 97; }
+        double sr = 0.0, si = 0.0;
+        for (int n = n_lo; n <= 48; ++n) {
+            const double2 p = in[M * n + n2], q = in[M * (97 - n) + n2];
+            const double axr = p.x + q.x, axi = p.y + q.y, bxr = p.x - q.x, bxi = p.y - q.y;
+            if (g == 0) { sr += axr; si += axi; }
+#pragma unroll
+            for (int r = 0; r < D97_R; ++r) {
+                const double2 w = w97[t[r]];
+                ar[r] = fma(axr, w.x, ar[r]); ai[r] = fma(axi, w.x, ai[r]);
+                br[r] = fma(bxr, w.y, br[r]); bi[r] = fma(bxi, w.y, bi[r]);
+                t[r] += k0 + r; if (t[r] >= 97) t[r] -= 97;
+            }
+        }
+        const double2 v0 = in[n2];
+#pragma unroll
+        for (int r = 0; r < D97_R; ++r) {
+            const int k = k0 + r;
+            const double2 xp = make_double2(v0.x + ar[r] - bi[r], v0.y + ai[r] + br[r]), xm = make_double2(v0.x + ar[r] + bi[r], v0.y + ai[r] - br[r]);
+            double2 wk = tw[n2 * k], wn = tw[n2 * (97 - k)];
+            if (INV) { wk.y = -wk.y; wn.y = -wn.y; }
+            t0[k * M + n2] = cmul(INV ? xm : xp, wk);
+            t0[(97 - k) * M + n2] = cmul(INV ? xp : xm, wn);
+        }
+        if (g == 0) t0[n2] = make_double2(v0.x + sr, v0.y + si);
     }
     __syncthreads();
-    if (tid < 32) gmsk_viterbi_warp(cb, SD_NSYM, bits);
+    if ((M & (M - 1)) == 0) {
+        const int lm = 31 - __clz(M), half = M / 2;
+        const double2 *src = t0; double2 *dst = t1;
+        int tsh = lm - 1;
+        for (int Ns = 1; Ns < M; Ns <<= 1, --tsh) {
+            for (int i = tid; i < 97 * half; i += nt) {
+                const int row = i >> (lm - 1), j = i & (half - 1), k = j & (Ns - 1);
+                double2 w = wm[k << tsh]; if (INV) w.y = -w.y;
+                const double2 x0 = src[row * M + j], x1 = cmul(src[row * M + j + half], w);
+                const int o = row * M + ((j - k) << 1) + k;
+                dst[o] = make_double2(x0.x + x1.x, x0.y + x1.y);
+                dst[o + Ns] = make_double2(x0.x - x1.x, x0.y - x1.y);
+            }
+            __syncthreads();
+            const double2 *sw = src; src = dst; dst = const_cast<double2 *>(sw);
+        }
+        for (int i = tid; i < N; i += nt) {
+            const int k1 = i / M, k2 = i - k1 * M;
+            const double2 v = src[i];
+            out[k1 + 97 * k2] = INV ? make_double2(v.x / (double)N, v.y / (double)N) : v;
+        }
+    } else {
+        for (int i = tid; i < N; i += nt) {
+            const int k1 = i % 97, k2 = i / 97;
+            double xr = 0.0, xi = 0.0;
+            int tt = 0; const int stp = 97 * k2;
+            for (int n2 = 0; n2 < M; ++n2) {
+                const double2 x = t0[k1 * M + n2];
+                double2 w = tw[tt]; if (INV) w.y = -w.y;
+                xr = fma(x.x, w.x, fma(-x.y, w.y, xr));
+                xi = fma(x.x, w.y, fma(x.y, w.x, xi));
+                tt += stp; if (tt >= N) tt -= N;
+            }
+            out[i] = INV ? make_double2(xr / (double)N, xi / (double)N) : make_double2(xr, xi);
+        }
+    }
     __syncthreads();
-    // :94-110
-    const unsigned char *db = bits + SD_TB + SD_EX;
-    for (int i = tid; i < 148; i += SD_THREADS) {
-        demod_bits[(i64)burst * 148 + i] = db[i];
-        const int nb = 1 - db[i], pb = (i > 0) ? 1 - db[i - 1] : 0;
-        dec_bits[(i64)burst * 148 + i] = (unsigned char)(nb != pb);
+}
+
+// r_correct(j0+1 : j0+count) = dst .* exp(1i*(j0:j0+count-1)*dphi2) in place; ph0 = exp(1i*j0*dphi2) (exact sincos, one thread)
+__device__ __forceinline__ void derotate_post(double2 *dst, int count, double dphi2, double2 ph0) {
+    const int tid = threadIdx.x, nt = blockDim.x;
+    double sn, cs;
+    sincos((double)tid * dphi2, &sn, &cs);
+    double2 ph = cmul(ph0, make_double2(cs, sn));
+    sincos((double)nt * dphi2, &sn, &cs);
+    const double2 st = make_double2(cs, sn);
+    for (int i = tid; i < count; i += nt) { dst[i] = cmul(dst[i], ph); ph = cmul(ph, st); }
+}
+
+// SCH_demod.m:65-110 for one (SCH row, stream).  320 threads: the 1552-sample level-0 window of the loader is filtered by its unrolled
+// 5-outputs-per-thread path.  Shared: x[N] | b1[N] | b2[N] | b3[N] (the loader's scratch and the branch correlations alias b1..b3).
+#define SDB_THREADS 320
+__global__ void __launch_bounds__(SDB_THREADS, 2) sch_demod_batch_kernel(WinSrc src, const StreamCtl *__restrict__ ctl, const DemodResultDev *__restrict__ rec,
+                                                                        const double *__restrict__ sch_pos, const unsigned char *__restrict__ sch_ok, int cap, int osr,
+                                                                        const double2 *__restrict__ tw, const double2 *__restrict__ Ft,
+                                                                        const double2 *__restrict__ Wtab, const signed char *__restrict__ data_pm,
+                                                                        unsigned char *__restrict__ demod_bits, unsigned char *__restrict__ dec_bits,
+                                                                        double *__restrict__ corr_val) {
+    extern __shared__ double2 sm[];
+    __shared__ unsigned char bits[SD_NSYM + 2];
+    __shared__ signed char dpm[64];
+    __shared__ double2 w97[97], wm[8];
+    __shared__ double2 ph0;
+    const int row = blockIdx.x, stream = blockIdx.y, tid = threadIdx.x;
+    if (row >= rec[stream].n_sch) return;
+    const i64 o = (i64)stream * cap + row;
+    if (!sch_ok[o]) {                                           // the reference would stop at SCH_demod.m:81: zeros, sch_ok = 0
+        for (int i = tid; i < 148; i += SDB_THREADS) { demod_bits[o * 148 + i] = 0; dec_bits[o * 148 + i] = 0; }
+        for (int k = tid; k < 85; k += SDB_THREADS) corr_val[o * 85 + k] = 0.0;
+        return;
     }
-    for (int k = tid; k < 148 - 64 + 1; k += SD_THREADS) {
-        int acc = 0;
-        for (int i = 0; i < 64; ++i) acc += dpm[i] * (2 * (int)db[k + i] - 1);
-        corr_val[(i64)burst * 85 + k] = (double)acc;
+    const StreamCtl c = ctl[stream];
+    const int N = SD_NSYM * osr, M = 2 * osr, sp_tr = (SD_EX + 42) * osr, L = 64 * osr;
+    double2 *x = sm, *b1 = x + N, *b2 = b1 + N, *b3 = b2 + N;
+    const i64 j0 = (i64)sch_pos[o] - SD_EX * osr - 1;           // 0-based first sample of x = s(sp:ep) (:79-81)
+    if (tid < 64) dpm[tid] = data_pm[tid];
+    for (int j = tid; j < 97; j += SDB_THREADS) w97[j] = tw[M * j];
+    if (tid < M / 2) wm[tid] = tw[97 * tid];
+    if (tid == 0) { double sn, cs; sincos((double)j0 * c.dphi2, &sn, &cs); ph0 = make_double2(cs, sn); }
+    load_window(src, c, stream, j0, N, x, b1, b1 + GSMCAL_XCAP(N));          // ends with a barrier
+    derotate_post(x, N, c.dphi2, ph0);
+    __syncthreads();
+    for (int n = tid; n < N; n += SDB_THREADS) b1[n] = (n >= sp_tr && n < sp_tr + L) ? x[n] : make_double2(0.0, 0.0);     // :83-84
+    __syncthreads();
+    dft97<false>(b1, b2, b3, b1, M, (SD_EX + 42) / 2, tw, w97, wm);          // fd_received_training (outer indices 25..56)
+    for (int n = tid; n < N; n += SDB_THREADS) b1[n] = cdiv(b1[n], Ft[n]);  // fd_chn (:86)
+    __syncthreads();
+    dft97<false>(x, b2, b3, x, M, 1, tw, w97, wm);                           // fd_x (:88)
+    for (int n = tid; n < N; n += SDB_THREADS) x[n] = cdiv(x[n], b1[n]);    // :89
+    __syncthreads();
+    dft97<true>(x, b2, b3, x, M, 1, tw, w97, wm);                            // x = ifft(fd_x) (:90)
+    sch_bits_body(x, b1, osr, Wtab, dpm, bits, demod_bits + o * 148, dec_bits + o * 148, corr_val + o * 85);
+}
+
+// FCCH_demod.m:21-66 for one (FCCH row, stream): the window comes through the fine search's filtered-window cache where it covers it
+// (the windows the post-SCH tone stage reads), then derotation by dphi2 and fcch_demod_body.  A window outside r_correct: NaN.
+__global__ void __maxnreg__(80) fcch_demod_batch_kernel(WinSrc src, const StreamCtl *__restrict__ ctl, const DemodResultDev *__restrict__ rec,
+                                                                     const double *__restrict__ fcch_pos, const unsigned char *__restrict__ fcch_ok, int cap, int osr,
+                                                                     const double2 *__restrict__ tw, double *__restrict__ freq_out,
+                                                                     double *__restrict__ snr_out, double *__restrict__ idx_out) {
+    extern __shared__ double2 sm[];
+    __shared__ double2 ph0;
+    const int row = blockIdx.x, stream = blockIdx.y, tid = threadIdx.x;
+    if (row >= rec[stream].n_fcch) return;
+    const i64 o = (i64)stream * cap + row;
+    if (!fcch_ok[o]) {
+        if (tid == 0) { freq_out[o] = NAN; snr_out[o] = NAN; idx_out[o] = NAN; }
+        return;
     }
+    const StreamCtl c = ctl[stream];
+    const int N = 148 * osr;
+    double2 *u = sm, *A = u + N, *F = A + N;
+    double *P = (double *)(F + N);
+    const i64 j0 = (i64)fcch_pos[o] - 1;
+    if (tid == 0) { double sn, cs; sincos((double)j0 * c.dphi2, &sn, &cs); ph0 = make_double2(cs, sn); }
+    load_window(src, c, stream, j0, N, u, A, A + GSMCAL_XCAP(N), row);       // ends with a barrier
+    derotate_post(u, N, c.dphi2, ph0);
+    __syncthreads();
+    fcch_demod_body(u, A, F, P, osr, tw, freq_out, snr_out, idx_out, o);
+}
+
+// mean(freq) (FCCH_demod.m:43, ascending row order) and carrier_ppm (:46-47) when every FCCH window lies inside r_correct
+__global__ void demod_fcch_mean_kernel(DemodResultDev *rec, int n_streams, const double *__restrict__ freq, int cap, double carrier_freq) {
+    const int d = blockIdx.x * blockDim.x + threadIdx.x;
+    if (d >= n_streams) return;
+    DemodResultDev r = rec[d];
+    if (r.n_fcch <= 0 || (r.flags & DM_FCCH_RANGE)) return;
+    double acc = 0.0;
+    for (int i = 0; i < r.n_fcch; ++i) acc += freq[(i64)d * cap + i];
+    r.fcch_mean_freq = acc / (double)r.n_fcch;
+    r.fcch_carrier_ppm = 1e6 * (r.fcch_mean_freq - ((1625.0 / 6.0) * 1e3) / 4.0) / carrier_freq;
+    rec[d] = r;
 }

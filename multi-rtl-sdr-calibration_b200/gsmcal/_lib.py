@@ -19,6 +19,11 @@ class StreamResult(C.Structure):
                 ("total_sampling_ppm", C.c_double), ("total_carrier_ppm", C.c_double)]
 
 
+class DemodResult(C.Structure):
+    _fields_ = [("n_sch", C.c_int32), ("n_sch_ok", C.c_int32), ("n_fcch", C.c_int32), ("flags", C.c_int32),
+                ("fcch_mean_freq", C.c_double), ("fcch_carrier_ppm", C.c_double)]
+
+
 # every symbol include/gsmcal.h declares: name -> (restype, argtypes)
 SIGNATURES = {
     "gsmcal_abi_version": (C.c_int, []),
@@ -59,6 +64,9 @@ SIGNATURES = {
                                          C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "gsmcal_calibrate_batch_r": (C.c_int, [C.c_void_p, C.c_int, c_i64, c_i64, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                            C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, c_i64]),
+    "gsmcal_calibrate_demod_batch": (C.c_int, [C.c_void_p, C.c_int, c_i64, c_i64, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                               C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                               C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "gsmcal_calibrate_batch_submit": (C.c_int, [C.c_int, C.c_void_p, c_i64, c_i64, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "gsmcal_calibrate_batch_collect": (C.c_int, [C.c_int]),

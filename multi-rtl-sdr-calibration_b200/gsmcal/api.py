@@ -11,7 +11,7 @@ import ctypes as C
 
 import numpy as np
 
-from ._lib import GsmcalError, StreamResult, check, lib  # noqa: F401
+from ._lib import DemodResult, GsmcalError, StreamResult, check, lib  # noqa: F401
 
 SYMBOL_RATE = (1625.0 / 6.0) * 1e3
 
@@ -348,6 +348,54 @@ def calibrate_batch(raw, carrier_freq: float, sch_training_sequence, coef, osr: 
     return _unpack_results(res, D, cap, coarse_pos, coarse_snr, fcch_pos, pos_info)
 
 
+DEMOD_NO_POS_INFO, DEMOD_NO_R_CORRECT, DEMOD_SCH_RANGE, DEMOD_FCCH_RANGE = 1, 2, 4, 8
+
+
+def calibrate_demod_batch(raw, carrier_freq: float, sch_training_sequence, coef, osr: int = 8, coarse_dr: int = 8,
+                          device_ptr: int | None = None, n_iq: int | None = None, n_streams: int | None = None, cuda_stream: int = 0):
+    """calibrate_batch followed by SCH_demod / FCCH_demod on every stream's r_correct (gsm_sync_demod.m:144-145), which is never
+    materialised.  Same inputs as calibrate_batch.  Each per-stream dict holds calibrate_batch's keys plus
+      sch:  dict(demod_bits [n x 148], bits_to_decoder [n x 148], corr_val [n x 85], sch_ok [n] bool), n = SCH rows of pos_info;
+            a row whose equaliser window leaves r_correct has sch_ok False and zeros;
+      fcch: dict(freq, mean_freq, carrier_ppm, snr, max_idx) as FCCH_demod returns it; NaN for a window outside r_correct, and
+            mean_freq / carrier_ppm NaN unless every window lies inside;
+      demod_flags: DEMOD_* bits.
+    sch and fcch are None where the demodulators do not run: pos_info == -1 (DEMOD_NO_POS_INFO) or r_correct == -1
+    (DEMOD_NO_R_CORRECT)."""
+    tpl = _stream(sch_training_sequence)
+    coef = np.ascontiguousarray(coef, dtype=np.float64)
+    if device_ptr is None:
+        raw = np.ascontiguousarray(raw, dtype=np.uint8)
+        if raw.ndim == 1:
+            raw = raw[None, :]
+        D, n_iq = raw.shape[0], raw.shape[1] // 2
+        ptr, mem = _ptr(raw), 0
+    else:
+        D, ptr, mem = int(n_streams), C.c_void_p(int(device_ptr)), 1
+    cap = max_bursts(n_iq, osr, coarse_dr)
+    res, dem = (StreamResult * D)(), (DemodResult * D)()
+    coarse_pos, coarse_snr, fcch_pos = np.empty((D, cap)), np.empty((D, cap)), np.empty((D, cap))
+    pos_info = np.empty((D, 6 * cap, 2))
+    sch_ok = np.zeros((D, cap), dtype=np.uint8)
+    bits, dec = np.zeros((D, cap, 148), dtype=np.uint8), np.zeros((D, cap, 148), dtype=np.uint8)
+    corr = np.zeros((D, cap, 85))
+    freq, snr, idx = np.empty((D, cap)), np.empty((D, cap)), np.empty((D, cap))
+    check(lib().gsmcal_calibrate_demod_batch(ptr, mem, int(n_iq), D, float(carrier_freq), _ptr(tpl), _ptr(coef), len(coef), int(osr), int(coarse_dr),
+                                             C.cast(res, C.c_void_p), _ptr(coarse_pos), _ptr(coarse_snr), _ptr(fcch_pos), _ptr(pos_info),
+                                             C.c_void_p(cuda_stream), C.cast(dem, C.c_void_p), _ptr(sch_ok), _ptr(bits), _ptr(dec), _ptr(corr),
+                                             _ptr(freq), _ptr(snr), _ptr(idx)))
+    out = _unpack_results(res, D, cap, coarse_pos, coarse_snr, fcch_pos, pos_info)
+    for d, item in enumerate(out):
+        r = dem[d]
+        item["demod_flags"] = r.flags
+        ns, nf = r.n_sch, r.n_fcch
+        item["sch"] = None if ns < 0 else dict(demod_bits=bits[d, :ns].astype(np.int64), bits_to_decoder=dec[d, :ns].astype(np.int64),
+                                               corr_val=corr[d, :ns].copy(), sch_ok=sch_ok[d, :ns].astype(bool))
+        item["fcch"] = None if nf < 0 else dict(freq=freq[d, :nf].copy(), mean_freq=r.fcch_mean_freq, carrier_ppm=r.fcch_carrier_ppm,
+                                                snr=snr[d, :nf].copy(), max_idx=idx[d, :nf].copy())
+    return out
+
+
 class PendingBatch:
     """A batch submitted with calibrate_batch_submit: owns the output arrays until collect() fills them."""
 
@@ -396,7 +444,7 @@ def calibrate_batch_submit(slot: int, device_ptr: int, n_iq: int, n_streams: int
     return PendingBatch(int(slot), D, cap, res, arrays, (tpl, coef))
 
 
-STAGE_NAMES = ("colsum_u8", "coarse", "fine_peak", "fine_tone", "sch", "post")
+STAGE_NAMES = ("colsum_u8", "coarse", "fine_peak", "fine_tone", "sch", "post", "demod")
 
 
 def last_batch_stage_ms() -> dict:

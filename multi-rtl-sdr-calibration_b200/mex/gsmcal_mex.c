@@ -301,6 +301,74 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
     mxFree(res); mxFree(pi); if (own) mxFree((void *)tpl);
 }
 
+#elif defined(GSMCAL_MEX_gsm_calibrate_demod_batch)
+/* [sampling_ppm, carrier_ppm, n_pos_info, pos_info, sch, fcch] = gsm_calibrate_demod_batch(raw_uint8, carrier_freq, sch_training_sequence, coef)
+ * gsm_calibrate_batch (outputs 1-4 as there) followed by SCH_demod / FCCH_demod on every dongle's r_correct (gsm_sync_demod.m:144-145).
+ * sch, fcch: 1 x D struct arrays, one element per dongle.
+ *   sch(d):  demod_bits, bits_to_decoder (148 x n_sch), corr_val (85 x n_sch), sch_ok (1 x n_sch), flags;
+ *   fcch(d): freq, snr, max_idx (1 x n_fcch), mean_freq, carrier_ppm, flags.
+ * Where the reference would not get that far (pos_info == -1, r_correct == -1: flags 1 / 2) the fields are empty and n_sch = -1 is
+ * reported as empty arrays; flags 4 / 8: a window leaves r_correct (sch_ok 0 / NaN rows, NaN mean).  See include/gsmcal.h. */
+void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
+    init_once(); need(nrhs, 4, "[sampling_ppm,carrier_ppm,n_pos_info,pos_info,sch,fcch] = gsm_calibrate_demod_batch(raw_uint8,carrier_freq,sch_training_sequence,coef)");
+    if (!mxIsUint8(prhs[0])) mexErrMsgIdAndTxt("gsmcal:type", "raw must be uint8");
+    size_t rows = mxGetM(prhs[0]), D = mxGetN(prhs[0]);
+    int own; const double *tpl = get_c128(prhs[2], &own);
+    size_t nt; const double *coef = real_vector(prhs[3], &nt);
+    int64_t n_iq = (int64_t)(rows / 2);
+    size_t B = (size_t)gsmcal_max_bursts((n_iq + 63) / 64, 8), R = D * B;
+    gsmcal_stream_result *res = (gsmcal_stream_result *)mxMalloc(D * sizeof(*res));
+    gsmcal_demod_result *dem = (gsmcal_demod_result *)mxMalloc(D * sizeof(*dem));
+    double *pi = (double *)mxMalloc(D * 12 * B * sizeof(double));
+    uint8_t *ok = (uint8_t *)mxMalloc(R * (1 + 2 * 148)), *bits = ok + R, *dec = bits + 148 * R;
+    double *corr = (double *)mxMalloc(R * 88 * sizeof(double)), *freq = corr + 85 * R, *snr = freq + R, *idx = snr + R;
+    fail_on(gsmcal_calibrate_demod_batch((const uint8_t *)mxGetData(prhs[0]), GSMCAL_MEM_HOST, n_iq, (int64_t)D, mxGetScalar(prhs[1]), tpl, coef, (int)nt, 8, 8,
+                                         res, NULL, NULL, NULL, pi, NULL, dem, ok, bits, dec, corr, freq, snr, idx), "gsm_calibrate_demod_batch");
+    plhs[0] = mxCreateDoubleMatrix(3, D, mxREAL);
+    if (nlhs > 1) plhs[1] = mxCreateDoubleMatrix(3, D, mxREAL);
+    if (nlhs > 2) plhs[2] = mxCreateDoubleMatrix(1, D, mxREAL);
+    for (size_t d = 0; d < D; ++d) {
+        double *sp = mxGetPr(plhs[0]) + 3 * d;
+        sp[0] = res[d].sampling_ppm[0]; sp[1] = res[d].sampling_ppm[1]; sp[2] = res[d].total_sampling_ppm;
+        if (nlhs > 1) { double *cp = mxGetPr(plhs[1]) + 3 * d; cp[0] = res[d].carrier_ppm[0]; cp[1] = res[d].carrier_ppm[1]; cp[2] = res[d].total_carrier_ppm; }
+        if (nlhs > 2) mxGetPr(plhs[2])[d] = res[d].n_pos_info;
+    }
+    if (nlhs > 3) {
+        size_t dims[3] = {6 * B, 2, D};
+        plhs[3] = mxCreateNumericArray(3, dims, mxDOUBLE_CLASS, mxREAL);
+        double *o = mxGetPr(plhs[3]);
+        for (size_t d = 0; d < D; ++d)
+            for (size_t i = 0; i < 6 * B; ++i)
+                for (int c = 0; c < 2; ++c)
+                    o[d * 12 * B + c * 6 * B + i] = ((int64_t)i < res[d].n_pos_info) ? pi[d * 12 * B + 2 * i + c] : mxGetNaN();
+    }
+    if (nlhs > 4) {
+        const char *f[] = {"demod_bits", "bits_to_decoder", "corr_val", "sch_ok", "flags"};
+        plhs[4] = mxCreateStructMatrix(1, D, 5, f);
+        for (size_t d = 0; d < D; ++d) {
+            size_t k = dem[d].n_sch < 0 ? 0 : (size_t)dem[d].n_sch;
+            mxArray *a = mxCreateDoubleMatrix(148, k, mxREAL), *b = mxCreateDoubleMatrix(148, k, mxREAL);
+            mxArray *cv = mxCreateDoubleMatrix(85, k, mxREAL), *so = mxCreateDoubleMatrix(1, k, mxREAL);
+            for (size_t i = 0; i < 148 * k; ++i) { mxGetPr(a)[i] = bits[148 * d * B + i]; mxGetPr(b)[i] = dec[148 * d * B + i]; }
+            if (k) memcpy(mxGetPr(cv), corr + 85 * d * B, 85 * k * sizeof(double));
+            for (size_t i = 0; i < k; ++i) mxGetPr(so)[i] = ok[d * B + i];
+            mxSetField(plhs[4], d, "demod_bits", a); mxSetField(plhs[4], d, "bits_to_decoder", b); mxSetField(plhs[4], d, "corr_val", cv);
+            mxSetField(plhs[4], d, "sch_ok", so); mxSetField(plhs[4], d, "flags", scalar(dem[d].flags));
+        }
+    }
+    if (nlhs > 5) {
+        const char *f[] = {"freq", "snr", "max_idx", "mean_freq", "carrier_ppm", "flags"};
+        plhs[5] = mxCreateStructMatrix(1, D, 6, f);
+        for (size_t d = 0; d < D; ++d) {
+            size_t k = dem[d].n_fcch < 0 ? 0 : (size_t)dem[d].n_fcch;
+            mxSetField(plhs[5], d, "freq", row_vector(freq + d * B, k)); mxSetField(plhs[5], d, "snr", row_vector(snr + d * B, k));
+            mxSetField(plhs[5], d, "max_idx", row_vector(idx + d * B, k)); mxSetField(plhs[5], d, "mean_freq", scalar(dem[d].fcch_mean_freq));
+            mxSetField(plhs[5], d, "carrier_ppm", scalar(dem[d].fcch_carrier_ppm)); mxSetField(plhs[5], d, "flags", scalar(dem[d].flags));
+        }
+    }
+    mxFree(res); mxFree(dem); mxFree(pi); mxFree(ok); mxFree(corr); if (own) mxFree((void *)tpl);
+}
+
 #elif defined(GSMCAL_MEX_gsm_normal_training_sequence_gen)
 /* s = gsm_normal_training_sequence_gen(oversampling_ratio)                 gsm_normal_training_sequence_gen.m:5 */
 void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {

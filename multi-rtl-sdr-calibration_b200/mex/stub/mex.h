@@ -11,10 +11,11 @@
 #include <string.h>
 
 typedef enum { mxREAL = 0, mxCOMPLEX = 1 } mxComplexity;
-typedef enum { mxDOUBLE_CLASS = 6, mxUINT8_CLASS = 9, mxLOGICAL_CLASS = 3 } mxClassID;
+typedef enum { mxDOUBLE_CLASS = 6, mxUINT8_CLASS = 9, mxLOGICAL_CLASS = 3, mxSTRUCT_CLASS = 2 } mxClassID;
 typedef struct mxArray_tag {
     mxClassID cls; int is_complex; size_t ndim; size_t dims[3];
     void *re; void *im;
+    int nfields; const char **fnames;     /* struct arrays: re holds nfields mxArray* per element */
 } mxArray;
 typedef int bool_t_;
 
@@ -58,6 +59,18 @@ static double *mxGetDoubles(const mxArray *a) { return (double *)a->re; }
 static mxArray *mxCreateDoubleMatrix(size_t m, size_t n, mxComplexity c) { size_t d[2] = {m, n}; return mxCreateNumericArray(2, d, mxDOUBLE_CLASS, c); }
 static mxArray *mxCreateDoubleScalar(double v) { mxArray *a = mxCreateDoubleMatrix(1, 1, mxREAL); ((double *)a->re)[0] = v; return a; }
 static mxArray *mxCreateLogicalScalar(int v) { size_t d[2] = {1, 1}; mxArray *a = mxCreateNumericArray(2, d, mxLOGICAL_CLASS, mxREAL); ((unsigned char *)a->re)[0] = v ? 1 : 0; return a; }
+static mxArray *mxCreateStructMatrix(size_t m, size_t n, int nfields, const char **fieldnames) {
+    mxArray *a = (mxArray *)calloc(1, sizeof(mxArray));
+    a->cls = mxSTRUCT_CLASS; a->ndim = 2; a->dims[0] = m; a->dims[1] = n; a->nfields = nfields;
+    a->fnames = (const char **)calloc((size_t)nfields, sizeof(char *));
+    for (int f = 0; f < nfields; ++f) a->fnames[f] = fieldnames[f];
+    a->re = calloc((m * n ? m * n : 1) * (size_t)nfields, sizeof(mxArray *));
+    return a;
+}
+static int mxIsStruct(const mxArray *a) { return a->cls == mxSTRUCT_CLASS; }
+static int mx_field_(const mxArray *a, const char *name) { for (int f = 0; f < a->nfields; ++f) if (!strcmp(a->fnames[f], name)) return f; return -1; }
+static void mxSetField(mxArray *a, size_t i, const char *name, mxArray *v) { int f = mx_field_(a, name); if (f >= 0) ((mxArray **)a->re)[i * a->nfields + f] = v; }
+static mxArray *mxGetField(const mxArray *a, size_t i, const char *name) { int f = mx_field_(a, name); return f < 0 ? NULL : ((mxArray **)a->re)[i * a->nfields + f]; }
 static void mxDestroyArray(mxArray *a) { if (a) { free(a->re); free(a->im); free(a); } }
 
 void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]);
