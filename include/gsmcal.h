@@ -251,6 +251,44 @@ int gsmcal_calibrate_demod_batch(const uint8_t *raw, int raw_mem, int64_t n_iq, 
                                  uint8_t *demod_bits, uint8_t *bits_to_decoder, double *corr_val,
                                  double *fcch_freq, double *fcch_snr, double *fcch_max_idx);
 
+/* gsmcal_calibrate_demod_batch (every output as there, byte for byte) followed by BCCH_demod (gsm_sync_demod.m:146, BCCH_demod.m:5-106)
+ * on every stream's r_correct, again without materialising it.  BCCH_demod's carrier ppm is that of carrier_correct_post_SCH on
+ * r_correct: the FCCH rows' tone-frequency mean, i.e. gsmcal_demod_result.fcch_carrier_ppm (copied bit for bit).  The training windows
+ * r_bcch(p+61*osr : p+61*osr+26*osr-1) of the first four BCCH rows, r_bcch(j) = r_correct(j)*exp(1i*(j-1)*comp) with
+ * comp = (fs_sym/4 - mean_freq)*2*pi/fs (:72-73, :85-89), are correlated with the eight normal training sequences (:91).
+ * normal_training_sequence: (26*osr) x 8 complex128, column-major (gsmcal_normal_training_sequence_gen).  One record per stream;
+ * the first flag that applies decides, in this order:
+ *   GSMCAL_BCCH_NO_POS_INFO  pos_info == -1 (:9-11):                 carrier_ppm -1,  nts_idx -1, corr_abs NaN
+ *   GSMCAL_BCCH_FEW_BCCH     fewer than four BCCH rows (:13-17):      carrier_ppm -1,  nts_idx -1, corr_abs NaN
+ *                            (also every stream whose pos_info is valid but r_correct = -1: that happens only with too few BCCH rows)
+ *   GSMCAL_BCCH_FCCH_RANGE   no FCCH mean (no FCCH row, or an FCCH window leaves r_correct; gsmcal_BCCH_demod returns GSMCAL_ERR_RANGE):
+ *                            carrier_ppm NaN, nts_idx -1, corr_abs NaN
+ *   GSMCAL_BCCH_TRAIN_RANGE  a training window leaves r_correct (the reference would raise): that burst's column NaN, nts_idx -1
+ *   0                        nts_idx 1..8 when the first maxima of the four columns agree (:93-102), else -1. */
+typedef struct gsmcal_bcch_result {
+    double  carrier_ppm;      /* BCCH_demod.m:68 on r_correct (== gsmcal_demod_result.fcch_carrier_ppm); -1 / NaN per the flags */
+    int32_t nts_idx;          /* 1..8, or -1 */
+    int32_t flags;            /* GSMCAL_BCCH_* */
+    double  corr_abs[32];     /* abs(corr_val), 8 x 4 column-major (:91-93) */
+} gsmcal_bcch_result;         /* 272 bytes */
+
+#define GSMCAL_BCCH_NO_POS_INFO  1
+#define GSMCAL_BCCH_FEW_BCCH     2
+#define GSMCAL_BCCH_FCCH_RANGE   4
+#define GSMCAL_BCCH_TRAIN_RANGE  8
+
+int gsmcal_calibrate_demod_bcch_batch(const uint8_t *raw, int raw_mem, int64_t n_iq, int64_t n_streams,
+                                      double carrier_freq, const double *sch_training_sequence,
+                                      const double *coef, int n_taps, int oversampling_ratio, int coarse_decimation,
+                                      gsmcal_stream_result *results,
+                                      double *coarse_pos, double *coarse_snr, double *fcch_pos, double *pos_info,
+                                      void *cuda_stream,
+                                      gsmcal_demod_result *demod /* [n_streams], required */, uint8_t *sch_ok,
+                                      uint8_t *demod_bits, uint8_t *bits_to_decoder, double *corr_val,
+                                      double *fcch_freq, double *fcch_snr, double *fcch_max_idx,
+                                      const double *normal_training_sequence /* (26*osr) x 8 complex128, column-major */,
+                                      gsmcal_bcch_result *bcch /* [n_streams], required */);
+
 /* The same pipeline with several batches in flight (continuous captures): _submit enqueues batch `slot` (0..3) on the library's
  * own streams once the caller's `cuda_stream` has produced the DEVICE-resident capture, and returns; _collect waits for that batch
  * and fills the result pointers given to _submit (they must stay valid until then).  Batches are staggered on the device: the
@@ -272,7 +310,7 @@ int gsmcal_calibrate_batch_cancel(int slot);
 /* CUDA-event times (ms) of the stages of the last gsmcal_calibrate_batch call on this process:
  * [0] uint8 column sums (+ H2D when raw is on the host) [1] coarse FCCH [2] fine FCCH sliding-DFT peak search
  * [3] fine ppm + tone estimate + gate [4] SCH correlation + pos_info [5] post-SCH tone estimate + result records
- * [6] (gsmcal_calibrate_demod_batch only) SCH_demod + FCCH_demod.  Returns the number of stages written. */
+ * [6] (gsmcal_calibrate_demod_batch / _demod_bcch_batch only) SCH_demod + FCCH_demod (+ BCCH_demod).  Returns the number of stages written. */
 int gsmcal_last_batch_stage_ms(double *ms, int cap);
 
 /* FCCH scanner per-channel processing, multi_rtl_sdr_gsm_FCCH_scanner.m:132-135,163-186, for n_chan

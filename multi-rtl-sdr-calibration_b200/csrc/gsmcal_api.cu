@@ -8,6 +8,7 @@
 #include <atomic>
 #include <cmath>
 #include <cstdarg>
+#include <cstddef>
 #include <cstdio>
 #include <cstring>
 #include <map>
@@ -22,6 +23,10 @@ static_assert(sizeof(gsmcal_stream_result) == sizeof(StreamResultDev), "result r
 static_assert(sizeof(gsmcal_demod_result) == sizeof(DemodResultDev) && sizeof(gsmcal_demod_result) == 32, "demod record layout");
 static_assert(GSMCAL_DEMOD_NO_POS_INFO == DM_NO_POS_INFO && GSMCAL_DEMOD_NO_R_CORRECT == DM_NO_R_CORRECT && GSMCAL_DEMOD_SCH_RANGE == DM_SCH_RANGE &&
               GSMCAL_DEMOD_FCCH_RANGE == DM_FCCH_RANGE, "demod flags");
+static_assert(sizeof(gsmcal_bcch_result) == sizeof(BcchResultDev) && sizeof(gsmcal_bcch_result) == 272 && offsetof(gsmcal_bcch_result, nts_idx) == 8 &&
+              offsetof(gsmcal_bcch_result, flags) == 12 && offsetof(gsmcal_bcch_result, corr_abs) == 16, "BCCH record layout");
+static_assert(GSMCAL_BCCH_NO_POS_INFO == BC_NO_POS_INFO && GSMCAL_BCCH_FEW_BCCH == BC_FEW_BCCH && GSMCAL_BCCH_FCCH_RANGE == BC_FCCH_RANGE &&
+              GSMCAL_BCCH_TRAIN_RANGE == BC_TRAIN_RANGE, "BCCH flags");
 
 namespace {
 
@@ -501,20 +506,25 @@ void sch_training_pm(signed char *data_pm);
 // ---- batched SCH_demod / FCCH_demod stage of gsmcal_calibrate_demod_batch -----------------------------------------------------
 struct DemodOut {                    // the caller's host outputs (any per-row pointer may be NULL)
     gsmcal_demod_result *rec; uint8_t *sch_ok, *bits, *dec; double *corr, *freq, *snr, *idx;
+    const double *nts; gsmcal_bcch_result *bcch;     // BCCH_demod inputs / outputs (gsmcal_calibrate_demod_bcch_batch), else both NULL
 };
 struct DemodDev {                    // device buffers, [D][cap] rows unless noted
     DemodResultDev *rec; double *sch_pos, *fcch_pos, *corr /* x85 */, *freq, *snr, *idx;
     unsigned char *sch_ok, *fcch_ok, *bits /* x148 */, *dec /* x148 */; double2 *Ft /* N */, *Wtab /* 16*osr */; signed char *dpm /* 64 */;
+    double2 *nts /* (26*osr) x 8 */; BcchResultDev *bcch /* [D]; nullptr: no BCCH stage */;
 };
 DemodDev sub_demod(const DemodDev &a, i64 d0, int cap) {
     DemodDev s = a;
     const i64 r = d0 * cap;
     s.rec += d0; s.sch_pos += r; s.fcch_pos += r; s.corr += r * 85; s.freq += r; s.snr += r; s.idx += r;
     s.sch_ok += r; s.fcch_ok += r; s.bits += r * 148; s.dec += r * 148;
+    if (s.bcch) s.bcch += d0;
     return s;
 }
-// workspace, branch table, training bits and fft(template) (SCH_demod.m:47-59), once per call on `st` before the stream groups fork
-int demod_setup(Ctx &c, i64 D, int cap, int osr, const double2 *tpl_dev, std::vector<double> &W, signed char *data_pm, cudaStream_t st, DemodDev *dd) {
+// workspace, branch table, training bits and fft(template) (SCH_demod.m:47-59), and with nts (host, (26*osr) x 8 complex) the normal
+// training sequences and the BCCH records behind them; once per call on `st` before the stream groups fork
+int demod_setup(Ctx &c, i64 D, int cap, int osr, const double2 *tpl_dev, const double *nts, std::vector<double> &W, signed char *data_pm, cudaStream_t st,
+                DemodDev *dd) {
     const int N = SD_NSYM * osr;
     size_t off = 0;
     auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes); return o; };
@@ -522,12 +532,15 @@ int demod_setup(Ctx &c, i64 D, int cap, int osr, const double2 *tpl_dev, std::ve
     const size_t o_rec = take(sizeof(DemodResultDev) * D), o_sp = take(8 * rows), o_fp = take(8 * rows), o_corr = take(8 * 85 * rows),
                  o_fr = take(8 * rows), o_sn = take(8 * rows), o_ix = take(8 * rows), o_so = take(rows), o_fo = take(rows),
                  o_b = take(148 * rows), o_d = take(148 * rows), o_ft = take(sizeof(double2) * N), o_w = take(sizeof(double2) * 16 * osr), o_pm = take(64);
+    const size_t o_nts = nts ? take(sizeof(double2) * 8 * 26 * osr) : 0, o_bc = nts ? take(sizeof(BcchResultDev) * D) : 0;
     void *base; TRY(c.dem.get(off, &base));
     char *b = (char *)base;
     dd->rec = (DemodResultDev *)(b + o_rec); dd->sch_pos = (double *)(b + o_sp); dd->fcch_pos = (double *)(b + o_fp); dd->corr = (double *)(b + o_corr);
     dd->freq = (double *)(b + o_fr); dd->snr = (double *)(b + o_sn); dd->idx = (double *)(b + o_ix);
     dd->sch_ok = (unsigned char *)(b + o_so); dd->fcch_ok = (unsigned char *)(b + o_fo); dd->bits = (unsigned char *)(b + o_b); dd->dec = (unsigned char *)(b + o_d);
     dd->Ft = (double2 *)(b + o_ft); dd->Wtab = (double2 *)(b + o_w); dd->dpm = (signed char *)(b + o_pm);
+    dd->nts = nts ? (double2 *)(b + o_nts) : nullptr; dd->bcch = nts ? (BcchResultDev *)(b + o_bc) : nullptr;
+    if (nts) CU(cudaMemcpyAsync(dd->nts, nts, sizeof(double2) * 8 * 26 * (size_t)osr, cudaMemcpyHostToDevice, st));
     W.assign(2 * 16 * (size_t)osr, 0.0);
     gmsk_branch_table(osr, W.data());
     sch_training_pm(data_pm);
@@ -537,7 +550,7 @@ int demod_setup(Ctx &c, i64 D, int cap, int osr, const double2 *tpl_dev, std::ve
     LAUNCH(fde_template_kernel, 1, SD_THREADS, 3 * (size_t)N * sizeof(double2), st, tpl_dev, osr, tw, dd->Ft);
     return GSMCAL_OK;
 }
-// one stream group: row lists + sentinels, SCH bursts, FCCH bursts, FCCH means
+// one stream group: row lists + sentinels, SCH bursts, FCCH bursts, FCCH means, and BCCH_demod when its outputs were asked for
 int run_demod(Ctx &c, WinSrc src, const Work &ws, const DemodDev &dd, int osr, double carrier_freq, i64 nd, int cap, cudaStream_t st) {
     const double2 *tw_s, *tw_f;
     TRY(get_twiddle(c, SD_NSYM * osr, st, &tw_s));
@@ -549,6 +562,11 @@ int run_demod(Ctx &c, WinSrc src, const Work &ws, const DemodDev &dd, int osr, d
     LAUNCH(fcch_demod_batch_kernel, dim3((unsigned)cap, (unsigned)nd), FD_THREADS, fs > fs_load ? fs : fs_load, st, with_cache(src, ws, cap), ws.ctl, dd.rec,
            dd.fcch_pos, dd.fcch_ok, cap, osr, tw_f, dd.freq, dd.snr, dd.idx);
     LAUNCH(demod_fcch_mean_kernel, (unsigned)((nd + 127) / 128), 128, 0, st, dd.rec, (int)nd, dd.freq, cap, carrier_freq);
+    if (dd.bcch) {
+        const int L = 26 * osr;
+        LAUNCH(bcch_demod_batch_kernel, (unsigned)nd, BC_THREADS, sizeof(double2) * (size_t)(L + GSMCAL_XCAP(L) + L + 8), st, src, ws.ctl, dd.rec, ws.pos_info,
+               cap, osr, dd.nts, dd.bcch);
+    }
     return GSMCAL_OK;
 }
 
@@ -1097,7 +1115,7 @@ static int calibrate_batch_impl(const uint8_t *raw, int raw_mem, int64_t n_iq, i
     CU(cudaMemsetAsync(w.pass_hist, 0, sizeof(unsigned) * 16 + sizeof(unsigned long long) * 64, st));
     DemodDev dd;
     std::vector<double> dm_w; signed char dm_pm[64];                 // host sources of the uploads, alive until the final synchronise
-    if (dm) TRY(demod_setup(*c, D, cap, osr, w.tpl, dm_w, dm_pm, st, &dd));
+    if (dm) TRY(demod_setup(*c, D, cap, osr, w.tpl, dm->nts, dm_w, dm_pm, st, &dd));
     g_stage_n = 0;
     // Streams are independent, so the batch is cut into groups that run the stage sequence on their own CUDA
     // streams: the latency-bound stages of one group (burst chain, per-stream solves) overlap the FP64-bound
@@ -1214,6 +1232,7 @@ static int calibrate_batch_impl(const uint8_t *raw, int raw_mem, int64_t n_iq, i
         if (dm->freq) TRY(copy_d2h(c->ring, g_device, dm->freq, dd.freq, sizeof(double) * rows, st));
         if (dm->snr) TRY(copy_d2h(c->ring, g_device, dm->snr, dd.snr, sizeof(double) * rows, st));
         if (dm->idx) TRY(copy_d2h(c->ring, g_device, dm->idx, dd.idx, sizeof(double) * rows, st));
+        if (dm->bcch) CU(cudaMemcpyAsync(dm->bcch, dd.bcch, sizeof(BcchResultDev) * D, cudaMemcpyDeviceToHost, st));
     }
     CU(cudaStreamSynchronize(st));
     if (timing) for (int i = 0; i + 1 < g_stage_n; ++i) CU(cudaEventElapsedTime(&g_stage_ms[i], c->stage_ev[i], c->stage_ev[i + 1]));
@@ -1243,7 +1262,19 @@ int gsmcal_calibrate_demod_batch(const uint8_t *raw, int raw_mem, int64_t n_iq, 
                                  gsmcal_demod_result *demod, uint8_t *sch_ok, uint8_t *demod_bits, uint8_t *bits_to_decoder, double *corr_val,
                                  double *fcch_freq, double *fcch_snr, double *fcch_max_idx) {
     if (!demod) return fail(GSMCAL_ERR_ARG, "calibrate_demod_batch: null demod");
-    const DemodOut o = {demod, sch_ok, demod_bits, bits_to_decoder, corr_val, fcch_freq, fcch_snr, fcch_max_idx};
+    const DemodOut o = {demod, sch_ok, demod_bits, bits_to_decoder, corr_val, fcch_freq, fcch_snr, fcch_max_idx, nullptr, nullptr};
+    return calibrate_batch_impl(raw, raw_mem, n_iq, D, carrier_freq, tpl, coef, n_taps, osr, coarse_dr, results, coarse_pos, coarse_snr, fcch_pos, pos_info,
+                                cuda_stream, nullptr, GSMCAL_MEM_DEVICE, 0, &o);
+}
+
+int gsmcal_calibrate_demod_bcch_batch(const uint8_t *raw, int raw_mem, int64_t n_iq, int64_t D, double carrier_freq, const double *tpl,
+                                      const double *coef, int n_taps, int osr, int coarse_dr, gsmcal_stream_result *results,
+                                      double *coarse_pos, double *coarse_snr, double *fcch_pos, double *pos_info, void *cuda_stream,
+                                      gsmcal_demod_result *demod, uint8_t *sch_ok, uint8_t *demod_bits, uint8_t *bits_to_decoder, double *corr_val,
+                                      double *fcch_freq, double *fcch_snr, double *fcch_max_idx,
+                                      const double *normal_training_sequence, gsmcal_bcch_result *bcch) {
+    if (!demod || !normal_training_sequence || !bcch) return fail(GSMCAL_ERR_ARG, "calibrate_demod_bcch_batch: null demod, normal_training_sequence or bcch");
+    const DemodOut o = {demod, sch_ok, demod_bits, bits_to_decoder, corr_val, fcch_freq, fcch_snr, fcch_max_idx, normal_training_sequence, bcch};
     return calibrate_batch_impl(raw, raw_mem, n_iq, D, carrier_freq, tpl, coef, n_taps, osr, coarse_dr, results, coarse_pos, coarse_snr, fcch_pos, pos_info,
                                 cuda_stream, nullptr, GSMCAL_MEM_DEVICE, 0, &o);
 }

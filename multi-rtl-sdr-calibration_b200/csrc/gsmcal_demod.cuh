@@ -495,3 +495,104 @@ __global__ void demod_fcch_mean_kernel(DemodResultDev *rec, int n_streams, const
     r.fcch_carrier_ppm = 1e6 * (r.fcch_mean_freq - ((1625.0 / 6.0) * 1e3) / 4.0) / carrier_freq;
     rec[d] = r;
 }
+
+// ===================================================================================================
+// Batched BCCH_demod (gsm_sync_demod.m:146) for every stream of gsmcal_calibrate_demod_bcch_batch.  Its carrier_correct_post_SCH on
+// r_correct (BCCH_demod.m:47-70) runs tone_freq_estimate over the FCCH rows and takes their mean: the statements and windows of
+// FCCH_demod.m:36-47, so the carrier ppm is rec.fcch_carrier_ppm and the compensation phase comes from rec.fcch_mean_freq.  Left to do:
+// the first four BCCH rows, their training windows r_bcch(p+61*osr : p+61*osr+26*osr-1) with r_bcch(j) = r_correct(j)*exp(1i*(j-1)*comp)
+// (:72-73, :85-89), the 8 x 4 correlations with the normal training sequences (:91) and the agreement decision (:93-102).
+// ===================================================================================================
+struct BcchResultDev {               // mirrors gsmcal_bcch_result (include/gsmcal.h)
+    double carrier_ppm;
+    int nts_idx, flags;
+    double corr_abs[32];             // 8 x 4 column-major
+};
+#define BC_NO_POS_INFO  1
+#define BC_FEW_BCCH     2
+#define BC_FCCH_RANGE   4
+#define BC_TRAIN_RANGE  8
+
+// One block per stream, one warp per normal training sequence (as nts_corr_kernel).  Shared: window w[26*osr] | the loader's scratch
+// X[GSMCAL_XCAP(26*osr)] | Y[26*osr + 8].  Sentinels, in the reference's order: pos_info == -1 (BCCH_demod.m:9-11), fewer than four
+// BCCH rows (:13-17), no FCCH mean (no FCCH row, or an FCCH window outside r_correct), then per burst a training window outside
+// r_correct (NaN column, nts_idx = -1).
+#define BC_THREADS 256
+__global__ void __launch_bounds__(BC_THREADS) bcch_demod_batch_kernel(WinSrc src, const StreamCtl *__restrict__ ctl, const DemodResultDev *__restrict__ rec,
+                                                                     const double *__restrict__ pos_info /* [stream][6*cap][2] */, int cap, int osr,
+                                                                     const double2 *__restrict__ nts /* (26*osr) x 8 column-major */,
+                                                                     BcchResultDev *__restrict__ out) {
+    extern __shared__ double2 sm[];
+    __shared__ double bpos[4];
+    __shared__ int n_bcch;
+    __shared__ double mag[32];
+    __shared__ double2 ph_a, ph_b;
+    const int stream = blockIdx.x, tid = threadIdx.x, q = tid >> 5, lane = tid & 31;
+    const int L = 26 * osr;
+    const DemodResultDev r = rec[stream];
+    BcchResultDev *o = out + stream;
+    int flags = 0;
+    if (r.flags & DM_NO_POS_INFO) flags = BC_NO_POS_INFO;
+    else {
+        if (q == 0) {                                           // the first four type-2 rows of pos_info, in pos_info order
+            const double *pi = pos_info + (i64)stream * 6 * cap * 2;
+            const int rows = ctl[stream].n_pos_info;
+            const unsigned below = (1u << lane) - 1u;
+            int nb = 0;
+            for (int i0 = 0; i0 < rows && nb < 4; i0 += 32) {
+                const int i = i0 + lane;
+                const bool is_b = i < rows && pi[2 * i + 1] == 2.0;
+                const unsigned mb = __ballot_sync(0xffffffffu, is_b);
+                const int k = nb + __popc(mb & below);
+                if (is_b && k < 4) bpos[k] = pi[2 * i];
+                nb += __popc(mb);
+            }
+            if (lane == 0) n_bcch = nb;
+        }
+        __syncthreads();
+        if (n_bcch < 4) flags = BC_FEW_BCCH;
+        else if (isnan(r.fcch_mean_freq)) flags = BC_FCCH_RANGE;
+    }
+    if (flags) {
+        if (tid < 32) o->corr_abs[tid] = NAN;
+        if (tid == 0) { o->carrier_ppm = (flags == BC_FCCH_RANGE) ? NAN : -1.0; o->nts_idx = -1; o->flags = flags; }
+        return;
+    }
+    const StreamCtl c = ctl[stream];
+    const double symbol_rate = (1625.0 / 6.0) * 1e3, target = symbol_rate / 4.0;
+    const double comp = (target - r.fcch_mean_freq) * 2 * GSMCAL_PI / (symbol_rate * osr);      // carrier_correct_post_SCH's comp_phase_rotate
+    double2 *w = sm, *X = w + L, *Y = X + GSMCAL_XCAP(L);
+    for (int b = 0; b < 4; ++b) {
+        const double p = bpos[b];
+        if (!(p == floor(p) && p + 61 * osr >= 1.0 && p + 61 * osr + L - 1 <= (double)c.len3)) {       // the reference would raise (:85-89)
+            flags = BC_TRAIN_RANGE;
+            if (lane == 0) mag[b * 8 + q] = NAN;
+            continue;
+        }
+        const i64 j0 = (i64)p + 61 * osr - 1;                  // 0-based first training sample
+        if (tid == 0) { double sn, cs; sincos((double)j0 * c.dphi2, &sn, &cs); ph_a = make_double2(cs, sn); }
+        if (tid == 32) { double sn, cs; sincos((double)j0 * comp, &sn, &cs); ph_b = make_double2(cs, sn); }
+        load_window(src, c, stream, j0, L, w, X, Y);           // ends with a barrier
+        derotate_post(w, L, c.dphi2, ph_a);                    // r_correct (carrier_correct_post_SCH.m:83)
+        derotate_post(w, L, comp, ph_b);                       // r_bcch (BCCH_demod.m:72-73); each thread rotates its own samples twice
+        __syncthreads();
+        double ar = 0.0, ai = 0.0;
+        for (int n = lane; n < L; n += 32) {
+            const double2 t = nts[(i64)q * L + n], v = w[n];
+            ar += t.x * v.x + t.y * v.y;                         // conj(t) * v
+            ai += t.x * v.y - t.y * v.x;
+        }
+        ar = warp_sum(ar); ai = warp_sum(ai);
+        if (lane == 0) mag[b * 8 + q] = hypot(ar, ai);
+        __syncthreads();                                       // w is reloaded for the next burst
+    }
+    __syncthreads();
+    if (tid < 32) o->corr_abs[tid] = mag[tid];
+    if (tid == 0) {
+        int idx[4];
+        for (int b = 0; b < 4; ++b) { idx[b] = 0; for (int k = 1; k < 8; ++k) if (mag[b * 8 + k] > mag[b * 8 + idx[b]]) idx[b] = k; }   // first maximum (:93)
+        o->carrier_ppm = r.fcch_carrier_ppm;
+        o->nts_idx = (!flags && idx[0] == idx[1] && idx[1] == idx[2] && idx[2] == idx[3]) ? idx[0] + 1 : -1;                   // :94-102
+        o->flags = flags;
+    }
+}

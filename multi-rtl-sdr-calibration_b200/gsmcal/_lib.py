@@ -24,6 +24,10 @@ class DemodResult(C.Structure):
                 ("fcch_mean_freq", C.c_double), ("fcch_carrier_ppm", C.c_double)]
 
 
+class BcchResult(C.Structure):
+    _fields_ = [("carrier_ppm", C.c_double), ("nts_idx", C.c_int32), ("flags", C.c_int32), ("corr_abs", C.c_double * 32)]
+
+
 # every symbol include/gsmcal.h declares: name -> (restype, argtypes)
 SIGNATURES = {
     "gsmcal_abi_version": (C.c_int, []),
@@ -67,6 +71,10 @@ SIGNATURES = {
     "gsmcal_calibrate_demod_batch": (C.c_int, [C.c_void_p, C.c_int, c_i64, c_i64, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                                C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                                C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "gsmcal_calibrate_demod_bcch_batch": (C.c_int, [C.c_void_p, C.c_int, c_i64, c_i64, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                    C.c_void_p, C.c_void_p]),
     "gsmcal_calibrate_batch_submit": (C.c_int, [C.c_int, C.c_void_p, c_i64, c_i64, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "gsmcal_calibrate_batch_collect": (C.c_int, [C.c_int]),

@@ -11,7 +11,7 @@ import ctypes as C
 
 import numpy as np
 
-from ._lib import DemodResult, GsmcalError, StreamResult, check, lib  # noqa: F401
+from ._lib import BcchResult, DemodResult, GsmcalError, StreamResult, check, lib  # noqa: F401
 
 SYMBOL_RATE = (1625.0 / 6.0) * 1e3
 
@@ -349,10 +349,12 @@ def calibrate_batch(raw, carrier_freq: float, sch_training_sequence, coef, osr: 
 
 
 DEMOD_NO_POS_INFO, DEMOD_NO_R_CORRECT, DEMOD_SCH_RANGE, DEMOD_FCCH_RANGE = 1, 2, 4, 8
+BCCH_NO_POS_INFO, BCCH_FEW_BCCH, BCCH_FCCH_RANGE, BCCH_TRAIN_RANGE = 1, 2, 4, 8
 
 
 def calibrate_demod_batch(raw, carrier_freq: float, sch_training_sequence, coef, osr: int = 8, coarse_dr: int = 8,
-                          device_ptr: int | None = None, n_iq: int | None = None, n_streams: int | None = None, cuda_stream: int = 0):
+                          device_ptr: int | None = None, n_iq: int | None = None, n_streams: int | None = None, cuda_stream: int = 0,
+                          normal_training_sequence=None):
     """calibrate_batch followed by SCH_demod / FCCH_demod on every stream's r_correct (gsm_sync_demod.m:144-145), which is never
     materialised.  Same inputs as calibrate_batch.  Each per-stream dict holds calibrate_batch's keys plus
       sch:  dict(demod_bits [n x 148], bits_to_decoder [n x 148], corr_val [n x 85], sch_ok [n] bool), n = SCH rows of pos_info;
@@ -361,7 +363,13 @@ def calibrate_demod_batch(raw, carrier_freq: float, sch_training_sequence, coef,
             mean_freq / carrier_ppm NaN unless every window lies inside;
       demod_flags: DEMOD_* bits.
     sch and fcch are None where the demodulators do not run: pos_info == -1 (DEMOD_NO_POS_INFO) or r_correct == -1
-    (DEMOD_NO_R_CORRECT)."""
+    (DEMOD_NO_R_CORRECT).
+    With normal_training_sequence ((26*osr) x 8, gsm_normal_training_sequence_gen) BCCH_demod (gsm_sync_demod.m:146) runs as well and
+    each dict gains
+      bcch: dict(carrier_ppm, nts_idx, corr_abs, flags): carrier_ppm of r_correct (== fcch carrier_ppm), nts_idx 1..8 or -1, corr_abs
+            abs(corr_val) 8 x 4 (NaN columns for training windows outside r_correct, BCCH_TRAIN_RANGE), flags BCCH_* bits; carrier_ppm,
+            nts_idx, corr_abs are (-1, -1, None) for BCCH_NO_POS_INFO / BCCH_FEW_BCCH as BCCH_demod returns them, (NaN, -1, None) for
+            BCCH_FCCH_RANGE (no FCCH mean to correct with)."""
     tpl = _stream(sch_training_sequence)
     coef = np.ascontiguousarray(coef, dtype=np.float64)
     if device_ptr is None:
@@ -380,10 +388,18 @@ def calibrate_demod_batch(raw, carrier_freq: float, sch_training_sequence, coef,
     bits, dec = np.zeros((D, cap, 148), dtype=np.uint8), np.zeros((D, cap, 148), dtype=np.uint8)
     corr = np.zeros((D, cap, 85))
     freq, snr, idx = np.empty((D, cap)), np.empty((D, cap)), np.empty((D, cap))
-    check(lib().gsmcal_calibrate_demod_batch(ptr, mem, int(n_iq), D, float(carrier_freq), _ptr(tpl), _ptr(coef), len(coef), int(osr), int(coarse_dr),
-                                             C.cast(res, C.c_void_p), _ptr(coarse_pos), _ptr(coarse_snr), _ptr(fcch_pos), _ptr(pos_info),
-                                             C.c_void_p(cuda_stream), C.cast(dem, C.c_void_p), _ptr(sch_ok), _ptr(bits), _ptr(dec), _ptr(corr),
-                                             _ptr(freq), _ptr(snr), _ptr(idx)))
+    args = [ptr, mem, int(n_iq), D, float(carrier_freq), _ptr(tpl), _ptr(coef), len(coef), int(osr), int(coarse_dr),
+            C.cast(res, C.c_void_p), _ptr(coarse_pos), _ptr(coarse_snr), _ptr(fcch_pos), _ptr(pos_info),
+            C.c_void_p(cuda_stream), C.cast(dem, C.c_void_p), _ptr(sch_ok), _ptr(bits), _ptr(dec), _ptr(corr), _ptr(freq), _ptr(snr), _ptr(idx)]
+    if normal_training_sequence is None:
+        check(lib().gsmcal_calibrate_demod_batch(*args))
+    else:
+        nts_m = np.asarray(normal_training_sequence)
+        if nts_m.shape != (26 * int(osr), 8):
+            raise ValueError("normal_training_sequence must be (26*osr) x 8")
+        nts = np.ascontiguousarray(nts_m.T, dtype=np.complex128)                # column-major (26*osr) x 8
+        bc = (BcchResult * D)()
+        check(lib().gsmcal_calibrate_demod_bcch_batch(*args, _ptr(nts), C.cast(bc, C.c_void_p)))
     out = _unpack_results(res, D, cap, coarse_pos, coarse_snr, fcch_pos, pos_info)
     for d, item in enumerate(out):
         r = dem[d]
@@ -393,6 +409,11 @@ def calibrate_demod_batch(raw, carrier_freq: float, sch_training_sequence, coef,
                                                corr_val=corr[d, :ns].copy(), sch_ok=sch_ok[d, :ns].astype(bool))
         item["fcch"] = None if nf < 0 else dict(freq=freq[d, :nf].copy(), mean_freq=r.fcch_mean_freq, carrier_ppm=r.fcch_carrier_ppm,
                                                 snr=snr[d, :nf].copy(), max_idx=idx[d, :nf].copy())
+        if normal_training_sequence is not None:
+            b = bc[d]
+            none = b.flags & (BCCH_NO_POS_INFO | BCCH_FEW_BCCH | BCCH_FCCH_RANGE)
+            item["bcch"] = dict(carrier_ppm=b.carrier_ppm, nts_idx=b.nts_idx, flags=b.flags,
+                                corr_abs=None if none else np.array(b.corr_abs).reshape(4, 8).T.copy())
     return out
 
 

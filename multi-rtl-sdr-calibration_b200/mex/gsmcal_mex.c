@@ -302,28 +302,46 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
 }
 
 #elif defined(GSMCAL_MEX_gsm_calibrate_demod_batch)
-/* [sampling_ppm, carrier_ppm, n_pos_info, pos_info, sch, fcch] = gsm_calibrate_demod_batch(raw_uint8, carrier_freq, sch_training_sequence, coef)
- * gsm_calibrate_batch (outputs 1-4 as there) followed by SCH_demod / FCCH_demod on every dongle's r_correct (gsm_sync_demod.m:144-145).
- * sch, fcch: 1 x D struct arrays, one element per dongle.
+/* [sampling_ppm, carrier_ppm, n_pos_info, pos_info, sch, fcch, bcch] =
+ *     gsm_calibrate_demod_batch(raw_uint8, carrier_freq, sch_training_sequence, coef [, normal_training_sequence])
+ * gsm_calibrate_batch (outputs 1-4 as there) followed by SCH_demod / FCCH_demod on every dongle's r_correct (gsm_sync_demod.m:144-145),
+ * and with normal_training_sequence ((26*8) x 8, gsm_normal_training_sequence_gen(8)) BCCH_demod as well (:146).
+ * sch, fcch, bcch: 1 x D struct arrays, one element per dongle.
  *   sch(d):  demod_bits, bits_to_decoder (148 x n_sch), corr_val (85 x n_sch), sch_ok (1 x n_sch), flags;
- *   fcch(d): freq, snr, max_idx (1 x n_fcch), mean_freq, carrier_ppm, flags.
+ *   fcch(d): freq, snr, max_idx (1 x n_fcch), mean_freq, carrier_ppm, flags;
+ *   bcch(d): carrier_ppm, idx (1..8 or -1), corr_abs (8 x 4, abs(corr_val)), flags.
  * Where the reference would not get that far (pos_info == -1, r_correct == -1: flags 1 / 2) the fields are empty and n_sch = -1 is
- * reported as empty arrays; flags 4 / 8: a window leaves r_correct (sch_ok 0 / NaN rows, NaN mean).  See include/gsmcal.h. */
+ * reported as empty arrays; flags 4 / 8: a window leaves r_correct (sch_ok 0 / NaN rows, NaN mean).  bcch(d).flags: 1 pos_info == -1,
+ * 2 fewer than four BCCH rows (carrier_ppm = idx = -1), 4 no FCCH mean (carrier_ppm NaN, idx -1), 8 a training window leaves
+ * r_correct (NaN column, idx -1); corr_abs is NaN where it was not computed.  See include/gsmcal.h. */
 void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
-    init_once(); need(nrhs, 4, "[sampling_ppm,carrier_ppm,n_pos_info,pos_info,sch,fcch] = gsm_calibrate_demod_batch(raw_uint8,carrier_freq,sch_training_sequence,coef)");
+    init_once();
+    if (nrhs < 4 || nrhs > 5 || (nlhs > 6 && nrhs < 5))
+        mexErrMsgIdAndTxt("gsmcal:nargin", "usage: [sampling_ppm,carrier_ppm,n_pos_info,pos_info,sch,fcch,bcch] = "
+                          "gsm_calibrate_demod_batch(raw_uint8,carrier_freq,sch_training_sequence,coef[,normal_training_sequence]) (bcch needs the fifth input)");
     if (!mxIsUint8(prhs[0])) mexErrMsgIdAndTxt("gsmcal:type", "raw must be uint8");
     size_t rows = mxGetM(prhs[0]), D = mxGetN(prhs[0]);
-    int own; const double *tpl = get_c128(prhs[2], &own);
+    int own, own_n = 0; const double *tpl = get_c128(prhs[2], &own), *nts = NULL;
     size_t nt; const double *coef = real_vector(prhs[3], &nt);
+    if (nrhs > 4) {
+        if (mxGetM(prhs[4]) != 26 * 8 || mxGetN(prhs[4]) != 8) mexErrMsgIdAndTxt("gsmcal:size", "normal_training_sequence must be (26*8) x 8");
+        nts = get_c128(prhs[4], &own_n);
+    }
     int64_t n_iq = (int64_t)(rows / 2);
     size_t B = (size_t)gsmcal_max_bursts((n_iq + 63) / 64, 8), R = D * B;
     gsmcal_stream_result *res = (gsmcal_stream_result *)mxMalloc(D * sizeof(*res));
     gsmcal_demod_result *dem = (gsmcal_demod_result *)mxMalloc(D * sizeof(*dem));
+    gsmcal_bcch_result *bc = nts ? (gsmcal_bcch_result *)mxMalloc(D * sizeof(*bc)) : NULL;
     double *pi = (double *)mxMalloc(D * 12 * B * sizeof(double));
     uint8_t *ok = (uint8_t *)mxMalloc(R * (1 + 2 * 148)), *bits = ok + R, *dec = bits + 148 * R;
     double *corr = (double *)mxMalloc(R * 88 * sizeof(double)), *freq = corr + 85 * R, *snr = freq + R, *idx = snr + R;
-    fail_on(gsmcal_calibrate_demod_batch((const uint8_t *)mxGetData(prhs[0]), GSMCAL_MEM_HOST, n_iq, (int64_t)D, mxGetScalar(prhs[1]), tpl, coef, (int)nt, 8, 8,
-                                         res, NULL, NULL, NULL, pi, NULL, dem, ok, bits, dec, corr, freq, snr, idx), "gsm_calibrate_demod_batch");
+    if (nts)
+        fail_on(gsmcal_calibrate_demod_bcch_batch((const uint8_t *)mxGetData(prhs[0]), GSMCAL_MEM_HOST, n_iq, (int64_t)D, mxGetScalar(prhs[1]), tpl, coef, (int)nt,
+                                                  8, 8, res, NULL, NULL, NULL, pi, NULL, dem, ok, bits, dec, corr, freq, snr, idx, nts, bc),
+                "gsm_calibrate_demod_batch");
+    else
+        fail_on(gsmcal_calibrate_demod_batch((const uint8_t *)mxGetData(prhs[0]), GSMCAL_MEM_HOST, n_iq, (int64_t)D, mxGetScalar(prhs[1]), tpl, coef, (int)nt, 8, 8,
+                                             res, NULL, NULL, NULL, pi, NULL, dem, ok, bits, dec, corr, freq, snr, idx), "gsm_calibrate_demod_batch");
     plhs[0] = mxCreateDoubleMatrix(3, D, mxREAL);
     if (nlhs > 1) plhs[1] = mxCreateDoubleMatrix(3, D, mxREAL);
     if (nlhs > 2) plhs[2] = mxCreateDoubleMatrix(1, D, mxREAL);
@@ -366,7 +384,17 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
             mxSetField(plhs[5], d, "carrier_ppm", scalar(dem[d].fcch_carrier_ppm)); mxSetField(plhs[5], d, "flags", scalar(dem[d].flags));
         }
     }
-    mxFree(res); mxFree(dem); mxFree(pi); mxFree(ok); mxFree(corr); if (own) mxFree((void *)tpl);
+    if (nlhs > 6) {
+        const char *f[] = {"carrier_ppm", "idx", "corr_abs", "flags"};
+        plhs[6] = mxCreateStructMatrix(1, D, 4, f);
+        for (size_t d = 0; d < D; ++d) {
+            mxArray *ca = mxCreateDoubleMatrix(8, 4, mxREAL);
+            memcpy(mxGetPr(ca), bc[d].corr_abs, sizeof bc[d].corr_abs);
+            mxSetField(plhs[6], d, "carrier_ppm", scalar(bc[d].carrier_ppm)); mxSetField(plhs[6], d, "idx", scalar(bc[d].nts_idx));
+            mxSetField(plhs[6], d, "corr_abs", ca); mxSetField(plhs[6], d, "flags", scalar(bc[d].flags));
+        }
+    }
+    mxFree(res); mxFree(dem); mxFree(pi); mxFree(ok); mxFree(corr); if (bc) mxFree(bc); if (own) mxFree((void *)tpl); if (own_n) mxFree((void *)nts);
 }
 
 #elif defined(GSMCAL_MEX_gsm_normal_training_sequence_gen)
