@@ -333,11 +333,14 @@ int gsmcal_fcch_scan(const uint8_t *raw, int raw_mem, int64_t n_iq, int64_t n_ch
  * batches in lockstep); 17 = 4 KB ring stages per block of the TMA column-sum kernel of _submit (default 2; 0 = plain launches);
  * 18 = its blocks per SM (default 3); 19, value 1 = SCH correlation kernel capped at 56 registers; 21, value 1 = the burst chains of a
  * batch's stream groups one after the other; 22, value 1 = burst chains on normal-priority streams; 23 = KB of shared memory per block
- * of an extra kernel of sleeping blocks behind the chain (experiment: what the chain's SM slots cost) */
+ * of an extra kernel of sleeping blocks behind the chain (experiment: what the chain's SM slots cost); 24 = the osr-8 SCH correlation:
+ * value 0 = fp32 screen of the 89 lags, fp64 only for the lags that can hold the maximum (default), 1 = fp64 correlation of every lag
+ * (A/B), 2 = run the screen, then the fp64 fallback as if it had failed (tests) */
 int gsmcal_debug_set(int key, int value);
 /* key 1: number of bursts of the last fine FCCH search whose band certificate failed (all-bin fallback ran); 2: bursts that needed the
  * 64-bin band kernel; 10 + p: bursts the osr-8 tier-1 kernel proved after p passes (p = 0: left open); 30: bytes moved through the
- * pinned staging ring so far */
+ * pinned staging ring so far; over the last call that ran the SCH stage: 120 = bursts the osr-8 SCH screen decided, 121 = bursts that ran
+ * the full fp64 SCH correlation (fallback, or debug key 24 != 0), 121 + c (c = 1..8) = decided bursts with c candidate lags */
 int64_t gsmcal_debug_get(int key);
 
 /* kernel-launch counter (all launches since the last reset, this process) - for bench.py's gpu_launches */

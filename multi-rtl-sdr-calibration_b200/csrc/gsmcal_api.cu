@@ -49,6 +49,8 @@ int g_debug_occupy = 0;            // debug key 23: KB of shared memory per bloc
 int g_debug_chain_serial = 0;      // debug key 21: the burst chains of a batch's stream groups run one after the other
 int g_debug_chain_lo = 0;          // debug key 22: ... on normal-priority streams (they only take what the FP64 blocks leave free)
 int g_debug_sch56 = 0;             // debug key 19: sch_corr_kernel capped at 56 registers
+int g_debug_sch_mode = 0;          // debug key 24: sch_corr_kernel at osr 8: 0 = fp32 screen, 1 = always fp64, 2 = screen + forced fallback
+unsigned *g_last_sch_stats = nullptr;   // SCH_NSTAT counters of the last call that ran the SCH stage (debug_get 120..)
 int g_debug_trickle = 2;           // debug key 17: ring stages (x 4 KB) of colsum_u8_trickle_kernel in submit/collect, 0 = off (plain column-sum launches)
 int g_debug_trickle_blocks = 3;    // debug key 18: its blocks per SM (3 x 2 stages: 22 GB in 7 ms under the FP64 stages, profiles/r2q)
 int g_debug_gate = 1;              // debug key 16: submit/collect staggers the batches - the FP64 stages of batch k+1 wait for batch k, its front runs under them
@@ -249,12 +251,32 @@ struct Work {
     StreamCtl *ctl; StreamResultDev *res;
     double *coarse_pos, *coarse_snr, *fine_raw, *fcch_pos, *fo, *gate, *sch_raw, *sch_pos, *post_pos, *pos_info, *snr_map, *power;
     int *sch_edge, *need_full, *need_band, *tone_need, *fall_list, *fall_count, *fall_m; double *fall_best; unsigned char *kind; double2 *tpl;
+    const float2 *tplf; const double *tpl_e;   // behind tpl: the screen's padded fp32 template and the template energy (tpl_pack)
+    unsigned *sch_stats;          // [SCH_NSTAT] sch_corr_kernel counters
     i64 snr_stride;
     unsigned *pass_hist;          // [16] fine_core8_kernel: bursts proven after p passes ([0] = left to the band kernel)
     double2 *wcache;              // [D][cap][B8_WLEN] or nullptr (set by attach_wcache)
     bool wc_valid;                // the fine search of this call filled the cache
 };
 size_t align_up(size_t x) { return (x + 255) & ~(size_t)255; }
+// the SCH template as the device reads it: fp64 [L] | fp32 with one pad slot per 16 samples [sch_tplf_len(L)], 16-byte aligned for the
+// TMA copy | the fp64 energy sum |t|^2, rounded up (the screen's bound needs an upper bound)
+size_t tplf_off(int L) { return sizeof(double2) * (size_t)L; }
+size_t tpl_e_off(int L) { return tplf_off(L) + ((sizeof(float2) * (size_t)sch_tplf_len(L) + 15) & ~(size_t)15); }
+size_t tpl_pack_bytes(int L) { return tpl_e_off(L) + 16; }
+void tpl_pack(const double *tpl, int L, unsigned char *dst) {
+    memset(dst, 0, tpl_pack_bytes(L));
+    memcpy(dst, tpl, sizeof(double2) * (size_t)L);
+    float2 *f = reinterpret_cast<float2 *>(dst + tplf_off(L));
+    double e = 0.0;
+    for (int i = 0; i < L; ++i) {
+        const double x = tpl[2 * i], y = tpl[2 * i + 1];
+        f[i + (i >> 4)] = make_float2((float)x, (float)y);
+        e += x * x + y * y;
+    }
+    e *= 1.0 + 1e-12;                                    // L <= 512: the sum's relative error is below 1e-13
+    memcpy(dst + tpl_e_off(L), &e, sizeof e);
+}
 constexpr int kMaxGroups = 32;     // stream groups per batch (tier-3 scratch is per group); ceil(148*8/64) = 19 <= 24 bands
 
 int make_work(DevBuf &wb, i64 D, int cap, i64 snr_len, int tpl_len, Work *w) {
@@ -264,7 +286,7 @@ int make_work(DevBuf &wb, i64 D, int cap, i64 snr_len, int tpl_len, Work *w) {
     size_t per = sizeof(double) * D * cap;
     size_t o_cp = take(per), o_cs = take(per), o_fr = take(per), o_fp = take(per), o_fo = take(per), o_g = take(per), o_sr = take(per), o_sp = take(per), o_pp = take(per);
     size_t o_pi = take(per * 12), o_snr = take(sizeof(double) * D * snr_len), o_pw = take(sizeof(double) * D);
-    size_t o_se = take(sizeof(int) * D * cap), o_nf = take(sizeof(int) * D * cap), o_nb = take(sizeof(int) * D * cap), o_tn = take(sizeof(int) * D * cap), o_fl = take(sizeof(int) * D * cap), o_fc = take(sizeof(int) * D), o_fm = take(sizeof(int) * (size_t)FALL_GRID * 24 * kMaxGroups), o_fb = take(sizeof(double) * (size_t)FALL_GRID * 24 * kMaxGroups), o_k = take(D * cap), o_tpl = take(sizeof(double2) * (tpl_len > 0 ? tpl_len : 1)), o_ph = take(sizeof(unsigned) * 16 + sizeof(unsigned long long) * 64);
+    size_t o_se = take(sizeof(int) * D * cap), o_nf = take(sizeof(int) * D * cap), o_nb = take(sizeof(int) * D * cap), o_tn = take(sizeof(int) * D * cap), o_fl = take(sizeof(int) * D * cap), o_fc = take(sizeof(int) * D), o_fm = take(sizeof(int) * (size_t)FALL_GRID * 24 * kMaxGroups), o_fb = take(sizeof(double) * (size_t)FALL_GRID * 24 * kMaxGroups), o_k = take(D * cap), o_tpl = take(tpl_pack_bytes(tpl_len > 0 ? tpl_len : 1)), o_ph = take(sizeof(unsigned) * 16 + sizeof(unsigned long long) * 64), o_ss = take(sizeof(unsigned) * SCH_NSTAT);
     void *base;
     TRY(wb.get(off, &base));
     char *b = static_cast<char *>(base);
@@ -273,6 +295,7 @@ int make_work(DevBuf &wb, i64 D, int cap, i64 snr_len, int tpl_len, Work *w) {
     w->fo = (double *)(b + o_fo); w->gate = (double *)(b + o_g); w->sch_raw = (double *)(b + o_sr); w->sch_pos = (double *)(b + o_sp); w->post_pos = (double *)(b + o_pp);
     w->pos_info = (double *)(b + o_pi); w->snr_map = (double *)(b + o_snr); w->power = (double *)(b + o_pw);
     w->sch_edge = (int *)(b + o_se); w->need_full = (int *)(b + o_nf); w->need_band = (int *)(b + o_nb); w->tone_need = (int *)(b + o_tn); w->fall_list = (int *)(b + o_fl); w->fall_count = (int *)(b + o_fc); w->fall_m = (int *)(b + o_fm); w->fall_best = (double *)(b + o_fb); w->kind = (unsigned char *)(b + o_k); w->tpl = (double2 *)(b + o_tpl);
+    w->tplf = (const float2 *)(b + o_tpl + tplf_off(tpl_len)); w->tpl_e = (const double *)(b + o_tpl + tpl_e_off(tpl_len)); w->sch_stats = (unsigned *)(b + o_ss);
     w->snr_stride = snr_len;
     w->pass_hist = (unsigned *)(b + o_ph);
     w->wcache = nullptr; w->wc_valid = false;
@@ -437,8 +460,10 @@ int run_fine(Ctx &c, WinSrc src_peak, WinSrc src_tone, i64 n_iq, int osr, double
 }
 
 int run_sch(WinSrc src, int osr, i64 D, int cap, Work &w, cudaStream_t st) {
-    if (g_debug_sch56) LAUNCH(sch_corr_kernel<56>, dim3((unsigned)cap, (unsigned)D), SCH_THREADS, sch_smem(osr), st, src, w.ctl, w.fcch_pos, cap, osr, w.tpl, w.sch_raw, w.sch_edge);
-    else               LAUNCH(sch_corr_kernel<64>, dim3((unsigned)cap, (unsigned)D), SCH_THREADS, sch_smem(osr), st, src, w.ctl, w.fcch_pos, cap, osr, w.tpl, w.sch_raw, w.sch_edge);
+#define SCH_ARGS src, w.ctl, w.fcch_pos, cap, osr, w.tpl, w.tplf, w.tpl_e, g_debug_sch_mode, w.sch_stats, w.sch_raw, w.sch_edge
+    if (g_debug_sch56) LAUNCH(sch_corr_kernel<56>, dim3((unsigned)cap, (unsigned)D), SCH_THREADS, sch_smem(osr), st, SCH_ARGS);
+    else               LAUNCH(sch_corr_kernel<64>, dim3((unsigned)cap, (unsigned)D), SCH_THREADS, sch_smem(osr), st, SCH_ARGS);
+#undef SCH_ARGS
     LAUNCH(sch_ppm_kernel, (unsigned)D, PS_THREADS, (size_t)cap * 21 + 16, st, w.ctl, (int)D, cap, osr, w.sch_raw, w.sch_edge, w.sch_pos, w.kind, w.pos_info, w.post_pos);
     return GSMCAL_OK;
 }
@@ -590,7 +615,7 @@ int gsmcal_set_device(int device) {
 }
 void gsmcal_release(void) {
     std::lock_guard<std::mutex> lk(g_mu);
-    g_last_need_full = nullptr; g_last_need_band = nullptr; g_last_need_full_n = 0; g_last_pass_hist = nullptr; g_prev_pass_hist = nullptr;   // they point into the workspaces freed below
+    g_last_need_full = nullptr; g_last_need_band = nullptr; g_last_need_full_n = 0; g_last_pass_hist = nullptr; g_prev_pass_hist = nullptr; g_last_sch_stats = nullptr;   // they point into the workspaces freed below
     for (auto &kv : g_ctx) {
         cudaSetDevice(kv.first);
         kv.second.ring.release(); kv.second.in.release(); kv.second.out.release(); kv.second.work.release(); kv.second.tplbuf.release(); kv.second.wc.release(); kv.second.dem.release();
@@ -633,6 +658,13 @@ int64_t gsmcal_debug_get(int key) {
         if (cudaMemcpy(&v, (unsigned long long *)(g_last_pass_hist + 16) + (key - 50), sizeof v, cudaMemcpyDeviceToHost) != cudaSuccess) return -1;
         return (int64_t)v;
     }
+    if (key >= 120 && key < 121 + SCH_NSTAT) {                  // sch_corr_kernel counters of the last call (SCH_NSTAT)
+        if (!g_last_sch_stats) return 0;
+        unsigned h[SCH_NSTAT];
+        if (cudaMemcpy(h, g_last_sch_stats, sizeof h, cudaMemcpyDeviceToHost) != cudaSuccess) return -1;
+        if (key == 120) { int64_t n = 0; for (int k = 1; k < SCH_NSTAT; ++k) n += h[k]; return n; }
+        return (int64_t)h[key - 121];
+    }
     if (key == 30) return (int64_t)g_staged_bytes.load();           // bytes that went through the pinned staging ring (pageable host buffers)
     if (key >= 10 && key < 26) {                                 // 10 + p: bursts the osr-8 tier-1 kernel proved after p passes (p = 0: left open)
         if (!g_last_pass_hist) return 0;
@@ -666,6 +698,7 @@ int gsmcal_debug_set(int key, int value) {
     if (key == 21) { g_debug_chain_serial = value != 0; return GSMCAL_OK; }
     if (key == 22) { g_debug_chain_lo = value != 0; return GSMCAL_OK; }
     if (key == 19) { g_debug_sch56 = value != 0; return GSMCAL_OK; }
+    if (key == 24) { if (value < 0 || value > 2) return fail(GSMCAL_ERR_ARG, "debug_set 24: 0, 1 or 2"); g_debug_sch_mode = value; return GSMCAL_OK; }
     if (key == 17) { g_debug_trickle = value < 0 ? 0 : (value > 24 ? 24 : value); return GSMCAL_OK; }
     if (key == 18) { g_debug_trickle_blocks = value < 1 ? 1 : (value > 4 ? 4 : value); return GSMCAL_OK; }
     if (key == 15) { g_debug_persist_threads = (value == 64 || value == 128) ? value : 256; return GSMCAL_OK; }
@@ -999,7 +1032,11 @@ int gsmcal_SCH_corr_rate_correction(const double *s, int64_t n, const double *FC
     TRY(c->in.get(sizeof(double2) * (size_t)n, &din));
     TRY(make_work(c->work, 1, cap, 1, L, &w));
     TRY(copy_h2d(c->ring, g_device, din, s, sizeof(double2) * (size_t)n, st));
-    CU(cudaMemcpyAsync(w.tpl, tpl, sizeof(double2) * L, cudaMemcpyHostToDevice, st));
+    std::vector<unsigned char> tpk(tpl_pack_bytes(L));
+    tpl_pack(tpl, L, tpk.data());
+    CU(cudaMemcpyAsync((void *)w.tpl, tpk.data(), tpk.size(), cudaMemcpyHostToDevice, st));
+    g_last_sch_stats = w.sch_stats;
+    CU(cudaMemsetAsync(w.sch_stats, 0, sizeof(unsigned) * SCH_NSTAT, st));
     CU(cudaMemcpyAsync(w.fcch_pos, FCCH_pos, sizeof(double) * cap, cudaMemcpyHostToDevice, st));
     StreamCtl h; memset(&h, 0, sizeof h); h.n_fcch = cap; h.sch_enable = 1; h.len1 = n;
     CU(cudaMemcpyAsync(w.ctl, &h, sizeof h, cudaMemcpyHostToDevice, st));
@@ -1108,7 +1145,11 @@ static int calibrate_batch_impl(const uint8_t *raw, int raw_mem, int64_t n_iq, i
     CU(cudaMemsetAsync(w.ctl, 0, sizeof(StreamCtl) * D, st));
     CU(cudaMemsetAsync(w.need_full, 0, sizeof(int) * D * cap, st));
     CU(cudaMemsetAsync(w.need_band, 0, sizeof(int) * D * cap, st));
-    CU(cudaMemcpyAsync(w.tpl, tpl, sizeof(double2) * 64 * osr, cudaMemcpyHostToDevice, st));
+    std::vector<unsigned char> tpk(tpl_pack_bytes(64 * osr));
+    tpl_pack(tpl, 64 * osr, tpk.data());
+    CU(cudaMemcpyAsync((void *)w.tpl, tpk.data(), tpk.size(), cudaMemcpyHostToDevice, st));      // pageable: staged before the call returns
+    g_last_sch_stats = w.sch_stats;
+    CU(cudaMemsetAsync(w.sch_stats, 0, sizeof(unsigned) * SCH_NSTAT, st));
     { const double2 *twp; TRY(get_twiddle(*c, 148 * osr, st, &twp)); }        // built on `st` before the groups fork
     g_last_need_full = w.need_full; g_last_need_band = w.need_band; g_last_need_full_n = (long long)D * cap;
     g_last_pass_hist = w.pass_hist;
@@ -1309,7 +1350,7 @@ int gsmcal_calibrate_batch_submit(int slot, const uint8_t *raw_dev, int64_t n_iq
     TRY(set_taps(coef, n_taps, st));
     // pinned staging: records | coarse_pos | coarse_snr | fcch_pos | pos_info (x12)
     sl.n_res = sizeof(StreamResultDev) * (size_t)D; sl.n_per = sizeof(double) * (size_t)D * cap;
-    const size_t need = align_up(sl.n_res) + 15 * sl.n_per + 64 * osr * sizeof(double2);
+    const size_t need = align_up(sl.n_res) + 15 * sl.n_per + tpl_pack_bytes(64 * osr);
     if (need > sl.stage_cap) {
         if (sl.stage) cudaFreeHost(sl.stage);
         sl.stage = nullptr; sl.stage_cap = 0;
@@ -1317,7 +1358,7 @@ int gsmcal_calibrate_batch_submit(int slot, const uint8_t *raw_dev, int64_t n_iq
         sl.stage_cap = need;
     }
     char *h_res = sl.stage, *h_arr = sl.stage + align_up(sl.n_res), *h_tpl = h_arr + 15 * sl.n_per;
-    memcpy(h_tpl, tpl, sizeof(double2) * 64 * osr);              // the caller's template may be pageable and short-lived
+    tpl_pack(tpl, 64 * osr, (unsigned char *)h_tpl);           // the caller's template may be pageable and short-lived
     { const double2 *twp; TRY(get_twiddle(*c, 148 * osr, st, &twp)); }
     // normal-priority kernels of different streams are dispatched in arrival order: behind the 10^5 queued blocks of the previous batch's fine
     // search even a memset waits milliseconds (device timeline, debug key 14), so the staggered mode runs the whole front at high priority
@@ -1327,7 +1368,9 @@ int gsmcal_calibrate_batch_submit(int slot, const uint8_t *raw_dev, int64_t n_iq
     CU(cudaMemsetAsync(w.ctl, 0, sizeof(StreamCtl) * D, fr));
     CU(cudaMemsetAsync(w.need_full, 0, sizeof(int) * D * cap, fr));
     CU(cudaMemsetAsync(w.need_band, 0, sizeof(int) * D * cap, fr));
-    CU(cudaMemcpyAsync(w.tpl, h_tpl, sizeof(double2) * 64 * osr, cudaMemcpyHostToDevice, fr));
+    CU(cudaMemcpyAsync(w.tpl, h_tpl, tpl_pack_bytes(64 * osr), cudaMemcpyHostToDevice, fr));
+    g_last_sch_stats = w.sch_stats;
+    CU(cudaMemsetAsync(w.sch_stats, 0, sizeof(unsigned) * SCH_NSTAT, fr));
     g_last_need_full = w.need_full; g_last_need_band = w.need_band; g_last_need_full_n = (long long)D * cap;
     g_prev_pass_hist = g_last_pass_hist; g_last_pass_hist = w.pass_hist;
     CU(cudaMemsetAsync(w.pass_hist, 0, sizeof(unsigned) * 16 + sizeof(unsigned long long) * 64, fr));

@@ -2059,16 +2059,108 @@ __global__ void __launch_bounds__(TONE_THREADS, 3) tone_est_kernel(WinSrc src, c
 // K9  SCH training-sequence correlation   SCH_corr_rate_correction.m:37-63
 // ===================================================================================================
 #define SCH_THREADS 256
-#define SCH_LPG 6       // lags per warp and pass
+#define SCH_LPG 6       // lags per warp and pass of the fp64 correlation
 #define SCH_PASSES 2
 #define SCH_NSL 16      // template samples per lane
+#define SCH_SLPW 12     // lags per warp of the fp32 screen: one pass, 8 x 12 = 96 >= 89
+#define SCH_MAXC 8      // candidate lags the screen may leave (one warp each); more -> the full fp64 correlation
+#define SCH_NSTAT 9     // counters: [0] bursts that ran the full fp64 correlation, [c] bursts the screen decided with c candidates
+// screen bound eps = SCH_EPS_K * 2^-24 * sqrt(E_win * E_tpl) + SCH_EPS_ABS * (1 + sqrt(L * E_tpl) + sqrt(L * E_win)), valid while both
+// energies are <= SCH_E_MAX (no fp32 overflow); derivation in DESIGN.md section 4
+#define SCH_EPS_K   64.0
+#define SCH_EPS_ABS 7.888609052210118e-31       // 2^-100
+#define SCH_E_MAX   1.329227995784916e36        // 2^120
+__host__ __device__ constexpr int sch_tplf_len(int L) { return L + (L >> 4); }   // float2 entries of the padded fp32 template
+
+// fp64 register-tiled correlation of all n_lag lags into corr / corr_i: per pass warp w owns lags [6(8p+w), +6), lane owns template
+// samples [16*lane, 16*lane+16); a 6-deep sliding register window of the burst is advanced one sample per step (2 shared loads per 6
+// complex MACs).  wp / tp hold window and template with one pad slot per 16 samples so the 256-byte lane stride is conflict free.  Two
+// passes of 6 lags (instead of one of 12) keep the kernel at 64 registers, and the lane partials are folded to 8 lanes by shuffles
+// before they go through shared memory (7 KB instead of 50 KB): 4 blocks per SM instead of 2.  Not inlined: next to the screen, the
+// 56-register build spilled inside this loop.
+__device__ __noinline__ void sch_corr_tiled_fp64(const double2 *wp, const double2 *tp, double *part, double *corr, double *corr_i,
+                                                    int n_lag, int n_smp) {
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = SCH_THREADS >> 5;
+    const int nb = SCH_NSL * lane;
+#pragma unroll 1
+    for (int pass = 0; pass < SCH_PASSES; ++pass) {
+        double ar[SCH_LPG], ai[SCH_LPG];
+        double2 wr_[SCH_LPG];
+#pragma unroll
+        for (int l = 0; l < SCH_LPG; ++l) { ar[l] = 0.0; ai[l] = 0.0; }
+        const int l0 = SCH_LPG * (pass * nw + w);
+#pragma unroll
+        for (int l = 0; l < SCH_LPG - 1; ++l) { const int i = l0 + nb + l; wr_[l] = (i < n_smp) ? wp[i + (i >> 4)] : make_double2(0.0, 0.0); }
+#pragma unroll
+        for (int n = 0; n < SCH_NSL; ++n) {
+            const int iw = l0 + nb + n + SCH_LPG - 1, it = nb + n;
+            wr_[SCH_LPG - 1] = (iw < n_smp) ? wp[iw + (iw >> 4)] : make_double2(0.0, 0.0);
+            const double2 tt = tp[it + (it >> 4)];
+#pragma unroll
+            for (int l = 0; l < SCH_LPG; ++l) {              // conj(ts) .* window
+                ar[l] = fma(wr_[l].x, tt.x, fma(wr_[l].y, tt.y, ar[l]));
+                ai[l] = fma(wr_[l].y, tt.x, fma(-wr_[l].x, tt.y, ai[l]));
+            }
+#pragma unroll
+            for (int l = 0; l < SCH_LPG - 1; ++l) wr_[l] = wr_[l + 1];
+        }
+        // fold 32 lanes to 8 (lanes 0..7 hold the sums of lanes {i, i+8, i+16, i+24}), then rows (lag, re|im) of 9 doubles
+#pragma unroll
+        for (int l = 0; l < SCH_LPG; ++l) {
+            ar[l] += __shfl_down_sync(0xffffffffu, ar[l], 16); ai[l] += __shfl_down_sync(0xffffffffu, ai[l], 16);
+            ar[l] += __shfl_down_sync(0xffffffffu, ar[l], 8);  ai[l] += __shfl_down_sync(0xffffffffu, ai[l], 8);
+        }
+        if (pass > 0) __syncthreads();                       // the rows of the previous pass have been consumed
+        if (lane < 8) {
+#pragma unroll
+            for (int l = 0; l < SCH_LPG; ++l) {
+                part[(2 * (SCH_LPG * w + l)) * 9 + lane] = ar[l];
+                part[(2 * (SCH_LPG * w + l) + 1) * 9 + lane] = ai[l];
+            }
+        }
+        __syncthreads();
+        if (threadIdx.x < 2 * nw * SCH_LPG) {
+            const double *row = part + threadIdx.x * 9;
+            const double s0 = (row[0] + row[1]) + (row[2] + row[3]), s1 = (row[4] + row[5]) + (row[6] + row[7]);
+            const int lag = SCH_LPG * pass * nw + (threadIdx.x >> 1);
+            if (lag < n_lag) { if (threadIdx.x & 1) corr_i[lag] = s0 + s1; else corr[lag] = s0 + s1; }
+        }
+    }
+}
+
+// |corr|^2 of ONE lag, evaluated by one warp in sch_corr_tiled_fp64's exact operation order (the same lane chains, the fold by 16 and 8,
+// the same row sums, then abs2_ref): the value is bit-identical to the tiled correlation's.  The template comes from global memory (8 KB,
+// L2/L1 resident); lane j reads 16 consecutive samples of it.
+__device__ __forceinline__ double sch_lag_fp64(const double2 *wp, const double2 *__restrict__ tpl, int lag, int lane) {
+    const int nb = SCH_NSL * lane;
+    double ar = 0.0, ai = 0.0;
+#pragma unroll
+    for (int n = 0; n < SCH_NSL; ++n) {
+        const int iw = lag + nb + n;
+        const double2 x = wp[iw + (iw >> 4)], tt = __ldg(tpl + nb + n);
+        ar = fma(x.x, tt.x, fma(x.y, tt.y, ar));
+        ai = fma(x.y, tt.x, fma(-x.x, tt.y, ai));
+    }
+    ar += __shfl_down_sync(0xffffffffu, ar, 16); ai += __shfl_down_sync(0xffffffffu, ai, 16);
+    ar += __shfl_down_sync(0xffffffffu, ar, 8);  ai += __shfl_down_sync(0xffffffffu, ai, 8);
+    // the row sum ((r0 + r1) + (r2 + r3)) + ((r4 + r5) + (r6 + r7)) by three more halvings: lane 0 ends with the same value
+#pragma unroll
+    for (int k = 1; k < 8; k <<= 1) { ar += __shfl_down_sync(0xffffffffu, ar, k); ai += __shfl_down_sync(0xffffffffu, ai, k); }
+    return abs2_ref(make_double2(ar, ai));                   // (lane 0's)
+}
+
+// tplf: the template in fp32, padded like tp (sch_tplf_len(L) entries); tpl_e: its energy in fp64, rounded up.  mode: 0 = fp32 screen,
+// 1 = always the fp64 correlation, 2 = screen, then take the fallback as if it had failed.  stats: SCH_NSTAT counters (see SCH_NSTAT).
 template <int MAXR>     // 64: four blocks fill the register file; 56 (a few spilled values) leaves room for the trickle column sums of the next batch
 __global__ void __maxnreg__(MAXR) sch_corr_kernel(WinSrc src, const StreamCtl *__restrict__ ctl, const double *__restrict__ fcch_pos, int cap,
-                                                              int osr, const double2 *__restrict__ tpl, double *__restrict__ sch_raw, int *__restrict__ sch_edge) {
+                                                              int osr, const double2 *__restrict__ tpl, const float2 *__restrict__ tplf,
+                                                              const double *__restrict__ tpl_e, int mode, unsigned *__restrict__ stats,
+                                                              double *__restrict__ sch_raw, int *__restrict__ sch_edge) {
     extern __shared__ double2 sm[];
     __shared__ double red_v[8];
     __shared__ int red_i[8];
     __shared__ double corr[160], corr_i[160];
+    __shared__ unsigned cmask[3];
     const int burst = blockIdx.x, stream = blockIdx.y;
     const StreamCtl c = ctl[stream];
     if (!c.sch_enable || burst >= c.n_fcch) return;
@@ -2086,12 +2178,19 @@ __global__ void __maxnreg__(MAXR) sch_corr_kernel(WinSrc src, const StreamCtl *_
     const i64 sp = training_sp - max_offset;
     const int n_lag = 2 * max_offset - 5 * osr + 1;            // 89 at osr 8
     const int n_smp = n_lag + L - 1;
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = SCH_THREADS >> 5;
+    // the tiled paths are written for osr 8: L = 32 * SCH_NSL and n_lag = 89 <= SCH_PASSES * nw * SCH_LPG = nw * SCH_SLPW
+    const bool tiled = (osr == 8);
+    const bool screen = tiled && mode != 1;
     double2 *win = sm, *t = win + n_smp, *X = t + L, *Y = X + GSMCAL_XCAP(n_smp);
-    // the 64*osr-sample template (8 KB at osr 8) is staged by ONE TMA bulk copy (cp.async.bulk -> UBLKCP) that completes on an
-    // mbarrier while all threads evaluate the burst window; it is consumed only after the wait below
+    // the template (the fp64 one, 8 KB at osr 8, or the padded fp32 one of the screen, 4.25 KB) is staged by ONE TMA bulk copy
+    // (cp.async.bulk -> UBLKCP) that completes on an mbarrier while all threads evaluate the burst window; it is consumed only after the
+    // wait below
     __shared__ __align__(8) unsigned long long tpl_bar;
     const unsigned bar_a = (unsigned)__cvta_generic_to_shared(&tpl_bar);
-    const bool tma_ok = (((uintptr_t)tpl & 15) == 0) && (((uintptr_t)t & 15) == 0);
+    const void *tsrc = screen ? (const void *)tplf : (const void *)tpl;
+    const unsigned tbytes = screen ? (unsigned)(sch_tplf_len(L) * sizeof(float2)) : (unsigned)(L * sizeof(double2));
+    const bool tma_ok = (((uintptr_t)tsrc & 15) == 0) && (((uintptr_t)t & 15) == 0) && ((tbytes & 15) == 0);
     if (tma_ok) {
         if (threadIdx.x == 0) {
             asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar_a));
@@ -2099,11 +2198,12 @@ __global__ void __maxnreg__(MAXR) sch_corr_kernel(WinSrc src, const StreamCtl *_
         }
         __syncthreads();
         if (threadIdx.x == 0) {
-            const unsigned bytes = (unsigned)(L * sizeof(double2));
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_a), "r"(bytes));
+            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_a), "r"(tbytes));
             asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                         ::"r"((unsigned)__cvta_generic_to_shared(t)), "l"(tpl), "r"(bytes), "r"(bar_a) : "memory");
+                         ::"r"((unsigned)__cvta_generic_to_shared(t)), "l"(tsrc), "r"(tbytes), "r"(bar_a) : "memory");
         }
+    } else if (screen) {
+        for (int i = threadIdx.x; i < sch_tplf_len(L); i += SCH_THREADS) reinterpret_cast<float2 *>(t)[i] = tplf[i];
     } else {
         for (int i = threadIdx.x; i < L; i += SCH_THREADS) t[i] = tpl[i];
     }
@@ -2115,63 +2215,133 @@ __global__ void __maxnreg__(MAXR) sch_corr_kernel(WinSrc src, const StreamCtl *_
                          : "=r"(done) : "r"(bar_a), "r"(0u) : "memory");
         }
     }
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = SCH_THREADS >> 5;
-    if (L == 32 * SCH_NSL && n_lag <= SCH_PASSES * nw * SCH_LPG) {
-        // register-tiled correlation: per pass warp w owns lags [6(8p+w), +6), lane owns template samples [16*lane, 16*lane+16);
-        // a 6-deep sliding register window of the burst is advanced one sample per step (2 shared loads per 6 complex MACs).
-        // Both arrays are re-laid out with one pad slot per 16 samples so the 256-byte lane stride is conflict free.  Two passes
-        // of 6 lags (instead of one of 12) keep the kernel at 64 registers, and the lane partials are folded to 8 lanes by shuffles
-        // before they go through shared memory (7 KB instead of 50 KB): 4 blocks per SM instead of 2.
+    if (tiled) {
         double2 *wp = X, *tp = X + (n_smp + (n_smp >> 4) + 2);      // X and Y are contiguous: 924 + 608 slots >= 640 + 544
-        for (int i = threadIdx.x; i < n_smp; i += SCH_THREADS) wp[i + (i >> 4)] = win[i];
-        for (int i = threadIdx.x; i < L; i += SCH_THREADS) tp[i + (i >> 4)] = t[i];
-        __syncthreads();
         double *part = reinterpret_cast<double *>(tp + (L + (L >> 4) + 2));      // [2 * nw * SCH_LPG][9]
-        const int nb = SCH_NSL * lane;
+        if (screen) {
+            // fp32 screen.  Only the index of the first maximum of |corr|^2 leaves the kernel, so every lag is correlated in fp32 and
+            // the bound eps >= |screened corr - fp64 corr| (DESIGN.md section 4) rules out the lags that cannot hold the maximum; the
+            // few that can are evaluated in fp64 exactly as the tiled correlation does, so the index is the one it would give.
+            float2 *wf = reinterpret_cast<float2 *>(tp);            // the fp64 template is not staged: its slots hold the fp32 window
+            float *part_f = reinterpret_cast<float *>(wf + (n_smp + (n_smp >> 4) + 2));  // [2 * nw * SCH_SLPW][9]
+            const float2 *tf = reinterpret_cast<const float2 *>(t);
+            double e = 0.0;
+            for (int i = threadIdx.x; i < n_smp; i += SCH_THREADS) {
+                const double2 v = win[i];
+                wp[i + (i >> 4)] = v;
+                wf[i + (i >> 4)] = make_float2((float)v.x, (float)v.y);
+                e = fma(v.x, v.x, fma(v.y, v.y, e));
+            }
+            const double e_win = block_sum(e, red_v) * (1.0 + 1e-12);   // its barriers also publish wp / wf; rounded up
+            const double e_tpl = *tpl_e;
+            const bool bounded = e_win <= SCH_E_MAX && e_tpl <= SCH_E_MAX;         // false for inf / NaN too
+            const double eps = SCH_EPS_K * 5.9604644775390625e-8 * sqrt(e_win * e_tpl) * (1.0 + 1e-12)
+                             + SCH_EPS_ABS * (1.0 + sqrt((double)L * e_tpl) + sqrt((double)L * e_win));
+            if (bounded) {
+                // per pass warp w owns lags [SLPW(8p+w), +SLPW), lane owns template samples [16*lane, +16); an SLPW-deep sliding register
+                // window of the burst advances one sample per step: 2 LDS.64 (2 wavefronts each, conflict free with the pad) per 4*SLPW
+                // FFMA.  One pass of 12 at 64 registers; the 56-register build takes two passes of 6 (12 would spill)
+                constexpr int SLPW = (MAXR >= 64) ? SCH_SLPW : SCH_SLPW / 2;
+                const int nb = SCH_NSL * lane;
 #pragma unroll 1
-        for (int pass = 0; pass < SCH_PASSES; ++pass) {
-            double ar[SCH_LPG], ai[SCH_LPG];
-            double2 wr_[SCH_LPG];
+                for (int pass = 0; pass < SCH_SLPW / SLPW; ++pass) {
+                    const int l0 = SLPW * (pass * nw + w);
+                    float ar[SLPW], ai[SLPW];
+                    float2 wr_[SLPW];
 #pragma unroll
-            for (int l = 0; l < SCH_LPG; ++l) { ar[l] = 0.0; ai[l] = 0.0; }
-            const int l0 = SCH_LPG * (pass * nw + w);
+                    for (int l = 0; l < SLPW; ++l) { ar[l] = 0.0f; ai[l] = 0.0f; }
 #pragma unroll
-            for (int l = 0; l < SCH_LPG - 1; ++l) { const int i = l0 + nb + l; wr_[l] = (i < n_smp) ? wp[i + (i >> 4)] : make_double2(0.0, 0.0); }
+                    for (int l = 0; l < SLPW - 1; ++l) { const int i = l0 + nb + l; wr_[l] = (i < n_smp) ? wf[i + (i >> 4)] : make_float2(0.0f, 0.0f); }
 #pragma unroll
-            for (int n = 0; n < SCH_NSL; ++n) {
-                const int iw = l0 + nb + n + SCH_LPG - 1, it = nb + n;
-                wr_[SCH_LPG - 1] = (iw < n_smp) ? wp[iw + (iw >> 4)] : make_double2(0.0, 0.0);
-                const double2 tt = tp[it + (it >> 4)];
+                    for (int n = 0; n < SCH_NSL; ++n) {
+                        const int iw = l0 + nb + n + SLPW - 1, it = nb + n;
+                        wr_[SLPW - 1] = (iw < n_smp) ? wf[iw + (iw >> 4)] : make_float2(0.0f, 0.0f);
+                        const float2 tt = tf[it + (it >> 4)];
 #pragma unroll
-                for (int l = 0; l < SCH_LPG; ++l) {              // conj(ts) .* window
-                    ar[l] = fma(wr_[l].x, tt.x, fma(wr_[l].y, tt.y, ar[l]));
-                    ai[l] = fma(wr_[l].y, tt.x, fma(-wr_[l].x, tt.y, ai[l]));
-                }
+                        for (int l = 0; l < SLPW; ++l) {
+                            ar[l] = fmaf(wr_[l].x, tt.x, fmaf(wr_[l].y, tt.y, ar[l]));
+                            ai[l] = fmaf(wr_[l].y, tt.x, fmaf(-wr_[l].x, tt.y, ai[l]));
+                        }
 #pragma unroll
-                for (int l = 0; l < SCH_LPG - 1; ++l) wr_[l] = wr_[l + 1];
-            }
-            // fold 32 lanes to 8 (lanes 0..7 hold the sums of lanes {i, i+8, i+16, i+24}), then rows (lag, re|im) of 9 doubles
+                        for (int l = 0; l < SLPW - 1; ++l) wr_[l] = wr_[l + 1];
+                    }
 #pragma unroll
-            for (int l = 0; l < SCH_LPG; ++l) {
-                ar[l] += __shfl_down_sync(0xffffffffu, ar[l], 16); ai[l] += __shfl_down_sync(0xffffffffu, ai[l], 16);
-                ar[l] += __shfl_down_sync(0xffffffffu, ar[l], 8);  ai[l] += __shfl_down_sync(0xffffffffu, ai[l], 8);
-            }
-            if (pass > 0) __syncthreads();                       // the rows of the previous pass have been consumed
-            if (lane < 8) {
+                    for (int l = 0; l < SLPW; ++l) {
+                        ar[l] += __shfl_down_sync(0xffffffffu, ar[l], 16); ai[l] += __shfl_down_sync(0xffffffffu, ai[l], 16);
+                        ar[l] += __shfl_down_sync(0xffffffffu, ar[l], 8);  ai[l] += __shfl_down_sync(0xffffffffu, ai[l], 8);
+                    }
+                    if (lane < 8) {                                 // rows (lag, re|im) of 9 floats, every lag of the burst
 #pragma unroll
-                for (int l = 0; l < SCH_LPG; ++l) {
-                    part[(2 * (SCH_LPG * w + l)) * 9 + lane] = ar[l];
-                    part[(2 * (SCH_LPG * w + l) + 1) * 9 + lane] = ai[l];
+                        for (int l = 0; l < SLPW; ++l) {
+                            part_f[(2 * (l0 + l)) * 9 + lane] = ar[l];
+                            part_f[(2 * (l0 + l) + 1) * 9 + lane] = ai[l];
+                        }
+                    }
                 }
             }
             __syncthreads();
-            if (threadIdx.x < 2 * nw * SCH_LPG) {
-                const double *row = part + threadIdx.x * 9;
-                const double s0 = (row[0] + row[1]) + (row[2] + row[3]), s1 = (row[4] + row[5]) + (row[6] + row[7]);
-                const int lag = SCH_LPG * pass * nw + (threadIdx.x >> 1);
-                if (lag < n_lag) { if (threadIdx.x & 1) corr_i[lag] = s0 + s1; else corr[lag] = s0 + s1; }
+            if (bounded && threadIdx.x < 2 * nw * SCH_SLPW) {
+                const float *row = part_f + threadIdx.x * 9;
+                const float s0 = (row[0] + row[1]) + (row[2] + row[3]), s1 = (row[4] + row[5]) + (row[6] + row[7]);
+                const int lag = threadIdx.x >> 1;
+                if (lag < n_lag) { if (threadIdx.x & 1) corr_i[lag] = (double)(s0 + s1); else corr[lag] = (double)(s0 + s1); }
             }
+            __syncthreads();
+            // candidates: M = max (|c^| - eps); a lag whose |c^| + eps stays below M (with the certificates' relative margin) is below
+            // the lag that attains M, whatever the exact values are
+            double a = 0.0, lo = -INFINITY;
+            if (bounded && threadIdx.x < n_lag) {
+                const double cr = corr[threadIdx.x], ci = corr_i[threadIdx.x];
+                a = sqrt(cr * cr + ci * ci);
+                lo = a - eps;
+            }
+#pragma unroll
+            for (int k = 16; k > 0; k >>= 1) lo = fmax(lo, __shfl_xor_sync(0xffffffffu, lo, k));
+            if (lane == 0) red_v[w] = lo;
+            __syncthreads();
+            double M = red_v[0];
+#pragma unroll
+            for (int k = 1; k < nw; ++k) M = fmax(M, red_v[k]);
+            const bool cand = bounded && threadIdx.x < n_lag && (a + eps) * (1.0 + 1e-9) >= M * (1.0 - 1e-9);
+            const unsigned bal = __ballot_sync(0xffffffffu, cand);
+            if (lane == 0 && w < 3) cmask[w] = bal;                 // n_lag <= 96
+            const int n_c = __syncthreads_count(cand);              // also orders the red_v reads before any later write
+            if (bounded && mode == 0 && n_c >= 1 && n_c <= SCH_MAXC) {
+                if (w < n_c) {                                      // warp w: the w-th candidate in lag order
+                    int k = w, lag = 0;
+#pragma unroll 1
+                    for (int q = 0; q < 3; ++q) {
+                        unsigned m = cmask[q];
+                        const int pc = __popc(m);
+                        if (k < pc) {
+                            for (; k > 0; --k) m &= m - 1;
+                            lag = 32 * q + __ffs(m) - 1;
+                            break;
+                        }
+                        k -= pc;
+                    }
+                    const double v = sch_lag_fp64(wp, tpl, lag, lane);
+                    if (lane == 0) { corr_i[w] = v; red_i[w] = lag; }
+                }
+                __syncthreads();
+                if (threadIdx.x == 0) {
+                    double v = -1.0; int bi = 0x7fffffff;
+                    for (int k = 0; k < n_c; ++k) argmax_combine(v, bi, corr_i[k], red_i[k]);
+                    *o = (double)(sp + bi);
+                    sch_edge[(i64)stream * cap + burst] = (bi == 0 || bi == n_lag - 1) ? 1 : 0;
+                    atomicAdd(stats + n_c, 1u);
+                }
+                return;
+            }
+            // fallback: the full fp64 correlation; the fp64 template goes over the fp32 window (read before the barriers above)
+            for (int i = threadIdx.x; i < L; i += SCH_THREADS) tp[i + (i >> 4)] = __ldg(tpl + i);
+        } else {
+            for (int i = threadIdx.x; i < n_smp; i += SCH_THREADS) wp[i + (i >> 4)] = win[i];
+            for (int i = threadIdx.x; i < L; i += SCH_THREADS) tp[i + (i >> 4)] = t[i];
         }
+        if (threadIdx.x == 0) atomicAdd(stats, 1u);
+        __syncthreads();
+        sch_corr_tiled_fp64(wp, tp, part, corr, corr_i, n_lag, n_smp);
     } else {
         for (int lag = w; lag < n_lag; lag += nw) {              // generic shapes: one warp per lag
             double ar = 0.0, ai = 0.0;
