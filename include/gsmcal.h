@@ -323,19 +323,15 @@ int gsmcal_fcch_scan(const uint8_t *raw, int raw_mem, int64_t n_iq, int64_t n_ch
 
 /* test / tuning hooks: key 0, value 1 = run the all-bin fine FCCH search for every burst (no band-limited fast path);
  * 3 = stream groups of gsmcal_calibrate_batch; 4 = pretend the tier-1/2 certificates failed; 5 = tier-3 list limit;
- * 6 = burst chain on high-priority streams (default 1); 7 = blocks per SM of a persistent high-priority column-sum kernel in
- * _submit (default 0 = off); 8 = stream groups inside a submitted batch (default 2); 9, value 1 = the generic tier-1 fine
- * search without the osr-8 fast path and its filtered-window cache (A/B and tests); 10 = passes of 8 tracked bins in the osr-8 tier-1
- * kernel (1..8, default 8); 11, value 1 = generic tone estimator for every burst (no tone8_kernel); 12, value 1 = plain cudaMemcpyAsync
- * for pageable host buffers instead of the library's multi-threaded pinned staging ring; 13, value 1 = per-phase clock64 counters in
- * fine_core8_kernel / tone8_kernel / coarse_chain_kernel (gsmcal_debug_get 50.. / 150..); 14, value 1 = device timeline of every
- * submitted batch on stderr; 15 = threads of the persistent column-sum kernel; 16 = stagger submitted batches (default 1; 0 = two
- * batches in lockstep); 17 = 4 KB ring stages per block of the TMA column-sum kernel of _submit (default 2; 0 = plain launches);
- * 18 = its blocks per SM (default 3); 19, value 1 = SCH correlation kernel capped at 56 registers; 21, value 1 = the burst chains of a
- * batch's stream groups one after the other; 22, value 1 = burst chains on normal-priority streams; 23 = KB of shared memory per block
- * of an extra kernel of sleeping blocks behind the chain (experiment: what the chain's SM slots cost); 24 = the osr-8 SCH correlation:
- * value 0 = fp32 screen of the 89 lags, fp64 only for the lags that can hold the maximum (default), 1 = fp64 correlation of every lag
- * (A/B), 2 = run the screen, then the fp64 fallback as if it had failed (tests) */
+ * 6 = burst chain on high-priority streams (default 1); 8 = stream groups inside a submitted batch (default 2); 9, value 1 = the
+ * generic tier-1 fine search without the osr-8 fast path and its filtered-window cache (A/B and tests); 10 = passes of 8 tracked bins
+ * in the osr-8 tier-1 kernel (1..8, default 8); 11, value 1 = generic tone estimator for every burst (no tone8_kernel); 12, value 1 =
+ * plain cudaMemcpyAsync for pageable host buffers instead of the library's multi-threaded pinned staging ring; 13, value 1 = per-phase
+ * clock64 counters in fine_core8_kernel / tone8_kernel / coarse_chain_kernel (gsmcal_debug_get 50.. / 150..); 14, value 1 = device
+ * timeline of every submitted batch on stderr; 17 = 4 KB ring stages per block of the TMA column-sum kernel of _submit (1..24,
+ * default 2); 18 = its blocks per SM (default 3); 24 = the osr-8 SCH correlation: value 0 = fp32 screen of the 89 lags, fp64 only for
+ * the lags that can hold the maximum (default), 1 = fp64 correlation of every lag (A/B), 2 = run the screen, then the fp64 fallback as
+ * if it had failed (tests).  Any other key: GSMCAL_ERR_ARG */
 int gsmcal_debug_set(int key, int value);
 /* key 1: number of bursts of the last fine FCCH search whose band certificate failed (all-bin fallback ran); 2: bursts that needed the
  * 64-bin band kernel; 10 + p: bursts the osr-8 tier-1 kernel proved after p passes (p = 0: left open); 30: bytes moved through the

@@ -40,20 +40,13 @@ int g_debug_fall_limit = FALL_GRID;  // tier 3 handles work lists up to this len
 int g_debug_fail_tier2 = 0;       // tests: pretend the 64-bin certificate failed
 int g_debug_force_full = 0;       // tests: run the all-bin fine search for every burst
 int g_debug_submit_groups = 2;    // stream groups inside a submitted batch (debug key 8)
-int g_debug_persist_colsum = 0;   // submit/collect: blocks per SM of the persistent high-priority column-sum kernel (0 = per-group launches)
 int g_debug_hi_prio = 1;          // burst chain of each stream group on a high-priority CUDA stream
 int g_debug_core8_passes = B8_NPASS; // passes of 8 tracked bins in fine_core8_kernel (1..8)
 unsigned *g_last_pass_hist = nullptr, *g_prev_pass_hist = nullptr;   // counters of the last / the one-before-last batch (debug_get 50.., 150..)
-int g_debug_persist_threads = 256;  // block size of the persistent column-sum kernel (debug key 15)
-int g_debug_occupy = 0;            // debug key 23: KB of shared memory per block of an extra occupy_kernel launch behind the chain (0 = none)
-int g_debug_chain_serial = 0;      // debug key 21: the burst chains of a batch's stream groups run one after the other
-int g_debug_chain_lo = 0;          // debug key 22: ... on normal-priority streams (they only take what the FP64 blocks leave free)
-int g_debug_sch56 = 0;             // debug key 19: sch_corr_kernel capped at 56 registers
 int g_debug_sch_mode = 0;          // debug key 24: sch_corr_kernel at osr 8: 0 = fp32 screen, 1 = always fp64, 2 = screen + forced fallback
 unsigned *g_last_sch_stats = nullptr;   // SCH_NSTAT counters of the last call that ran the SCH stage (debug_get 120..)
-int g_debug_trickle = 2;           // debug key 17: ring stages (x 4 KB) of colsum_u8_trickle_kernel in submit/collect, 0 = off (plain column-sum launches)
+int g_debug_trickle = 2;           // debug key 17: ring stages (x 4 KB, 1..24) of colsum_u8_trickle_kernel in submit/collect
 int g_debug_trickle_blocks = 3;    // debug key 18: its blocks per SM (3 x 2 stages: 22 GB in 7 ms under the FP64 stages, profiles/r2q)
-int g_debug_gate = 1;              // debug key 16: submit/collect staggers the batches - the FP64 stages of batch k+1 wait for batch k, its front runs under them
 int g_debug_timeline = 0;          // submit/collect print the device timeline of every batch to stderr (A/B of overlap)
 cudaEvent_t g_tl_base = nullptr;
 int g_debug_prof = 0;              // fine_core8_kernel accumulates per-phase cycle counts (debug_get 50..65)
@@ -99,8 +92,7 @@ struct DevBuf {
 constexpr int kSlots = 4;
 struct Slot {
     DevBuf work, wc;                                            // wc: filtered-window cache of the osr-8 fast path
-    cudaStream_t front = nullptr, front_hi = nullptr;
-    std::vector<cudaStream_t> co;                               // debug key 22: normal-priority streams for the burst chains
+    cudaStream_t front_hi = nullptr;
     std::vector<cudaStream_t> grp, hi;
     cudaEvent_t done = nullptr;
     cudaEvent_t tl[8] = {};                                     // debug key 14: front start, column sums done, burst chain done, FP64 stages done,
@@ -190,10 +182,8 @@ int get_ctx(Ctx **out) {
         CU(cudaFuncSetAttribute(tone8_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, T8_SMEM));
         CU(cudaFuncSetAttribute(tone8_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, T8_SMEM));
         CU(cudaFuncSetAttribute(tone_est_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-        CU(cudaFuncSetAttribute(sch_corr_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
-        CU(cudaFuncSetAttribute(sch_corr_kernel<56>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
+        CU(cudaFuncSetAttribute(sch_corr_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
         CU(cudaFuncSetAttribute(colsum_u8_trickle_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 24 * (TRK_STAGE + 8)));
-        CU(cudaFuncSetAttribute(occupy_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
         CU(cudaFuncSetAttribute(colsum_u8_trickle_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
         CU(cudaFuncSetAttribute(materialise_r_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
         CU(cudaFuncSetAttribute(fir_full_tma_kernel<48>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
@@ -352,14 +342,6 @@ int run_colsum_u8(const uint8_t *raw, i64 n_iq, i64 D, StreamCtl *ctl, cudaStrea
     return GSMCAL_OK;
 }
 
-int run_colsum_u8_persist(const uint8_t *raw, i64 n_iq, i64 D, StreamCtl *ctl, int blocks, cudaStream_t st) {
-    if (((uintptr_t)raw & 1) != 0) return fail(GSMCAL_ERR_ARG, "uint8 capture must start on an even address");
-    const i64 chunk = 512 * 1024;
-    i64 chunks = (2 * n_iq + chunk - 1) / chunk; if (chunks < 1) chunks = 1;
-    LAUNCH(colsum_u8_persist_kernel, (unsigned)blocks, g_debug_persist_threads, 0, st, raw, n_iq, chunk, chunks, D, ctl);
-    return GSMCAL_OK;
-}
-
 int run_colsum_u8_trickle(const uint8_t *raw, i64 n_iq, i64 D, StreamCtl *ctl, int blocks, int n_stage, cudaStream_t st) {
     if (((uintptr_t)raw & 1) != 0) return fail(GSMCAL_ERR_ARG, "uint8 capture must start on an even address");
     const i64 chunk = 512 * 1024;
@@ -460,10 +442,8 @@ int run_fine(Ctx &c, WinSrc src_peak, WinSrc src_tone, i64 n_iq, int osr, double
 }
 
 int run_sch(WinSrc src, int osr, i64 D, int cap, Work &w, cudaStream_t st) {
-#define SCH_ARGS src, w.ctl, w.fcch_pos, cap, osr, w.tpl, w.tplf, w.tpl_e, g_debug_sch_mode, w.sch_stats, w.sch_raw, w.sch_edge
-    if (g_debug_sch56) LAUNCH(sch_corr_kernel<56>, dim3((unsigned)cap, (unsigned)D), SCH_THREADS, sch_smem(osr), st, SCH_ARGS);
-    else               LAUNCH(sch_corr_kernel<64>, dim3((unsigned)cap, (unsigned)D), SCH_THREADS, sch_smem(osr), st, SCH_ARGS);
-#undef SCH_ARGS
+    LAUNCH(sch_corr_kernel, dim3((unsigned)cap, (unsigned)D), SCH_THREADS, sch_smem(osr), st,
+           src, w.ctl, w.fcch_pos, cap, osr, w.tpl, w.tplf, w.tpl_e, g_debug_sch_mode, w.sch_stats, w.sch_raw, w.sch_edge);
     LAUNCH(sch_ppm_kernel, (unsigned)D, PS_THREADS, (size_t)cap * 21 + 16, st, w.ctl, (int)D, cap, osr, w.sch_raw, w.sch_edge, w.sch_pos, w.kind, w.pos_info, w.post_pos);
     return GSMCAL_OK;
 }
@@ -595,6 +575,69 @@ int run_demod(Ctx &c, WinSrc src, const Work &ws, const DemodDev &dd, int osr, d
     return GSMCAL_OK;
 }
 
+// ---- what gsmcal_calibrate_batch* and gsmcal_calibrate_batch_submit share ---------------------------------------------------------
+// `to` waits for what has been enqueued on `from` so far
+int hand_off(cudaStream_t from, cudaStream_t to) {
+    cudaEvent_t ev; CU(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+    CU(cudaEventRecord(ev, from)); CU(cudaStreamWaitEvent(to, ev, 0)); CU(cudaEventDestroy(ev));
+    return GSMCAL_OK;
+}
+
+struct Batch { CoarseParams p; int dec; i64 len_dec; int cap; Work w; };
+// argument checks and sizes; no device is touched, so a malformed call fails the same way on every machine
+int batch_args(const char *name, const void *raw, const double *tpl, const double *coef, const void *results, i64 n_iq, i64 D, int osr,
+               int coarse_dr, Batch *b) {
+    if (!raw || !tpl || !coef || !results || n_iq < 1 || D < 1 || osr < 1 || osr > 8) return fail(GSMCAL_ERR_ARG, "%s: bad arguments (osr 1..8)", name);
+    TRY(coarse_params(coarse_dr, &b->p));
+    b->dec = osr * coarse_dr;
+    b->len_dec = (n_iq + b->dec - 1) / b->dec;
+    if (b->p.n_first > b->len_dec) return fail(GSMCAL_ERR_RANGE, "%s: capture shorter than 23 frames", name);
+    b->cap = (int)gsmcal_max_bursts(b->len_dec, coarse_dr);
+    return GSMCAL_OK;
+}
+// the per-call set-up on st: workspace and window cache, FIR taps, zeroed control blocks and counters, the packed SCH template (through
+// h_tpl, tpl_pack_bytes(64 * osr) bytes that stay valid until the copy has run) and the twiddles, built before the stream groups fork
+int batch_setup(Ctx &c, DevBuf &work, DevBuf &wc, const double *tpl, const double *coef, int n_taps, int osr, i64 D, unsigned char *h_tpl,
+                cudaStream_t st, Batch *b) {
+    Work &w = b->w;
+    const int cap = b->cap;
+    TRY(make_work(work, D, cap, b->p.n_first, 64 * osr, &w));
+    TRY(attach_wcache(wc, D, cap, osr, &w));
+    TRY(set_taps(coef, n_taps, st));
+    CU(cudaMemsetAsync(w.ctl, 0, sizeof(StreamCtl) * D, st));
+    CU(cudaMemsetAsync(w.need_full, 0, sizeof(int) * D * cap, st));
+    CU(cudaMemsetAsync(w.need_band, 0, sizeof(int) * D * cap, st));
+    tpl_pack(tpl, 64 * osr, h_tpl);
+    CU(cudaMemcpyAsync((void *)w.tpl, h_tpl, tpl_pack_bytes(64 * osr), cudaMemcpyHostToDevice, st));
+    CU(cudaMemsetAsync(w.sch_stats, 0, sizeof(unsigned) * SCH_NSTAT, st));
+    { const double2 *twp; TRY(get_twiddle(c, 148 * osr, st, &twp)); }
+    CU(cudaMemsetAsync(w.pass_hist, 0, sizeof(unsigned) * 16 + sizeof(unsigned long long) * 64, st));
+    g_last_sch_stats = w.sch_stats;
+    g_last_need_full = w.need_full; g_last_need_band = w.need_band; g_last_need_full_n = (long long)D * cap;
+    g_last_pass_hist = w.pass_hist;
+    return GSMCAL_OK;
+}
+
+// the burst stages of one stream group, in order on sg: fine peak, fine rest (ppm, tone, carrier), SCH, post-SCH and, with dd, the demod
+// stage.  With marks, marks[i] is recorded on sg behind stage i (null entries are skipped)
+int run_burst_stages(Ctx &c, const uint8_t *graw, i64 n_iq, int n_taps, int osr, double carrier_freq, i64 nd, int cap, Work &ws,
+                     const DemodDev *dd, cudaStream_t sg, const cudaEvent_t *marks) {
+    auto mark = [&](int i) { if (marks && marks[i]) CU(cudaEventRecord(marks[i], sg)); return GSMCAL_OK; };
+    TRY(run_fine_peak(c, lazy_src(graw, n_iq, n_taps, 0, 1), n_iq, osr, nd, cap, ws, sg));
+    TRY(mark(0));
+    TRY(run_fine_rest(c, with_cache(lazy_src(graw, n_iq, n_taps, 1, 1), ws, cap), n_iq, osr, carrier_freq, nd, cap, ws, sg));
+    TRY(mark(1));
+    TRY(run_sch(lazy_src(graw, n_iq, n_taps, 2, 1), osr, nd, cap, ws, sg));
+    TRY(mark(2));
+    TRY(run_post(c, with_cache(lazy_src(graw, n_iq, n_taps, 3, 1), ws, cap), osr, carrier_freq, nd, cap, ws, true, sg));
+    TRY(mark(3));
+    if (dd) {
+        TRY(run_demod(c, lazy_src(graw, n_iq, n_taps, 3, 1), ws, *dd, osr, carrier_freq, nd, cap, sg));
+        TRY(mark(4));
+    }
+    return GSMCAL_OK;
+}
+
 }  // namespace
 
 // ====================================================================================================
@@ -630,12 +673,9 @@ void gsmcal_release(void) {
             if (sl.done) { cudaEventSynchronize(sl.done); cudaEventDestroy(sl.done); sl.done = nullptr; }
             for (cudaStream_t s2 : sl.grp) cudaStreamDestroy(s2);
             for (cudaStream_t s2 : sl.hi) cudaStreamDestroy(s2);
-            for (cudaStream_t s2 : sl.co) cudaStreamDestroy(s2);
-            sl.co.clear();
-            if (sl.front) cudaStreamDestroy(sl.front);
             if (sl.front_hi) cudaStreamDestroy(sl.front_hi);
             sl.front_hi = nullptr;
-            sl.grp.clear(); sl.hi.clear(); sl.front = nullptr;
+            sl.grp.clear(); sl.hi.clear();
             if (sl.stage) cudaFreeHost(sl.stage);
             sl.stage = nullptr; sl.stage_cap = 0; sl.busy = false;
             sl.work.release(); sl.wc.release();
@@ -693,18 +733,11 @@ int gsmcal_debug_set(int key, int value) {
     if (key == 12) { g_debug_no_staging = value ? 1 : 0; return GSMCAL_OK; }
     if (key == 13) { g_debug_prof = value ? 1 : 0; return GSMCAL_OK; }
     if (key == 14) { g_debug_timeline = value ? 1 : 0; return GSMCAL_OK; }
-    if (key == 16) { g_debug_gate = value ? 1 : 0; return GSMCAL_OK; }
-    if (key == 23) { g_debug_occupy = value < 0 ? 0 : (value > 96 ? 96 : value); return GSMCAL_OK; }
-    if (key == 21) { g_debug_chain_serial = value != 0; return GSMCAL_OK; }
-    if (key == 22) { g_debug_chain_lo = value != 0; return GSMCAL_OK; }
-    if (key == 19) { g_debug_sch56 = value != 0; return GSMCAL_OK; }
     if (key == 24) { if (value < 0 || value > 2) return fail(GSMCAL_ERR_ARG, "debug_set 24: 0, 1 or 2"); g_debug_sch_mode = value; return GSMCAL_OK; }
-    if (key == 17) { g_debug_trickle = value < 0 ? 0 : (value > 24 ? 24 : value); return GSMCAL_OK; }
+    if (key == 17) { g_debug_trickle = value < 1 ? 1 : (value > 24 ? 24 : value); return GSMCAL_OK; }
     if (key == 18) { g_debug_trickle_blocks = value < 1 ? 1 : (value > 4 ? 4 : value); return GSMCAL_OK; }
-    if (key == 15) { g_debug_persist_threads = (value == 64 || value == 128) ? value : 256; return GSMCAL_OK; }
     if (key == 10) { g_debug_core8_passes = value < 1 ? 1 : (value > 8 ? 8 : value); return GSMCAL_OK; }
     if (key == 8) { g_debug_submit_groups = value < 1 ? 1 : (value > kMaxGroups / 2 ? kMaxGroups / 2 : value); return GSMCAL_OK; }
-    if (key == 7) { g_debug_persist_colsum = value < 0 ? 0 : (value > 8 ? 8 : value); return GSMCAL_OK; }
     if (key == 3) { g_debug_groups = value < 1 ? 1 : (value > kMaxGroups / 2 ? kMaxGroups / 2 : value); return GSMCAL_OK; }
     return fail(GSMCAL_ERR_ARG, "debug_set: unknown key");
 }
@@ -1125,35 +1158,18 @@ static int calibrate_batch_impl(const uint8_t *raw, int raw_mem, int64_t n_iq, i
                                 double *r_out, int r_mem, int64_t r_stride, const DemodOut *dm = nullptr) {
     std::lock_guard<std::mutex> lk(g_mu);
     if (r_out && r_stride < n_iq) return fail(GSMCAL_ERR_ARG, "calibrate_batch_r: r_stride must be >= n_iq");
-    if (!raw || !tpl || !coef || !results || n_iq < 1 || D < 1 || osr < 1 || osr > 8) return fail(GSMCAL_ERR_ARG, "calibrate_batch: bad arguments (osr 1..8)");
-    CoarseParams p; TRY(coarse_params(coarse_dr, &p));
-    const int dec = osr * coarse_dr;
-    const i64 len_dec = (n_iq + dec - 1) / dec;
-    if (p.n_first > len_dec) return fail(GSMCAL_ERR_RANGE, "calibrate_batch: capture shorter than 23 frames");
-    const int cap = (int)gsmcal_max_bursts(len_dec, coarse_dr);
+    Batch b; TRY(batch_args("calibrate_batch", raw, tpl, coef, results, n_iq, D, osr, coarse_dr, &b));
+    const int cap = b.cap;
     Ctx *c; TRY(get_ctx(&c));
     cudaStream_t st = (cudaStream_t)cuda_stream;
-    Work w;
-    TRY(make_work(c->work, D, cap, p.n_first, 64 * osr, &w));
-    TRY(attach_wcache(c->wc, D, cap, osr, &w));
-    TRY(set_taps(coef, n_taps, st));
+    std::vector<unsigned char> tpk(tpl_pack_bytes(64 * osr));       // pageable: cudaMemcpyAsync stages it before it returns
+    TRY(batch_setup(*c, c->work, c->wc, tpl, coef, n_taps, osr, D, tpk.data(), st, &b));
+    Work &w = b.w;
     const uint8_t *draw = raw;
     if (raw_mem == GSMCAL_MEM_HOST) {
         void *din; TRY(c->in.get((size_t)2 * n_iq * D, &din));
         draw = (const uint8_t *)din;
     }
-    CU(cudaMemsetAsync(w.ctl, 0, sizeof(StreamCtl) * D, st));
-    CU(cudaMemsetAsync(w.need_full, 0, sizeof(int) * D * cap, st));
-    CU(cudaMemsetAsync(w.need_band, 0, sizeof(int) * D * cap, st));
-    std::vector<unsigned char> tpk(tpl_pack_bytes(64 * osr));
-    tpl_pack(tpl, 64 * osr, tpk.data());
-    CU(cudaMemcpyAsync((void *)w.tpl, tpk.data(), tpk.size(), cudaMemcpyHostToDevice, st));      // pageable: staged before the call returns
-    g_last_sch_stats = w.sch_stats;
-    CU(cudaMemsetAsync(w.sch_stats, 0, sizeof(unsigned) * SCH_NSTAT, st));
-    { const double2 *twp; TRY(get_twiddle(*c, 148 * osr, st, &twp)); }        // built on `st` before the groups fork
-    g_last_need_full = w.need_full; g_last_need_band = w.need_band; g_last_need_full_n = (long long)D * cap;
-    g_last_pass_hist = w.pass_hist;
-    CU(cudaMemsetAsync(w.pass_hist, 0, sizeof(unsigned) * 16 + sizeof(unsigned long long) * 64, st));
     DemodDev dd;
     std::vector<double> dm_w; signed char dm_pm[64];                 // host sources of the uploads, alive until the final synchronise
     if (dm) TRY(demod_setup(*c, D, cap, osr, w.tpl, dm->nts, dm_w, dm_pm, st, &dd));
@@ -1185,25 +1201,14 @@ static int calibrate_batch_impl(const uint8_t *raw, int raw_mem, int64_t n_iq, i
         const uint8_t *graw = draw + d0 * per;
         if (raw_mem == GSMCAL_MEM_HOST) {
             TRY(copy_h2d(c->ring, g_device, (void *)graw, raw + d0 * per, per * nd, cp));
-            cudaEvent_t ev; CU(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-            CU(cudaEventRecord(ev, cp)); CU(cudaStreamWaitEvent(sg, ev, 0)); CU(cudaEventDestroy(ev));
+            TRY(hand_off(cp, sg));
             TRY(run_colsum_u8(graw, n_iq, nd, ws.ctl, sg));
         } else if (sg == st) {
             TRY(run_colsum_u8(graw, n_iq, nd, ws.ctl, sg));
-        } else if (g_debug_persist_colsum > 0 && g_debug_hi_prio && g > 0) {
-            // device input, groups after the first: the column sums as ONE persistent launch of small fixed footprint on the group's
-            // high-priority stream, so they run BESIDE the FP64 stages of the previous group (which the gate below keeps ahead)
-            cudaStream_t sh = c->side_hi[g];
-            int n_sm = 148; CU(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, g_device));
-            CU(cudaStreamWaitEvent(sh, ev_fork, 0));
-            TRY(run_colsum_u8_persist(graw, n_iq, nd, ws.ctl, n_sm * g_debug_persist_colsum, sh));
-            cudaEvent_t ev; CU(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-            CU(cudaEventRecord(ev, sh)); CU(cudaStreamWaitEvent(sg, ev, 0)); CU(cudaEventDestroy(ev));
         } else {
             // device input: the HBM-bound column sums run on the caller's stream (group 0 gets the whole bandwidth first)
             TRY(run_colsum_u8(graw, n_iq, nd, ws.ctl, st));
-            cudaEvent_t ev; CU(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-            CU(cudaEventRecord(ev, st)); CU(cudaStreamWaitEvent(sg, ev, 0)); CU(cudaEventDestroy(ev));
+            TRY(hand_off(st, sg));
         }
         LAUNCH(mean_kernel, (unsigned)((nd + 127) / 128), 128, 0, sg, ws.ctl, (int)nd, n_iq);
         if (timing) TRY(stage_mark(*c, sg));
@@ -1212,28 +1217,17 @@ static int calibrate_batch_impl(const uint8_t *raw, int raw_mem, int64_t n_iq, i
             // their blocks queue behind the thousands of pending blocks of the other groups' FP64 kernels.  A high-priority stream
             // lets the block scheduler place them as soon as a slot frees, so the chain runs underneath the heavy kernels.
             cudaStream_t sh = c->side_hi[g];
-            cudaEvent_t e1, e2; CU(cudaEventCreateWithFlags(&e1, cudaEventDisableTiming)); CU(cudaEventCreateWithFlags(&e2, cudaEventDisableTiming));
-            CU(cudaEventRecord(e1, sg)); CU(cudaStreamWaitEvent(sh, e1, 0));
-            TRY(run_coarse(lazy_src(graw, n_iq, n_taps, 0, dec), len_dec, p, nd, cap, ws, sh));
-            CU(cudaEventRecord(e2, sh)); CU(cudaStreamWaitEvent(sg, e2, 0));
-            CU(cudaEventDestroy(e1)); CU(cudaEventDestroy(e2));
+            TRY(hand_off(sg, sh));
+            TRY(run_coarse(lazy_src(graw, n_iq, n_taps, 0, b.dec), b.len_dec, b.p, nd, cap, ws, sh));
+            TRY(hand_off(sh, sg));
         } else
-        TRY(run_coarse(lazy_src(graw, n_iq, n_taps, 0, dec), len_dec, p, nd, cap, ws, sg));
+        TRY(run_coarse(lazy_src(graw, n_iq, n_taps, 0, b.dec), b.len_dec, b.p, nd, cap, ws, sg));
         if (timing) TRY(stage_mark(*c, sg));
         // stagger the groups (see gsmcal_calibrate_batch_submit): the FP64 stages of group g wait for group g-1, its front does not
-        if (g_debug_gate && sg != st && !ev_done.empty()) CU(cudaStreamWaitEvent(sg, ev_done.back(), 0));
-        TRY(run_fine_peak(*c, lazy_src(graw, n_iq, n_taps, 0, 1), n_iq, osr, nd, cap, ws, sg));
-        if (timing) TRY(stage_mark(*c, sg));
-        TRY(run_fine_rest(*c, with_cache(lazy_src(graw, n_iq, n_taps, 1, 1), ws, cap), n_iq, osr, carrier_freq, nd, cap, ws, sg));
-        if (timing) TRY(stage_mark(*c, sg));
-        TRY(run_sch(lazy_src(graw, n_iq, n_taps, 2, 1), osr, nd, cap, ws, sg));
-        if (timing) TRY(stage_mark(*c, sg));
-        TRY(run_post(*c, with_cache(lazy_src(graw, n_iq, n_taps, 3, 1), ws, cap), osr, carrier_freq, nd, cap, ws, true, sg));
-        if (timing) TRY(stage_mark(*c, sg));
-        if (dm) {
-            TRY(run_demod(*c, lazy_src(graw, n_iq, n_taps, 3, 1), ws, sub_demod(dd, d0, cap), osr, carrier_freq, nd, cap, sg));
-            if (timing) TRY(stage_mark(*c, sg));
-        }
+        if (!ev_done.empty()) CU(cudaStreamWaitEvent(sg, ev_done.back(), 0));
+        const DemodDev gdd = dm ? sub_demod(dd, d0, cap) : DemodDev{};
+        TRY(run_burst_stages(*c, graw, n_iq, n_taps, osr, carrier_freq, nd, cap, ws, dm ? &gdd : nullptr, sg, timing ? c->stage_ev + g_stage_n : nullptr));
+        if (timing) g_stage_n += dm ? 5 : 4;                     // 3 + 5 <= kNumStageEvents
         if (sg != st) {
             cudaEvent_t ev; CU(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
             CU(cudaEventRecord(ev, sg));
@@ -1326,12 +1320,8 @@ int gsmcal_calibrate_batch_submit(int slot, const uint8_t *raw_dev, int64_t n_iq
                                   double *coarse_pos, double *coarse_snr, double *fcch_pos, double *pos_info, void *cuda_stream) {
     std::lock_guard<std::mutex> lk(g_mu);
     if (slot < 0 || slot >= kSlots) return fail(GSMCAL_ERR_ARG, "calibrate_batch_submit: slot must be 0..%d", kSlots - 1);
-    if (!raw_dev || !tpl || !coef || !results || n_iq < 1 || D < 1 || osr < 1 || osr > 8) return fail(GSMCAL_ERR_ARG, "calibrate_batch_submit: bad arguments (osr 1..8)");
-    CoarseParams p; TRY(coarse_params(coarse_dr, &p));
-    const int dec = osr * coarse_dr;
-    const i64 len_dec = (n_iq + dec - 1) / dec;
-    if (p.n_first > len_dec) return fail(GSMCAL_ERR_RANGE, "calibrate_batch_submit: capture shorter than 23 frames");
-    const int cap = (int)gsmcal_max_bursts(len_dec, coarse_dr);
+    Batch b; TRY(batch_args("calibrate_batch_submit", raw_dev, tpl, coef, results, n_iq, D, osr, coarse_dr, &b));
+    const int cap = b.cap;
     Ctx *c; TRY(get_ctx(&c));
     Slot &sl = c->slots[slot];
     if (sl.busy) return fail(GSMCAL_ERR_ARG, "calibrate_batch_submit: slot %d still holds an uncollected batch", slot);
@@ -1339,16 +1329,13 @@ int gsmcal_calibrate_batch_submit(int slot, const uint8_t *raw_dev, int64_t n_iq
     int n_groups = g_debug_submit_groups;                       // 2: in the staggered pipeline a batch's stages run alone, so the per-stream kernels and
                                                                 // the grid tails of one half overlap the burst kernels of the other (31.15 -> 30.85 ms, profiles/r2x)
     if (D < 2 * n_groups) n_groups = 1;
-    if (!sl.front) { CU(cudaStreamCreateWithFlags(&sl.front, cudaStreamNonBlocking)); CU(cudaEventCreateWithFlags(&sl.done, cudaEventDisableTiming)); }
+    if (!sl.done) CU(cudaEventCreateWithFlags(&sl.done, cudaEventDisableTiming));
     int lo_p = 0, hi_p = 0; CU(cudaDeviceGetStreamPriorityRange(&lo_p, &hi_p));
     if (!sl.front_hi) CU(cudaStreamCreateWithPriority(&sl.front_hi, cudaStreamNonBlocking, hi_p));
     while ((int)sl.grp.size() < n_groups) { cudaStream_t s2; CU(cudaStreamCreateWithFlags(&s2, cudaStreamNonBlocking)); sl.grp.push_back(s2); }
     while ((int)sl.hi.size() < n_groups) { cudaStream_t s2; CU(cudaStreamCreateWithPriority(&s2, cudaStreamNonBlocking, hi_p)); sl.hi.push_back(s2); }
-    Work w;
-    TRY(make_work(sl.work, D, cap, p.n_first, 64 * osr, &w));
-    TRY(attach_wcache(sl.wc, D, cap, osr, &w));
-    TRY(set_taps(coef, n_taps, st));
-    // pinned staging: records | coarse_pos | coarse_snr | fcch_pos | pos_info (x12)
+    // pinned staging: records | coarse_pos | coarse_snr | fcch_pos | pos_info (x12) | the packed SCH template (the caller's template may be
+    // pageable and short-lived)
     sl.n_res = sizeof(StreamResultDev) * (size_t)D; sl.n_per = sizeof(double) * (size_t)D * cap;
     const size_t need = align_up(sl.n_res) + 15 * sl.n_per + tpl_pack_bytes(64 * osr);
     if (need > sl.stage_cap) {
@@ -1358,97 +1345,52 @@ int gsmcal_calibrate_batch_submit(int slot, const uint8_t *raw_dev, int64_t n_iq
         sl.stage_cap = need;
     }
     char *h_res = sl.stage, *h_arr = sl.stage + align_up(sl.n_res), *h_tpl = h_arr + 15 * sl.n_per;
-    tpl_pack(tpl, 64 * osr, (unsigned char *)h_tpl);           // the caller's template may be pageable and short-lived
-    { const double2 *twp; TRY(get_twiddle(*c, 148 * osr, st, &twp)); }
     // normal-priority kernels of different streams are dispatched in arrival order: behind the 10^5 queued blocks of the previous batch's fine
-    // search even a memset waits milliseconds (device timeline, debug key 14), so the staggered mode runs the whole front at high priority
-    cudaStream_t fr = (g_debug_trickle > 0 || g_debug_gate) ? sl.front_hi : sl.front;
-    cudaEvent_t ev_in; CU(cudaEventCreateWithFlags(&ev_in, cudaEventDisableTiming));
-    CU(cudaEventRecord(ev_in, st)); CU(cudaStreamWaitEvent(fr, ev_in, 0)); CU(cudaEventDestroy(ev_in));     // the capture is ready on the caller's stream
-    CU(cudaMemsetAsync(w.ctl, 0, sizeof(StreamCtl) * D, fr));
-    CU(cudaMemsetAsync(w.need_full, 0, sizeof(int) * D * cap, fr));
-    CU(cudaMemsetAsync(w.need_band, 0, sizeof(int) * D * cap, fr));
-    CU(cudaMemcpyAsync(w.tpl, h_tpl, tpl_pack_bytes(64 * osr), cudaMemcpyHostToDevice, fr));
-    g_last_sch_stats = w.sch_stats;
-    CU(cudaMemsetAsync(w.sch_stats, 0, sizeof(unsigned) * SCH_NSTAT, fr));
-    g_last_need_full = w.need_full; g_last_need_band = w.need_band; g_last_need_full_n = (long long)D * cap;
-    g_prev_pass_hist = g_last_pass_hist; g_last_pass_hist = w.pass_hist;
-    CU(cudaMemsetAsync(w.pass_hist, 0, sizeof(unsigned) * 16 + sizeof(unsigned long long) * 64, fr));
+    // search even a memset waits milliseconds (device timeline, debug key 14), so the whole front runs at high priority
+    cudaStream_t fr = sl.front_hi;
+    TRY(hand_off(st, fr));                                       // the capture is ready on the caller's stream
+    unsigned *prev_pass_hist = g_last_pass_hist;
+    TRY(batch_setup(*c, sl.work, sl.wc, tpl, coef, n_taps, osr, D, (unsigned char *)h_tpl, fr, &b));
+    g_prev_pass_hist = prev_pass_hist;
+    Work &w = b.w;
     const size_t per = (size_t)2 * n_iq;
-    std::vector<cudaEvent_t> ev_done;
-    cudaEvent_t e_sum = nullptr;
     sl.tl_on = g_debug_timeline != 0;
     if (sl.tl_on) {
         if (!sl.tl[0]) for (auto &e : sl.tl) CU(cudaEventCreate(&e));
         if (!g_tl_base) { CU(cudaEventCreate(&g_tl_base)); CU(cudaEventRecord(g_tl_base, fr)); }
         CU(cudaEventRecord(sl.tl[0], fr));
     }
-    std::vector<cudaEvent_t> e_sum_g;                            // per stream group: its column sums are done
-    if (g_debug_persist_colsum > 0 || g_debug_trickle > 0) {
-        // the column sums as persistent launches of fixed footprint on the high-priority front stream (see colsum_u8_persist_kernel,
-        // colsum_u8_trickle_kernel), one per stream group, back to back: the burst chain of group g starts under the sums of group g+1
-        int n_sm = 148; CU(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, g_device));
-        cudaEvent_t e_in; CU(cudaEventCreateWithFlags(&e_in, cudaEventDisableTiming)); CU(cudaEventCreateWithFlags(&e_sum, cudaEventDisableTiming));
-        CU(cudaEventRecord(e_in, fr)); CU(cudaStreamWaitEvent(sl.front_hi, e_in, 0)); CU(cudaEventDestroy(e_in));
-        for (int g = 0; g < n_groups; ++g) {
-            const i64 d0 = D * g / n_groups, d1 = D * (g + 1) / n_groups;
-            if (g_debug_persist_colsum > 0) TRY(run_colsum_u8_persist(raw_dev + d0 * per, n_iq, d1 - d0, w.ctl + d0, n_sm * g_debug_persist_colsum, sl.front_hi));
-            else TRY(run_colsum_u8_trickle(raw_dev + d0 * per, n_iq, d1 - d0, w.ctl + d0, n_sm * g_debug_trickle_blocks, g_debug_trickle, sl.front_hi));
-            cudaEvent_t eg; CU(cudaEventCreateWithFlags(&eg, cudaEventDisableTiming));
-            CU(cudaEventRecord(eg, sl.front_hi));
-            e_sum_g.push_back(eg);
-        }
-        CU(cudaEventRecord(e_sum, sl.front_hi));
-        if (sl.tl_on) CU(cudaEventRecord(sl.tl[1], sl.front_hi));
+    // the column sums as launches of fixed footprint on the front stream (see colsum_u8_trickle_kernel), one per stream group, back to back:
+    // the burst chain of group g starts under the sums of group g+1
+    int n_sm = 148; CU(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, g_device));
+    for (int g = 0; g < n_groups; ++g) {
+        const i64 d0 = D * g / n_groups, d1 = D * (g + 1) / n_groups;
+        TRY(run_colsum_u8_trickle(raw_dev + d0 * per, n_iq, d1 - d0, w.ctl + d0, n_sm * g_debug_trickle_blocks, g_debug_trickle, fr));
+        TRY(hand_off(fr, sl.hi[g]));
     }
-    if (g_debug_chain_lo) while ((int)sl.co.size() < n_groups) { cudaStream_t s2; CU(cudaStreamCreateWithFlags(&s2, cudaStreamNonBlocking)); sl.co.push_back(s2); }
-    cudaEvent_t e_chain_prev = nullptr;
+    if (sl.tl_on) CU(cudaEventRecord(sl.tl[1], fr));
     for (int g = 0; g < n_groups; ++g) {
         const i64 d0 = D * g / n_groups, d1 = D * (g + 1) / n_groups, nd = d1 - d0;
-        cudaStream_t sg = sl.grp[g], sh = g_debug_chain_lo ? sl.co[g] : sl.hi[g];
+        cudaStream_t sg = sl.grp[g], sh = sl.hi[g];
         Work ws = sub_work(w, d0, cap, g);
         const uint8_t *graw = raw_dev + d0 * per;
-        cudaEvent_t e0, e1; CU(cudaEventCreateWithFlags(&e0, cudaEventDisableTiming)); CU(cudaEventCreateWithFlags(&e1, cudaEventDisableTiming));
-        if (e_sum) CU(cudaStreamWaitEvent(sh, e_sum_g[g], 0));
-        else {
-            TRY(run_colsum_u8(graw, n_iq, nd, ws.ctl, fr));     // HBM-bound sums back to back on the front stream (group 0 first)
-            CU(cudaEventRecord(e0, fr)); CU(cudaStreamWaitEvent(sh, e0, 0));
-            if (sl.tl_on && g == n_groups - 1) CU(cudaEventRecord(sl.tl[1], fr));
-        }
-        if (g_debug_chain_serial && e_chain_prev) CU(cudaStreamWaitEvent(sh, e_chain_prev, 0));
         LAUNCH(mean_kernel, (unsigned)((nd + 127) / 128), 128, 0, sh, ws.ctl, (int)nd, n_iq);
-        TRY(run_coarse(lazy_src(graw, n_iq, n_taps, 0, dec), len_dec, p, nd, cap, ws, sh));      // latency-bound chain: high priority
-        if (g_debug_occupy > 0) LAUNCH(occupy_kernel, (unsigned)nd, 64, (size_t)g_debug_occupy * 1024, sh, (long long)4500000, w.fine_raw);   // ~2.3 ms at 1.965 GHz
-        CU(cudaEventRecord(e1, sh)); CU(cudaStreamWaitEvent(sg, e1, 0));
-        if (e_chain_prev) CU(cudaEventDestroy(e_chain_prev));
-        e_chain_prev = e1;
-        if (sl.tl_on && g == n_groups - 1) CU(cudaEventRecord(sl.tl[2], sh));
-        // Staggered batches (debug key 16, default on).  Ungated, two batches in flight run in lockstep (normal-priority kernels are dispatched
-        // in arrival order, so their stages interleave and both finish together) and both fronts execute while nothing else does.  Gated,
-        // the FP64 stages of batch k+1 start when batch k is done and the front of batch k+1 - on the high-priority stream, with the
-        // column sums as the small-footprint TMA-ring kernel - runs UNDER the FP64 stages of batch k.  Device timelines and the cost of the
-        // overlap (the ring's shared-memory traffic, the burst chain): profiles/r2n, r2p, r2q, r2z, r2ak and DESIGN.md section 4.
-        if (g_debug_gate && c->last_slot >= 0 && c->last_slot != slot && c->slots[c->last_slot].busy)
-            CU(cudaStreamWaitEvent(sg, c->slots[c->last_slot].done, 0));
-        CU(cudaEventDestroy(e0));
+        TRY(run_coarse(lazy_src(graw, n_iq, n_taps, 0, b.dec), b.len_dec, b.p, nd, cap, ws, sh));      // latency-bound chain: high priority
+        TRY(hand_off(sh, sg));
         const bool tl_g = sl.tl_on && g == n_groups - 1;
+        if (tl_g) CU(cudaEventRecord(sl.tl[2], sh));
+        // Staggered batches: the FP64 stages of batch k+1 start when batch k is done, and the front of batch k+1 - on the high-priority
+        // streams, with the column sums as the small-footprint TMA-ring kernel - runs UNDER the FP64 stages of batch k.  Without this wait
+        // two batches in flight run in lockstep (normal-priority kernels are dispatched in arrival order, so their stages interleave and
+        // both finish together) and both fronts execute while nothing else does.  Device timelines and the cost of the overlap (the ring's
+        // shared-memory traffic, the burst chain): profiles/r2n, r2p, r2q, r2z, r2ak and DESIGN.md section 4.
+        if (c->last_slot >= 0 && c->last_slot != slot && c->slots[c->last_slot].busy)
+            CU(cudaStreamWaitEvent(sg, c->slots[c->last_slot].done, 0));
         if (tl_g) CU(cudaEventRecord(sl.tl[4], sg));
-        TRY(run_fine_peak(*c, lazy_src(graw, n_iq, n_taps, 0, 1), n_iq, osr, nd, cap, ws, sg));
-        if (tl_g) CU(cudaEventRecord(sl.tl[5], sg));
-        TRY(run_fine_rest(*c, with_cache(lazy_src(graw, n_iq, n_taps, 1, 1), ws, cap), n_iq, osr, carrier_freq, nd, cap, ws, sg));
-        if (tl_g) CU(cudaEventRecord(sl.tl[6], sg));
-        TRY(run_sch(lazy_src(graw, n_iq, n_taps, 2, 1), osr, nd, cap, ws, sg));
-        if (tl_g) CU(cudaEventRecord(sl.tl[7], sg));
-        TRY(run_post(*c, with_cache(lazy_src(graw, n_iq, n_taps, 3, 1), ws, cap), osr, carrier_freq, nd, cap, ws, true, sg));
-        cudaEvent_t ev; CU(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-        CU(cudaEventRecord(ev, sg));
-        if (sl.tl_on && g == n_groups - 1) CU(cudaEventRecord(sl.tl[3], sg));
-        ev_done.push_back(ev);
+        const cudaEvent_t marks[4] = {sl.tl[5], sl.tl[6], sl.tl[7], sl.tl[3]};
+        TRY(run_burst_stages(*c, graw, n_iq, n_taps, osr, carrier_freq, nd, cap, ws, nullptr, sg, tl_g ? marks : nullptr));
+        TRY(hand_off(sg, fr));
     }
-    if (e_sum) CU(cudaEventDestroy(e_sum));
-    for (cudaEvent_t eg : e_sum_g) CU(cudaEventDestroy(eg));
-    if (e_chain_prev) CU(cudaEventDestroy(e_chain_prev));
-    for (cudaEvent_t ev : ev_done) { CU(cudaStreamWaitEvent(fr, ev, 0)); CU(cudaEventDestroy(ev)); }
     CU(cudaMemcpyAsync(h_res, w.res, sl.n_res, cudaMemcpyDeviceToHost, fr));
     if (coarse_pos) CU(cudaMemcpyAsync(h_arr, w.coarse_pos, sl.n_per, cudaMemcpyDeviceToHost, fr));
     if (coarse_snr) CU(cudaMemcpyAsync(h_arr + sl.n_per, w.coarse_snr, sl.n_per, cudaMemcpyDeviceToHost, fr));

@@ -445,7 +445,7 @@ __device__ __forceinline__ void colsum_u8_chunk(const uint8_t *__restrict__ raw,
         i64 c1 = c0 + chunk_bytes; if (c1 > body) c1 = body;
         const uint4 *v = reinterpret_cast<const uint4 *>(p + head);
         const i64 i0 = c0 / 16, i1 = c1 / 16;
-        const int nt = blockDim.x;                               // 256 (grid form) or a smaller persistent block
+        const int nt = blockDim.x;                               // 256
         i64 i = i0 + threadIdx.x;
         for (; i + 3 * nt < i1; i += 4 * nt) {
             uint4 a = __ldg(v + i), b = __ldg(v + i + nt), c = __ldg(v + i + 2 * nt), d = __ldg(v + i + 3 * nt);
@@ -479,12 +479,6 @@ __device__ __forceinline__ void colsum_u8_chunk(const uint8_t *__restrict__ raw,
 
 __global__ void __launch_bounds__(256) colsum_u8_kernel(const uint8_t *__restrict__ raw, i64 n_iq, i64 chunk_bytes, StreamCtl *ctl) {
     colsum_u8_chunk(raw, n_iq, chunk_bytes, ctl, blockIdx.y, blockIdx.x);
-}
-// persistent form for the submit/collect pipeline: a FIXED small footprint (2 blocks per SM) launched on a high-priority stream, so the
-// HBM-bound sums of batch k+1 share the SMs with the register-file-filling FP64 kernels of batch k instead of waiting behind them
-__global__ void __launch_bounds__(256) colsum_u8_persist_kernel(const uint8_t *__restrict__ raw, i64 n_iq, i64 chunk_bytes, i64 n_chunks, i64 n_streams, StreamCtl *ctl) {
-    const i64 total = n_chunks * n_streams;
-    for (i64 w = blockIdx.x; w < total; w += gridDim.x) colsum_u8_chunk(raw, n_iq, chunk_bytes, ctl, (int)(w / n_chunks), w % n_chunks);
 }
 
 // "trickle" form for the staggered submit/collect pipeline (debug key 17): ONE warp per block, one block per SM, the bytes brought in by
@@ -1254,17 +1248,6 @@ __global__ void __maxnreg__(112) coarse_chain_kernel(WinSrc src, StreamCtl *ctl,
     asm volatile("cp.async.wait_group 0;");                      // no copy may still be in flight when the block retires
     if (prof && tid == 0) atomicAdd(prof + 6, 1ull);
     if (tid == 0) ctl[stream].n_coarse = count;
-}
-
-// Experiment hook (debug key 23): blocks that only OCCUPY - `cycles` of spinning with the footprint given at launch (64 threads, dynamic
-// shared memory) - launched behind the burst chain on its high-priority stream, to tell what the chain costs the burst kernels of the
-// previous batch: the SM slots it holds, or the instructions it executes.
-__global__ void __launch_bounds__(64) occupy_kernel(long long cycles, double *sink) {
-    extern __shared__ double occ_sm[];
-    const long long t0 = clock64();
-    double acc = 0.0;
-    while (clock64() - t0 < cycles) { acc += occ_sm[threadIdx.x]; __nanosleep(200); }
-    if (acc == 12345.678) *sink = acc;
 }
 
 // ===================================================================================================
@@ -2151,8 +2134,8 @@ __device__ __forceinline__ double sch_lag_fp64(const double2 *wp, const double2 
 
 // tplf: the template in fp32, padded like tp (sch_tplf_len(L) entries); tpl_e: its energy in fp64, rounded up.  mode: 0 = fp32 screen,
 // 1 = always the fp64 correlation, 2 = screen, then take the fallback as if it had failed.  stats: SCH_NSTAT counters (see SCH_NSTAT).
-template <int MAXR>     // 64: four blocks fill the register file; 56 (a few spilled values) leaves room for the trickle column sums of the next batch
-__global__ void __maxnreg__(MAXR) sch_corr_kernel(WinSrc src, const StreamCtl *__restrict__ ctl, const double *__restrict__ fcch_pos, int cap,
+// 64 registers: four blocks fill the register file
+__global__ void __maxnreg__(64) sch_corr_kernel(WinSrc src, const StreamCtl *__restrict__ ctl, const double *__restrict__ fcch_pos, int cap,
                                                               int osr, const double2 *__restrict__ tpl, const float2 *__restrict__ tplf,
                                                               const double *__restrict__ tpl_e, int mode, unsigned *__restrict__ stats,
                                                               double *__restrict__ sch_raw, int *__restrict__ sch_edge) {
@@ -2238,44 +2221,41 @@ __global__ void __maxnreg__(MAXR) sch_corr_kernel(WinSrc src, const StreamCtl *_
             const double eps = SCH_EPS_K * 5.9604644775390625e-8 * sqrt(e_win * e_tpl) * (1.0 + 1e-12)
                              + SCH_EPS_ABS * (1.0 + sqrt((double)L * e_tpl) + sqrt((double)L * e_win));
             if (bounded) {
-                // per pass warp w owns lags [SLPW(8p+w), +SLPW), lane owns template samples [16*lane, +16); an SLPW-deep sliding register
+                // warp w owns lags [SLPW*w, +SLPW), lane owns template samples [16*lane, +16); an SLPW-deep sliding register
                 // window of the burst advances one sample per step: 2 LDS.64 (2 wavefronts each, conflict free with the pad) per 4*SLPW
-                // FFMA.  One pass of 12 at 64 registers; the 56-register build takes two passes of 6 (12 would spill)
-                constexpr int SLPW = (MAXR >= 64) ? SCH_SLPW : SCH_SLPW / 2;
+                // FFMA.  One pass of 12 lags at 64 registers
+                constexpr int SLPW = SCH_SLPW;
                 const int nb = SCH_NSL * lane;
-#pragma unroll 1
-                for (int pass = 0; pass < SCH_SLPW / SLPW; ++pass) {
-                    const int l0 = SLPW * (pass * nw + w);
-                    float ar[SLPW], ai[SLPW];
-                    float2 wr_[SLPW];
+                const int l0 = SLPW * w;
+                float ar[SLPW], ai[SLPW];
+                float2 wr_[SLPW];
 #pragma unroll
-                    for (int l = 0; l < SLPW; ++l) { ar[l] = 0.0f; ai[l] = 0.0f; }
+                for (int l = 0; l < SLPW; ++l) { ar[l] = 0.0f; ai[l] = 0.0f; }
 #pragma unroll
-                    for (int l = 0; l < SLPW - 1; ++l) { const int i = l0 + nb + l; wr_[l] = (i < n_smp) ? wf[i + (i >> 4)] : make_float2(0.0f, 0.0f); }
+                for (int l = 0; l < SLPW - 1; ++l) { const int i = l0 + nb + l; wr_[l] = (i < n_smp) ? wf[i + (i >> 4)] : make_float2(0.0f, 0.0f); }
 #pragma unroll
-                    for (int n = 0; n < SCH_NSL; ++n) {
-                        const int iw = l0 + nb + n + SLPW - 1, it = nb + n;
-                        wr_[SLPW - 1] = (iw < n_smp) ? wf[iw + (iw >> 4)] : make_float2(0.0f, 0.0f);
-                        const float2 tt = tf[it + (it >> 4)];
-#pragma unroll
-                        for (int l = 0; l < SLPW; ++l) {
-                            ar[l] = fmaf(wr_[l].x, tt.x, fmaf(wr_[l].y, tt.y, ar[l]));
-                            ai[l] = fmaf(wr_[l].y, tt.x, fmaf(-wr_[l].x, tt.y, ai[l]));
-                        }
-#pragma unroll
-                        for (int l = 0; l < SLPW - 1; ++l) wr_[l] = wr_[l + 1];
-                    }
+                for (int n = 0; n < SCH_NSL; ++n) {
+                    const int iw = l0 + nb + n + SLPW - 1, it = nb + n;
+                    wr_[SLPW - 1] = (iw < n_smp) ? wf[iw + (iw >> 4)] : make_float2(0.0f, 0.0f);
+                    const float2 tt = tf[it + (it >> 4)];
 #pragma unroll
                     for (int l = 0; l < SLPW; ++l) {
-                        ar[l] += __shfl_down_sync(0xffffffffu, ar[l], 16); ai[l] += __shfl_down_sync(0xffffffffu, ai[l], 16);
-                        ar[l] += __shfl_down_sync(0xffffffffu, ar[l], 8);  ai[l] += __shfl_down_sync(0xffffffffu, ai[l], 8);
+                        ar[l] = fmaf(wr_[l].x, tt.x, fmaf(wr_[l].y, tt.y, ar[l]));
+                        ai[l] = fmaf(wr_[l].y, tt.x, fmaf(-wr_[l].x, tt.y, ai[l]));
                     }
-                    if (lane < 8) {                                 // rows (lag, re|im) of 9 floats, every lag of the burst
 #pragma unroll
-                        for (int l = 0; l < SLPW; ++l) {
-                            part_f[(2 * (l0 + l)) * 9 + lane] = ar[l];
-                            part_f[(2 * (l0 + l) + 1) * 9 + lane] = ai[l];
-                        }
+                    for (int l = 0; l < SLPW - 1; ++l) wr_[l] = wr_[l + 1];
+                }
+#pragma unroll
+                for (int l = 0; l < SLPW; ++l) {
+                    ar[l] += __shfl_down_sync(0xffffffffu, ar[l], 16); ai[l] += __shfl_down_sync(0xffffffffu, ai[l], 16);
+                    ar[l] += __shfl_down_sync(0xffffffffu, ar[l], 8);  ai[l] += __shfl_down_sync(0xffffffffu, ai[l], 8);
+                }
+                if (lane < 8) {                                 // rows (lag, re|im) of 9 floats, every lag of the burst
+#pragma unroll
+                    for (int l = 0; l < SLPW; ++l) {
+                        part_f[(2 * (l0 + l)) * 9 + lane] = ar[l];
+                        part_f[(2 * (l0 + l) + 1) * 9 + lane] = ai[l];
                     }
                 }
             }
@@ -2341,7 +2321,11 @@ __global__ void __maxnreg__(MAXR) sch_corr_kernel(WinSrc src, const StreamCtl *_
         }
         if (threadIdx.x == 0) atomicAdd(stats, 1u);
         __syncthreads();
-        sch_corr_tiled_fp64(wp, tp, part, corr, corr_i, n_lag, n_smp);
+        // corr / corr_i reach the helper as opaque shared addresses: as its only caller this kernel would otherwise have them folded into
+        // the helper, and then ptxas spills 8 bytes here at 64 registers
+        unsigned a_c = (unsigned)__cvta_generic_to_shared(corr), a_ci = (unsigned)__cvta_generic_to_shared(corr_i);
+        asm("" : "+r"(a_c), "+r"(a_ci));
+        sch_corr_tiled_fp64(wp, tp, part, (double *)__cvta_shared_to_generic(a_c), (double *)__cvta_shared_to_generic(a_ci), n_lag, n_smp);
     } else {
         for (int lag = w; lag < n_lag; lag += nw) {              // generic shapes: one warp per lag
             double ar = 0.0, ai = 0.0;

@@ -117,18 +117,28 @@ def test_demod_family_sentinels_and_loud_failure(built_lib):
         assert e.value.code == -2
 
 
-def test_every_debug_set_key_is_documented_in_the_header():
-    """gsmcal_debug_set's keys are the tuning surface the profiles/ scripts use: each key the library accepts must be described in the
-    comment above its declaration (include/gsmcal.h)."""
+def test_debug_set_accepts_exactly_the_documented_keys():
+    """gsmcal_debug_set's keys are the tuning surface the profiles/ scripts use: the library accepts exactly the keys listed here, and each
+    must be described in the comment above its declaration (include/gsmcal.h)."""
     import re
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     src = open(os.path.join(root, "multi-rtl-sdr-calibration_b200", "csrc", "gsmcal_api.cu")).read()
     body = src[src.index("int gsmcal_debug_set(int key, int value)"):]
     body = body[:body.index("\n}\n")]
     keys = sorted({int(k) for k in re.findall(r"key == (\d+)", body)})
-    assert len(keys) >= 20
+    assert keys == [0, 3, 4, 5, 6, 8, 9, 10, 11, 12, 13, 14, 17, 18, 24]
     hdr = open(os.path.join(root, "include", "gsmcal.h")).read()
     doc = hdr[hdr.index("test / tuning hooks"):hdr.index("int gsmcal_debug_set")]
     documented = {int(k) for k in re.findall(r"(?:key |; |, |\* )(\d+)(?:,| =)", doc)}
     missing = [k for k in keys if k not in documented]
     assert not missing, f"debug keys without a line in include/gsmcal.h: {missing}"
+
+
+def test_debug_set_rejects_removed_and_unknown_keys(built_lib):
+    """Keys of the removed overlap experiments (7, 15, 16, 19, 21, 22, 23) and keys that never existed are argument errors; no device
+    is needed to reject them."""
+    from gsmcal import _lib
+    lib = _lib.lib()
+    for key in (7, 15, 16, 19, 21, 22, 23, 99):
+        assert lib.gsmcal_debug_set(key, 1) == -1, key
+        assert "unknown key" in lib.gsmcal_last_error().decode()

@@ -717,13 +717,11 @@ def test_submit_collect_matches_synchronous_call(gpu, captures, coef47, tpl):
     assert [x["pos_info"].tolist() for x in again] == [y["pos_info"].tolist() for y in ref_b]
 
 
-@pytest.mark.parametrize("gate,stages,blocks,sch56,chain", [(1, 7, 1, 1, 0), (1, 2, 3, 0, 0), (1, 24, 1, 1, 0), (0, 0, 1, 0, 0), (1, 0, 1, 0, 0),
-                                                            (0, 3, 2, 0, 0), (1, 2, 3, 0, 1), (1, 2, 3, 0, 2)])
-def test_submit_collect_trickle_column_sums_and_staggered_batches(gpu, captures, coef47, tpl, gate, stages, blocks, sch56, chain):
-    """debug keys 16-19: column sums by the TMA-ring kernel (ragged stream starts: 2*N_RAG is not a multiple of 16) or by plain launches,
-    FP64 stages gated behind the previous batch or in lockstep, SCH kernel at 56 registers - same records as the synchronous call,
-    bit for bit.  (The default is gate on, 2 stages x 3 blocks per SM.)  chain 1 / 2: the burst chains of the stream groups serialised (key 21) /
-    on normal-priority streams (key 22)."""
+@pytest.mark.parametrize("stages,blocks", [(7, 1), (2, 3), (24, 1), (3, 2), (1, 1)])
+def test_submit_collect_trickle_column_sums_and_staggered_batches(gpu, captures, coef47, tpl, stages, blocks):
+    """debug keys 17-18: column sums by the TMA-ring kernel at several ring sizes (ragged stream starts: 2*N_RAG is not a multiple of 16),
+    FP64 stages gated behind the previous batch - same records as the synchronous call, bit for bit.  (The default is 2 stages x 3
+    blocks per SM.)"""
     import torch
     from gsmcal._lib import lib
     _, raw = captures
@@ -734,8 +732,8 @@ def test_submit_collect_trickle_column_sums_and_staggered_batches(gpu, captures,
     st = torch.cuda.current_stream().cuda_stream
     ref_a = gpu.calibrate_batch(None, CARRIER, tpl, coef47, device_ptr=a.data_ptr(), n_iq=N_RAG, n_streams=3, cuda_stream=st)
     ref_b = gpu.calibrate_batch(None, CARRIER, tpl, coef47, device_ptr=b.data_ptr(), n_iq=N_RAG, n_streams=5, cuda_stream=st)
-    for key, val in ((16, gate), (17, stages), (18, blocks), (19, sch56), (21, int(chain == 1)), (22, int(chain == 2))):
-        lib().gsmcal_debug_set(key, val)
+    for key, val in ((17, stages), (18, blocks)):
+        assert lib().gsmcal_debug_set(key, val) == 0
     try:
         pend = [gpu.calibrate_batch_submit(0, a.data_ptr(), N_RAG, 3, CARRIER, tpl, coef47, cuda_stream=st, details=True),
                 gpu.calibrate_batch_submit(1, b.data_ptr(), N_RAG, 5, CARRIER, tpl, coef47, cuda_stream=st, details=True)]
@@ -743,7 +741,7 @@ def test_submit_collect_trickle_column_sums_and_staggered_batches(gpu, captures,
         pend.append(gpu.calibrate_batch_submit(0, b.data_ptr(), N_RAG, 5, CARRIER, tpl, coef47, cuda_stream=st, details=True))
         got += [pend[1].collect(), pend[2].collect()]
     finally:
-        for key, val in ((16, 1), (17, 2), (18, 3), (19, 0), (21, 0), (22, 0)):       # the library defaults
+        for key, val in ((17, 2), (18, 3)):                                       # the library defaults
             lib().gsmcal_debug_set(key, val)
     for g, ref in zip(got, (ref_a, ref_b, ref_b)):
         assert len(g) == len(ref)

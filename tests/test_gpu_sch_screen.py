@@ -2,8 +2,7 @@
 bound eps of DESIGN.md section 4, and the few that can are evaluated in fp64 in the tiled correlation's operation order.
 CPU: a NumPy emulation of the screen in the kernel's order on random and adversarial windows, |screen - fp64| <= eps for every lag.
 GPU: the screen (debug key 24 = 0) against the fp64 correlation of every lag (= 1) and the forced fallback (= 2): identical outputs on
-the captures, on the Appendix-A SCH paths, on a noise-only stream, on a planted near-tie, through the drop-in and in the 56-register
-build (debug key 19)."""
+the captures, on the Appendix-A SCH paths, on a noise-only stream, on a planted near-tie and through the drop-in."""
 import math
 import os
 import re
@@ -186,14 +185,9 @@ def test_debug_key_24_rejects_other_values(gpu):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("sch56", [0, 1])
-def test_batch_identical_across_modes(gpu, captures, coef47, tpl, sch56):
+def test_batch_identical_across_modes(gpu, captures, coef47, tpl):
     _, raw = captures
-    _lib().gsmcal_debug_set(19, sch56)
-    try:
-        out, stats = _run_modes(lambda: gpu.calibrate_batch(raw, CARRIER, tpl, coef47))
-    finally:
-        _lib().gsmcal_debug_set(19, 0)
+    out, stats = _run_modes(lambda: gpu.calibrate_batch(raw, CARRIER, tpl, coef47))
     _same_batch(out[0], out[1])
     _same_batch(out[0], out[2])
     assert stats[0]["screened"] > 0 and stats[0]["screened"] == sum(stats[0]["hist"])
