@@ -502,6 +502,52 @@ int check_fir_args(const double *coef, int n_taps, const void *s, i64 n, i64 n_c
     return GSMCAL_OK;
 }
 
+// ---- what the drop-in entry points share (they run on stream 0; fcch_scan passes the caller's stream) ---------------------------
+// They touch the device, so every entry point calls them after its host-decided sentinels and argument errors.
+// one complex128 stream: the device's context, s (n samples) on the device and a one-stream workspace of cap bursts
+int upload_s(const double *s, i64 n, int cap, i64 snr_len, int tpl_len, cudaStream_t st, Ctx **c, const double2 **din, Work *w) {
+    TRY(get_ctx(c));
+    void *p; TRY((*c)->in.get(sizeof(double2) * (size_t)n, &p));
+    TRY(make_work((*c)->work, 1, cap, snr_len, tpl_len, w));
+    TRY(copy_h2d((*c)->ring, g_device, p, s, sizeof(double2) * (size_t)n, st));
+    *din = (const double2 *)p;
+    return GSMCAL_OK;
+}
+// n_col columns of n_iq uint8 I/Q pairs as the kernels read them: a workspace of n_col streams x cap bursts, the FIR taps when coef is
+// given, a device copy of a host capture, and the column sums behind zeroed control blocks
+int u8_input(Ctx &c, const uint8_t *a, int mem, i64 n_iq, i64 n_col, int cap, i64 snr_len, const double *coef, int n_taps, cudaStream_t st,
+             const uint8_t **draw, Work *w) {
+    const size_t bytes = (size_t)2 * n_iq * n_col;
+    void *p = (void *)a;
+    if (mem == GSMCAL_MEM_HOST) TRY(c.in.get(bytes, &p));
+    TRY(make_work(c.work, n_col, cap, snr_len, 0, w));
+    if (coef) TRY(set_taps(coef, n_taps, st));
+    if (mem == GSMCAL_MEM_HOST) TRY(copy_h2d(c.ring, g_device, p, a, bytes, st));
+    CU(cudaMemsetAsync(w->ctl, 0, sizeof(StreamCtl) * n_col, st));
+    *draw = (const uint8_t *)p;
+    return run_colsum_u8(*draw, n_iq, n_col, w->ctl, st);
+}
+unsigned raw2iq_grid(i64 n_iq) { i64 gx = (n_iq + 256 * 8 - 1) / (256 * 8); if (gx > 148 * 16) gx = 148 * 16; return (unsigned)gx; }
+// one stream's control block to / from the host, complete on return
+int put_ctl(StreamCtl *dev, const StreamCtl &h, cudaStream_t st) {
+    CU(cudaMemcpyAsync(dev, &h, sizeof h, cudaMemcpyHostToDevice, st));
+    CU(cudaStreamSynchronize(st));
+    return GSMCAL_OK;
+}
+int get_ctl(const StreamCtl *dev, StreamCtl *h, cudaStream_t st) {
+    CU(cudaMemcpyAsync(h, dev, sizeof *h, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return GSMCAL_OK;
+}
+// r (len samples) of a correction drop-in: s (n samples, din on the device) resampled by (1+e) and / or derotated by dphi, or s itself
+int return_r(Ctx &c, const double *s, const double2 *din, i64 n, i64 len, double e, int do_interp, double dphi, int do_derot, double *r,
+             cudaStream_t st) {
+    if (!do_interp && !do_derot) { memcpy(r, s, sizeof(double2) * (size_t)len); return GSMCAL_OK; }
+    void *dout; TRY(c.out.get(sizeof(double2) * (size_t)len, &dout));
+    TRY(run_resample_derotate(din, n, e, do_interp, dphi, do_derot, (double2 *)dout, len, st));
+    return copy_d2h(c.ring, g_device, r, dout, sizeof(double2) * (size_t)len, st);
+}
+
 void gmsk_template(int osr, double *out);
 size_t fcch_demod_smem(int osr);
 size_t sch_demod_smem(int osr);
@@ -527,7 +573,8 @@ DemodDev sub_demod(const DemodDev &a, i64 d0, int cap) {
     return s;
 }
 // workspace, branch table, training bits and fft(template) (SCH_demod.m:47-59), and with nts (host, (26*osr) x 8 complex) the normal
-// training sequences and the BCCH records behind them; once per call on `st` before the stream groups fork
+// training sequences and the BCCH records behind them; once per call on `st` before the stream groups fork (gsmcal_SCH_demod: one
+// stream of its H bursts)
 int demod_setup(Ctx &c, i64 D, int cap, int osr, const double2 *tpl_dev, const double *nts, std::vector<double> &W, signed char *data_pm, cudaStream_t st,
                 DemodDev *dd) {
     const int N = SD_NSYM * osr;
@@ -755,15 +802,10 @@ int gsmcal_raw2iq_u8(const uint8_t *a, int64_t n_iq, int64_t n_col, double *b) {
     if (n_iq == 0) return GSMCAL_OK;
     Ctx *c; TRY(get_ctx(&c));
     cudaStream_t st = 0;
-    void *din, *dout; Work w;
-    TRY(c->in.get((size_t)2 * n_iq * n_col, &din));
+    const uint8_t *din; void *dout; Work w;
     TRY(c->out.get(sizeof(double2) * (size_t)n_iq * n_col, &dout));
-    TRY(make_work(c->work, n_col, 1, 1, 0, &w));
-    TRY(copy_h2d(c->ring, g_device, din, a, (size_t)2 * n_iq * n_col, st));
-    CU(cudaMemsetAsync(w.ctl, 0, sizeof(StreamCtl) * n_col, st));
-    TRY(run_colsum_u8((const uint8_t *)din, n_iq, n_col, w.ctl, st));
-    i64 gx = (n_iq + 256 * 8 - 1) / (256 * 8); if (gx > 148 * 16) gx = 148 * 16; if (gx < 1) gx = 1;
-    LAUNCH(raw2iq_store_kernel, dim3((unsigned)gx, (unsigned)n_col), 256, 0, st, (const uint8_t *)din, n_iq, w.ctl, (double2 *)dout);
+    TRY(u8_input(*c, a, GSMCAL_MEM_HOST, n_iq, n_col, 1, 1, nullptr, 0, st, &din, &w));
+    LAUNCH(raw2iq_store_kernel, dim3(raw2iq_grid(n_iq), (unsigned)n_col), 256, 0, st, din, n_iq, w.ctl, (double2 *)dout);
     TRY(copy_d2h(c->ring, g_device, b, dout, sizeof(double2) * (size_t)n_iq * n_col, st));
     return GSMCAL_OK;
 }
@@ -783,9 +825,9 @@ int gsmcal_raw2iq_f64(const double *a, int64_t n_iq, int64_t n_col, double *b) {
     TRY(make_work(c->work, n_col, 1, 1, 0, &w));
     TRY(copy_h2d(c->ring, g_device, din, a, sizeof(double) * (size_t)2 * n_iq * n_col, st));
     CU(cudaMemsetAsync(w.ctl, 0, sizeof(StreamCtl) * n_col, st));
-    i64 gx = (n_iq + 256 * 8 - 1) / (256 * 8); if (gx > 148 * 16) gx = 148 * 16; if (gx < 1) gx = 1;
-    LAUNCH(colsum_f64_kernel, dim3((unsigned)gx, (unsigned)n_col), 256, 0, st, (const double *)din, n_iq, w.ctl);
-    LAUNCH(raw2iq_store_f64_kernel, dim3((unsigned)gx, (unsigned)n_col), 256, 0, st, (const double *)din, n_iq, w.ctl, (double2 *)dout);
+    const dim3 grid(raw2iq_grid(n_iq), (unsigned)n_col);
+    LAUNCH(colsum_f64_kernel, grid, 256, 0, st, (const double *)din, n_iq, w.ctl);
+    LAUNCH(raw2iq_store_f64_kernel, grid, 256, 0, st, (const double *)din, n_iq, w.ctl, (double2 *)dout);
     TRY(copy_d2h(c->ring, g_device, b, dout, sizeof(double2) * (size_t)n_iq * n_col, st));
     return GSMCAL_OK;
 }
@@ -833,14 +875,9 @@ int gsmcal_raw2iq_fir_u8(const uint8_t *a, int64_t n_iq, int64_t n_col, const do
     Ctx *c; TRY(get_ctx(&c));
     cudaStream_t st = 0;
     const i64 n_out = (n_iq + decim - 1) / decim;
-    void *din, *dout; Work w;
-    TRY(c->in.get((size_t)2 * n_iq * n_col, &din));
+    const uint8_t *din; void *dout; Work w;
     TRY(c->out.get(sizeof(double2) * (size_t)n_out * n_col, &dout));
-    TRY(make_work(c->work, n_col, 1, 1, 0, &w));
-    TRY(set_taps(coef, n_taps, st));
-    TRY(copy_h2d(c->ring, g_device, din, a, (size_t)2 * n_iq * n_col, st));
-    CU(cudaMemsetAsync(w.ctl, 0, sizeof(StreamCtl) * n_col, st));
-    TRY(run_colsum_u8((const uint8_t *)din, n_iq, n_col, w.ctl, st));
+    TRY(u8_input(*c, a, GSMCAL_MEM_HOST, n_iq, n_col, 1, 1, coef, n_taps, st, &din, &w));
     TRY(run_fir<true>(din, n_iq, 2 * n_iq, w.ctl, n_taps, decim, n_col, (double2 *)dout, n_out, nullptr, st));
     TRY(copy_d2h(c->ring, g_device, r, dout, sizeof(double2) * (size_t)n_out * n_col, st));
     return GSMCAL_OK;
@@ -860,20 +897,15 @@ int gsmcal_band_power_u8(const uint8_t *a, int64_t n_iq, int64_t n_col, const do
     if (!a || !power || n_iq < 1 || n_col < 1 || decim < 1) return fail(GSMCAL_ERR_ARG, "band_power: bad arguments");
     Ctx *c; TRY(get_ctx(&c));
     cudaStream_t st = 0;
-    void *din; Work w;
-    TRY(c->in.get((size_t)2 * n_iq * n_col, &din));
-    TRY(make_work(c->work, n_col, 1, 1, 0, &w));
-    if (coef) TRY(set_taps(coef, n_taps, st));
-    TRY(copy_h2d(c->ring, g_device, din, a, (size_t)2 * n_iq * n_col, st));
-    CU(cudaMemsetAsync(w.ctl, 0, sizeof(StreamCtl) * n_col, st));
+    const uint8_t *din; Work w;
+    TRY(u8_input(*c, a, GSMCAL_MEM_HOST, n_iq, n_col, 1, 1, coef, n_taps, st, &din, &w));
     CU(cudaMemsetAsync(w.power, 0, sizeof(double) * n_col, st));
-    TRY(run_colsum_u8((const uint8_t *)din, n_iq, n_col, w.ctl, st));
     const i64 n_out = (n_iq + decim - 1) / decim;
     if (coef) {
         TRY(run_fir<true>(din, n_iq, 2 * n_iq, w.ctl, n_taps, decim, n_col, nullptr, n_out, w.power, st));
     } else {
         i64 gx = (n_out + 2047) / 2048; if (gx > 1024) gx = 1024;
-        LAUNCH(power_u8_kernel, dim3((unsigned)gx, (unsigned)n_col), 256, 0, st, (const uint8_t *)din, n_iq, w.ctl, decim, w.power);
+        LAUNCH(power_u8_kernel, dim3((unsigned)gx, (unsigned)n_col), 256, 0, st, din, n_iq, w.ctl, decim, w.power);
     }
     CU(cudaMemcpyAsync(power, w.power, sizeof(double) * n_col, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
@@ -889,14 +921,9 @@ int gsmcal_diversity_power_u8(const uint8_t *s_all, int64_t n_iq, int64_t n_freq
     const i64 n_col = n_freq * n_dongle;
     Ctx *c; TRY(get_ctx(&c));
     cudaStream_t st = 0;
-    void *din; Work w;
-    TRY(c->in.get((size_t)2 * n_iq * n_col, &din));
-    TRY(make_work(c->work, n_col, 3, 1, 0, &w));                  // cap 3: room for power | per-dongle spectrum | combination in the [D][cap] arrays
-    TRY(set_taps(coef, n_taps, st));
-    TRY(copy_h2d(c->ring, g_device, din, s_all, (size_t)2 * n_iq * n_col, st));
-    CU(cudaMemsetAsync(w.ctl, 0, sizeof(StreamCtl) * n_col, st));
+    const uint8_t *din; Work w;
+    TRY(u8_input(*c, s_all, GSMCAL_MEM_HOST, n_iq, n_col, 3, 1, coef, n_taps, st, &din, &w));   // cap 3: room for power | per-dongle spectrum | combination in the [D][cap] arrays
     CU(cudaMemsetAsync(w.power, 0, sizeof(double) * n_col, st));
-    TRY(run_colsum_u8((const uint8_t *)din, n_iq, n_col, w.ctl, st));
     const i64 n_out = (n_iq + decim - 1) / decim;
     TRY(run_fir<true>(din, n_iq, 2 * n_iq, w.ctl, n_taps, decim, n_col, nullptr, n_out, w.power, st));
     LAUNCH(diversity_combine_kernel, (unsigned)((n_freq + 127) / 128), 128, 0, st, w.power, n_out, (int)n_freq, (int)n_dongle, w.fo, w.gate);
@@ -909,18 +936,14 @@ int gsmcal_diversity_power_u8(const uint8_t *s_all, int64_t n_iq, int64_t n_freq
 // ---------------------------------------------------------------------------------------------------
 static int snr_windows(const double *s, int64_t len, int fft_len, i64 w0, i64 n_win, Ctx **cout, Work *w, cudaStream_t st) {
     if (!s || len < 1 || fft_len < 1 || fft_len > 128) return fail(GSMCAL_ERR_ARG, "moving fft: bad arguments (fft_len <= 128)");
-    Ctx *c; TRY(get_ctx(&c));
-    void *din;
-    TRY(c->in.get(sizeof(double2) * (size_t)len, &din));
-    TRY(make_work(c->work, 1, 1, n_win > 0 ? n_win : 1, 0, w));
-    TRY(copy_h2d(c->ring, g_device, din, s, sizeof(double2) * (size_t)len, st));
+    const double2 *din;
+    TRY(upload_s(s, len, 1, n_win > 0 ? n_win : 1, 0, st, cout, &din, w));
     CU(cudaMemsetAsync(w->ctl, 0, sizeof(StreamCtl), st));
     if (n_win > 0) {
-        WinSrc src = mat_src((const double2 *)din, len, len, 0);
         size_t smem = sizeof(double2) * (fft_len + SNR_THREADS + fft_len);
-        LAUNCH(snr_map_kernel, dim3((unsigned)((n_win + SNR_THREADS - 1) / SNR_THREADS), 1), SNR_THREADS, smem, st, src, w->ctl, w0, n_win, fft_len, w->snr_map, w->snr_stride);
+        LAUNCH(snr_map_kernel, dim3((unsigned)((n_win + SNR_THREADS - 1) / SNR_THREADS), 1), SNR_THREADS, smem, st, mat_src(din, len, len, 0), w->ctl, w0, n_win, fft_len,
+               w->snr_map, w->snr_stride);
     }
-    *cout = c;
     return GSMCAL_OK;
 }
 
@@ -934,8 +957,7 @@ int gsmcal_move_fft_snr_runtime_avg(const double *s, int64_t len, int mv_len, in
     StreamCtl h; memset(&h, 0, sizeof h); h.first_hit = -1;
     if (n_win > 0) {
         LAUNCH(first_hit_scan_kernel, 1, 32, 0, st, w.snr_map, w.snr_stride, n_win, mv_len, th, w.ctl, 1);
-        CU(cudaMemcpyAsync(&h, w.ctl, sizeof h, cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
+        TRY(get_ctl(w.ctl, &h, st));
     }
     if (h.first_hit > 0) { *hit_flag = 1; *hit_idx = h.first_hit; *hit_avg_snr = h.hit_avg_snr; *hit_snr = h.hit_snr; }
     else { *hit_flag = 0; *hit_idx = -1; *hit_avg_snr = INFINITY; *hit_snr = INFINITY; }
@@ -979,16 +1001,11 @@ int gsmcal_FCCH_coarse_position(const double *s, int64_t len, int decimation_rat
     CoarseParams p; TRY(coarse_params(decimation_ratio, &p));
     if (p.n_first > len) return fail(GSMCAL_ERR_RANGE, "FCCH_coarse_position: stream shorter than 23 frames (s(1:%lld) would raise an index error)", (long long)p.n_first);
     const int cap = (int)gsmcal_max_bursts(len, decimation_ratio);
-    Ctx *c; TRY(get_ctx(&c));
-    cudaStream_t st = 0; void *din; Work w;
-    TRY(c->in.get(sizeof(double2) * (size_t)len, &din));
-    TRY(make_work(c->work, 1, cap, p.n_first, 0, &w));
-    TRY(copy_h2d(c->ring, g_device, din, s, sizeof(double2) * (size_t)len, st));
+    cudaStream_t st = 0; Ctx *c; const double2 *din; Work w;
+    TRY(upload_s(s, len, cap, p.n_first, 0, st, &c, &din, &w));
     CU(cudaMemsetAsync(w.ctl, 0, sizeof(StreamCtl), st));
-    TRY(run_coarse(mat_src((const double2 *)din, len, len, 0), len, p, 1, cap, w, st));
-    StreamCtl h;
-    CU(cudaMemcpyAsync(&h, w.ctl, sizeof h, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
+    TRY(run_coarse(mat_src(din, len, len, 0), len, p, 1, cap, w, st));
+    StreamCtl h; TRY(get_ctl(w.ctl, &h, st));
     if (h.n_coarse < 0) { *n_out = -1; return GSMCAL_OK; }
     if (h.n_coarse > cap_out) return fail(GSMCAL_ERR_CAPACITY, "FCCH_coarse_position: %d hits, capacity %lld", h.n_coarse, (long long)cap_out);
     CU(cudaMemcpy(position, w.coarse_pos, sizeof(double) * h.n_coarse, cudaMemcpyDeviceToHost));
@@ -1012,19 +1029,14 @@ int gsmcal_FCCH_fine_correction(const double *s, int64_t n, const double *base_p
         if (p + 64 > (double)(len_s - 148 + 1)) break;
         if (p != floor(p) || p - 64 < 1) return fail(GSMCAL_ERR_RANGE, "FCCH_fine_correction: base_position(%lld)=%g puts the search window before the first sample", (long long)i + 1, p);
     }
-    Ctx *c; TRY(get_ctx(&c));
-    cudaStream_t st = 0; void *din; Work w;
     const int cap = (int)n_base;
-    TRY(c->in.get(sizeof(double2) * (size_t)n, &din));
-    TRY(make_work(c->work, 1, cap, 1, 0, &w));
-    TRY(copy_h2d(c->ring, g_device, din, s, sizeof(double2) * (size_t)n, st));
-    StreamCtl h; memset(&h, 0, sizeof h); h.n_coarse = cap;
-    CU(cudaMemcpyAsync(w.ctl, &h, sizeof h, cudaMemcpyHostToDevice, st));
+    cudaStream_t st = 0; Ctx *c; const double2 *din; Work w;
+    TRY(upload_s(s, n, cap, 1, 0, st, &c, &din, &w));
     CU(cudaMemcpyAsync(w.coarse_pos, base_position, sizeof(double) * cap, cudaMemcpyHostToDevice, st));
-    CU(cudaStreamSynchronize(st));
-    TRY(run_fine(*c, mat_src((const double2 *)din, n, n, 0), mat_src((const double2 *)din, n, n, 1), n, osr, carrier_freq, 1, cap, w, st));
-    CU(cudaMemcpyAsync(&h, w.ctl, sizeof h, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
+    StreamCtl h; memset(&h, 0, sizeof h); h.n_coarse = cap;
+    TRY(put_ctl(w.ctl, h, st));
+    TRY(run_fine(*c, mat_src(din, n, n, 0), mat_src(din, n, n, 1), n, osr, carrier_freq, 1, cap, w, st));
+    TRY(get_ctl(w.ctl, &h, st));
     *sampling_ppm = h.sppm1; *carrier_ppm = h.cppm1; *n_pos = h.n_fcch;
     if (h.n_fcch > 0) {
         if (h.n_fcch > pos_cap) return fail(GSMCAL_ERR_CAPACITY, "FCCH_fine_correction: FCCH_pos capacity");
@@ -1033,12 +1045,7 @@ int gsmcal_FCCH_fine_correction(const double *s, int64_t n, const double *base_p
     *r_len = h.len1;
     if (h.len1 >= 0) {
         if (!r || h.len1 > r_cap) return fail(GSMCAL_ERR_CAPACITY, "FCCH_fine_correction: r capacity %lld < %lld", (long long)r_cap, (long long)h.len1);
-        if (!h.interp1_on && !h.derot1_on) memcpy(r, s, sizeof(double2) * (size_t)h.len1);     // r = s (:72)
-        else {
-            void *dout; TRY(c->out.get(sizeof(double2) * (size_t)h.len1, &dout));
-            TRY(run_resample_derotate((const double2 *)din, n, h.e1, h.interp1_on, h.dphi1, h.derot1_on, (double2 *)dout, h.len1, st));
-            TRY(copy_d2h(c->ring, g_device, r, dout, sizeof(double2) * (size_t)h.len1, st));
-        }
+        TRY(return_r(*c, s, din, n, h.len1, h.e1, h.interp1_on, h.dphi1, h.derot1_on, r, st));     // r = s when neither is on (:72)
     }
     return GSMCAL_OK;
 }
@@ -1060,11 +1067,8 @@ int gsmcal_SCH_corr_rate_correction(const double *s, int64_t n, const double *FC
     const int L = 64 * osr;
     for (int i = 0; i < cap; ++i) if (FCCH_pos[i] != floor(FCCH_pos[i]) || FCCH_pos[i] + (625 * osr / 4) * 8 + 42 * osr - 8 * osr < 1)
         return fail(GSMCAL_ERR_RANGE, "SCH_corr_rate_correction: FCCH_pos(%d) puts the search window before the first sample", i + 1);
-    Ctx *c; TRY(get_ctx(&c));
-    cudaStream_t st = 0; void *din; Work w;
-    TRY(c->in.get(sizeof(double2) * (size_t)n, &din));
-    TRY(make_work(c->work, 1, cap, 1, L, &w));
-    TRY(copy_h2d(c->ring, g_device, din, s, sizeof(double2) * (size_t)n, st));
+    cudaStream_t st = 0; Ctx *c; const double2 *din; Work w;
+    TRY(upload_s(s, n, cap, 1, L, st, &c, &din, &w));
     std::vector<unsigned char> tpk(tpl_pack_bytes(L));
     tpl_pack(tpl, L, tpk.data());
     CU(cudaMemcpyAsync((void *)w.tpl, tpk.data(), tpk.size(), cudaMemcpyHostToDevice, st));
@@ -1072,11 +1076,9 @@ int gsmcal_SCH_corr_rate_correction(const double *s, int64_t n, const double *FC
     CU(cudaMemsetAsync(w.sch_stats, 0, sizeof(unsigned) * SCH_NSTAT, st));
     CU(cudaMemcpyAsync(w.fcch_pos, FCCH_pos, sizeof(double) * cap, cudaMemcpyHostToDevice, st));
     StreamCtl h; memset(&h, 0, sizeof h); h.n_fcch = cap; h.sch_enable = 1; h.len1 = n;
-    CU(cudaMemcpyAsync(w.ctl, &h, sizeof h, cudaMemcpyHostToDevice, st));
-    CU(cudaStreamSynchronize(st));
-    TRY(run_sch(mat_src((const double2 *)din, n, n, 0), osr, 1, cap, w, st));
-    CU(cudaMemcpyAsync(&h, w.ctl, sizeof h, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
+    TRY(put_ctl(w.ctl, h, st));
+    TRY(run_sch(mat_src(din, n, n, 0), osr, 1, cap, w, st));
+    TRY(get_ctl(w.ctl, &h, st));
     *sampling_ppm = h.sppm2; *n_rows = h.n_pos_info;
     if (h.n_pos_info > 0) {
         if (h.n_pos_info > rows_cap) return fail(GSMCAL_ERR_CAPACITY, "SCH_corr_rate_correction: pos_info capacity %lld < %d", (long long)rows_cap, h.n_pos_info);
@@ -1087,12 +1089,7 @@ int gsmcal_SCH_corr_rate_correction(const double *s, int64_t n, const double *FC
     *r_len = h.len2;
     if (h.len2 >= 0) {
         if (!r || h.len2 > r_cap) return fail(GSMCAL_ERR_CAPACITY, "SCH_corr_rate_correction: r capacity");
-        if (!h.interp2_on) memcpy(r, s, sizeof(double2) * (size_t)h.len2);                    // r = s (:87,:120)
-        else {
-            void *dout; TRY(c->out.get(sizeof(double2) * (size_t)h.len2, &dout));
-            TRY(run_resample_derotate((const double2 *)din, n, h.e2, 1, 0.0, 0, (double2 *)dout, h.len2, st));
-            TRY(copy_d2h(c->ring, g_device, r, dout, sizeof(double2) * (size_t)h.len2, st));
-        }
+        TRY(return_r(*c, s, din, n, h.len2, h.e2, h.interp2_on, 0.0, 0, r, st));                // r = s without resampling (:87,:120)
     }
     return GSMCAL_OK;
 }
@@ -1117,24 +1114,17 @@ int gsmcal_carrier_correct_post_SCH(const double *s, int64_t n, const double *po
     for (double p : fpos) if (p != floor(p) || p < 1 || p + N - 1 > (double)n) return fail(GSMCAL_ERR_RANGE, "carrier_correct_post_SCH: FCCH window outside the stream");
     if (fpos.empty()) return fail(GSMCAL_ERR_RANGE, "carrier_correct_post_SCH: no FCCH rows (mean of empty is NaN in the reference)");
     if (!r || n > r_cap) return fail(GSMCAL_ERR_CAPACITY, "carrier_correct_post_SCH: r capacity");
-    Ctx *c; TRY(get_ctx(&c));
-    cudaStream_t st = 0; void *din, *dout; Work w;
     const int cap = (int)fpos.size();
-    TRY(c->in.get(sizeof(double2) * (size_t)n, &din));
-    TRY(c->out.get(sizeof(double2) * (size_t)n, &dout));
-    TRY(make_work(c->work, 1, cap, 1, 0, &w));
-    TRY(copy_h2d(c->ring, g_device, din, s, sizeof(double2) * (size_t)n, st));
+    cudaStream_t st = 0; Ctx *c; const double2 *din; Work w;
+    TRY(upload_s(s, n, cap, 1, 0, st, &c, &din, &w));
     CU(cudaMemcpyAsync(w.post_pos, fpos.data(), sizeof(double) * cap, cudaMemcpyHostToDevice, st));
     StreamCtl h; memset(&h, 0, sizeof h); h.post_enable = 1; h.n_post_fcch = cap; h.len2 = n;
     h.sppm1 = h.sppm2 = h.cppm1 = INFINITY;
-    CU(cudaMemcpyAsync(w.ctl, &h, sizeof h, cudaMemcpyHostToDevice, st));
-    CU(cudaStreamSynchronize(st));
-    TRY(run_post(*c, mat_src((const double2 *)din, n, n, 0), osr, carrier_freq, 1, cap, w, false, st));
-    CU(cudaMemcpyAsync(&h, w.ctl, sizeof h, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
+    TRY(put_ctl(w.ctl, h, st));
+    TRY(run_post(*c, mat_src(din, n, n, 0), osr, carrier_freq, 1, cap, w, false, st));
+    TRY(get_ctl(w.ctl, &h, st));
     *carrier_ppm = h.cppm2;
-    TRY(run_resample_derotate((const double2 *)din, n, 0.0, 0, h.dphi2, 1, (double2 *)dout, n, st));
-    TRY(copy_d2h(c->ring, g_device, r, dout, sizeof(double2) * (size_t)n, st));
+    TRY(return_r(*c, s, din, n, n, 0.0, 0, h.dphi2, 1, r, st));
     *r_len = n;
     return GSMCAL_OK;
 }
@@ -1472,17 +1462,8 @@ int gsmcal_fcch_scan(const uint8_t *raw, int raw_mem, int64_t n_iq, int64_t n_ch
     const int cap = (int)gsmcal_max_bursts(len_dec, coarse_dr);
     Ctx *c; TRY(get_ctx(&c));
     cudaStream_t st = (cudaStream_t)cuda_stream;
-    Work w;
-    TRY(make_work(c->work, n_chan, cap, p.n_first, 0, &w));
-    TRY(set_taps(coef, n_taps, st));
-    const uint8_t *draw = raw;
-    if (raw_mem == GSMCAL_MEM_HOST) {
-        void *din; TRY(c->in.get((size_t)2 * n_iq * n_chan, &din));
-        TRY(copy_h2d(c->ring, g_device, din, raw, (size_t)2 * n_iq * n_chan, st));
-        draw = (const uint8_t *)din;
-    }
-    CU(cudaMemsetAsync(w.ctl, 0, sizeof(StreamCtl) * n_chan, st));
-    TRY(run_colsum_u8(draw, n_iq, n_chan, w.ctl, st));
+    const uint8_t *draw; Work w;
+    TRY(u8_input(*c, raw, raw_mem, n_iq, n_chan, cap, p.n_first, coef, n_taps, st, &draw, &w));
     LAUNCH(mean_kernel, (unsigned)((n_chan + 127) / 128), 128, 0, st, w.ctl, (int)n_chan, n_iq);
     TRY(run_coarse(lazy_src(draw, n_iq, n_taps, 0, dec), len_dec, p, n_chan, cap, w, st));
     LAUNCH(scan_accept_kernel, (unsigned)((n_chan + 63) / 64), 64, 0, st, w.ctl, (int)n_chan, cap, w.coarse_pos, w.coarse_snr, w.fo, w.gate);
@@ -1524,17 +1505,15 @@ int gsmcal_stage_launch(int stage, const void *in, void *out, int64_t n_iq, int6
     std::lock_guard<std::mutex> lk(g_mu);
     Ctx *c; TRY(get_ctx(&c));
     cudaStream_t st = (cudaStream_t)cuda_stream;
-    static Work w; static i64 w_cols = 0;
-    if (stage == 0 || w_cols != n_col) { TRY(make_work(c->work, n_col, 1, 1, 0, &w)); w_cols = n_col; }
+    Work w; TRY(make_work(c->work, n_col, 1, 1, 0, &w));       // the control blocks of stage 0's column sums stay at offset 0
     if (coef) TRY(set_taps(coef, n_taps, st));
     switch (stage) {
     case 0:
         CU(cudaMemsetAsync(w.ctl, 0, sizeof(StreamCtl) * n_col, st));
         return run_colsum_u8((const uint8_t *)in, n_iq, n_col, w.ctl, st);
-    case 1: {
-        i64 gx = (n_iq + 256 * 8 - 1) / (256 * 8); if (gx > 148 * 16) gx = 148 * 16;
-        LAUNCH(raw2iq_store_kernel, dim3((unsigned)gx, (unsigned)n_col), 256, 0, st, (const uint8_t *)in, n_iq, w.ctl, (double2 *)out);
-        return GSMCAL_OK; }
+    case 1:
+        LAUNCH(raw2iq_store_kernel, dim3(raw2iq_grid(n_iq), (unsigned)n_col), 256, 0, st, (const uint8_t *)in, n_iq, w.ctl, (double2 *)out);
+        return GSMCAL_OK;
     case 2: return run_fir<false>(in, n_iq, n_iq, nullptr, n_taps, 1, n_col, (double2 *)out, n_iq, nullptr, st);
     case 3: return run_fir<true>(in, n_iq, 2 * n_iq, w.ctl, n_taps, 1, n_col, (double2 *)out, n_iq, nullptr, st);
     case 4: for (i64 d = 0; d < n_col; ++d) TRY(run_resample_derotate((const double2 *)in + d * n_iq, n_iq, -35e-6, 1, 0.0, 0, (double2 *)out + d * n_iq, n_iq, st)); return GSMCAL_OK;

@@ -72,6 +72,37 @@ def test_sentinels_need_no_device(built_lib):
     assert p[0].tolist() == [[-1.0, -1.0]] and p[1] is None and p[2] == math.inf
     c = gsmcal.carrier_correct_post_SCH(s, [[-1.0, -1.0]], 8, 957.4e6)
     assert c == (None, math.inf)
+    assert gsmcal.carrier_correct_post_SCH(s, [[10.0, 0.0]] + [[20.0 + k, 2.0] for k in range(3)], 8, 957.4e6) == (None, math.inf)   # < 4 BCCH rows
+    assert gsmcal.specific_fft_snr_fix_avg(s, (5, 4), 16, 10.0, 1.0) == (False, -1.0, math.inf)                                 # empty target set
+
+
+def test_host_decided_range_errors_need_no_device(built_lib):
+    """Every window the drop-ins can check on the host is checked before any device work: the reference's index errors come out as
+    GSMCAL_ERR_RANGE with the same text on a machine without a GPU (not as GSMCAL_ERR_CUDA), and launch nothing on one with a GPU."""
+    import gsmcal
+    s = np.zeros(20000, dtype=np.complex128)
+    tpl, nts = np.ones(512, complex), np.ones((208, 8), complex)
+    bcch = [[3000.0 + k * 1250, 2.0] for k in range(4)]
+    cases = [
+        ("base_position(1)=10 puts the search window before the first sample",
+         lambda: gsmcal.FCCH_fine_correction(np.zeros(80000, complex), [10.0, 2000.0, 3000.0, 4000.0, 5000.0], 8, 957.4e6)),
+        ("FCCH_pos(1) puts the search window before the first sample",
+         lambda: gsmcal.SCH_corr_rate_correction(s, [-20000.0, 1.0, 2.0, 3.0, 4.0], tpl, 8)),
+        ("carrier_correct_post_SCH: FCCH window outside the stream",
+         lambda: gsmcal.carrier_correct_post_SCH(s, [[19000.0, 0.0]] + bcch, 8, 957.4e6)),
+        ("FCCH_demod: no FCCH rows", lambda: gsmcal.FCCH_demod(s, bcch, 8, 957.4e6)),
+        ("SCH_demod: equaliser window of the SCH burst at 19900 outside the stream", lambda: gsmcal.SCH_demod(s, [[19900.0, 1.0]], tpl, 8)),
+        ("BCCH_demod: training window of BCCH burst 4 outside the stream",
+         lambda: gsmcal.BCCH_demod(s, [[1001.0, 0.0]] + bcch[:3] + [[19900.0, 2.0]], nts, 8, 957.4e6)),
+        ("specific_fft_snr_fix_avg: window outside the stream", lambda: gsmcal.specific_fft_snr_fix_avg(s, (0, 100), 64, 10.0, 1.0)),
+        ("FCCH_coarse_position: stream shorter than 23 frames", lambda: gsmcal.FCCH_coarse_position(s[:1000], 8)),
+    ]
+    launches = gsmcal.launch_count()
+    for text, call in cases:
+        with pytest.raises(gsmcal.GsmcalError) as e:
+            call()
+        assert e.value.code == -4 and text in str(e.value), str(e.value)
+    assert gsmcal.launch_count() == launches
 
 
 def test_compute_fails_loudly_without_a_gpu(built_lib):
