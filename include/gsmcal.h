@@ -289,6 +289,44 @@ int gsmcal_calibrate_demod_bcch_batch(const uint8_t *raw, int raw_mem, int64_t n
                                       const double *normal_training_sequence /* (26*osr) x 8 complex128, column-major */,
                                       gsmcal_bcch_result *bcch /* [n_streams], required */);
 
+/* gsmcal_calibrate_batch (every output as there, byte for byte) followed by sub-sample timing of every SCH burst and a least-squares
+ * line through the burst times: each dongle's sample clock measured from the burst positions themselves instead of the integer
+ * lattice of sampling_ppm, and the time of its bursts in its own capture.  Only oversampling_ratio 8.  For stream d, with
+ * e1 = sampling_ppm[0]*1e-6, e2 = sampling_ppm[1]*1e-6, r = r_correct (1-based, the samples gsmcal_calibrate_batch_r writes) and
+ * p_i the position of the i-th SCH row (type 1) of pos_info:
+ *   g_i = p_i + 42*8 (training start); c_i(l) = |sum_{n=0..511} conj(t_n) r(g_i+l+n)|^2 (fp64, abs then square) for l = -64..24
+ *   (the 89 lags of SCH_corr_rate_correction.m:36,45-48), l* = the first maximum;
+ *   GSMCAL_TIMING_RANGE: the 600-sample window leaves r, GSMCAL_TIMING_EDGE: l* is the first or last lag; both give tau_i = NaN;
+ *   delta = 0.5*(y- - y+)/(y- - 2*y0 + y+) of y = c_i(l*-1, l*, l*+1) (0 when the denominator is 0), tau_i = g_i + l* + delta;
+ *   x_i = ((tau_i - 1)*(1 + e2))*(1 + e1): tau_i in 0-based samples of the uint8 capture (r(j) sits at raw time (j-1)(1+e2)(1+e1));
+ *   over the n_fit rows with finite x_i, m_i = p_i - p_first: b = sum (m-mean m)(x-mean x) / sum (m-mean m)^2 (row order),
+ *   a = mean x - b*mean m, t0 = a, fit_ppm = (b - 1)*1e6, rms = sqrt(sum (x - a - b*m)^2 / n_fit); n_fit < 3: GSMCAL_TIMING_FEW, NaN.
+ * sch_tau, sch_x [n_streams][B] (B as above; NULL = not copied): tau_i and x_i by SCH row, NaN where excluded. */
+typedef struct gsmcal_sch_timing_result {
+    int32_t n_sch;        /* type-1 rows of pos_info; -1 when the step did not run (flags say why) */
+    int32_t n_fit;        /* rows with a finite tau */
+    int32_t flags;        /* GSMCAL_TIMING_* */
+    int32_t reserved;
+    double  t0;           /* fit intercept, raw-capture samples (0-based): the raw time of the first SCH row's training start */
+    double  fit_ppm;      /* (slope - 1) * 1e6 */
+    double  rms;          /* fit residual RMS, raw-capture samples */
+} gsmcal_sch_timing_result;   /* 40 bytes */
+
+#define GSMCAL_TIMING_NO_POS_INFO  1   /* pos_info == -1: nothing to time */
+#define GSMCAL_TIMING_NO_R_CORRECT 2   /* pos_info valid but results.r_len[2] == -1 */
+#define GSMCAL_TIMING_RANGE        4   /* some row's 600-sample correlation window leaves r_correct */
+#define GSMCAL_TIMING_EDGE         8   /* some row's maximum sits on the first or last lag */
+#define GSMCAL_TIMING_FEW         16   /* fewer than 3 rows with a finite tau: t0, fit_ppm, rms NaN */
+
+int gsmcal_calibrate_sch_timing_batch(const uint8_t *raw, int raw_mem, int64_t n_iq, int64_t n_streams,
+                                      double carrier_freq, const double *sch_training_sequence,
+                                      const double *coef, int n_taps, int oversampling_ratio, int coarse_decimation,
+                                      gsmcal_stream_result *results,
+                                      double *coarse_pos, double *coarse_snr, double *fcch_pos, double *pos_info,
+                                      void *cuda_stream,
+                                      gsmcal_sch_timing_result *timing /* [n_streams], required */,
+                                      double *sch_tau, double *sch_x);
+
 /* The same pipeline with several batches in flight (continuous captures): _submit enqueues batch `slot` (0..3) on the library's
  * own streams once the caller's `cuda_stream` has produced the DEVICE-resident capture, and returns; _collect waits for that batch
  * and fills the result pointers given to _submit (they must stay valid until then).  Batches are staggered on the device: the
@@ -310,7 +348,8 @@ int gsmcal_calibrate_batch_cancel(int slot);
 /* CUDA-event times (ms) of the stages of the last gsmcal_calibrate_batch call on this process:
  * [0] uint8 column sums (+ H2D when raw is on the host) [1] coarse FCCH [2] fine FCCH sliding-DFT peak search
  * [3] fine ppm + tone estimate + gate [4] SCH correlation + pos_info [5] post-SCH tone estimate + result records
- * [6] (gsmcal_calibrate_demod_batch / _demod_bcch_batch only) SCH_demod + FCCH_demod (+ BCCH_demod).  Returns the number of stages written. */
+ * [6] (gsmcal_calibrate_demod_batch / _demod_bcch_batch only) SCH_demod + FCCH_demod (+ BCCH_demod);
+ *     (gsmcal_calibrate_sch_timing_batch only) SCH row list, sub-sample SCH timing and the clock fit.  Returns the number of stages written. */
 int gsmcal_last_batch_stage_ms(double *ms, int cap);
 
 /* FCCH scanner per-channel processing, multi_rtl_sdr_gsm_FCCH_scanner.m:132-135,163-186, for n_chan

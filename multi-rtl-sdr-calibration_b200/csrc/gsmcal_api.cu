@@ -27,6 +27,10 @@ static_assert(sizeof(gsmcal_bcch_result) == sizeof(BcchResultDev) && sizeof(gsmc
               offsetof(gsmcal_bcch_result, flags) == 12 && offsetof(gsmcal_bcch_result, corr_abs) == 16, "BCCH record layout");
 static_assert(GSMCAL_BCCH_NO_POS_INFO == BC_NO_POS_INFO && GSMCAL_BCCH_FEW_BCCH == BC_FEW_BCCH && GSMCAL_BCCH_FCCH_RANGE == BC_FCCH_RANGE &&
               GSMCAL_BCCH_TRAIN_RANGE == BC_TRAIN_RANGE, "BCCH flags");
+static_assert(sizeof(gsmcal_sch_timing_result) == sizeof(TimingResultDev) && sizeof(gsmcal_sch_timing_result) == 40 &&
+              offsetof(gsmcal_sch_timing_result, t0) == 16 && offsetof(gsmcal_sch_timing_result, rms) == 32, "SCH timing record layout");
+static_assert(GSMCAL_TIMING_NO_POS_INFO == TM_NO_POS_INFO && GSMCAL_TIMING_NO_R_CORRECT == TM_NO_R_CORRECT && GSMCAL_TIMING_RANGE == TM_RANGE &&
+              GSMCAL_TIMING_EDGE == TM_EDGE && GSMCAL_TIMING_FEW == TM_FEW, "SCH timing flags");
 
 namespace {
 
@@ -622,6 +626,39 @@ int run_demod(Ctx &c, WinSrc src, const Work &ws, const DemodDev &dd, int osr, d
     return GSMCAL_OK;
 }
 
+// ---- sub-sample SCH timing stage of gsmcal_calibrate_sch_timing_batch ----------------------------------------------------------
+struct TimingOut { gsmcal_sch_timing_result *rec; double *tau, *x; };    // the caller's host outputs (tau, x may be NULL)
+struct TimingDev {                   // device buffers, [D][cap] rows unless noted
+    DemodResultDev *rows /* [D] */; double *sch_pos, *fcch_pos, *tau, *x; unsigned char *sch_ok, *fcch_ok, *row_flag; TimingResultDev *rec /* [D] */;
+};
+TimingDev sub_timing(const TimingDev &a, i64 d0, int cap) {
+    TimingDev s = a;
+    const i64 r = d0 * cap;
+    s.rows += d0; s.rec += d0; s.sch_pos += r; s.fcch_pos += r; s.tau += r; s.x += r; s.sch_ok += r; s.fcch_ok += r; s.row_flag += r;
+    return s;
+}
+int timing_setup(Ctx &c, i64 D, int cap, TimingDev *td) {
+    size_t off = 0;
+    auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes); return o; };
+    const size_t rows = (size_t)D * cap;
+    const size_t o_rows = take(sizeof(DemodResultDev) * D), o_rec = take(sizeof(TimingResultDev) * D), o_sp = take(8 * rows), o_fp = take(8 * rows),
+                 o_tau = take(8 * rows), o_x = take(8 * rows), o_so = take(rows), o_fo = take(rows), o_rf = take(rows);
+    void *base; TRY(c.dem.get(off, &base));
+    char *b = (char *)base;
+    td->rows = (DemodResultDev *)(b + o_rows); td->rec = (TimingResultDev *)(b + o_rec); td->sch_pos = (double *)(b + o_sp);
+    td->fcch_pos = (double *)(b + o_fp); td->tau = (double *)(b + o_tau); td->x = (double *)(b + o_x);
+    td->sch_ok = (unsigned char *)(b + o_so); td->fcch_ok = (unsigned char *)(b + o_fo); td->row_flag = (unsigned char *)(b + o_rf);
+    return GSMCAL_OK;
+}
+// one stream group: the row lists of the demod stage, the timing of every SCH row, the per-stream fit (osr 8)
+int run_timing(WinSrc src, const Work &ws, const TimingDev &td, i64 nd, int cap, cudaStream_t st) {
+    LAUNCH(demod_compact_kernel, (unsigned)nd, 32, 0, st, ws.ctl, ws.pos_info, cap, 8, td.rows, td.sch_pos, td.sch_ok, td.fcch_pos, td.fcch_ok);
+    LAUNCH(sch_timing_batch_kernel, dim3((unsigned)cap, (unsigned)nd), SCH_THREADS, TM_SMEM, st, src, ws.ctl, td.rows, td.sch_pos, cap, ws.tpl,
+           td.tau, td.row_flag);
+    LAUNCH(sch_timing_fit_kernel, (unsigned)nd, 32, 0, st, ws.ctl, td.rows, td.sch_pos, td.row_flag, td.tau, cap, td.x, td.rec);
+    return GSMCAL_OK;
+}
+
 // ---- what gsmcal_calibrate_batch* and gsmcal_calibrate_batch_submit share ---------------------------------------------------------
 // `to` waits for what has been enqueued on `from` so far
 int hand_off(cudaStream_t from, cudaStream_t to) {
@@ -666,9 +703,9 @@ int batch_setup(Ctx &c, DevBuf &work, DevBuf &wc, const double *tpl, const doubl
 }
 
 // the burst stages of one stream group, in order on sg: fine peak, fine rest (ppm, tone, carrier), SCH, post-SCH and, with dd, the demod
-// stage.  With marks, marks[i] is recorded on sg behind stage i (null entries are skipped)
+// stage or, with td, the SCH timing stage.  With marks, marks[i] is recorded on sg behind stage i (null entries are skipped)
 int run_burst_stages(Ctx &c, const uint8_t *graw, i64 n_iq, int n_taps, int osr, double carrier_freq, i64 nd, int cap, Work &ws,
-                     const DemodDev *dd, cudaStream_t sg, const cudaEvent_t *marks) {
+                     const DemodDev *dd, const TimingDev *td, cudaStream_t sg, const cudaEvent_t *marks) {
     auto mark = [&](int i) { if (marks && marks[i]) CU(cudaEventRecord(marks[i], sg)); return GSMCAL_OK; };
     TRY(run_fine_peak(c, lazy_src(graw, n_iq, n_taps, 0, 1), n_iq, osr, nd, cap, ws, sg));
     TRY(mark(0));
@@ -680,6 +717,9 @@ int run_burst_stages(Ctx &c, const uint8_t *graw, i64 n_iq, int n_taps, int osr,
     TRY(mark(3));
     if (dd) {
         TRY(run_demod(c, lazy_src(graw, n_iq, n_taps, 3, 1), ws, *dd, osr, carrier_freq, nd, cap, sg));
+        TRY(mark(4));
+    } else if (td) {
+        TRY(run_timing(lazy_src(graw, n_iq, n_taps, 3, 1), ws, *td, nd, cap, sg));
         TRY(mark(4));
     }
     return GSMCAL_OK;
@@ -1145,7 +1185,7 @@ int gsmcal_total_ppm_calculation(const double *ppm_in, int64_t n, double *ppm_ou
 static int calibrate_batch_impl(const uint8_t *raw, int raw_mem, int64_t n_iq, int64_t D, double carrier_freq, const double *tpl,
                                 const double *coef, int n_taps, int osr, int coarse_dr, gsmcal_stream_result *results,
                                 double *coarse_pos, double *coarse_snr, double *fcch_pos, double *pos_info, void *cuda_stream,
-                                double *r_out, int r_mem, int64_t r_stride, const DemodOut *dm = nullptr) {
+                                double *r_out, int r_mem, int64_t r_stride, const DemodOut *dm = nullptr, const TimingOut *tm = nullptr) {
     std::lock_guard<std::mutex> lk(g_mu);
     if (r_out && r_stride < n_iq) return fail(GSMCAL_ERR_ARG, "calibrate_batch_r: r_stride must be >= n_iq");
     Batch b; TRY(batch_args("calibrate_batch", raw, tpl, coef, results, n_iq, D, osr, coarse_dr, &b));
@@ -1163,6 +1203,8 @@ static int calibrate_batch_impl(const uint8_t *raw, int raw_mem, int64_t n_iq, i
     DemodDev dd;
     std::vector<double> dm_w; signed char dm_pm[64];                 // host sources of the uploads, alive until the final synchronise
     if (dm) TRY(demod_setup(*c, D, cap, osr, w.tpl, dm->nts, dm_w, dm_pm, st, &dd));
+    TimingDev td;
+    if (tm) TRY(timing_setup(*c, D, cap, &td));
     g_stage_n = 0;
     // Streams are independent, so the batch is cut into groups that run the stage sequence on their own CUDA
     // streams: the latency-bound stages of one group (burst chain, per-stream solves) overlap the FP64-bound
@@ -1216,8 +1258,10 @@ static int calibrate_batch_impl(const uint8_t *raw, int raw_mem, int64_t n_iq, i
         // stagger the groups (see gsmcal_calibrate_batch_submit): the FP64 stages of group g wait for group g-1, its front does not
         if (!ev_done.empty()) CU(cudaStreamWaitEvent(sg, ev_done.back(), 0));
         const DemodDev gdd = dm ? sub_demod(dd, d0, cap) : DemodDev{};
-        TRY(run_burst_stages(*c, graw, n_iq, n_taps, osr, carrier_freq, nd, cap, ws, dm ? &gdd : nullptr, sg, timing ? c->stage_ev + g_stage_n : nullptr));
-        if (timing) g_stage_n += dm ? 5 : 4;                     // 3 + 5 <= kNumStageEvents
+        const TimingDev gtd = tm ? sub_timing(td, d0, cap) : TimingDev{};
+        TRY(run_burst_stages(*c, graw, n_iq, n_taps, osr, carrier_freq, nd, cap, ws, dm ? &gdd : nullptr, tm ? &gtd : nullptr, sg,
+                             timing ? c->stage_ev + g_stage_n : nullptr));
+        if (timing) g_stage_n += (dm || tm) ? 5 : 4;             // 3 + 5 <= kNumStageEvents
         if (sg != st) {
             cudaEvent_t ev; CU(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
             CU(cudaEventRecord(ev, sg));
@@ -1258,6 +1302,11 @@ static int calibrate_batch_impl(const uint8_t *raw, int raw_mem, int64_t n_iq, i
         if (dm->snr) TRY(copy_d2h(c->ring, g_device, dm->snr, dd.snr, sizeof(double) * rows, st));
         if (dm->idx) TRY(copy_d2h(c->ring, g_device, dm->idx, dd.idx, sizeof(double) * rows, st));
         if (dm->bcch) CU(cudaMemcpyAsync(dm->bcch, dd.bcch, sizeof(BcchResultDev) * D, cudaMemcpyDeviceToHost, st));
+    }
+    if (tm) {
+        CU(cudaMemcpyAsync(tm->rec, td.rec, sizeof(TimingResultDev) * D, cudaMemcpyDeviceToHost, st));
+        if (tm->tau) TRY(copy_d2h(c->ring, g_device, tm->tau, td.tau, sizeof(double) * D * cap, st));
+        if (tm->x) TRY(copy_d2h(c->ring, g_device, tm->x, td.x, sizeof(double) * D * cap, st));
     }
     CU(cudaStreamSynchronize(st));
     if (timing) for (int i = 0; i + 1 < g_stage_n; ++i) CU(cudaEventElapsedTime(&g_stage_ms[i], c->stage_ev[i], c->stage_ev[i + 1]));
@@ -1302,6 +1351,17 @@ int gsmcal_calibrate_demod_bcch_batch(const uint8_t *raw, int raw_mem, int64_t n
     const DemodOut o = {demod, sch_ok, demod_bits, bits_to_decoder, corr_val, fcch_freq, fcch_snr, fcch_max_idx, normal_training_sequence, bcch};
     return calibrate_batch_impl(raw, raw_mem, n_iq, D, carrier_freq, tpl, coef, n_taps, osr, coarse_dr, results, coarse_pos, coarse_snr, fcch_pos, pos_info,
                                 cuda_stream, nullptr, GSMCAL_MEM_DEVICE, 0, &o);
+}
+
+int gsmcal_calibrate_sch_timing_batch(const uint8_t *raw, int raw_mem, int64_t n_iq, int64_t D, double carrier_freq, const double *tpl,
+                                      const double *coef, int n_taps, int osr, int coarse_dr, gsmcal_stream_result *results,
+                                      double *coarse_pos, double *coarse_snr, double *fcch_pos, double *pos_info, void *cuda_stream,
+                                      gsmcal_sch_timing_result *timing, double *sch_tau, double *sch_x) {
+    if (!timing) return fail(GSMCAL_ERR_ARG, "calibrate_sch_timing_batch: null timing");
+    if (osr != 8) return fail(GSMCAL_ERR_ARG, "calibrate_sch_timing_batch: oversampling_ratio must be 8");
+    const TimingOut o = {timing, sch_tau, sch_x};
+    return calibrate_batch_impl(raw, raw_mem, n_iq, D, carrier_freq, tpl, coef, n_taps, osr, coarse_dr, results, coarse_pos, coarse_snr, fcch_pos, pos_info,
+                                cuda_stream, nullptr, GSMCAL_MEM_DEVICE, 0, nullptr, &o);
 }
 
 // ---- submit / collect: the same pipeline, several batches in flight -----------------------------------------------------------
@@ -1378,7 +1438,7 @@ int gsmcal_calibrate_batch_submit(int slot, const uint8_t *raw_dev, int64_t n_iq
             CU(cudaStreamWaitEvent(sg, c->slots[c->last_slot].done, 0));
         if (tl_g) CU(cudaEventRecord(sl.tl[4], sg));
         const cudaEvent_t marks[4] = {sl.tl[5], sl.tl[6], sl.tl[7], sl.tl[3]};
-        TRY(run_burst_stages(*c, graw, n_iq, n_taps, osr, carrier_freq, nd, cap, ws, nullptr, sg, tl_g ? marks : nullptr));
+        TRY(run_burst_stages(*c, graw, n_iq, n_taps, osr, carrier_freq, nd, cap, ws, nullptr, nullptr, sg, tl_g ? marks : nullptr));
         TRY(hand_off(sg, fr));
     }
     CU(cudaMemcpyAsync(h_res, w.res, sl.n_res, cudaMemcpyDeviceToHost, fr));

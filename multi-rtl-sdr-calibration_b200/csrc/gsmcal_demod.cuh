@@ -596,3 +596,140 @@ __global__ void __launch_bounds__(BC_THREADS) bcch_demod_batch_kernel(WinSrc src
         o->flags = flags;
     }
 }
+
+// ===================================================================================================
+// Sub-sample SCH timing and the per-stream clock fit of gsmcal_calibrate_sch_timing_batch (definition: include/gsmcal.h).  The SCH row
+// list is demod_compact_kernel's; its sch_ok is SCH_demod's 194*osr-sample window check, so the 600-sample correlation window is checked
+// here.  osr 8 only: the correlation is sch_corr_kernel's register-tiled fp64 one (sch_corr_tiled_fp64, 256 threads, 89 lags of 512).
+// ===================================================================================================
+struct TimingResultDev {             // mirrors gsmcal_sch_timing_result (include/gsmcal.h)
+    int n_sch, n_fit, flags, reserved;
+    double t0, fit_ppm, rms;
+};
+#define TM_NO_POS_INFO  1
+#define TM_NO_R_CORRECT 2
+#define TM_RANGE        4
+#define TM_EDGE         8
+#define TM_FEW         16
+#define TM_L     512                   // 64 * osr template samples
+#define TM_LAG0  64                    // lags -8*osr .. +3*osr (SCH_corr_rate_correction.m:36,45-48)
+#define TM_NLAG  89
+#define TM_NSMP  (TM_NLAG + TM_L - 1)  // 600
+// shared: window [TM_NSMP] | scratch: the loader's X, Y, later the padded window and template and the row sums of sch_corr_tiled_fp64
+#define TM_PADW  (TM_NSMP + (TM_NSMP >> 4) + 2)
+#define TM_PADT  (TM_L + (TM_L >> 4) + 2)
+#define TM_PART  ((2 * (SCH_THREADS >> 5) * SCH_LPG * 9 + 1) / 2 + 1)
+#define TM_SCRATCH ((GSMCAL_XCAP(TM_NSMP) + TM_NSMP + 8) > (TM_PADW + TM_PADT + TM_PART) ? (GSMCAL_XCAP(TM_NSMP) + TM_NSMP + 8) : (TM_PADW + TM_PADT + TM_PART))
+#define TM_SMEM  ((size_t)(TM_NSMP + TM_SCRATCH) * sizeof(double2))
+
+// One block per (SCH row, stream): c(l) = |sum conj(t) r_correct(g+l : g+l+511)|^2 for the 89 lags, g = p + 42*8, the first maximum
+// and the three-point parabola through it.  tau = NaN and row_flag = TM_RANGE / TM_EDGE where the row is excluded.
+__global__ void __launch_bounds__(SCH_THREADS) sch_timing_batch_kernel(WinSrc src, const StreamCtl *__restrict__ ctl, const DemodResultDev *__restrict__ rec,
+                                                                      const double *__restrict__ sch_pos, int cap, const double2 *__restrict__ tpl,
+                                                                      double *__restrict__ tau, unsigned char *__restrict__ row_flag) {
+    extern __shared__ double2 sm[];
+    __shared__ double corr[96], corr_i[96];
+    __shared__ double2 ph0;
+    const int row = blockIdx.x, stream = blockIdx.y, tid = threadIdx.x;
+    if (row >= rec[stream].n_sch) return;                      // also n_sch = -1: the step does not run for this stream
+    const i64 o = (i64)stream * cap + row;
+    const StreamCtl c = ctl[stream];
+    const double p = sch_pos[o], g = p + 42.0 * 8.0;
+    if (!(p == floor(p) && g - TM_LAG0 >= 1.0 && g + (TM_NLAG - 1 - TM_LAG0) + (TM_L - 1) <= (double)c.len3)) {
+        if (tid == 0) { tau[o] = NAN; row_flag[o] = TM_RANGE; }
+        return;
+    }
+    const i64 j0 = (i64)g - TM_LAG0 - 1;                       // 0-based first sample of the window r(g-64 : g+24+511)
+    double2 *win = sm, *X = win + TM_NSMP, *Y = X + GSMCAL_XCAP(TM_NSMP);
+    if (tid == 0) { double sn, cs; sincos((double)j0 * c.dphi2, &sn, &cs); ph0 = make_double2(cs, sn); }
+    load_window(src, c, stream, j0, TM_NSMP, win, X, Y);        // level 3; ends with a barrier
+    derotate_post(win, TM_NSMP, c.dphi2, ph0);                 // r_correct (carrier_correct_post_SCH.m:83)
+    __syncthreads();
+    double2 *wp = X, *tp = wp + TM_PADW;
+    double *part = reinterpret_cast<double *>(tp + TM_PADT);
+    for (int i = tid; i < TM_NSMP; i += SCH_THREADS) wp[i + (i >> 4)] = win[i];
+    for (int i = tid; i < TM_L; i += SCH_THREADS) tp[i + (i >> 4)] = __ldg(tpl + i);
+    __syncthreads();
+    sch_corr_tiled_fp64(wp, tp, part, corr, corr_i, TM_NLAG, TM_NSMP);
+    __syncthreads();
+    if (tid < TM_NLAG) corr[tid] = abs2_ref(make_double2(corr[tid], corr_i[tid]));
+    __syncthreads();
+    if (tid == 0) {
+        int k = 0;
+        for (int l = 1; l < TM_NLAG; ++l) if (corr[l] > corr[k]) k = l;      // first maximum, scanning the lags upwards
+        if (k == 0 || k == TM_NLAG - 1) { tau[o] = NAN; row_flag[o] = TM_EDGE; return; }
+        const double ym = corr[k - 1], y0 = corr[k], yp = corr[k + 1];
+        const double den = __dadd_rn(__dsub_rn(ym, 2.0 * y0), yp);
+        const double delta = (den == 0.0) ? 0.0 : __ddiv_rn(0.5 * __dsub_rn(ym, yp), den);
+        tau[o] = __dadd_rn(g + (double)(k - TM_LAG0), delta);
+        row_flag[o] = 0;
+    }
+}
+
+// One warp per stream: the lanes map tau to raw-capture time, x = ((tau - 1)*(1 + e2))*(1 + e1), and lane 0 fits the line in row
+// order (the sums exactly as include/gsmcal.h states them, every product and sum rounded on its own).
+__global__ void __launch_bounds__(32) sch_timing_fit_kernel(const StreamCtl *__restrict__ ctl, const DemodResultDev *__restrict__ rec,
+                                                            const double *__restrict__ sch_pos, const unsigned char *__restrict__ row_flag,
+                                                            const double *__restrict__ tau, int cap, double *__restrict__ x_out,
+                                                            TimingResultDev *__restrict__ out) {
+    const int stream = blockIdx.x, lane = threadIdx.x;
+    const DemodResultDev r = rec[stream];
+    TimingResultDev t;
+    t.n_sch = -1; t.n_fit = 0; t.flags = 0; t.reserved = 0; t.t0 = NAN; t.fit_ppm = NAN; t.rms = NAN;
+    if (r.flags & (DM_NO_POS_INFO | DM_NO_R_CORRECT)) {
+        t.flags = (r.flags & DM_NO_POS_INFO) ? TM_NO_POS_INFO : TM_NO_R_CORRECT;
+        if (lane == 0) out[stream] = t;
+        return;
+    }
+    const StreamCtl c = ctl[stream];
+    const double s1 = __dadd_rn(1.0, __dmul_rn(c.sppm1, 1e-6)), s2 = __dadd_rn(1.0, __dmul_rn(c.sppm2, 1e-6));   // sampling_ppm[0], [1] of the record
+    const i64 base = (i64)stream * cap;
+    const int n = r.n_sch;
+    unsigned fl = 0, nf = 0;
+    for (int i = lane; i < n; i += 32) {
+        const double x = __dmul_rn(__dmul_rn(tau[base + i] - 1.0, s2), s1);
+        x_out[base + i] = x;
+        fl |= row_flag[base + i];
+        nf += isfinite(x) ? 1u : 0u;
+    }
+    fl = __reduce_or_sync(0xffffffffu, fl);
+    nf = __reduce_add_sync(0xffffffffu, nf);
+    __syncwarp();                                              // x_out of every lane is visible to lane 0
+    if (lane != 0) return;
+    t.n_sch = n; t.n_fit = (int)nf; t.flags = (int)fl;
+    if (nf < 3) {
+        t.flags |= TM_FEW;
+        out[stream] = t;
+        return;
+    }
+    double p_first = 0.0, sm = 0.0, sx = 0.0;
+    bool first = true;
+    for (int i = 0; i < n; ++i) {
+        const double x = x_out[base + i];
+        if (!isfinite(x)) continue;
+        if (first) { p_first = sch_pos[base + i]; first = false; }
+        sm = __dadd_rn(sm, sch_pos[base + i] - p_first);
+        sx = __dadd_rn(sx, x);
+    }
+    const double m_bar = sm / (double)nf, x_bar = sx / (double)nf;
+    double sxy = 0.0, smm = 0.0;
+    for (int i = 0; i < n; ++i) {
+        const double x = x_out[base + i];
+        if (!isfinite(x)) continue;
+        const double dm = __dsub_rn(sch_pos[base + i] - p_first, m_bar), dx = __dsub_rn(x, x_bar);
+        sxy = __dadd_rn(sxy, __dmul_rn(dm, dx));
+        smm = __dadd_rn(smm, __dmul_rn(dm, dm));
+    }
+    const double b = sxy / smm, a = __dsub_rn(x_bar, __dmul_rn(b, m_bar));
+    double ss = 0.0;
+    for (int i = 0; i < n; ++i) {
+        const double x = x_out[base + i];
+        if (!isfinite(x)) continue;
+        const double e = __dsub_rn(__dsub_rn(x, a), __dmul_rn(b, sch_pos[base + i] - p_first));
+        ss = __dadd_rn(ss, __dmul_rn(e, e));
+    }
+    t.t0 = a;
+    t.fit_ppm = __dmul_rn(b - 1.0, 1e6);
+    t.rms = sqrt(ss / (double)nf);
+    out[stream] = t;
+}

@@ -28,6 +28,11 @@ class BcchResult(C.Structure):
     _fields_ = [("carrier_ppm", C.c_double), ("nts_idx", C.c_int32), ("flags", C.c_int32), ("corr_abs", C.c_double * 32)]
 
 
+class SchTimingResult(C.Structure):
+    _fields_ = [("n_sch", C.c_int32), ("n_fit", C.c_int32), ("flags", C.c_int32), ("reserved", C.c_int32),
+                ("t0", C.c_double), ("fit_ppm", C.c_double), ("rms", C.c_double)]
+
+
 # every symbol include/gsmcal.h declares: name -> (restype, argtypes)
 SIGNATURES = {
     "gsmcal_abi_version": (C.c_int, []),
@@ -75,6 +80,9 @@ SIGNATURES = {
                                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                                     C.c_void_p, C.c_void_p]),
+    "gsmcal_calibrate_sch_timing_batch": (C.c_int, [C.c_void_p, C.c_int, c_i64, c_i64, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                    C.c_void_p, C.c_void_p, C.c_void_p]),
     "gsmcal_calibrate_batch_submit": (C.c_int, [C.c_int, C.c_void_p, c_i64, c_i64, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "gsmcal_calibrate_batch_collect": (C.c_int, [C.c_int]),

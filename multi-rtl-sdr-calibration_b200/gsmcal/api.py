@@ -11,7 +11,7 @@ import ctypes as C
 
 import numpy as np
 
-from ._lib import BcchResult, DemodResult, GsmcalError, StreamResult, check, lib  # noqa: F401
+from ._lib import BcchResult, DemodResult, GsmcalError, SchTimingResult, StreamResult, check, lib  # noqa: F401
 
 SYMBOL_RATE = (1625.0 / 6.0) * 1e3
 
@@ -307,11 +307,19 @@ def _unpack_results(res, D, cap, coarse_pos, coarse_snr, fcch_pos, pos_info):
 
 def calibrate_batch(raw, carrier_freq: float, sch_training_sequence, coef, osr: int = 8, coarse_dr: int = 8,
                     device_ptr: int | None = None, n_iq: int | None = None, n_streams: int | None = None,
-                    cuda_stream: int = 0, details: bool = True, r_correct=None, r_device_ptr: int | None = None):
+                    cuda_stream: int = 0, details: bool = True, r_correct=None, r_device_ptr: int | None = None,
+                    sch_timing: bool = False):
     """gsm_sync_demod.m:107-124 for every row of `raw` ([D, 2N] uint8, row d == dongle d's fread column).
 
     `raw` is a host NumPy array, or pass device_ptr/n_iq/n_streams for a capture already resident in HBM.
-    Returns a list of per-stream dicts with the same keys as the function-by-function chain."""
+    Returns a list of per-stream dicts with the same keys as the function-by-function chain.
+
+    sch_timing=True (osr 8, not with r_correct / r_device_ptr, implies details) also times every SCH burst of pos_info to a fraction
+    of a sample on r_correct and fits a line through the burst times (gsmcal_calibrate_sch_timing_batch, include/gsmcal.h); each dict
+    gains timing: dict(t0, fit_ppm, rms, n_fit, flags, tau, x): t0 the raw-capture time (0-based samples) of the first fitted burst's
+    training start, fit_ppm the sample clock error of the fit, rms its residual (samples), flags TIMING_* bits, and per SCH row tau (time
+    in r_correct, 1-based) and x (time in the uint8 capture, 0-based), NaN where excluded; tau and x are None when the step did not
+    run (TIMING_NO_POS_INFO / TIMING_NO_R_CORRECT)."""
     tpl = _stream(sch_training_sequence)
     coef = np.ascontiguousarray(coef, dtype=np.float64)
     if device_ptr is None:
@@ -324,6 +332,9 @@ def calibrate_batch(raw, carrier_freq: float, sch_training_sequence, coef, osr: 
         D, ptr, mem = int(n_streams), C.c_void_p(int(device_ptr)), 1
     cap = max_bursts(n_iq, osr, coarse_dr)
     res = (StreamResult * D)()
+    if sch_timing and (r_correct is not None or r_device_ptr is not None):
+        raise ValueError("sch_timing does not combine with r_correct / r_device_ptr")
+    details = details or sch_timing
     if details:
         coarse_pos, coarse_snr, fcch_pos = np.empty((D, cap)), np.empty((D, cap)), np.empty((D, cap))
         pos_info = np.empty((D, 6 * cap, 2))
@@ -331,7 +342,13 @@ def calibrate_batch(raw, carrier_freq: float, sch_training_sequence, coef, osr: 
     else:
         coarse_pos = coarse_snr = fcch_pos = pos_info = None
         ptrs = [None] * 4
-    if r_correct is None and r_device_ptr is None:
+    if sch_timing:
+        tm = (SchTimingResult * D)()
+        tau, x = np.empty((D, cap)), np.empty((D, cap))
+        check(lib().gsmcal_calibrate_sch_timing_batch(ptr, mem, int(n_iq), D, float(carrier_freq), _ptr(tpl), _ptr(coef), len(coef),
+                                                      int(osr), int(coarse_dr), C.cast(res, C.c_void_p), *ptrs, C.c_void_p(cuda_stream),
+                                                      C.cast(tm, C.c_void_p), _ptr(tau), _ptr(x)))
+    elif r_correct is None and r_device_ptr is None:
         check(lib().gsmcal_calibrate_batch(ptr, mem, int(n_iq), D, float(carrier_freq), _ptr(tpl), _ptr(coef), len(coef),
                                            int(osr), int(coarse_dr), C.cast(res, C.c_void_p), *ptrs, C.c_void_p(cuda_stream)))
     else:
@@ -345,9 +362,17 @@ def calibrate_batch(raw, carrier_freq: float, sch_training_sequence, coef, osr: 
                                              int(osr), int(coarse_dr), C.cast(res, C.c_void_p), *ptrs, C.c_void_p(cuda_stream), rp, rmem, int(n_iq)))
     if not details:
         return res
-    return _unpack_results(res, D, cap, coarse_pos, coarse_snr, fcch_pos, pos_info)
+    out = _unpack_results(res, D, cap, coarse_pos, coarse_snr, fcch_pos, pos_info)
+    if sch_timing:
+        for d, item in enumerate(out):
+            t = tm[d]
+            n = t.n_sch
+            item["timing"] = dict(t0=t.t0, fit_ppm=t.fit_ppm, rms=t.rms, n_fit=t.n_fit, flags=t.flags,
+                                  tau=None if n < 0 else tau[d, :n].copy(), x=None if n < 0 else x[d, :n].copy())
+    return out
 
 
+TIMING_NO_POS_INFO, TIMING_NO_R_CORRECT, TIMING_RANGE, TIMING_EDGE, TIMING_FEW = 1, 2, 4, 8, 16
 DEMOD_NO_POS_INFO, DEMOD_NO_R_CORRECT, DEMOD_SCH_RANGE, DEMOD_FCCH_RANGE = 1, 2, 4, 8
 BCCH_NO_POS_INFO, BCCH_FEW_BCCH, BCCH_FCCH_RANGE, BCCH_TRAIN_RANGE = 1, 2, 4, 8
 

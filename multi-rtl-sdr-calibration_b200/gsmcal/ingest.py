@@ -203,13 +203,15 @@ class DongleIngest:
 
 
 def calibrate_from_dongles(endpoints, num_sample: int, freq: float, n_captures: int = 1, osr: int = 8,
-                           coarse_dr: int = 8, gain: float = 0, details: bool = True, demod: bool = False, **kw):
+                           coarse_dr: int = 8, gain: float = 0, details: bool = True, demod: bool = False,
+                           sch_timing: bool = False, **kw):
     """gsm_sync_demod.m:57-124 with every dongle of `endpoints` in one batched library call per capture.
 
     Returns a list (one entry per capture) of the per-dongle result lists of `calibrate_batch`.  With demod=True the call is
     `calibrate_demod_batch` with the normal training sequences of gsm_sync_demod.m:39, so the whole per-dongle loop (:57-147: SCH_demod,
     FCCH_demod and BCCH_demod on every r_correct) runs, and each per-dongle dict carries its sch / fcch / bcch entries (details is
-    ignored then)."""
+    ignored then).  With sch_timing=True (and demod False) the call is `calibrate_batch(..., sch_timing=True)`: each per-dongle dict
+    carries its timing entry, every SCH burst timed to a fraction of a sample and the least-squares clock fit of the dongle."""
     from . import api
     fs = (1625.0 / 6.0) * 1e3 * osr
     coef = api.fir1(46, 200e3 / fs)                                 # gsm_sync_demod.m:34
@@ -221,5 +223,5 @@ def calibrate_from_dongles(endpoints, num_sample: int, freq: float, n_captures: 
             if demod:
                 out.append(api.calibrate_demod_batch(buf, freq, tpl, coef, osr, coarse_dr, normal_training_sequence=nts))
             else:
-                out.append(api.calibrate_batch(buf, freq, tpl, coef, osr, coarse_dr, details=details))
+                out.append(api.calibrate_batch(buf, freq, tpl, coef, osr, coarse_dr, details=details, sch_timing=sch_timing))
     return out

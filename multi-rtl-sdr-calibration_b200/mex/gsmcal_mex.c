@@ -265,11 +265,18 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
 }
 
 #elif defined(GSMCAL_MEX_gsm_calibrate_batch)
-/* [sampling_ppm, carrier_ppm, n_pos_info, pos_info] = gsm_calibrate_batch(raw_uint8, carrier_freq, sch_training_sequence, coef)
+/* [sampling_ppm, carrier_ppm, n_pos_info, pos_info, timing] = gsm_calibrate_batch(raw_uint8, carrier_freq, sch_training_sequence, coef)
  * raw_uint8: 2N x D uint8 (one dongle per column) - gsm_sync_demod.m:107-124 for all dongles in one call.
- * sampling_ppm, carrier_ppm: 3 x D ([FCCH stage; SCH/post stage; total]); pos_info: (6B) x 2 x D, rows beyond n_pos_info(d) are NaN. */
+ * sampling_ppm, carrier_ppm: 3 x D ([FCCH stage; SCH/post stage; total]); pos_info: (6B) x 2 x D, rows beyond n_pos_info(d) are NaN.
+ * timing (asked for only: with four outputs nothing more runs): 1 x D struct array of the sub-sample SCH timing and clock fit of
+ * gsmcal_calibrate_sch_timing_batch: t0 (raw-capture samples, 0-based), fit_ppm, rms, n_fit, flags (1 pos_info == -1, 2 r_correct == -1,
+ * 4 a correlation window leaves r_correct, 8 a maximum on the first or last lag, 16 fewer than 3 fitted bursts), tau and x (1 x n_sch:
+ * each SCH burst's time in r_correct and in the capture, NaN where excluded; empty when the step did not run).  See include/gsmcal.h. */
 void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
-    init_once(); need(nrhs, 4, "[sampling_ppm,carrier_ppm,n_pos_info,pos_info] = gsm_calibrate_batch(raw_uint8,carrier_freq,sch_training_sequence,coef)");
+    init_once();
+    if (nrhs != 4 || nlhs > 5)
+        mexErrMsgIdAndTxt("gsmcal:nargin", "usage: [sampling_ppm,carrier_ppm,n_pos_info,pos_info,timing] = "
+                          "gsm_calibrate_batch(raw_uint8,carrier_freq,sch_training_sequence,coef)");
     if (!mxIsUint8(prhs[0])) mexErrMsgIdAndTxt("gsmcal:type", "raw must be uint8");
     size_t rows = mxGetM(prhs[0]), D = mxGetN(prhs[0]);
     int own; const double *tpl = get_c128(prhs[2], &own);
@@ -278,8 +285,16 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
     int64_t B = gsmcal_max_bursts((n_iq + 63) / 64, 8);
     gsmcal_stream_result *res = (gsmcal_stream_result *)mxMalloc(D * sizeof(*res));
     double *pi = (double *)mxMalloc(D * 12 * (size_t)B * sizeof(double));
-    fail_on(gsmcal_calibrate_batch((const uint8_t *)mxGetData(prhs[0]), GSMCAL_MEM_HOST, n_iq, (int64_t)D, mxGetScalar(prhs[1]), tpl, coef, (int)nt, 8, 8,
-                                   res, NULL, NULL, NULL, pi, NULL), "gsm_calibrate_batch");
+    gsmcal_sch_timing_result *tm = NULL;
+    double *tau = NULL, *xr = NULL;
+    if (nlhs > 4) {
+        tm = (gsmcal_sch_timing_result *)mxMalloc(D * sizeof(*tm));
+        tau = (double *)mxMalloc(2 * D * (size_t)B * sizeof(double)); xr = tau + D * (size_t)B;
+        fail_on(gsmcal_calibrate_sch_timing_batch((const uint8_t *)mxGetData(prhs[0]), GSMCAL_MEM_HOST, n_iq, (int64_t)D, mxGetScalar(prhs[1]), tpl, coef,
+                                                  (int)nt, 8, 8, res, NULL, NULL, NULL, pi, NULL, tm, tau, xr), "gsm_calibrate_batch");
+    } else
+        fail_on(gsmcal_calibrate_batch((const uint8_t *)mxGetData(prhs[0]), GSMCAL_MEM_HOST, n_iq, (int64_t)D, mxGetScalar(prhs[1]), tpl, coef, (int)nt, 8, 8,
+                                       res, NULL, NULL, NULL, pi, NULL), "gsm_calibrate_batch");
     plhs[0] = mxCreateDoubleMatrix(3, D, mxREAL);
     if (nlhs > 1) plhs[1] = mxCreateDoubleMatrix(3, D, mxREAL);
     if (nlhs > 2) plhs[2] = mxCreateDoubleMatrix(1, D, mxREAL);
@@ -297,6 +312,19 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
             for (size_t i = 0; i < (size_t)(6 * B); ++i)
                 for (int c = 0; c < 2; ++c)
                     o[d * 12 * B + c * 6 * B + i] = ((int64_t)i < res[d].n_pos_info) ? pi[d * 12 * B + 2 * i + c] : mxGetNaN();
+    }
+    if (nlhs > 4) {
+        const char *f[] = {"t0", "fit_ppm", "rms", "n_fit", "flags", "tau", "x"};
+        plhs[4] = mxCreateStructMatrix(1, D, 7, f);
+        for (size_t d = 0; d < D; ++d) {
+            const size_t n = tm[d].n_sch > 0 ? (size_t)tm[d].n_sch : 0;
+            mxArray *ta = mxCreateDoubleMatrix(1, n, mxREAL), *xa = mxCreateDoubleMatrix(1, n, mxREAL);
+            if (n) { memcpy(mxGetPr(ta), tau + d * B, n * sizeof(double)); memcpy(mxGetPr(xa), xr + d * B, n * sizeof(double)); }
+            mxSetField(plhs[4], d, "t0", scalar(tm[d].t0)); mxSetField(plhs[4], d, "fit_ppm", scalar(tm[d].fit_ppm));
+            mxSetField(plhs[4], d, "rms", scalar(tm[d].rms)); mxSetField(plhs[4], d, "n_fit", scalar(tm[d].n_fit));
+            mxSetField(plhs[4], d, "flags", scalar(tm[d].flags)); mxSetField(plhs[4], d, "tau", ta); mxSetField(plhs[4], d, "x", xa);
+        }
+        mxFree(tm); mxFree(tau);
     }
     mxFree(res); mxFree(pi); if (own) mxFree((void *)tpl);
 }
