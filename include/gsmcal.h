@@ -327,6 +327,65 @@ int gsmcal_calibrate_sch_timing_batch(const uint8_t *raw, int raw_mem, int64_t n
                                       gsmcal_sch_timing_result *timing /* [n_streams], required */,
                                       double *sch_tau, double *sch_x);
 
+/* gsmcal_calibrate_demod_batch (every output as there, byte for byte; with normal_training_sequence and bcch, both set or both NULL,
+ * gsmcal_calibrate_demod_bcch_batch's) followed by SCH channel decoding: the BSIC and the TDMA frame number (FN) each SCH burst carries,
+ * and each dongle's capture start on the cell's frame clock.  Per type-1 row of pos_info, in row order (the rows SCH_demod
+ * demodulates), with m = its demod_bits and k* = the first maximum of its corr_val (0..84):
+ *   1. skip: sch_ok = 0 -> GSMCAL_SCHDEC_ROW_WINDOW; k* < 39 or k* > 45 (the coded bits would leave the 148) -> GSMCAL_SCHDEC_ROW_ALIGN.
+ *   2. burst bits: m_i = 1 exactly when b_i = b_(i-1) (demod_bits are differentially encoded; bits_to_decoder is not used).  With
+ *      b_(k*+j) = SCH training bit j (j = 0..63): b_i = b_(i+1) xor (1 - m_(i+1)) for i = k*-1 down to k*-39, b_i = b_(i-1) xor (1 - m_i)
+ *      for i = k*+64 up to k*+102.  Coded bits e(0..38) = b(k*-39 .. k*-1), e(39..77) = b(k*+64 .. k*+102) (TS 45.002 5.2.5, k* = 42).
+ *   3. convolutional code (TS 45.003 4.7): e(2k) = u(k)+u(k-3)+u(k-4), e(2k+1) = u(k)+u(k-1)+u(k-3)+u(k-4) mod 2, k = 0..38, u(k<0) = 0.
+ *      Hard-decision Viterbi over the 16 states (u(k), u(k-1), u(k-2), u(k-3)), Hamming branch metrics, from and back to state 0
+ *      (u(35..38) = 0 are the tail).  A state keeps the predecessor with the smaller metric, on a tie the one whose dropped (oldest)
+ *      bit is 0.  hamming = the final metric of state 0: the number of coded bits the decision disagrees with.
+ *   4. CRC (TS 45.003 4.7): d(0)D^34 + ... + d(24)D^10 + p(0)D^9 + ... + p(9), u(0..24) = d, u(25..34) = p, divided by
+ *      D^10 + D^8 + D^6 + D^5 + D^4 + D^2 + 1 must leave 1 + D + ... + D^9, else GSMCAL_SCHDEC_ROW_CRC.
+ *   5. fields (TS 44.018 9.1.30, d(0) = bit 1 of octet 1, OsmocomBB's packing): d(0), d(1) = T1 bits 9, 10; d(2..7) = BSIC bits 0..5;
+ *      d(8..15) = T1 bits 1..8; d(16), d(17) = T3' bits 1, 2; d(18..22) = T2 bits 0..4; d(23) = T1 bit 0; d(24) = T3' bit 0.
+ *      T3 = 10*T3' + 1, FN = 51*((T3 - T2) mod 26) + T3 + 1326*T1 (TS 45.002 3.3.2.2).  T2 > 25 or T3' > 4: GSMCAL_SCHDEC_ROW_FIELD.
+ *      No recorded capture pins this bit order against a live cell: like the GMSK modulator's, its parity is unverified.
+ *   6. vote: with F = 1250*osr samples per frame (10,000 at osr 8) and p_i the SCH rows' pos_info positions (one regridded frame grid,
+ *      so f_i = (p_i - p_first)/F is an integer; p_first = the first SCH row's), every row that passes 1-5 votes for
+ *      (fn_first = (FN_i - f_i) mod 2,715,648, BSIC_i).  Most votes wins, equal votes: the pair whose earliest voting row comes first.
+ *      n_agree = its votes; GSMCAL_SCHDEC_DISAGREE when some valid row voted otherwise; GSMCAL_SCHDEC_NONE when no row passed.
+ *   7. frame_clock_start = (fn_first*F - (p_first - 1)) mod (2,715,648*F): the GSM time of raw capture sample 0 in nominal samples since
+ *      FN 0 of the hyperframe (r_correct(j) sits at raw time (j-1)(1+e2)(1+e1) and its spacing is nominal).  An integer-valued double,
+ *      as accurate as pos_info (a few samples), not sub-sample.
+ * sch_fn, sch_bsic [n_streams][B] int32 (-1 where not decoded), sch_hamming, sch_row_flags [n_streams][B] uint8 (B as above); any may be
+ * NULL (not copied back).  Rows beyond the record's n_sch hold -1 / -1 / 0 / 0. */
+typedef struct gsmcal_sch_decode_result {
+    int32_t n_sch;             /* type-1 rows; -1: not run (flags say why: GSMCAL_SCHDEC_NO_POS_INFO / _NO_R_CORRECT only) */
+    int32_t n_crc_ok;          /* rows with a valid CRC and valid fields */
+    int32_t n_agree;           /* of those, rows that voted for the winning (fn_first, bsic) */
+    int32_t flags;             /* GSMCAL_SCHDEC_* */
+    int32_t bsic;              /* 0..63 (NCC*8 + BCC), or -1 */
+    int32_t fn_first;          /* FN of the frame holding the first SCH row of pos_info, or -1 */
+    double  frame_clock_start; /* see 7.; NaN without a winner */
+} gsmcal_sch_decode_result;    /* 32 bytes */
+
+#define GSMCAL_SCHDEC_NO_POS_INFO   1  /* as GSMCAL_DEMOD_NO_POS_INFO */
+#define GSMCAL_SCHDEC_NO_R_CORRECT  2  /* as GSMCAL_DEMOD_NO_R_CORRECT */
+#define GSMCAL_SCHDEC_NONE          4  /* no row passed the CRC and field checks */
+#define GSMCAL_SCHDEC_DISAGREE      8  /* some valid row voted for another (fn_first, bsic) */
+#define GSMCAL_SCHDEC_ROW_WINDOW    1  /* row flags: sch_ok = 0 */
+#define GSMCAL_SCHDEC_ROW_ALIGN     2  /* k* outside 39..45 */
+#define GSMCAL_SCHDEC_ROW_CRC       4  /* CRC check failed */
+#define GSMCAL_SCHDEC_ROW_FIELD     8  /* T2 > 25 or T3' > 4 */
+
+int gsmcal_calibrate_sch_decode_batch(const uint8_t *raw, int raw_mem, int64_t n_iq, int64_t n_streams,
+                                      double carrier_freq, const double *sch_training_sequence,
+                                      const double *coef, int n_taps, int oversampling_ratio, int coarse_decimation,
+                                      gsmcal_stream_result *results,
+                                      double *coarse_pos, double *coarse_snr, double *fcch_pos, double *pos_info,
+                                      void *cuda_stream,
+                                      gsmcal_demod_result *demod /* [n_streams], required */, uint8_t *sch_ok,
+                                      uint8_t *demod_bits, uint8_t *bits_to_decoder, double *corr_val,
+                                      double *fcch_freq, double *fcch_snr, double *fcch_max_idx,
+                                      const double *normal_training_sequence /* or NULL */, gsmcal_bcch_result *bcch /* or NULL */,
+                                      gsmcal_sch_decode_result *dec /* [n_streams], required */,
+                                      int32_t *sch_fn, int32_t *sch_bsic, uint8_t *sch_hamming, uint8_t *sch_row_flags);
+
 /* The same pipeline with several batches in flight (continuous captures): _submit enqueues batch `slot` (0..3) on the library's
  * own streams once the caller's `cuda_stream` has produced the DEVICE-resident capture, and returns; _collect waits for that batch
  * and fills the result pointers given to _submit (they must stay valid until then).  Batches are staggered on the device: the
@@ -348,7 +407,7 @@ int gsmcal_calibrate_batch_cancel(int slot);
 /* CUDA-event times (ms) of the stages of the last gsmcal_calibrate_batch call on this process:
  * [0] uint8 column sums (+ H2D when raw is on the host) [1] coarse FCCH [2] fine FCCH sliding-DFT peak search
  * [3] fine ppm + tone estimate + gate [4] SCH correlation + pos_info [5] post-SCH tone estimate + result records
- * [6] (gsmcal_calibrate_demod_batch / _demod_bcch_batch only) SCH_demod + FCCH_demod (+ BCCH_demod);
+ * [6] (gsmcal_calibrate_demod_batch / _demod_bcch_batch / _sch_decode_batch only) SCH_demod (+ SCH decoding) + FCCH_demod (+ BCCH_demod);
  *     (gsmcal_calibrate_sch_timing_batch only) SCH row list, sub-sample SCH timing and the clock fit.  Returns the number of stages written. */
 int gsmcal_last_batch_stage_ms(double *ms, int cap);
 

@@ -31,6 +31,11 @@ static_assert(sizeof(gsmcal_sch_timing_result) == sizeof(TimingResultDev) && siz
               offsetof(gsmcal_sch_timing_result, t0) == 16 && offsetof(gsmcal_sch_timing_result, rms) == 32, "SCH timing record layout");
 static_assert(GSMCAL_TIMING_NO_POS_INFO == TM_NO_POS_INFO && GSMCAL_TIMING_NO_R_CORRECT == TM_NO_R_CORRECT && GSMCAL_TIMING_RANGE == TM_RANGE &&
               GSMCAL_TIMING_EDGE == TM_EDGE && GSMCAL_TIMING_FEW == TM_FEW, "SCH timing flags");
+static_assert(sizeof(gsmcal_sch_decode_result) == sizeof(SchDecodeResultDev) && sizeof(gsmcal_sch_decode_result) == 32 &&
+              offsetof(gsmcal_sch_decode_result, fn_first) == 20 && offsetof(gsmcal_sch_decode_result, frame_clock_start) == 24, "SCH decode record layout");
+static_assert(GSMCAL_SCHDEC_NO_POS_INFO == SC_NO_POS_INFO && GSMCAL_SCHDEC_NO_R_CORRECT == SC_NO_R_CORRECT && GSMCAL_SCHDEC_NONE == SC_NONE &&
+              GSMCAL_SCHDEC_DISAGREE == SC_DISAGREE && GSMCAL_SCHDEC_ROW_WINDOW == SC_ROW_WINDOW && GSMCAL_SCHDEC_ROW_ALIGN == SC_ROW_ALIGN &&
+              GSMCAL_SCHDEC_ROW_CRC == SC_ROW_CRC && GSMCAL_SCHDEC_ROW_FIELD == SC_ROW_FIELD, "SCH decode flags");
 
 namespace {
 
@@ -562,11 +567,13 @@ void sch_training_pm(signed char *data_pm);
 struct DemodOut {                    // the caller's host outputs (any per-row pointer may be NULL)
     gsmcal_demod_result *rec; uint8_t *sch_ok, *bits, *dec; double *corr, *freq, *snr, *idx;
     const double *nts; gsmcal_bcch_result *bcch;     // BCCH_demod inputs / outputs (gsmcal_calibrate_demod_bcch_batch), else both NULL
+    gsmcal_sch_decode_result *sdec; int32_t *fn, *bsic; uint8_t *ham, *rflag;   // SCH decoding (gsmcal_calibrate_sch_decode_batch), else NULL
 };
 struct DemodDev {                    // device buffers, [D][cap] rows unless noted
     DemodResultDev *rec; double *sch_pos, *fcch_pos, *corr /* x85 */, *freq, *snr, *idx;
     unsigned char *sch_ok, *fcch_ok, *bits /* x148 */, *dec /* x148 */; double2 *Ft /* N */, *Wtab /* 16*osr */; signed char *dpm /* 64 */;
     double2 *nts /* (26*osr) x 8 */; BcchResultDev *bcch /* [D]; nullptr: no BCCH stage */;
+    SchDecodeResultDev *sdec /* [D]; nullptr: no SCH decoding */; int *key, *fn, *bsic; unsigned char *ham, *rflag;
 };
 DemodDev sub_demod(const DemodDev &a, i64 d0, int cap) {
     DemodDev s = a;
@@ -574,13 +581,14 @@ DemodDev sub_demod(const DemodDev &a, i64 d0, int cap) {
     s.rec += d0; s.sch_pos += r; s.fcch_pos += r; s.corr += r * 85; s.freq += r; s.snr += r; s.idx += r;
     s.sch_ok += r; s.fcch_ok += r; s.bits += r * 148; s.dec += r * 148;
     if (s.bcch) s.bcch += d0;
+    if (s.sdec) { s.sdec += d0; s.key += r; s.fn += r; s.bsic += r; s.ham += r; s.rflag += r; }
     return s;
 }
 // workspace, branch table, training bits and fft(template) (SCH_demod.m:47-59), and with nts (host, (26*osr) x 8 complex) the normal
-// training sequences and the BCCH records behind them; once per call on `st` before the stream groups fork (gsmcal_SCH_demod: one
-// stream of its H bursts)
-int demod_setup(Ctx &c, i64 D, int cap, int osr, const double2 *tpl_dev, const double *nts, std::vector<double> &W, signed char *data_pm, cudaStream_t st,
-                DemodDev *dd) {
+// training sequences and the BCCH records behind them, and with sch_decode the SCH decoding's records and row buffers; once per call on
+// `st` before the stream groups fork (gsmcal_SCH_demod: one stream of its H bursts)
+int demod_setup(Ctx &c, i64 D, int cap, int osr, const double2 *tpl_dev, const double *nts, bool sch_decode, std::vector<double> &W, signed char *data_pm,
+                cudaStream_t st, DemodDev *dd) {
     const int N = SD_NSYM * osr;
     size_t off = 0;
     auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes); return o; };
@@ -589,6 +597,9 @@ int demod_setup(Ctx &c, i64 D, int cap, int osr, const double2 *tpl_dev, const d
                  o_fr = take(8 * rows), o_sn = take(8 * rows), o_ix = take(8 * rows), o_so = take(rows), o_fo = take(rows),
                  o_b = take(148 * rows), o_d = take(148 * rows), o_ft = take(sizeof(double2) * N), o_w = take(sizeof(double2) * 16 * osr), o_pm = take(64);
     const size_t o_nts = nts ? take(sizeof(double2) * 8 * 26 * osr) : 0, o_bc = nts ? take(sizeof(BcchResultDev) * D) : 0;
+    const size_t o_sd = sch_decode ? take(sizeof(SchDecodeResultDev) * D) : 0, o_key = sch_decode ? take(4 * rows) : 0,
+                 o_fn = sch_decode ? take(4 * rows) : 0, o_bs = sch_decode ? take(4 * rows) : 0, o_hm = sch_decode ? take(rows) : 0,
+                 o_rf = sch_decode ? take(rows) : 0;
     void *base; TRY(c.dem.get(off, &base));
     char *b = (char *)base;
     dd->rec = (DemodResultDev *)(b + o_rec); dd->sch_pos = (double *)(b + o_sp); dd->fcch_pos = (double *)(b + o_fp); dd->corr = (double *)(b + o_corr);
@@ -596,6 +607,9 @@ int demod_setup(Ctx &c, i64 D, int cap, int osr, const double2 *tpl_dev, const d
     dd->sch_ok = (unsigned char *)(b + o_so); dd->fcch_ok = (unsigned char *)(b + o_fo); dd->bits = (unsigned char *)(b + o_b); dd->dec = (unsigned char *)(b + o_d);
     dd->Ft = (double2 *)(b + o_ft); dd->Wtab = (double2 *)(b + o_w); dd->dpm = (signed char *)(b + o_pm);
     dd->nts = nts ? (double2 *)(b + o_nts) : nullptr; dd->bcch = nts ? (BcchResultDev *)(b + o_bc) : nullptr;
+    dd->sdec = sch_decode ? (SchDecodeResultDev *)(b + o_sd) : nullptr; dd->key = sch_decode ? (int *)(b + o_key) : nullptr;
+    dd->fn = sch_decode ? (int *)(b + o_fn) : nullptr; dd->bsic = sch_decode ? (int *)(b + o_bs) : nullptr;
+    dd->ham = sch_decode ? (unsigned char *)(b + o_hm) : nullptr; dd->rflag = sch_decode ? (unsigned char *)(b + o_rf) : nullptr;
     if (nts) CU(cudaMemcpyAsync(dd->nts, nts, sizeof(double2) * 8 * 26 * (size_t)osr, cudaMemcpyHostToDevice, st));
     W.assign(2 * 16 * (size_t)osr, 0.0);
     gmsk_branch_table(osr, W.data());
@@ -606,7 +620,7 @@ int demod_setup(Ctx &c, i64 D, int cap, int osr, const double2 *tpl_dev, const d
     LAUNCH(fde_template_kernel, 1, SD_THREADS, 3 * (size_t)N * sizeof(double2), st, tpl_dev, osr, tw, dd->Ft);
     return GSMCAL_OK;
 }
-// one stream group: row lists + sentinels, SCH bursts, FCCH bursts, FCCH means, and BCCH_demod when its outputs were asked for
+// one stream group: row lists + sentinels, SCH bursts, SCH decoding and BCCH_demod when their outputs were asked for, FCCH bursts, FCCH means
 int run_demod(Ctx &c, WinSrc src, const Work &ws, const DemodDev &dd, int osr, double carrier_freq, i64 nd, int cap, cudaStream_t st) {
     const double2 *tw_s, *tw_f;
     TRY(get_twiddle(c, SD_NSYM * osr, st, &tw_s));
@@ -614,6 +628,9 @@ int run_demod(Ctx &c, WinSrc src, const Work &ws, const DemodDev &dd, int osr, d
     LAUNCH(demod_compact_kernel, (unsigned)nd, 32, 0, st, ws.ctl, ws.pos_info, cap, osr, dd.rec, dd.sch_pos, dd.sch_ok, dd.fcch_pos, dd.fcch_ok);
     LAUNCH(sch_demod_batch_kernel, dim3((unsigned)cap, (unsigned)nd), SDB_THREADS, sch_demod_smem(osr), st, src, ws.ctl, dd.rec, dd.sch_pos, dd.sch_ok,
            cap, osr, tw_s, dd.Ft, dd.Wtab, dd.dpm, dd.bits, dd.dec, dd.corr);
+    if (dd.sdec)
+        LAUNCH(sch_decode_batch_kernel, (unsigned)nd, 32, 0, st, dd.rec, dd.sch_pos, dd.sch_ok, dd.bits, dd.corr, cap, osr, dd.key, dd.fn, dd.bsic,
+               dd.ham, dd.rflag, dd.sdec);
     const size_t fs = fcch_demod_smem(osr), fs_load = sizeof(double2) * (3 * 148 * (size_t)osr + 144);      // + the loader's scratch behind u
     LAUNCH(fcch_demod_batch_kernel, dim3((unsigned)cap, (unsigned)nd), FD_THREADS, fs > fs_load ? fs : fs_load, st, with_cache(src, ws, cap), ws.ctl, dd.rec,
            dd.fcch_pos, dd.fcch_ok, cap, osr, tw_f, dd.freq, dd.snr, dd.idx);
@@ -1202,7 +1219,7 @@ static int calibrate_batch_impl(const uint8_t *raw, int raw_mem, int64_t n_iq, i
     }
     DemodDev dd;
     std::vector<double> dm_w; signed char dm_pm[64];                 // host sources of the uploads, alive until the final synchronise
-    if (dm) TRY(demod_setup(*c, D, cap, osr, w.tpl, dm->nts, dm_w, dm_pm, st, &dd));
+    if (dm) TRY(demod_setup(*c, D, cap, osr, w.tpl, dm->nts, dm->sdec != nullptr, dm_w, dm_pm, st, &dd));
     TimingDev td;
     if (tm) TRY(timing_setup(*c, D, cap, &td));
     g_stage_n = 0;
@@ -1302,6 +1319,11 @@ static int calibrate_batch_impl(const uint8_t *raw, int raw_mem, int64_t n_iq, i
         if (dm->snr) TRY(copy_d2h(c->ring, g_device, dm->snr, dd.snr, sizeof(double) * rows, st));
         if (dm->idx) TRY(copy_d2h(c->ring, g_device, dm->idx, dd.idx, sizeof(double) * rows, st));
         if (dm->bcch) CU(cudaMemcpyAsync(dm->bcch, dd.bcch, sizeof(BcchResultDev) * D, cudaMemcpyDeviceToHost, st));
+        if (dm->sdec) CU(cudaMemcpyAsync(dm->sdec, dd.sdec, sizeof(SchDecodeResultDev) * D, cudaMemcpyDeviceToHost, st));
+        if (dm->fn) TRY(copy_d2h(c->ring, g_device, dm->fn, dd.fn, sizeof(int) * rows, st));
+        if (dm->bsic) TRY(copy_d2h(c->ring, g_device, dm->bsic, dd.bsic, sizeof(int) * rows, st));
+        if (dm->ham) TRY(copy_d2h(c->ring, g_device, dm->ham, dd.ham, rows, st));
+        if (dm->rflag) TRY(copy_d2h(c->ring, g_device, dm->rflag, dd.rflag, rows, st));
     }
     if (tm) {
         CU(cudaMemcpyAsync(tm->rec, td.rec, sizeof(TimingResultDev) * D, cudaMemcpyDeviceToHost, st));
@@ -1336,7 +1358,8 @@ int gsmcal_calibrate_demod_batch(const uint8_t *raw, int raw_mem, int64_t n_iq, 
                                  gsmcal_demod_result *demod, uint8_t *sch_ok, uint8_t *demod_bits, uint8_t *bits_to_decoder, double *corr_val,
                                  double *fcch_freq, double *fcch_snr, double *fcch_max_idx) {
     if (!demod) return fail(GSMCAL_ERR_ARG, "calibrate_demod_batch: null demod");
-    const DemodOut o = {demod, sch_ok, demod_bits, bits_to_decoder, corr_val, fcch_freq, fcch_snr, fcch_max_idx, nullptr, nullptr};
+    const DemodOut o = {demod, sch_ok, demod_bits, bits_to_decoder, corr_val, fcch_freq, fcch_snr, fcch_max_idx, nullptr, nullptr,
+                        nullptr, nullptr, nullptr, nullptr, nullptr};
     return calibrate_batch_impl(raw, raw_mem, n_iq, D, carrier_freq, tpl, coef, n_taps, osr, coarse_dr, results, coarse_pos, coarse_snr, fcch_pos, pos_info,
                                 cuda_stream, nullptr, GSMCAL_MEM_DEVICE, 0, &o);
 }
@@ -1348,7 +1371,23 @@ int gsmcal_calibrate_demod_bcch_batch(const uint8_t *raw, int raw_mem, int64_t n
                                       double *fcch_freq, double *fcch_snr, double *fcch_max_idx,
                                       const double *normal_training_sequence, gsmcal_bcch_result *bcch) {
     if (!demod || !normal_training_sequence || !bcch) return fail(GSMCAL_ERR_ARG, "calibrate_demod_bcch_batch: null demod, normal_training_sequence or bcch");
-    const DemodOut o = {demod, sch_ok, demod_bits, bits_to_decoder, corr_val, fcch_freq, fcch_snr, fcch_max_idx, normal_training_sequence, bcch};
+    const DemodOut o = {demod, sch_ok, demod_bits, bits_to_decoder, corr_val, fcch_freq, fcch_snr, fcch_max_idx, normal_training_sequence, bcch,
+                        nullptr, nullptr, nullptr, nullptr, nullptr};
+    return calibrate_batch_impl(raw, raw_mem, n_iq, D, carrier_freq, tpl, coef, n_taps, osr, coarse_dr, results, coarse_pos, coarse_snr, fcch_pos, pos_info,
+                                cuda_stream, nullptr, GSMCAL_MEM_DEVICE, 0, &o);
+}
+
+int gsmcal_calibrate_sch_decode_batch(const uint8_t *raw, int raw_mem, int64_t n_iq, int64_t D, double carrier_freq, const double *tpl,
+                                      const double *coef, int n_taps, int osr, int coarse_dr, gsmcal_stream_result *results,
+                                      double *coarse_pos, double *coarse_snr, double *fcch_pos, double *pos_info, void *cuda_stream,
+                                      gsmcal_demod_result *demod, uint8_t *sch_ok, uint8_t *demod_bits, uint8_t *bits_to_decoder, double *corr_val,
+                                      double *fcch_freq, double *fcch_snr, double *fcch_max_idx,
+                                      const double *normal_training_sequence, gsmcal_bcch_result *bcch,
+                                      gsmcal_sch_decode_result *dec, int32_t *sch_fn, int32_t *sch_bsic, uint8_t *sch_hamming, uint8_t *sch_row_flags) {
+    if (!demod || !dec) return fail(GSMCAL_ERR_ARG, "calibrate_sch_decode_batch: null demod or dec");
+    if (!normal_training_sequence != !bcch) return fail(GSMCAL_ERR_ARG, "calibrate_sch_decode_batch: normal_training_sequence and bcch must both be set or both NULL");
+    const DemodOut o = {demod, sch_ok, demod_bits, bits_to_decoder, corr_val, fcch_freq, fcch_snr, fcch_max_idx, normal_training_sequence, bcch,
+                        dec, sch_fn, sch_bsic, sch_hamming, sch_row_flags};
     return calibrate_batch_impl(raw, raw_mem, n_iq, D, carrier_freq, tpl, coef, n_taps, osr, coarse_dr, results, coarse_pos, coarse_snr, fcch_pos, pos_info,
                                 cuda_stream, nullptr, GSMCAL_MEM_DEVICE, 0, &o);
 }

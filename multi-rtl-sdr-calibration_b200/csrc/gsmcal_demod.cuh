@@ -733,3 +733,155 @@ __global__ void __launch_bounds__(32) sch_timing_fit_kernel(const StreamCtl *__r
     t.rms = sqrt(ss / (double)nf);
     out[stream] = t;
 }
+
+// ===================================================================================================
+// SCH channel decoding of gsmcal_calibrate_sch_decode_batch (definition: include/gsmcal.h) on what sch_demod_batch_kernel wrote: BSIC
+// and FN of every SCH row, the per-stream vote and the capture start on the cell's frame clock.
+// ===================================================================================================
+struct SchDecodeResultDev {          // mirrors gsmcal_sch_decode_result (include/gsmcal.h)
+    int n_sch, n_crc_ok, n_agree, flags, bsic, fn_first;
+    double frame_clock_start;
+};
+#define SC_NO_POS_INFO  1
+#define SC_NO_R_CORRECT 2
+#define SC_NONE         4
+#define SC_DISAGREE     8
+#define SC_ROW_WINDOW   1
+#define SC_ROW_ALIGN    2
+#define SC_ROW_CRC      4
+#define SC_ROW_FIELD    8
+#define SC_FN_MOD 2715648
+
+// one row: the 78 coded bits around the training sequence at k (m: the 148 demodulated symbols), the 16-state Viterbi, CRC and fields.
+// Returns the row flag; fn, bsic, ham are written where the steps got that far.
+__device__ __forceinline__ int sch_decode_row(const unsigned char *__restrict__ m, int k, int &fn, int &bsic, int &ham) {
+    const unsigned long long T = 0xB962040F2D45761Bull;            // SCH training bits 0..63, bit j at position 63 - j (T_0 = MSB)
+    unsigned long long e = 0ull;                                   // e(0..63) at bits 63..0
+    unsigned e_hi = 0u;                                            // e(64..77) at bits 13..0
+    int b = (int)(T >> 63) & 1;                                    // backwards from b(k) = T_0
+    for (int i = k - 1; i >= k - 39; --i) {
+        b ^= 1 - m[i + 1];
+        e |= (unsigned long long)b << (63 - (i - (k - 39)));
+    }
+    b = (int)T & 1;                                                // forwards from b(k+63) = T_63
+    for (int i = k + 64; i <= k + 102; ++i) {
+        b ^= 1 - m[i];
+        const int j = 39 + i - (k + 64);
+        if (j < 64) e |= (unsigned long long)b << (63 - j);
+        else e_hi |= (unsigned)b << (77 - j);
+    }
+    // state s = u(k) | u(k-1) << 1 | u(k-2) << 2 | u(k-3) << 3; survivors: the 39 decided inputs, newest at bit 0
+    int metric[16];
+    unsigned long long path[16];
+#pragma unroll
+    for (int s = 0; s < 16; ++s) { metric[s] = (s == 0) ? 0 : 1 << 20; path[s] = 0ull; }
+    for (int t = 0; t < 39; ++t) {
+        const int c0 = (t < 32) ? (int)(e >> (63 - 2 * t)) & 1 : (int)(e_hi >> (77 - 2 * t)) & 1;      // e(2t), e(2t+1)
+        const int c1 = (t < 32) ? (int)(e >> (62 - 2 * t)) & 1 : (int)(e_hi >> (76 - 2 * t)) & 1;
+        int nm[16];
+        unsigned long long np[16];
+#pragma unroll
+        for (int s = 0; s < 16; ++s) {
+            const int u = s & 1;
+            const int p0 = s >> 1, p1 = (s >> 1) | 8;                // predecessors: dropped bit u(k-4) = 0 / 1
+            const int a0 = u ^ ((p0 >> 2) & 1) ^ ((p0 >> 3) & 1), a1 = u ^ (p0 & 1) ^ ((p0 >> 2) & 1) ^ ((p0 >> 3) & 1);
+            const int m0 = metric[p0] + (a0 ^ c0) + (a1 ^ c1);
+            const int m1 = metric[p1] + (a0 ^ 1 ^ c0) + (a1 ^ 1 ^ c1);      // the dropped bit enters both outputs
+            const bool take1 = m1 < m0;                              // a tie keeps dropped bit 0
+            nm[s] = take1 ? m1 : m0;
+            np[s] = ((take1 ? path[p1] : path[p0]) << 1) | (unsigned long long)u;
+        }
+#pragma unroll
+        for (int s = 0; s < 16; ++s) { metric[s] = nm[s]; path[s] = np[s]; }
+    }
+    ham = metric[0];
+    // u(0) at bit 38 ... u(34) at bit 4: the 35-bit word d(0)D^34 + ... + p(9) is path >> 4
+    unsigned long long v = path[0] >> 4;
+    for (int i = 34; i >= 10; --i)
+        if ((v >> i) & 1ull) v ^= 0x575ull << (i - 10);
+    if ((v & 0x3FFull) != 0x3FFull) return SC_ROW_CRC;
+    const unsigned long long w = path[0] >> 14;                    // d(i) at bit 24 - i
+    auto d = [&](int i) { return (int)(w >> (24 - i)) & 1; };
+    int bs = 0, t1 = (d(0) << 9) | (d(1) << 10) | d(23), t2 = 0;
+    for (int i = 0; i < 6; ++i) bs |= d(2 + i) << i;
+    for (int i = 0; i < 8; ++i) t1 |= d(8 + i) << (1 + i);
+    for (int i = 0; i < 5; ++i) t2 |= d(18 + i) << i;
+    const int t3p = (d(16) << 1) | (d(17) << 2) | d(24);
+    if (t2 > 25 || t3p > 4) return SC_ROW_FIELD;
+    const int t3 = 10 * t3p + 1;
+    fn = 51 * ((t3 - t2 + 26) % 26) + t3 + 1326 * t1;
+    bsic = bs;
+    return 0;
+}
+
+// One warp per stream: each lane decodes whole SCH rows (row = lane, lane + 32, ...), then the warp takes the vote over the rows' keys
+// (fn_first * 64 + bsic, -1 for rows that do not vote) and lane 0 writes the record.
+__global__ void __launch_bounds__(32) sch_decode_batch_kernel(const DemodResultDev *__restrict__ rec, const double *__restrict__ sch_pos,
+                                                              const unsigned char *__restrict__ sch_ok, const unsigned char *__restrict__ bits,
+                                                              const double *__restrict__ corr, int cap, int osr, int *__restrict__ key,
+                                                              int *__restrict__ fn_out, int *__restrict__ bsic_out,
+                                                              unsigned char *__restrict__ ham_out, unsigned char *__restrict__ flag_out,
+                                                              SchDecodeResultDev *__restrict__ out) {
+    const int stream = blockIdx.x, lane = threadIdx.x;
+    const DemodResultDev r = rec[stream];
+    const i64 base = (i64)stream * cap;
+    const int n = r.n_sch;                                         // -1 when SCH_demod did not run
+    const i64 frame = 1250 * (i64)osr;
+    const double p_first = (n > 0) ? sch_pos[base] : 0.0;
+    int n_ok = 0;
+    for (int i = lane; i < cap; i += 32) {
+        int fn = -1, bsic = -1, ham = 0, fl = 0, k_vote = -1;
+        if (i < n) {
+            if (!sch_ok[base + i]) fl = SC_ROW_WINDOW;
+            else {
+                const double *c = corr + (base + i) * 85;
+                int k = 0;
+                for (int l = 1; l < 85; ++l) if (c[l] > c[k]) k = l;   // first maximum
+                if (k < 39 || k > 45) fl = SC_ROW_ALIGN;
+                else fl = sch_decode_row(bits + (base + i) * 148, k, fn, bsic, ham);
+                if (fl) { fn = -1; bsic = -1; }
+                else {
+                    const i64 f = (i64)(sch_pos[base + i] - p_first) / frame;
+                    i64 ff = ((i64)fn - f) % SC_FN_MOD; if (ff < 0) ff += SC_FN_MOD;
+                    k_vote = (int)ff * 64 + bsic;
+                    ++n_ok;
+                }
+            }
+        }
+        fn_out[base + i] = fn; bsic_out[base + i] = bsic; ham_out[base + i] = (unsigned char)ham; flag_out[base + i] = (unsigned char)fl;
+        key[base + i] = k_vote;
+    }
+    n_ok = __reduce_add_sync(0xffffffffu, n_ok);
+    __syncwarp();                                                  // every lane's keys are visible to the warp
+    SchDecodeResultDev o;
+    o.n_sch = n; o.n_crc_ok = n_ok; o.n_agree = 0; o.flags = 0; o.bsic = -1; o.fn_first = -1; o.frame_clock_start = NAN;
+    if (n < 0) o.flags = (r.flags & DM_NO_POS_INFO) ? SC_NO_POS_INFO : SC_NO_R_CORRECT;
+    else if (n_ok == 0) o.flags = SC_NONE;
+    else {
+        // each lane scores the keys it owns: (votes, first row with that key); the best is the most votes, then the earliest first row
+        int best_cnt = 0, best_first = 0x7fffffff, best_key = -1;
+        for (int i = lane; i < n; i += 32) {
+            const int ki = key[base + i];
+            if (ki < 0) continue;
+            int cnt = 0, first = i;
+            for (int j = 0; j < n; ++j) {
+                if (key[base + j] != ki) continue;
+                ++cnt;
+                if (j < first) first = j;
+            }
+            if (cnt > best_cnt || (cnt == best_cnt && first < best_first)) { best_cnt = cnt; best_first = first; best_key = ki; }
+        }
+        for (int o2 = 16; o2 > 0; o2 >>= 1) {
+            const int c2 = __shfl_xor_sync(0xffffffffu, best_cnt, o2), f2 = __shfl_xor_sync(0xffffffffu, best_first, o2);
+            const int k2 = __shfl_xor_sync(0xffffffffu, best_key, o2);
+            if (c2 > best_cnt || (c2 == best_cnt && f2 < best_first)) { best_cnt = c2; best_first = f2; best_key = k2; }
+        }
+        o.n_agree = best_cnt;
+        o.fn_first = best_key >> 6; o.bsic = best_key & 63;
+        o.flags = (best_cnt < n_ok) ? SC_DISAGREE : 0;
+        const i64 hyper = (i64)SC_FN_MOD * frame;
+        i64 t = ((i64)o.fn_first * frame - ((i64)p_first - 1)) % hyper; if (t < 0) t += hyper;
+        o.frame_clock_start = (double)t;
+    }
+    if (lane == 0) out[stream] = o;
+}

@@ -33,6 +33,11 @@ class SchTimingResult(C.Structure):
                 ("t0", C.c_double), ("fit_ppm", C.c_double), ("rms", C.c_double)]
 
 
+class SchDecodeResult(C.Structure):
+    _fields_ = [("n_sch", C.c_int32), ("n_crc_ok", C.c_int32), ("n_agree", C.c_int32), ("flags", C.c_int32), ("bsic", C.c_int32),
+                ("fn_first", C.c_int32), ("frame_clock_start", C.c_double)]
+
+
 # every symbol include/gsmcal.h declares: name -> (restype, argtypes)
 SIGNATURES = {
     "gsmcal_abi_version": (C.c_int, []),
@@ -80,6 +85,10 @@ SIGNATURES = {
                                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                                     C.c_void_p, C.c_void_p]),
+    "gsmcal_calibrate_sch_decode_batch": (C.c_int, [C.c_void_p, C.c_int, c_i64, c_i64, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "gsmcal_calibrate_sch_timing_batch": (C.c_int, [C.c_void_p, C.c_int, c_i64, c_i64, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                                     C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -11,7 +11,7 @@ import ctypes as C
 
 import numpy as np
 
-from ._lib import BcchResult, DemodResult, GsmcalError, SchTimingResult, StreamResult, check, lib  # noqa: F401
+from ._lib import BcchResult, DemodResult, GsmcalError, SchDecodeResult, SchTimingResult, StreamResult, check, lib  # noqa: F401
 
 SYMBOL_RATE = (1625.0 / 6.0) * 1e3
 
@@ -375,11 +375,14 @@ def calibrate_batch(raw, carrier_freq: float, sch_training_sequence, coef, osr: 
 TIMING_NO_POS_INFO, TIMING_NO_R_CORRECT, TIMING_RANGE, TIMING_EDGE, TIMING_FEW = 1, 2, 4, 8, 16
 DEMOD_NO_POS_INFO, DEMOD_NO_R_CORRECT, DEMOD_SCH_RANGE, DEMOD_FCCH_RANGE = 1, 2, 4, 8
 BCCH_NO_POS_INFO, BCCH_FEW_BCCH, BCCH_FCCH_RANGE, BCCH_TRAIN_RANGE = 1, 2, 4, 8
+SCHDEC_NO_POS_INFO, SCHDEC_NO_R_CORRECT, SCHDEC_NONE, SCHDEC_DISAGREE = 1, 2, 4, 8
+SCHDEC_ROW_WINDOW, SCHDEC_ROW_ALIGN, SCHDEC_ROW_CRC, SCHDEC_ROW_FIELD = 1, 2, 4, 8
+FN_MOD = 2715648                                   # TDMA frames in a hyperframe
 
 
 def calibrate_demod_batch(raw, carrier_freq: float, sch_training_sequence, coef, osr: int = 8, coarse_dr: int = 8,
                           device_ptr: int | None = None, n_iq: int | None = None, n_streams: int | None = None, cuda_stream: int = 0,
-                          normal_training_sequence=None):
+                          normal_training_sequence=None, sch_decode: bool = False):
     """calibrate_batch followed by SCH_demod / FCCH_demod on every stream's r_correct (gsm_sync_demod.m:144-145), which is never
     materialised.  Same inputs as calibrate_batch.  Each per-stream dict holds calibrate_batch's keys plus
       sch:  dict(demod_bits [n x 148], bits_to_decoder [n x 148], corr_val [n x 85], sch_ok [n] bool), n = SCH rows of pos_info;
@@ -394,7 +397,14 @@ def calibrate_demod_batch(raw, carrier_freq: float, sch_training_sequence, coef,
       bcch: dict(carrier_ppm, nts_idx, corr_abs, flags): carrier_ppm of r_correct (== fcch carrier_ppm), nts_idx 1..8 or -1, corr_abs
             abs(corr_val) 8 x 4 (NaN columns for training windows outside r_correct, BCCH_TRAIN_RANGE), flags BCCH_* bits; carrier_ppm,
             nts_idx, corr_abs are (-1, -1, None) for BCCH_NO_POS_INFO / BCCH_FEW_BCCH as BCCH_demod returns them, (NaN, -1, None) for
-            BCCH_FCCH_RANGE (no FCCH mean to correct with)."""
+            BCCH_FCCH_RANGE (no FCCH mean to correct with).
+    sch_decode=True also decodes every SCH burst (gsmcal_calibrate_sch_decode_batch, definition in include/gsmcal.h) and each dict gains
+      cell: dict(bsic, ncc, bcc, fn_first, frame_clock_start, n_crc_ok, n_agree, flags, fn, bsic_rows, hamming, row_flags): the cell's
+            BSIC (ncc = bsic >> 3, bcc = bsic & 7; -1 without a winner), the TDMA frame number of the first SCH row of pos_info, the GSM
+            time of capture sample 0 in nominal samples since FN 0 (NaN without a winner), the rows that decoded and that voted for the
+            winner, flags SCHDEC_* bits, and per SCH row fn, bsic_rows (-1 where not decoded), hamming and row_flags (SCHDEC_ROW_*);
+            the per-row arrays are None where SCH_demod did not run.  A winner with n_agree 1 may be a false CRC pass (about 1 in 1024
+            rows of noise passes the 10-bit CRC)."""
     tpl = _stream(sch_training_sequence)
     coef = np.ascontiguousarray(coef, dtype=np.float64)
     if device_ptr is None:
@@ -416,15 +426,23 @@ def calibrate_demod_batch(raw, carrier_freq: float, sch_training_sequence, coef,
     args = [ptr, mem, int(n_iq), D, float(carrier_freq), _ptr(tpl), _ptr(coef), len(coef), int(osr), int(coarse_dr),
             C.cast(res, C.c_void_p), _ptr(coarse_pos), _ptr(coarse_snr), _ptr(fcch_pos), _ptr(pos_info),
             C.c_void_p(cuda_stream), C.cast(dem, C.c_void_p), _ptr(sch_ok), _ptr(bits), _ptr(dec), _ptr(corr), _ptr(freq), _ptr(snr), _ptr(idx)]
-    if normal_training_sequence is None:
-        check(lib().gsmcal_calibrate_demod_batch(*args))
-    else:
+    nts_args = [None, None]
+    if normal_training_sequence is not None:
         nts_m = np.asarray(normal_training_sequence)
         if nts_m.shape != (26 * int(osr), 8):
             raise ValueError("normal_training_sequence must be (26*osr) x 8")
         nts = np.ascontiguousarray(nts_m.T, dtype=np.complex128)                # column-major (26*osr) x 8
         bc = (BcchResult * D)()
-        check(lib().gsmcal_calibrate_demod_bcch_batch(*args, _ptr(nts), C.cast(bc, C.c_void_p)))
+        nts_args = [_ptr(nts), C.cast(bc, C.c_void_p)]
+    if sch_decode:
+        sd = (SchDecodeResult * D)()
+        fn, bsic = np.empty((D, cap), dtype=np.int32), np.empty((D, cap), dtype=np.int32)
+        ham, rfl = np.empty((D, cap), dtype=np.uint8), np.empty((D, cap), dtype=np.uint8)
+        check(lib().gsmcal_calibrate_sch_decode_batch(*args, *nts_args, C.cast(sd, C.c_void_p), _ptr(fn), _ptr(bsic), _ptr(ham), _ptr(rfl)))
+    elif normal_training_sequence is None:
+        check(lib().gsmcal_calibrate_demod_batch(*args))
+    else:
+        check(lib().gsmcal_calibrate_demod_bcch_batch(*args, *nts_args))
     out = _unpack_results(res, D, cap, coarse_pos, coarse_snr, fcch_pos, pos_info)
     for d, item in enumerate(out):
         r = dem[d]
@@ -439,6 +457,29 @@ def calibrate_demod_batch(raw, carrier_freq: float, sch_training_sequence, coef,
             none = b.flags & (BCCH_NO_POS_INFO | BCCH_FEW_BCCH | BCCH_FCCH_RANGE)
             item["bcch"] = dict(carrier_ppm=b.carrier_ppm, nts_idx=b.nts_idx, flags=b.flags,
                                 corr_abs=None if none else np.array(b.corr_abs).reshape(4, 8).T.copy())
+        if sch_decode:
+            c, n = sd[d], sd[d].n_sch
+            rows = lambda a: None if n < 0 else a[d, :n].astype(np.int64)      # noqa: E731
+            item["cell"] = dict(bsic=c.bsic, ncc=c.bsic >> 3 if c.bsic >= 0 else -1, bcc=c.bsic & 7 if c.bsic >= 0 else -1,
+                                fn_first=c.fn_first, frame_clock_start=c.frame_clock_start, n_crc_ok=c.n_crc_ok, n_agree=c.n_agree,
+                                flags=c.flags, fn=rows(fn), bsic_rows=rows(bsic), hamming=rows(ham), row_flags=rows(rfl))
+    return out
+
+
+def frame_clock_offsets(results, ref: int = 0, osr: int = 8) -> np.ndarray:
+    """Capture-start offsets on the cell's frame clock, from calibrate_demod_batch(..., sch_decode=True) results: for every stream that
+    decoded the same BSIC as stream `ref` (both with a winner), frame_clock_start[d] - frame_clock_start[ref] wrapped into (-H/2, H/2],
+    H = one hyperframe = 2,715,648 * 1250 * osr nominal samples; NaN for every other stream.  Positive: stream d started later."""
+    h = float(FN_MOD * 1250 * int(osr))
+    cells = [r["cell"] for r in results]
+    c0 = cells[ref]
+    out = np.full(len(cells), np.nan)
+    if c0["bsic"] < 0:
+        return out
+    for d, c in enumerate(cells):
+        if c["bsic"] == c0["bsic"] and c["n_agree"] > 0:
+            v = (c["frame_clock_start"] - c0["frame_clock_start"]) % h                # exact: integer-valued doubles below 2^53
+            out[d] = v - h if v > h / 2 else v
     return out
 
 

@@ -63,6 +63,8 @@ class StreamSpec:
     drop_fcch: tuple = field(default_factory=tuple)   # indices (0-based, in order of appearance) of FCCH bursts to replace by data
     noise_only: bool = False
     tsc: int | None = None          # normal training sequence code (0..7) put at bits 61..86 of every normal burst; None = random bits
+    bsic: int | None = None         # 0..63: every SCH burst carries the coded (BSIC, FN) of TS 45.003 4.7; None = random coded bits
+    fn0: int = 0                    # TDMA frame number of slot 0's frame (a multiple of 51, below FN_MOD)
 
 
 def random_spec(seed: int, n_samples: int, carrier_freq: float = 957.4e6) -> StreamSpec:
@@ -86,6 +88,37 @@ NORMAL_TRAINING_BITS = (      # gsm_normal_training_sequence_gen.m:17-24
     (0, 1, 0, 0, 1, 1, 1, 0, 1, 0, 1, 1, 0, 0, 0, 0, 0, 1, 0, 0, 1, 1, 1, 0, 1, 0),
     (1, 0, 1, 0, 0, 1, 1, 1, 1, 1, 0, 1, 1, 0, 0, 0, 1, 0, 1, 0, 0, 1, 1, 1, 1, 1),
     (1, 1, 1, 0, 1, 1, 1, 1, 0, 0, 0, 1, 0, 0, 1, 0, 1, 1, 1, 0, 1, 1, 1, 1, 0, 0))
+
+
+FN_MOD = 26 * 51 * 2048     # TDMA frames in a hyperframe (TS 45.002 3.3.2.2)
+
+
+def sch_fields(fn: int):
+    """(T1, T2, T3') of an SCH frame number (FN mod 51 in 1, 11, 21, 31, 41)"""
+    t3 = fn % 51
+    assert t3 % 10 == 1 and t3 <= 41, "not an SCH frame"
+    return fn // 1326, fn % 26, (t3 - 1) // 10
+
+
+def sch_encode(bsic: int, fn: int) -> np.ndarray:
+    """The 78 coded bits of an SCH burst (TS 45.003 4.7): the 25 information bits packed as TS 44.018 9.1.30 (OsmocomBB's order),
+    the 10 parity bits that leave the remainder 1 + D + ... + D^9 modulo D^10 + D^8 + D^6 + D^5 + D^4 + D^2 + 1, four tail bits, and the
+    rate-1/2 code G0 = 1 + D^3 + D^4, G1 = 1 + D + D^3 + D^4.  Parity with a live cell is unverified (no recorded capture)."""
+    t1, t2, t3p = sch_fields(fn)
+    bit = lambda v, i: (v >> i) & 1                                      # noqa: E731
+    d = [bit(t1, 9), bit(t1, 10)] + [bit(bsic, i) for i in range(6)] + [bit(t1, i) for i in range(1, 9)]
+    d += [bit(t3p, 1), bit(t3p, 2)] + [bit(t2, i) for i in range(5)] + [bit(t1, 0), bit(t3p, 0)]
+    rem = 0
+    for b in d + [0] * 10:                                              # d(D) * D^10 mod g(D)
+        rem = (rem << 1) | b
+        if rem & 0x400:
+            rem ^= 0x575
+    u = d + [((rem ^ 0x3FF) >> (9 - i)) & 1 for i in range(10)] + [0, 0, 0, 0]
+    c = []
+    for k in range(39):
+        v = lambda j: u[k - j] if k >= j else 0                         # noqa: E731
+        c += [v(0) ^ v(3) ^ v(4), v(0) ^ v(1) ^ v(3) ^ v(4)]
+    return np.array(c, dtype=np.int64)
 
 
 def _slot_bits(n_slots: int, gen: torch.Generator, device, drop_fcch=(), tsc=None) -> torch.Tensor:
@@ -114,6 +147,33 @@ def _slot_bits(n_slots: int, gen: torch.Generator, device, drop_fcch=(), tsc=Non
     return bits
 
 
+def stream_bits(spec: StreamSpec, gen: torch.Generator | None = None, device="cpu") -> torch.Tensor:
+    """[n_slots, 156] burst bits of the stream (what generate_stream modulates); gen: the stream's generator, seeded here when None.
+    With spec.bsic set, the coded SCH bits are written over bits 3..41 and 106..144 of every SCH burst after the random draws, so the
+    generator's later draws (the noise) and every other bit are those of bsic=None."""
+    dev = torch.device(device)
+    if gen is None:
+        gen = torch.Generator(device=dev)
+        gen.manual_seed(int(spec.seed))
+    inv = 1.0 / (1.0 + spec.sampling_ppm * 1e-6)
+    t_end = spec.start_offset + spec.n_samples * inv
+    n_slots = int(t_end // SLOT) + 3
+    bits = _slot_bits(n_slots, gen, dev, spec.drop_fcch, spec.tsc)
+    if spec.bsic is not None:
+        assert 0 <= spec.bsic < 64 and spec.fn0 % 51 == 0 and 0 <= spec.fn0 < FN_MOD
+        for s in range(0, n_slots, 8):
+            if (s // 8) % 51 % 10 == 1 and (s // 8) % 51 <= 41:
+                c = torch.from_numpy(sch_encode(spec.bsic, (spec.fn0 + s // 8) % FN_MOD)).to(dev)
+                bits[s, 3:42] = c[:39]
+                bits[s, 106:145] = c[39:]
+    return bits
+
+
+def true_frame_clock_start(spec: StreamSpec) -> float:
+    """GSM time of receiver sample 0 in nominal 8x samples since FN 0 (the quantity gsmcal_sch_decode_result.frame_clock_start measures)"""
+    return spec.fn0 * FRAME + spec.start_offset
+
+
 def generate_stream(spec: StreamSpec, device="cpu", out: torch.Tensor | None = None) -> torch.Tensor:
     """Returns 2*n_samples uint8 (I,Q interleaved).  `out` may be a preallocated uint8 view to fill."""
     dev = torch.device(device)
@@ -122,9 +182,7 @@ def generate_stream(spec: StreamSpec, device="cpu", out: torch.Tensor | None = N
     gen.manual_seed(int(spec.seed))
     f64 = torch.float64
     inv = 1.0 / (1.0 + spec.sampling_ppm * 1e-6)
-    t_end = spec.start_offset + n * inv
-    n_slots = int(t_end // SLOT) + 3
-    bits = _slot_bits(n_slots, gen, dev, spec.drop_fcch, spec.tsc).flatten()
+    bits = stream_bits(spec, gen, dev).flatten()
     prev = torch.cat([torch.ones(1, dtype=torch.int64, device=dev), bits[:-1]])
     a = (1 - 2 * (bits ^ prev)).to(torch.int64)                 # +1 where a bit equals its predecessor
     psum = torch.cumsum(a, 0)                                   # P[m] = sum_{i<=m} a_i

@@ -329,7 +329,7 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
     mxFree(res); mxFree(pi); if (own) mxFree((void *)tpl);
 }
 
-#elif defined(GSMCAL_MEX_gsm_calibrate_demod_batch)
+#elif defined(GSMCAL_MEX_gsm_calibrate_demod_batch) || defined(GSMCAL_MEX_gsm_calibrate_sch_decode_batch)
 /* [sampling_ppm, carrier_ppm, n_pos_info, pos_info, sch, fcch, bcch] =
  *     gsm_calibrate_demod_batch(raw_uint8, carrier_freq, sch_training_sequence, coef [, normal_training_sequence])
  * gsm_calibrate_batch (outputs 1-4 as there) followed by SCH_demod / FCCH_demod on every dongle's r_correct (gsm_sync_demod.m:144-145),
@@ -341,12 +341,25 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
  * Where the reference would not get that far (pos_info == -1, r_correct == -1: flags 1 / 2) the fields are empty and n_sch = -1 is
  * reported as empty arrays; flags 4 / 8: a window leaves r_correct (sch_ok 0 / NaN rows, NaN mean).  bcch(d).flags: 1 pos_info == -1,
  * 2 fewer than four BCCH rows (carrier_ppm = idx = -1), 4 no FCCH mean (carrier_ppm NaN, idx -1), 8 a training window leaves
- * r_correct (NaN column, idx -1); corr_abs is NaN where it was not computed.  See include/gsmcal.h. */
+ * r_correct (NaN column, idx -1); corr_abs is NaN where it was not computed.  See include/gsmcal.h.
+ *
+ * [sampling_ppm, carrier_ppm, n_pos_info, pos_info, sch, fcch, cell] = gsm_calibrate_sch_decode_batch(raw_uint8, carrier_freq, sch_training_sequence, coef)
+ * (GSMCAL_MEX_gsm_calibrate_sch_decode_batch) is the same call followed by SCH channel decoding (gsmcal_calibrate_sch_decode_batch):
+ *   cell(d): bsic (0..63 or -1), ncc, bcc, fn_first (TDMA frame number of the first SCH row of pos_info, or -1), frame_clock_start (GSM
+ *   time of capture sample 0 in samples since FN 0 of the hyperframe, NaN without a winner), n_crc_ok, n_agree, flags (1 pos_info == -1,
+ *   2 r_correct == -1, 4 no row decoded, 8 rows disagree), and per SCH row fn, bsic (-1 where not decoded), hamming, row_flags
+ *   (1 x n_sch; 1 window outside r_correct, 2 training peak too far from bit 42, 4 CRC, 8 invalid T2 / T3'). */
 void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
     init_once();
+#if defined(GSMCAL_MEX_gsm_calibrate_sch_decode_batch)
+    if (nrhs != 4 || nlhs > 7)
+        mexErrMsgIdAndTxt("gsmcal:nargin", "usage: [sampling_ppm,carrier_ppm,n_pos_info,pos_info,sch,fcch,cell] = "
+                          "gsm_calibrate_sch_decode_batch(raw_uint8,carrier_freq,sch_training_sequence,coef)");
+#else
     if (nrhs < 4 || nrhs > 5 || (nlhs > 6 && nrhs < 5))
         mexErrMsgIdAndTxt("gsmcal:nargin", "usage: [sampling_ppm,carrier_ppm,n_pos_info,pos_info,sch,fcch,bcch] = "
                           "gsm_calibrate_demod_batch(raw_uint8,carrier_freq,sch_training_sequence,coef[,normal_training_sequence]) (bcch needs the fifth input)");
+#endif
     if (!mxIsUint8(prhs[0])) mexErrMsgIdAndTxt("gsmcal:type", "raw must be uint8");
     size_t rows = mxGetM(prhs[0]), D = mxGetN(prhs[0]);
     int own, own_n = 0; const double *tpl = get_c128(prhs[2], &own), *nts = NULL;
@@ -363,6 +376,14 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
     double *pi = (double *)mxMalloc(D * 12 * B * sizeof(double));
     uint8_t *ok = (uint8_t *)mxMalloc(R * (1 + 2 * 148)), *bits = ok + R, *dec = bits + 148 * R;
     double *corr = (double *)mxMalloc(R * 88 * sizeof(double)), *freq = corr + 85 * R, *snr = freq + R, *idx = snr + R;
+#if defined(GSMCAL_MEX_gsm_calibrate_sch_decode_batch)
+    gsmcal_sch_decode_result *sd = (gsmcal_sch_decode_result *)mxMalloc(D * sizeof(*sd));
+    int32_t *sfn = (int32_t *)mxMalloc(R * 2 * sizeof(int32_t)), *sbs = sfn + R;
+    uint8_t *sham = (uint8_t *)mxMalloc(R * 2), *srf = sham + R;
+    fail_on(gsmcal_calibrate_sch_decode_batch((const uint8_t *)mxGetData(prhs[0]), GSMCAL_MEM_HOST, n_iq, (int64_t)D, mxGetScalar(prhs[1]), tpl, coef, (int)nt,
+                                              8, 8, res, NULL, NULL, NULL, pi, NULL, dem, ok, bits, dec, corr, freq, snr, idx, NULL, NULL,
+                                              sd, sfn, sbs, sham, srf), "gsm_calibrate_sch_decode_batch");
+#else
     if (nts)
         fail_on(gsmcal_calibrate_demod_bcch_batch((const uint8_t *)mxGetData(prhs[0]), GSMCAL_MEM_HOST, n_iq, (int64_t)D, mxGetScalar(prhs[1]), tpl, coef, (int)nt,
                                                   8, 8, res, NULL, NULL, NULL, pi, NULL, dem, ok, bits, dec, corr, freq, snr, idx, nts, bc),
@@ -370,6 +391,7 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
     else
         fail_on(gsmcal_calibrate_demod_batch((const uint8_t *)mxGetData(prhs[0]), GSMCAL_MEM_HOST, n_iq, (int64_t)D, mxGetScalar(prhs[1]), tpl, coef, (int)nt, 8, 8,
                                              res, NULL, NULL, NULL, pi, NULL, dem, ok, bits, dec, corr, freq, snr, idx), "gsm_calibrate_demod_batch");
+#endif
     plhs[0] = mxCreateDoubleMatrix(3, D, mxREAL);
     if (nlhs > 1) plhs[1] = mxCreateDoubleMatrix(3, D, mxREAL);
     if (nlhs > 2) plhs[2] = mxCreateDoubleMatrix(1, D, mxREAL);
@@ -412,6 +434,29 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
             mxSetField(plhs[5], d, "carrier_ppm", scalar(dem[d].fcch_carrier_ppm)); mxSetField(plhs[5], d, "flags", scalar(dem[d].flags));
         }
     }
+#if defined(GSMCAL_MEX_gsm_calibrate_sch_decode_batch)
+    if (nlhs > 6) {
+        const char *f[] = {"bsic", "ncc", "bcc", "fn_first", "frame_clock_start", "n_crc_ok", "n_agree", "flags", "fn", "bsic_rows", "hamming", "row_flags"};
+        plhs[6] = mxCreateStructMatrix(1, D, 12, f);
+        for (size_t d = 0; d < D; ++d) {
+            const gsmcal_sch_decode_result *c = sd + d;
+            const size_t k = c->n_sch < 0 ? 0 : (size_t)c->n_sch;
+            mxArray *a[4];
+            for (int j = 0; j < 4; ++j) a[j] = mxCreateDoubleMatrix(1, k, mxREAL);
+            for (size_t i = 0; i < k; ++i) {
+                mxGetPr(a[0])[i] = sfn[d * B + i]; mxGetPr(a[1])[i] = sbs[d * B + i];
+                mxGetPr(a[2])[i] = sham[d * B + i]; mxGetPr(a[3])[i] = srf[d * B + i];
+            }
+            mxSetField(plhs[6], d, "bsic", scalar(c->bsic)); mxSetField(plhs[6], d, "ncc", scalar(c->bsic < 0 ? -1 : c->bsic >> 3));
+            mxSetField(plhs[6], d, "bcc", scalar(c->bsic < 0 ? -1 : c->bsic & 7)); mxSetField(plhs[6], d, "fn_first", scalar(c->fn_first));
+            mxSetField(plhs[6], d, "frame_clock_start", scalar(c->frame_clock_start)); mxSetField(plhs[6], d, "n_crc_ok", scalar(c->n_crc_ok));
+            mxSetField(plhs[6], d, "n_agree", scalar(c->n_agree)); mxSetField(plhs[6], d, "flags", scalar(c->flags));
+            mxSetField(plhs[6], d, "fn", a[0]); mxSetField(plhs[6], d, "bsic_rows", a[1]);
+            mxSetField(plhs[6], d, "hamming", a[2]); mxSetField(plhs[6], d, "row_flags", a[3]);
+        }
+    }
+    mxFree(sd); mxFree(sfn); mxFree(sham);
+#else
     if (nlhs > 6) {
         const char *f[] = {"carrier_ppm", "idx", "corr_abs", "flags"};
         plhs[6] = mxCreateStructMatrix(1, D, 4, f);
@@ -422,6 +467,7 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
             mxSetField(plhs[6], d, "corr_abs", ca); mxSetField(plhs[6], d, "flags", scalar(bc[d].flags));
         }
     }
+#endif
     mxFree(res); mxFree(dem); mxFree(pi); mxFree(ok); mxFree(corr); if (bc) mxFree(bc); if (own) mxFree((void *)tpl); if (own_n) mxFree((void *)nts);
 }
 
