@@ -563,116 +563,97 @@ size_t sch_demod_smem(int osr);
 void gmsk_branch_table(int osr, double *W);
 void sch_training_pm(signed char *data_pm);
 
-// ---- batched SCH_demod / FCCH_demod stage of gsmcal_calibrate_demod_batch -----------------------------------------------------
-struct DemodOut {                    // the caller's host outputs (any per-row pointer may be NULL)
-    gsmcal_demod_result *rec; uint8_t *sch_ok, *bits, *dec; double *corr, *freq, *snr, *idx;
-    const double *nts; gsmcal_bcch_result *bcch;     // BCCH_demod inputs / outputs (gsmcal_calibrate_demod_bcch_batch), else both NULL
-    gsmcal_sch_decode_result *sdec; int32_t *fn, *bsic; uint8_t *ham, *rflag;   // SCH decoding (gsmcal_calibrate_sch_decode_batch), else NULL
+// ---- the stage behind post-SCH ("tail") of gsmcal_calibrate_demod_batch, _demod_bcch_batch, _sch_decode_batch and _sch_timing_batch --
+// It is the SCH timing block when `timing` is set, else the demod block (batched SCH_demod / FCCH_demod) with the BCCH block when `nts`
+// is set and the SCH decoding block when `sdec` is set.
+struct TailOut {                     // the caller's host outputs; an array left NULL is not read back
+    gsmcal_demod_result *demod; uint8_t *sch_ok, *bits, *dec; double *corr, *freq, *snr, *idx;
+    const double *nts; gsmcal_bcch_result *bcch;
+    gsmcal_sch_decode_result *sdec; int32_t *fn, *bsic; uint8_t *ham, *rflag;
+    gsmcal_sch_timing_result *timing; double *tau, *x;
 };
-struct DemodDev {                    // device buffers, [D][cap] rows unless noted
-    DemodResultDev *rec; double *sch_pos, *fcch_pos, *corr /* x85 */, *freq, *snr, *idx;
-    unsigned char *sch_ok, *fcch_ok, *bits /* x148 */, *dec /* x148 */; double2 *Ft /* N */, *Wtab /* 16*osr */; signed char *dpm /* 64 */;
-    double2 *nts /* (26*osr) x 8 */; BcchResultDev *bcch /* [D]; nullptr: no BCCH stage */;
-    SchDecodeResultDev *sdec /* [D]; nullptr: no SCH decoding */; int *key, *fn, *bsic; unsigned char *ham, *rflag;
+struct TailDev {                     // device buffers of the same blocks
+    DemodResultDev *rec; double *sch_pos, *fcch_pos; unsigned char *sch_ok, *fcch_ok;                       // the row lists
+    double *corr, *freq, *snr, *idx; unsigned char *bits, *dec; double2 *Ft /* N */, *Wtab /* 16*osr */; signed char *dpm /* 64 */;
+    double2 *nts /* (26*osr) x 8 */; BcchResultDev *bcch;
+    SchDecodeResultDev *sdec; int *key, *fn, *bsic; unsigned char *ham, *rflag;
+    TimingResultDev *timing; double *tau, *x; unsigned char *row_flag;
 };
-DemodDev sub_demod(const DemodDev &a, i64 d0, int cap) {
-    DemodDev s = a;
-    const i64 r = d0 * cap;
-    s.rec += d0; s.sch_pos += r; s.fcch_pos += r; s.corr += r * 85; s.freq += r; s.snr += r; s.idx += r;
-    s.sch_ok += r; s.fcch_ok += r; s.bits += r * 148; s.dec += r * 148;
-    if (s.bcch) s.bcch += d0;
-    if (s.sdec) { s.sdec += d0; s.key += r; s.fn += r; s.bsic += r; s.ham += r; s.rflag += r; }
-    return s;
+// every per-stream array ([D] records, [D][cap] rows) of the blocks `o` asks for: f(device pointer, bytes per stream, the caller's host
+// array or NULL).  Set-up, the slice of a stream group and the read-back all walk this one list.  The per-call constants (Ft, Wtab, dpm,
+// nts) are not in it.
+template <class F> void tail_arrays(TailDev &t, const TailOut &o, int cap, F &&f) {
+    const size_t r = (size_t)cap;
+    f(t.rec, sizeof(DemodResultDev), o.demod); f(t.sch_pos, 8 * r, nullptr); f(t.fcch_pos, 8 * r, nullptr);
+    f(t.sch_ok, r, o.sch_ok); f(t.fcch_ok, r, nullptr);
+    if (o.timing) {
+        f(t.timing, sizeof(TimingResultDev), o.timing); f(t.tau, 8 * r, o.tau); f(t.x, 8 * r, o.x); f(t.row_flag, r, nullptr);
+        return;
+    }
+    f(t.bits, 148 * r, o.bits); f(t.dec, 148 * r, o.dec); f(t.corr, 8 * 85 * r, o.corr); f(t.freq, 8 * r, o.freq); f(t.snr, 8 * r, o.snr);
+    f(t.idx, 8 * r, o.idx);
+    if (o.nts) f(t.bcch, sizeof(BcchResultDev), o.bcch);
+    if (o.sdec) {
+        f(t.sdec, sizeof(SchDecodeResultDev), o.sdec); f(t.key, 4 * r, nullptr); f(t.fn, 4 * r, o.fn); f(t.bsic, 4 * r, o.bsic);
+        f(t.ham, r, o.ham); f(t.rflag, r, o.rflag);
+    }
 }
-// workspace, branch table, training bits and fft(template) (SCH_demod.m:47-59), and with nts (host, (26*osr) x 8 complex) the normal
-// training sequences and the BCCH records behind them, and with sch_decode the SCH decoding's records and row buffers; once per call on
-// `st` before the stream groups fork (gsmcal_SCH_demod: one stream of its H bursts)
-int demod_setup(Ctx &c, i64 D, int cap, int osr, const double2 *tpl_dev, const double *nts, bool sch_decode, std::vector<double> &W, signed char *data_pm,
-                cudaStream_t st, DemodDev *dd) {
+template <class T> void place(T *&p, uintptr_t a) { p = (T *)a; }
+// the buffers of D streams in c.dem, and for the demod block the branch table, training bits and fft(template) (SCH_demod.m:47-59) and
+// with nts (host, (26*osr) x 8 complex) the normal training sequences; once per call on `st` before the stream groups fork
+// (gsmcal_SCH_demod: the demod block alone, one stream of its H bursts)
+int tail_setup(Ctx &c, i64 D, int cap, int osr, const double2 *tpl_dev, const TailOut &o, std::vector<double> &W, signed char *data_pm,
+               cudaStream_t st, TailDev *t) {
     const int N = SD_NSYM * osr;
-    size_t off = 0;
-    auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes); return o; };
-    const size_t rows = (size_t)D * cap;
-    const size_t o_rec = take(sizeof(DemodResultDev) * D), o_sp = take(8 * rows), o_fp = take(8 * rows), o_corr = take(8 * 85 * rows),
-                 o_fr = take(8 * rows), o_sn = take(8 * rows), o_ix = take(8 * rows), o_so = take(rows), o_fo = take(rows),
-                 o_b = take(148 * rows), o_d = take(148 * rows), o_ft = take(sizeof(double2) * N), o_w = take(sizeof(double2) * 16 * osr), o_pm = take(64);
-    const size_t o_nts = nts ? take(sizeof(double2) * 8 * 26 * osr) : 0, o_bc = nts ? take(sizeof(BcchResultDev) * D) : 0;
-    const size_t o_sd = sch_decode ? take(sizeof(SchDecodeResultDev) * D) : 0, o_key = sch_decode ? take(4 * rows) : 0,
-                 o_fn = sch_decode ? take(4 * rows) : 0, o_bs = sch_decode ? take(4 * rows) : 0, o_hm = sch_decode ? take(rows) : 0,
-                 o_rf = sch_decode ? take(rows) : 0;
-    void *base; TRY(c.dem.get(off, &base));
-    char *b = (char *)base;
-    dd->rec = (DemodResultDev *)(b + o_rec); dd->sch_pos = (double *)(b + o_sp); dd->fcch_pos = (double *)(b + o_fp); dd->corr = (double *)(b + o_corr);
-    dd->freq = (double *)(b + o_fr); dd->snr = (double *)(b + o_sn); dd->idx = (double *)(b + o_ix);
-    dd->sch_ok = (unsigned char *)(b + o_so); dd->fcch_ok = (unsigned char *)(b + o_fo); dd->bits = (unsigned char *)(b + o_b); dd->dec = (unsigned char *)(b + o_d);
-    dd->Ft = (double2 *)(b + o_ft); dd->Wtab = (double2 *)(b + o_w); dd->dpm = (signed char *)(b + o_pm);
-    dd->nts = nts ? (double2 *)(b + o_nts) : nullptr; dd->bcch = nts ? (BcchResultDev *)(b + o_bc) : nullptr;
-    dd->sdec = sch_decode ? (SchDecodeResultDev *)(b + o_sd) : nullptr; dd->key = sch_decode ? (int *)(b + o_key) : nullptr;
-    dd->fn = sch_decode ? (int *)(b + o_fn) : nullptr; dd->bsic = sch_decode ? (int *)(b + o_bs) : nullptr;
-    dd->ham = sch_decode ? (unsigned char *)(b + o_hm) : nullptr; dd->rflag = sch_decode ? (unsigned char *)(b + o_rf) : nullptr;
-    if (nts) CU(cudaMemcpyAsync(dd->nts, nts, sizeof(double2) * 8 * 26 * (size_t)osr, cudaMemcpyHostToDevice, st));
+    *t = TailDev{};
+    auto layout = [&](uintptr_t base) {          // points every buffer into [base, base + the size it returns)
+        size_t off = 0;
+        auto take = [&](auto *&p, size_t bytes) { place(p, base + off); off = align_up(off + bytes); };
+        tail_arrays(*t, o, cap, [&](auto *&p, size_t per, const void *) { take(p, per * D); });
+        if (!o.timing) { take(t->Ft, sizeof(double2) * N); take(t->Wtab, sizeof(double2) * 16 * osr); take(t->dpm, 64); }
+        if (o.nts) take(t->nts, sizeof(double2) * 8 * 26 * osr);
+        return off;
+    };
+    void *base; TRY(c.dem.get(layout(0), &base));
+    layout((uintptr_t)base);
+    if (o.timing) return GSMCAL_OK;
+    if (o.nts) CU(cudaMemcpyAsync(t->nts, o.nts, sizeof(double2) * 8 * 26 * (size_t)osr, cudaMemcpyHostToDevice, st));
     W.assign(2 * 16 * (size_t)osr, 0.0);
     gmsk_branch_table(osr, W.data());
     sch_training_pm(data_pm);
-    CU(cudaMemcpyAsync(dd->Wtab, W.data(), sizeof(double) * W.size(), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(dd->dpm, data_pm, 64, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(t->Wtab, W.data(), sizeof(double) * W.size(), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(t->dpm, data_pm, 64, cudaMemcpyHostToDevice, st));
     const double2 *tw; TRY(get_twiddle(c, N, st, &tw));
-    LAUNCH(fde_template_kernel, 1, SD_THREADS, 3 * (size_t)N * sizeof(double2), st, tpl_dev, osr, tw, dd->Ft);
+    LAUNCH(fde_template_kernel, 1, SD_THREADS, 3 * (size_t)N * sizeof(double2), st, tpl_dev, osr, tw, t->Ft);
     return GSMCAL_OK;
 }
-// one stream group: row lists + sentinels, SCH bursts, SCH decoding and BCCH_demod when their outputs were asked for, FCCH bursts, FCCH means
-int run_demod(Ctx &c, WinSrc src, const Work &ws, const DemodDev &dd, int osr, double carrier_freq, i64 nd, int cap, cudaStream_t st) {
-    const double2 *tw_s, *tw_f;
+// one stream group: row lists + sentinels, then either the timing of every SCH row and the per-stream fit (osr 8), or SCH bursts, SCH
+// decoding and BCCH_demod when their outputs were asked for, FCCH bursts, FCCH means
+int run_tail(Ctx &c, WinSrc src, const Work &ws, const TailDev &t, int osr, double carrier_freq, i64 nd, int cap, cudaStream_t st) {
+    LAUNCH(demod_compact_kernel, (unsigned)nd, 32, 0, st, ws.ctl, ws.pos_info, cap, osr, t.rec, t.sch_pos, t.sch_ok, t.fcch_pos, t.fcch_ok);
+    if (t.timing) {
+        LAUNCH(sch_timing_batch_kernel, dim3((unsigned)cap, (unsigned)nd), SCH_THREADS, TM_SMEM, st, src, ws.ctl, t.rec, t.sch_pos, cap, ws.tpl,
+               t.tau, t.row_flag);
+        LAUNCH(sch_timing_fit_kernel, (unsigned)nd, 32, 0, st, ws.ctl, t.rec, t.sch_pos, t.row_flag, t.tau, cap, t.x, t.timing);
+        return GSMCAL_OK;
+    }
+    const double2 *tw_s, *tw_f;                  // both built by the set-up: no launch here
     TRY(get_twiddle(c, SD_NSYM * osr, st, &tw_s));
     TRY(get_twiddle(c, 148 * osr, st, &tw_f));
-    LAUNCH(demod_compact_kernel, (unsigned)nd, 32, 0, st, ws.ctl, ws.pos_info, cap, osr, dd.rec, dd.sch_pos, dd.sch_ok, dd.fcch_pos, dd.fcch_ok);
-    LAUNCH(sch_demod_batch_kernel, dim3((unsigned)cap, (unsigned)nd), SDB_THREADS, sch_demod_smem(osr), st, src, ws.ctl, dd.rec, dd.sch_pos, dd.sch_ok,
-           cap, osr, tw_s, dd.Ft, dd.Wtab, dd.dpm, dd.bits, dd.dec, dd.corr);
-    if (dd.sdec)
-        LAUNCH(sch_decode_batch_kernel, (unsigned)nd, 32, 0, st, dd.rec, dd.sch_pos, dd.sch_ok, dd.bits, dd.corr, cap, osr, dd.key, dd.fn, dd.bsic,
-               dd.ham, dd.rflag, dd.sdec);
+    LAUNCH(sch_demod_batch_kernel, dim3((unsigned)cap, (unsigned)nd), SDB_THREADS, sch_demod_smem(osr), st, src, ws.ctl, t.rec, t.sch_pos, t.sch_ok,
+           cap, osr, tw_s, t.Ft, t.Wtab, t.dpm, t.bits, t.dec, t.corr);
+    if (t.sdec)
+        LAUNCH(sch_decode_batch_kernel, (unsigned)nd, 32, 0, st, t.rec, t.sch_pos, t.sch_ok, t.bits, t.corr, cap, osr, t.key, t.fn, t.bsic,
+               t.ham, t.rflag, t.sdec);
     const size_t fs = fcch_demod_smem(osr), fs_load = sizeof(double2) * (3 * 148 * (size_t)osr + 144);      // + the loader's scratch behind u
-    LAUNCH(fcch_demod_batch_kernel, dim3((unsigned)cap, (unsigned)nd), FD_THREADS, fs > fs_load ? fs : fs_load, st, with_cache(src, ws, cap), ws.ctl, dd.rec,
-           dd.fcch_pos, dd.fcch_ok, cap, osr, tw_f, dd.freq, dd.snr, dd.idx);
-    LAUNCH(demod_fcch_mean_kernel, (unsigned)((nd + 127) / 128), 128, 0, st, dd.rec, (int)nd, dd.freq, cap, carrier_freq);
-    if (dd.bcch) {
+    LAUNCH(fcch_demod_batch_kernel, dim3((unsigned)cap, (unsigned)nd), FD_THREADS, fs > fs_load ? fs : fs_load, st, with_cache(src, ws, cap), ws.ctl, t.rec,
+           t.fcch_pos, t.fcch_ok, cap, osr, tw_f, t.freq, t.snr, t.idx);
+    LAUNCH(demod_fcch_mean_kernel, (unsigned)((nd + 127) / 128), 128, 0, st, t.rec, (int)nd, t.freq, cap, carrier_freq);
+    if (t.bcch) {
         const int L = 26 * osr;
-        LAUNCH(bcch_demod_batch_kernel, (unsigned)nd, BC_THREADS, sizeof(double2) * (size_t)(L + GSMCAL_XCAP(L) + L + 8), st, src, ws.ctl, dd.rec, ws.pos_info,
-               cap, osr, dd.nts, dd.bcch);
+        LAUNCH(bcch_demod_batch_kernel, (unsigned)nd, BC_THREADS, sizeof(double2) * (size_t)(L + GSMCAL_XCAP(L) + L + 8), st, src, ws.ctl, t.rec, ws.pos_info,
+               cap, osr, t.nts, t.bcch);
     }
-    return GSMCAL_OK;
-}
-
-// ---- sub-sample SCH timing stage of gsmcal_calibrate_sch_timing_batch ----------------------------------------------------------
-struct TimingOut { gsmcal_sch_timing_result *rec; double *tau, *x; };    // the caller's host outputs (tau, x may be NULL)
-struct TimingDev {                   // device buffers, [D][cap] rows unless noted
-    DemodResultDev *rows /* [D] */; double *sch_pos, *fcch_pos, *tau, *x; unsigned char *sch_ok, *fcch_ok, *row_flag; TimingResultDev *rec /* [D] */;
-};
-TimingDev sub_timing(const TimingDev &a, i64 d0, int cap) {
-    TimingDev s = a;
-    const i64 r = d0 * cap;
-    s.rows += d0; s.rec += d0; s.sch_pos += r; s.fcch_pos += r; s.tau += r; s.x += r; s.sch_ok += r; s.fcch_ok += r; s.row_flag += r;
-    return s;
-}
-int timing_setup(Ctx &c, i64 D, int cap, TimingDev *td) {
-    size_t off = 0;
-    auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes); return o; };
-    const size_t rows = (size_t)D * cap;
-    const size_t o_rows = take(sizeof(DemodResultDev) * D), o_rec = take(sizeof(TimingResultDev) * D), o_sp = take(8 * rows), o_fp = take(8 * rows),
-                 o_tau = take(8 * rows), o_x = take(8 * rows), o_so = take(rows), o_fo = take(rows), o_rf = take(rows);
-    void *base; TRY(c.dem.get(off, &base));
-    char *b = (char *)base;
-    td->rows = (DemodResultDev *)(b + o_rows); td->rec = (TimingResultDev *)(b + o_rec); td->sch_pos = (double *)(b + o_sp);
-    td->fcch_pos = (double *)(b + o_fp); td->tau = (double *)(b + o_tau); td->x = (double *)(b + o_x);
-    td->sch_ok = (unsigned char *)(b + o_so); td->fcch_ok = (unsigned char *)(b + o_fo); td->row_flag = (unsigned char *)(b + o_rf);
-    return GSMCAL_OK;
-}
-// one stream group: the row lists of the demod stage, the timing of every SCH row, the per-stream fit (osr 8)
-int run_timing(WinSrc src, const Work &ws, const TimingDev &td, i64 nd, int cap, cudaStream_t st) {
-    LAUNCH(demod_compact_kernel, (unsigned)nd, 32, 0, st, ws.ctl, ws.pos_info, cap, 8, td.rows, td.sch_pos, td.sch_ok, td.fcch_pos, td.fcch_ok);
-    LAUNCH(sch_timing_batch_kernel, dim3((unsigned)cap, (unsigned)nd), SCH_THREADS, TM_SMEM, st, src, ws.ctl, td.rows, td.sch_pos, cap, ws.tpl,
-           td.tau, td.row_flag);
-    LAUNCH(sch_timing_fit_kernel, (unsigned)nd, 32, 0, st, ws.ctl, td.rows, td.sch_pos, td.row_flag, td.tau, cap, td.x, td.rec);
     return GSMCAL_OK;
 }
 
@@ -719,10 +700,10 @@ int batch_setup(Ctx &c, DevBuf &work, DevBuf &wc, const double *tpl, const doubl
     return GSMCAL_OK;
 }
 
-// the burst stages of one stream group, in order on sg: fine peak, fine rest (ppm, tone, carrier), SCH, post-SCH and, with dd, the demod
-// stage or, with td, the SCH timing stage.  With marks, marks[i] is recorded on sg behind stage i (null entries are skipped)
+// the burst stages of one stream group, in order on sg: fine peak, fine rest (ppm, tone, carrier), SCH, post-SCH and, with tail, the tail
+// stage.  With marks, marks[i] is recorded on sg behind stage i (null entries are skipped)
 int run_burst_stages(Ctx &c, const uint8_t *graw, i64 n_iq, int n_taps, int osr, double carrier_freq, i64 nd, int cap, Work &ws,
-                     const DemodDev *dd, const TimingDev *td, cudaStream_t sg, const cudaEvent_t *marks) {
+                     const TailDev *tail, cudaStream_t sg, const cudaEvent_t *marks) {
     auto mark = [&](int i) { if (marks && marks[i]) CU(cudaEventRecord(marks[i], sg)); return GSMCAL_OK; };
     TRY(run_fine_peak(c, lazy_src(graw, n_iq, n_taps, 0, 1), n_iq, osr, nd, cap, ws, sg));
     TRY(mark(0));
@@ -732,11 +713,8 @@ int run_burst_stages(Ctx &c, const uint8_t *graw, i64 n_iq, int n_taps, int osr,
     TRY(mark(2));
     TRY(run_post(c, with_cache(lazy_src(graw, n_iq, n_taps, 3, 1), ws, cap), osr, carrier_freq, nd, cap, ws, true, sg));
     TRY(mark(3));
-    if (dd) {
-        TRY(run_demod(c, lazy_src(graw, n_iq, n_taps, 3, 1), ws, *dd, osr, carrier_freq, nd, cap, sg));
-        TRY(mark(4));
-    } else if (td) {
-        TRY(run_timing(lazy_src(graw, n_iq, n_taps, 3, 1), ws, *td, nd, cap, sg));
+    if (tail) {
+        TRY(run_tail(c, lazy_src(graw, n_iq, n_taps, 3, 1), ws, *tail, osr, carrier_freq, nd, cap, sg));
         TRY(mark(4));
     }
     return GSMCAL_OK;
@@ -1202,7 +1180,7 @@ int gsmcal_total_ppm_calculation(const double *ppm_in, int64_t n, double *ppm_ou
 static int calibrate_batch_impl(const uint8_t *raw, int raw_mem, int64_t n_iq, int64_t D, double carrier_freq, const double *tpl,
                                 const double *coef, int n_taps, int osr, int coarse_dr, gsmcal_stream_result *results,
                                 double *coarse_pos, double *coarse_snr, double *fcch_pos, double *pos_info, void *cuda_stream,
-                                double *r_out, int r_mem, int64_t r_stride, const DemodOut *dm = nullptr, const TimingOut *tm = nullptr) {
+                                double *r_out, int r_mem, int64_t r_stride, const TailOut *tail = nullptr) {
     std::lock_guard<std::mutex> lk(g_mu);
     if (r_out && r_stride < n_iq) return fail(GSMCAL_ERR_ARG, "calibrate_batch_r: r_stride must be >= n_iq");
     Batch b; TRY(batch_args("calibrate_batch", raw, tpl, coef, results, n_iq, D, osr, coarse_dr, &b));
@@ -1217,11 +1195,9 @@ static int calibrate_batch_impl(const uint8_t *raw, int raw_mem, int64_t n_iq, i
         void *din; TRY(c->in.get((size_t)2 * n_iq * D, &din));
         draw = (const uint8_t *)din;
     }
-    DemodDev dd;
-    std::vector<double> dm_w; signed char dm_pm[64];                 // host sources of the uploads, alive until the final synchronise
-    if (dm) TRY(demod_setup(*c, D, cap, osr, w.tpl, dm->nts, dm->sdec != nullptr, dm_w, dm_pm, st, &dd));
-    TimingDev td;
-    if (tm) TRY(timing_setup(*c, D, cap, &td));
+    TailDev td;
+    std::vector<double> tail_w; signed char tail_pm[64];             // host sources of the uploads, alive until the final synchronise
+    if (tail) TRY(tail_setup(*c, D, cap, osr, w.tpl, *tail, tail_w, tail_pm, st, &td));
     g_stage_n = 0;
     // Streams are independent, so the batch is cut into groups that run the stage sequence on their own CUDA
     // streams: the latency-bound stages of one group (burst chain, per-stream solves) overlap the FP64-bound
@@ -1274,11 +1250,11 @@ static int calibrate_batch_impl(const uint8_t *raw, int raw_mem, int64_t n_iq, i
         if (timing) TRY(stage_mark(*c, sg));
         // stagger the groups (see gsmcal_calibrate_batch_submit): the FP64 stages of group g wait for group g-1, its front does not
         if (!ev_done.empty()) CU(cudaStreamWaitEvent(sg, ev_done.back(), 0));
-        const DemodDev gdd = dm ? sub_demod(dd, d0, cap) : DemodDev{};
-        const TimingDev gtd = tm ? sub_timing(td, d0, cap) : TimingDev{};
-        TRY(run_burst_stages(*c, graw, n_iq, n_taps, osr, carrier_freq, nd, cap, ws, dm ? &gdd : nullptr, tm ? &gtd : nullptr, sg,
+        TailDev gtd = td;                                        // the group's rows of every per-stream array
+        if (tail) tail_arrays(gtd, *tail, cap, [&](auto *&p, size_t per, const void *) { place(p, (uintptr_t)p + d0 * per); });
+        TRY(run_burst_stages(*c, graw, n_iq, n_taps, osr, carrier_freq, nd, cap, ws, tail ? &gtd : nullptr, sg,
                              timing ? c->stage_ev + g_stage_n : nullptr));
-        if (timing) g_stage_n += (dm || tm) ? 5 : 4;             // 3 + 5 <= kNumStageEvents
+        if (timing) g_stage_n += tail ? 5 : 4;                   // 3 + 5 <= kNumStageEvents
         if (sg != st) {
             cudaEvent_t ev; CU(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
             CU(cudaEventRecord(ev, sg));
@@ -1308,27 +1284,10 @@ static int calibrate_batch_impl(const uint8_t *raw, int raw_mem, int64_t n_iq, i
     if (coarse_snr) CU(cudaMemcpyAsync(coarse_snr, w.coarse_snr, sizeof(double) * D * cap, cudaMemcpyDeviceToHost, st));
     if (fcch_pos) CU(cudaMemcpyAsync(fcch_pos, w.fcch_pos, sizeof(double) * D * cap, cudaMemcpyDeviceToHost, st));
     if (pos_info) CU(cudaMemcpyAsync(pos_info, w.pos_info, sizeof(double) * D * cap * 12, cudaMemcpyDeviceToHost, st));
-    if (dm) {
-        const size_t rows = (size_t)D * cap;
-        CU(cudaMemcpyAsync(dm->rec, dd.rec, sizeof(DemodResultDev) * D, cudaMemcpyDeviceToHost, st));
-        if (dm->sch_ok) TRY(copy_d2h(c->ring, g_device, dm->sch_ok, dd.sch_ok, rows, st));
-        if (dm->bits) TRY(copy_d2h(c->ring, g_device, dm->bits, dd.bits, 148 * rows, st));
-        if (dm->dec) TRY(copy_d2h(c->ring, g_device, dm->dec, dd.dec, 148 * rows, st));
-        if (dm->corr) TRY(copy_d2h(c->ring, g_device, dm->corr, dd.corr, sizeof(double) * 85 * rows, st));
-        if (dm->freq) TRY(copy_d2h(c->ring, g_device, dm->freq, dd.freq, sizeof(double) * rows, st));
-        if (dm->snr) TRY(copy_d2h(c->ring, g_device, dm->snr, dd.snr, sizeof(double) * rows, st));
-        if (dm->idx) TRY(copy_d2h(c->ring, g_device, dm->idx, dd.idx, sizeof(double) * rows, st));
-        if (dm->bcch) CU(cudaMemcpyAsync(dm->bcch, dd.bcch, sizeof(BcchResultDev) * D, cudaMemcpyDeviceToHost, st));
-        if (dm->sdec) CU(cudaMemcpyAsync(dm->sdec, dd.sdec, sizeof(SchDecodeResultDev) * D, cudaMemcpyDeviceToHost, st));
-        if (dm->fn) TRY(copy_d2h(c->ring, g_device, dm->fn, dd.fn, sizeof(int) * rows, st));
-        if (dm->bsic) TRY(copy_d2h(c->ring, g_device, dm->bsic, dd.bsic, sizeof(int) * rows, st));
-        if (dm->ham) TRY(copy_d2h(c->ring, g_device, dm->ham, dd.ham, rows, st));
-        if (dm->rflag) TRY(copy_d2h(c->ring, g_device, dm->rflag, dd.rflag, rows, st));
-    }
-    if (tm) {
-        CU(cudaMemcpyAsync(tm->rec, td.rec, sizeof(TimingResultDev) * D, cudaMemcpyDeviceToHost, st));
-        if (tm->tau) TRY(copy_d2h(c->ring, g_device, tm->tau, td.tau, sizeof(double) * D * cap, st));
-        if (tm->x) TRY(copy_d2h(c->ring, g_device, tm->x, td.x, sizeof(double) * D * cap, st));
+    if (tail) {
+        int rc = GSMCAL_OK;
+        tail_arrays(td, *tail, cap, [&](auto *p, size_t per, void *h) { if (h && rc == GSMCAL_OK) rc = copy_d2h(c->ring, g_device, h, p, per * D, st); });
+        TRY(rc);
     }
     CU(cudaStreamSynchronize(st));
     if (timing) for (int i = 0; i + 1 < g_stage_n; ++i) CU(cudaEventElapsedTime(&g_stage_ms[i], c->stage_ev[i], c->stage_ev[i + 1]));
@@ -1358,8 +1317,9 @@ int gsmcal_calibrate_demod_batch(const uint8_t *raw, int raw_mem, int64_t n_iq, 
                                  gsmcal_demod_result *demod, uint8_t *sch_ok, uint8_t *demod_bits, uint8_t *bits_to_decoder, double *corr_val,
                                  double *fcch_freq, double *fcch_snr, double *fcch_max_idx) {
     if (!demod) return fail(GSMCAL_ERR_ARG, "calibrate_demod_batch: null demod");
-    const DemodOut o = {demod, sch_ok, demod_bits, bits_to_decoder, corr_val, fcch_freq, fcch_snr, fcch_max_idx, nullptr, nullptr,
-                        nullptr, nullptr, nullptr, nullptr, nullptr};
+    TailOut o{};
+    o.demod = demod; o.sch_ok = sch_ok; o.bits = demod_bits; o.dec = bits_to_decoder; o.corr = corr_val; o.freq = fcch_freq; o.snr = fcch_snr;
+    o.idx = fcch_max_idx;
     return calibrate_batch_impl(raw, raw_mem, n_iq, D, carrier_freq, tpl, coef, n_taps, osr, coarse_dr, results, coarse_pos, coarse_snr, fcch_pos, pos_info,
                                 cuda_stream, nullptr, GSMCAL_MEM_DEVICE, 0, &o);
 }
@@ -1371,8 +1331,9 @@ int gsmcal_calibrate_demod_bcch_batch(const uint8_t *raw, int raw_mem, int64_t n
                                       double *fcch_freq, double *fcch_snr, double *fcch_max_idx,
                                       const double *normal_training_sequence, gsmcal_bcch_result *bcch) {
     if (!demod || !normal_training_sequence || !bcch) return fail(GSMCAL_ERR_ARG, "calibrate_demod_bcch_batch: null demod, normal_training_sequence or bcch");
-    const DemodOut o = {demod, sch_ok, demod_bits, bits_to_decoder, corr_val, fcch_freq, fcch_snr, fcch_max_idx, normal_training_sequence, bcch,
-                        nullptr, nullptr, nullptr, nullptr, nullptr};
+    TailOut o{};
+    o.demod = demod; o.sch_ok = sch_ok; o.bits = demod_bits; o.dec = bits_to_decoder; o.corr = corr_val; o.freq = fcch_freq; o.snr = fcch_snr;
+    o.idx = fcch_max_idx; o.nts = normal_training_sequence; o.bcch = bcch;
     return calibrate_batch_impl(raw, raw_mem, n_iq, D, carrier_freq, tpl, coef, n_taps, osr, coarse_dr, results, coarse_pos, coarse_snr, fcch_pos, pos_info,
                                 cuda_stream, nullptr, GSMCAL_MEM_DEVICE, 0, &o);
 }
@@ -1386,8 +1347,10 @@ int gsmcal_calibrate_sch_decode_batch(const uint8_t *raw, int raw_mem, int64_t n
                                       gsmcal_sch_decode_result *dec, int32_t *sch_fn, int32_t *sch_bsic, uint8_t *sch_hamming, uint8_t *sch_row_flags) {
     if (!demod || !dec) return fail(GSMCAL_ERR_ARG, "calibrate_sch_decode_batch: null demod or dec");
     if (!normal_training_sequence != !bcch) return fail(GSMCAL_ERR_ARG, "calibrate_sch_decode_batch: normal_training_sequence and bcch must both be set or both NULL");
-    const DemodOut o = {demod, sch_ok, demod_bits, bits_to_decoder, corr_val, fcch_freq, fcch_snr, fcch_max_idx, normal_training_sequence, bcch,
-                        dec, sch_fn, sch_bsic, sch_hamming, sch_row_flags};
+    TailOut o{};
+    o.demod = demod; o.sch_ok = sch_ok; o.bits = demod_bits; o.dec = bits_to_decoder; o.corr = corr_val; o.freq = fcch_freq; o.snr = fcch_snr;
+    o.idx = fcch_max_idx; o.nts = normal_training_sequence; o.bcch = bcch;
+    o.sdec = dec; o.fn = sch_fn; o.bsic = sch_bsic; o.ham = sch_hamming; o.rflag = sch_row_flags;
     return calibrate_batch_impl(raw, raw_mem, n_iq, D, carrier_freq, tpl, coef, n_taps, osr, coarse_dr, results, coarse_pos, coarse_snr, fcch_pos, pos_info,
                                 cuda_stream, nullptr, GSMCAL_MEM_DEVICE, 0, &o);
 }
@@ -1398,9 +1361,10 @@ int gsmcal_calibrate_sch_timing_batch(const uint8_t *raw, int raw_mem, int64_t n
                                       gsmcal_sch_timing_result *timing, double *sch_tau, double *sch_x) {
     if (!timing) return fail(GSMCAL_ERR_ARG, "calibrate_sch_timing_batch: null timing");
     if (osr != 8) return fail(GSMCAL_ERR_ARG, "calibrate_sch_timing_batch: oversampling_ratio must be 8");
-    const TimingOut o = {timing, sch_tau, sch_x};
+    TailOut o{};
+    o.timing = timing; o.tau = sch_tau; o.x = sch_x;
     return calibrate_batch_impl(raw, raw_mem, n_iq, D, carrier_freq, tpl, coef, n_taps, osr, coarse_dr, results, coarse_pos, coarse_snr, fcch_pos, pos_info,
-                                cuda_stream, nullptr, GSMCAL_MEM_DEVICE, 0, nullptr, &o);
+                                cuda_stream, nullptr, GSMCAL_MEM_DEVICE, 0, &o);
 }
 
 // ---- submit / collect: the same pipeline, several batches in flight -----------------------------------------------------------
@@ -1477,7 +1441,7 @@ int gsmcal_calibrate_batch_submit(int slot, const uint8_t *raw_dev, int64_t n_iq
             CU(cudaStreamWaitEvent(sg, c->slots[c->last_slot].done, 0));
         if (tl_g) CU(cudaEventRecord(sl.tl[4], sg));
         const cudaEvent_t marks[4] = {sl.tl[5], sl.tl[6], sl.tl[7], sl.tl[3]};
-        TRY(run_burst_stages(*c, graw, n_iq, n_taps, osr, carrier_freq, nd, cap, ws, nullptr, nullptr, sg, tl_g ? marks : nullptr));
+        TRY(run_burst_stages(*c, graw, n_iq, n_taps, osr, carrier_freq, nd, cap, ws, nullptr, sg, tl_g ? marks : nullptr));
         TRY(hand_off(sg, fr));
     }
     CU(cudaMemcpyAsync(h_res, w.res, sl.n_res, cudaMemcpyDeviceToHost, fr));

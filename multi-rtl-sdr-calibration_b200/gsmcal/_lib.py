@@ -38,6 +38,10 @@ class SchDecodeResult(C.Structure):
                 ("fn_first", C.c_int32), ("frame_clock_start", C.c_double)]
 
 
+# the leading arguments of gsmcal_calibrate_batch and its variants: raw, raw_mem, n_iq, D, carrier_freq, tpl, coef, n_taps, osr,
+# coarse_dr, results, coarse_pos, coarse_snr, fcch_pos, pos_info, cuda_stream
+_BATCH = [C.c_void_p, C.c_int, c_i64, c_i64, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 6
+
 # every symbol include/gsmcal.h declares: name -> (restype, argtypes)
 SIGNATURES = {
     "gsmcal_abi_version": (C.c_int, []),
@@ -74,24 +78,12 @@ SIGNATURES = {
                                     C.POINTER(C.c_double), C.POINTER(C.c_int), C.c_void_p]),
     "gsmcal_SCH_demod": (C.c_int, [C.c_void_p, c_i64, C.c_void_p, c_i64, C.c_void_p, C.c_int, c_i64, C.POINTER(c_i64),
                                    C.c_void_p, C.c_void_p, C.c_void_p]),
-    "gsmcal_calibrate_batch": (C.c_int, [C.c_void_p, C.c_int, c_i64, c_i64, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
-                                         C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
-    "gsmcal_calibrate_batch_r": (C.c_int, [C.c_void_p, C.c_int, c_i64, c_i64, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
-                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, c_i64]),
-    "gsmcal_calibrate_demod_batch": (C.c_int, [C.c_void_p, C.c_int, c_i64, c_i64, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
-                                               C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
-                                               C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
-    "gsmcal_calibrate_demod_bcch_batch": (C.c_int, [C.c_void_p, C.c_int, c_i64, c_i64, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
-                                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
-                                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
-                                                    C.c_void_p, C.c_void_p]),
-    "gsmcal_calibrate_sch_decode_batch": (C.c_int, [C.c_void_p, C.c_int, c_i64, c_i64, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
-                                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
-                                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
-                                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
-    "gsmcal_calibrate_sch_timing_batch": (C.c_int, [C.c_void_p, C.c_int, c_i64, c_i64, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
-                                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
-                                                    C.c_void_p, C.c_void_p, C.c_void_p]),
+    "gsmcal_calibrate_batch": (C.c_int, _BATCH),
+    "gsmcal_calibrate_batch_r": (C.c_int, _BATCH + [C.c_void_p, C.c_int, c_i64]),
+    "gsmcal_calibrate_demod_batch": (C.c_int, _BATCH + [C.c_void_p] * 8),
+    "gsmcal_calibrate_demod_bcch_batch": (C.c_int, _BATCH + [C.c_void_p] * 10),
+    "gsmcal_calibrate_sch_decode_batch": (C.c_int, _BATCH + [C.c_void_p] * 15),
+    "gsmcal_calibrate_sch_timing_batch": (C.c_int, _BATCH + [C.c_void_p] * 3),
     "gsmcal_calibrate_batch_submit": (C.c_int, [C.c_int, C.c_void_p, c_i64, c_i64, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "gsmcal_calibrate_batch_collect": (C.c_int, [C.c_int]),

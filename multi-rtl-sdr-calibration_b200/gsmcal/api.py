@@ -305,6 +305,28 @@ def _unpack_results(res, D, cap, coarse_pos, coarse_snr, fcch_pos, pos_info):
     return out
 
 
+def _batch_args(raw, carrier_freq, sch_training_sequence, coef, osr, coarse_dr, device_ptr, n_iq, n_streams, cuda_stream, details):
+    """The 16 leading arguments of gsmcal_calibrate_batch and its variants, for `raw` ([D, 2N] uint8 on the host, or one row) or, with
+    device_ptr, a capture of n_streams x n_iq resident in HBM.  Returns (args, keep, D, n_iq, cap, res, arrays): keep holds the host
+    arrays args point into, res the D result records, arrays (coarse_pos, coarse_snr, fcch_pos, pos_info), or None without details."""
+    tpl = _stream(sch_training_sequence)
+    coef = np.ascontiguousarray(coef, dtype=np.float64)
+    if device_ptr is None:
+        raw = np.ascontiguousarray(raw, dtype=np.uint8)
+        if raw.ndim == 1:
+            raw = raw[None, :]
+        D, n_iq = raw.shape[0], raw.shape[1] // 2
+        ptr, mem = _ptr(raw), 0
+    else:
+        D, ptr, mem = int(n_streams), C.c_void_p(int(device_ptr)), 1
+    cap = max_bursts(n_iq, osr, coarse_dr)
+    res = (StreamResult * D)()
+    arrays = (np.empty((D, cap)), np.empty((D, cap)), np.empty((D, cap)), np.empty((D, 6 * cap, 2))) if details else None
+    args = [ptr, mem, int(n_iq), D, float(carrier_freq), _ptr(tpl), _ptr(coef), len(coef), int(osr), int(coarse_dr), C.cast(res, C.c_void_p),
+            *([_ptr(a) for a in arrays] if details else [None] * 4), C.c_void_p(cuda_stream)]
+    return args, (raw, tpl, coef), D, n_iq, cap, res, arrays
+
+
 def calibrate_batch(raw, carrier_freq: float, sch_training_sequence, coef, osr: int = 8, coarse_dr: int = 8,
                     device_ptr: int | None = None, n_iq: int | None = None, n_streams: int | None = None,
                     cuda_stream: int = 0, details: bool = True, r_correct=None, r_device_ptr: int | None = None,
@@ -320,37 +342,17 @@ def calibrate_batch(raw, carrier_freq: float, sch_training_sequence, coef, osr: 
     training start, fit_ppm the sample clock error of the fit, rms its residual (samples), flags TIMING_* bits, and per SCH row tau (time
     in r_correct, 1-based) and x (time in the uint8 capture, 0-based), NaN where excluded; tau and x are None when the step did not
     run (TIMING_NO_POS_INFO / TIMING_NO_R_CORRECT)."""
-    tpl = _stream(sch_training_sequence)
-    coef = np.ascontiguousarray(coef, dtype=np.float64)
-    if device_ptr is None:
-        raw = np.ascontiguousarray(raw, dtype=np.uint8)
-        if raw.ndim == 1:
-            raw = raw[None, :]
-        D, n_iq = raw.shape[0], raw.shape[1] // 2
-        ptr, mem = _ptr(raw), 0
-    else:
-        D, ptr, mem = int(n_streams), C.c_void_p(int(device_ptr)), 1
-    cap = max_bursts(n_iq, osr, coarse_dr)
-    res = (StreamResult * D)()
     if sch_timing and (r_correct is not None or r_device_ptr is not None):
         raise ValueError("sch_timing does not combine with r_correct / r_device_ptr")
     details = details or sch_timing
-    if details:
-        coarse_pos, coarse_snr, fcch_pos = np.empty((D, cap)), np.empty((D, cap)), np.empty((D, cap))
-        pos_info = np.empty((D, 6 * cap, 2))
-        ptrs = [_ptr(coarse_pos), _ptr(coarse_snr), _ptr(fcch_pos), _ptr(pos_info)]
-    else:
-        coarse_pos = coarse_snr = fcch_pos = pos_info = None
-        ptrs = [None] * 4
+    args, keep, D, n_iq, cap, res, arrays = _batch_args(raw, carrier_freq, sch_training_sequence, coef, osr, coarse_dr, device_ptr, n_iq,
+                                                        n_streams, cuda_stream, details)
     if sch_timing:
         tm = (SchTimingResult * D)()
         tau, x = np.empty((D, cap)), np.empty((D, cap))
-        check(lib().gsmcal_calibrate_sch_timing_batch(ptr, mem, int(n_iq), D, float(carrier_freq), _ptr(tpl), _ptr(coef), len(coef),
-                                                      int(osr), int(coarse_dr), C.cast(res, C.c_void_p), *ptrs, C.c_void_p(cuda_stream),
-                                                      C.cast(tm, C.c_void_p), _ptr(tau), _ptr(x)))
+        check(lib().gsmcal_calibrate_sch_timing_batch(*args, C.cast(tm, C.c_void_p), _ptr(tau), _ptr(x)))
     elif r_correct is None and r_device_ptr is None:
-        check(lib().gsmcal_calibrate_batch(ptr, mem, int(n_iq), D, float(carrier_freq), _ptr(tpl), _ptr(coef), len(coef),
-                                           int(osr), int(coarse_dr), C.cast(res, C.c_void_p), *ptrs, C.c_void_p(cuda_stream)))
+        check(lib().gsmcal_calibrate_batch(*args))
     else:
         # r_correct: a [D, n_iq] complex128 host array to fill, or r_device_ptr: a device buffer of D * n_iq complex128
         if r_device_ptr is not None:
@@ -358,11 +360,10 @@ def calibrate_batch(raw, carrier_freq: float, sch_training_sequence, coef, osr: 
         else:
             assert r_correct.dtype == np.complex128 and r_correct.flags.c_contiguous and r_correct.shape == (D, n_iq)
             rp, rmem = _ptr(r_correct), 0
-        check(lib().gsmcal_calibrate_batch_r(ptr, mem, int(n_iq), D, float(carrier_freq), _ptr(tpl), _ptr(coef), len(coef),
-                                             int(osr), int(coarse_dr), C.cast(res, C.c_void_p), *ptrs, C.c_void_p(cuda_stream), rp, rmem, int(n_iq)))
+        check(lib().gsmcal_calibrate_batch_r(*args, rp, rmem, int(n_iq)))
     if not details:
         return res
-    out = _unpack_results(res, D, cap, coarse_pos, coarse_snr, fcch_pos, pos_info)
+    out = _unpack_results(res, D, cap, *arrays)
     if sch_timing:
         for d, item in enumerate(out):
             t = tm[d]
@@ -405,27 +406,14 @@ def calibrate_demod_batch(raw, carrier_freq: float, sch_training_sequence, coef,
             winner, flags SCHDEC_* bits, and per SCH row fn, bsic_rows (-1 where not decoded), hamming and row_flags (SCHDEC_ROW_*);
             the per-row arrays are None where SCH_demod did not run.  A winner with n_agree 1 may be a false CRC pass (about 1 in 1024
             rows of noise passes the 10-bit CRC)."""
-    tpl = _stream(sch_training_sequence)
-    coef = np.ascontiguousarray(coef, dtype=np.float64)
-    if device_ptr is None:
-        raw = np.ascontiguousarray(raw, dtype=np.uint8)
-        if raw.ndim == 1:
-            raw = raw[None, :]
-        D, n_iq = raw.shape[0], raw.shape[1] // 2
-        ptr, mem = _ptr(raw), 0
-    else:
-        D, ptr, mem = int(n_streams), C.c_void_p(int(device_ptr)), 1
-    cap = max_bursts(n_iq, osr, coarse_dr)
-    res, dem = (StreamResult * D)(), (DemodResult * D)()
-    coarse_pos, coarse_snr, fcch_pos = np.empty((D, cap)), np.empty((D, cap)), np.empty((D, cap))
-    pos_info = np.empty((D, 6 * cap, 2))
+    args, keep, D, n_iq, cap, res, arrays = _batch_args(raw, carrier_freq, sch_training_sequence, coef, osr, coarse_dr, device_ptr, n_iq,
+                                                        n_streams, cuda_stream, True)
+    dem = (DemodResult * D)()
     sch_ok = np.zeros((D, cap), dtype=np.uint8)
     bits, dec = np.zeros((D, cap, 148), dtype=np.uint8), np.zeros((D, cap, 148), dtype=np.uint8)
     corr = np.zeros((D, cap, 85))
     freq, snr, idx = np.empty((D, cap)), np.empty((D, cap)), np.empty((D, cap))
-    args = [ptr, mem, int(n_iq), D, float(carrier_freq), _ptr(tpl), _ptr(coef), len(coef), int(osr), int(coarse_dr),
-            C.cast(res, C.c_void_p), _ptr(coarse_pos), _ptr(coarse_snr), _ptr(fcch_pos), _ptr(pos_info),
-            C.c_void_p(cuda_stream), C.cast(dem, C.c_void_p), _ptr(sch_ok), _ptr(bits), _ptr(dec), _ptr(corr), _ptr(freq), _ptr(snr), _ptr(idx)]
+    args += [C.cast(dem, C.c_void_p), _ptr(sch_ok), _ptr(bits), _ptr(dec), _ptr(corr), _ptr(freq), _ptr(snr), _ptr(idx)]
     nts_args = [None, None]
     if normal_training_sequence is not None:
         nts_m = np.asarray(normal_training_sequence)
@@ -443,7 +431,7 @@ def calibrate_demod_batch(raw, carrier_freq: float, sch_training_sequence, coef,
         check(lib().gsmcal_calibrate_demod_batch(*args))
     else:
         check(lib().gsmcal_calibrate_demod_bcch_batch(*args, *nts_args))
-    out = _unpack_results(res, D, cap, coarse_pos, coarse_snr, fcch_pos, pos_info)
+    out = _unpack_results(res, D, cap, *arrays)
     for d, item in enumerate(out):
         r = dem[d]
         item["demod_flags"] = r.flags
@@ -516,19 +504,10 @@ def calibrate_batch_submit(slot: int, device_ptr: int, n_iq: int, n_streams: int
                            osr: int = 8, coarse_dr: int = 8, cuda_stream: int = 0, details: bool = False) -> PendingBatch:
     """Enqueue gsm_sync_demod.m:107-124 for a capture resident in HBM and return at once; `.collect()` waits for the results.
     Up to 4 slots may be in flight: the front of batch k+1 overlaps the FP64-bound stages of batch k on the device."""
-    tpl = _stream(sch_training_sequence)
-    coef = np.ascontiguousarray(coef, dtype=np.float64)
-    D = int(n_streams)
-    cap = max_bursts(n_iq, osr, coarse_dr)
-    res = (StreamResult * D)()
-    if details:
-        arrays = (np.empty((D, cap)), np.empty((D, cap)), np.empty((D, cap)), np.empty((D, 6 * cap, 2)))
-        ptrs = [_ptr(a) for a in arrays]
-    else:
-        arrays, ptrs = None, [None] * 4
-    check(lib().gsmcal_calibrate_batch_submit(int(slot), C.c_void_p(int(device_ptr)), int(n_iq), D, float(carrier_freq), _ptr(tpl), _ptr(coef),
-                                              len(coef), int(osr), int(coarse_dr), C.cast(res, C.c_void_p), *ptrs, C.c_void_p(cuda_stream)))
-    return PendingBatch(int(slot), D, cap, res, arrays, (tpl, coef))
+    args, keep, D, n_iq, cap, res, arrays = _batch_args(None, carrier_freq, sch_training_sequence, coef, osr, coarse_dr, device_ptr, n_iq,
+                                                        n_streams, cuda_stream, details)
+    check(lib().gsmcal_calibrate_batch_submit(int(slot), args[0], *args[2:]))             # no raw_mem: the capture is on the device
+    return PendingBatch(int(slot), D, cap, res, arrays, keep)
 
 
 STAGE_NAMES = ("colsum_u8", "coarse", "fine_peak", "fine_tone", "sch", "post", "demod")

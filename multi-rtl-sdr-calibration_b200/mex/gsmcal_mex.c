@@ -87,6 +87,28 @@ static const double *real_vector(const mxArray *a, size_t *n) {
 static void need(int nrhs, int want, const char *usage) {
     if (nrhs != want) mexErrMsgIdAndTxt("gsmcal:nargin", "usage: %s", usage);
 }
+/* the first four outputs of the batch gateways, as many as asked for: sampling_ppm, carrier_ppm (3 x D), n_pos_info (1 x D) and pos_info
+ * ((6B) x 2 x D, NaN beyond n_pos_info(d)), from the D records and pi ([D][6B][2]) of a batch call */
+static void batch_outputs(int nlhs, mxArray *plhs[], const gsmcal_stream_result *res, const double *pi, size_t D, size_t B) {
+    plhs[0] = mxCreateDoubleMatrix(3, D, mxREAL);
+    if (nlhs > 1) plhs[1] = mxCreateDoubleMatrix(3, D, mxREAL);
+    if (nlhs > 2) plhs[2] = mxCreateDoubleMatrix(1, D, mxREAL);
+    for (size_t d = 0; d < D; ++d) {
+        double *sp = mxGetPr(plhs[0]) + 3 * d;
+        sp[0] = res[d].sampling_ppm[0]; sp[1] = res[d].sampling_ppm[1]; sp[2] = res[d].total_sampling_ppm;
+        if (nlhs > 1) { double *cp = mxGetPr(plhs[1]) + 3 * d; cp[0] = res[d].carrier_ppm[0]; cp[1] = res[d].carrier_ppm[1]; cp[2] = res[d].total_carrier_ppm; }
+        if (nlhs > 2) mxGetPr(plhs[2])[d] = res[d].n_pos_info;
+    }
+    if (nlhs > 3) {
+        size_t dims[3] = {6 * B, 2, D};
+        plhs[3] = mxCreateNumericArray(3, dims, mxDOUBLE_CLASS, mxREAL);
+        double *o = mxGetPr(plhs[3]);
+        for (size_t d = 0; d < D; ++d)
+            for (size_t i = 0; i < 6 * B; ++i)
+                for (int c = 0; c < 2; ++c)
+                    o[d * 12 * B + c * 6 * B + i] = ((int64_t)i < res[d].n_pos_info) ? pi[d * 12 * B + 2 * i + c] : mxGetNaN();
+    }
+}
 
 /* ------------------------------------------------------------------------------------------------ */
 #if defined(GSMCAL_MEX_raw2iq)
@@ -295,24 +317,7 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
     } else
         fail_on(gsmcal_calibrate_batch((const uint8_t *)mxGetData(prhs[0]), GSMCAL_MEM_HOST, n_iq, (int64_t)D, mxGetScalar(prhs[1]), tpl, coef, (int)nt, 8, 8,
                                        res, NULL, NULL, NULL, pi, NULL), "gsm_calibrate_batch");
-    plhs[0] = mxCreateDoubleMatrix(3, D, mxREAL);
-    if (nlhs > 1) plhs[1] = mxCreateDoubleMatrix(3, D, mxREAL);
-    if (nlhs > 2) plhs[2] = mxCreateDoubleMatrix(1, D, mxREAL);
-    for (size_t d = 0; d < D; ++d) {
-        double *sp = mxGetPr(plhs[0]) + 3 * d;
-        sp[0] = res[d].sampling_ppm[0]; sp[1] = res[d].sampling_ppm[1]; sp[2] = res[d].total_sampling_ppm;
-        if (nlhs > 1) { double *cp = mxGetPr(plhs[1]) + 3 * d; cp[0] = res[d].carrier_ppm[0]; cp[1] = res[d].carrier_ppm[1]; cp[2] = res[d].total_carrier_ppm; }
-        if (nlhs > 2) mxGetPr(plhs[2])[d] = res[d].n_pos_info;
-    }
-    if (nlhs > 3) {
-        size_t dims[3] = {(size_t)(6 * B), 2, D};
-        plhs[3] = mxCreateNumericArray(3, dims, mxDOUBLE_CLASS, mxREAL);
-        double *o = mxGetPr(plhs[3]);
-        for (size_t d = 0; d < D; ++d)
-            for (size_t i = 0; i < (size_t)(6 * B); ++i)
-                for (int c = 0; c < 2; ++c)
-                    o[d * 12 * B + c * 6 * B + i] = ((int64_t)i < res[d].n_pos_info) ? pi[d * 12 * B + 2 * i + c] : mxGetNaN();
-    }
+    batch_outputs(nlhs, plhs, res, pi, D, (size_t)B);
     if (nlhs > 4) {
         const char *f[] = {"t0", "fit_ppm", "rms", "n_fit", "flags", "tau", "x"};
         plhs[4] = mxCreateStructMatrix(1, D, 7, f);
@@ -392,24 +397,7 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
         fail_on(gsmcal_calibrate_demod_batch((const uint8_t *)mxGetData(prhs[0]), GSMCAL_MEM_HOST, n_iq, (int64_t)D, mxGetScalar(prhs[1]), tpl, coef, (int)nt, 8, 8,
                                              res, NULL, NULL, NULL, pi, NULL, dem, ok, bits, dec, corr, freq, snr, idx), "gsm_calibrate_demod_batch");
 #endif
-    plhs[0] = mxCreateDoubleMatrix(3, D, mxREAL);
-    if (nlhs > 1) plhs[1] = mxCreateDoubleMatrix(3, D, mxREAL);
-    if (nlhs > 2) plhs[2] = mxCreateDoubleMatrix(1, D, mxREAL);
-    for (size_t d = 0; d < D; ++d) {
-        double *sp = mxGetPr(plhs[0]) + 3 * d;
-        sp[0] = res[d].sampling_ppm[0]; sp[1] = res[d].sampling_ppm[1]; sp[2] = res[d].total_sampling_ppm;
-        if (nlhs > 1) { double *cp = mxGetPr(plhs[1]) + 3 * d; cp[0] = res[d].carrier_ppm[0]; cp[1] = res[d].carrier_ppm[1]; cp[2] = res[d].total_carrier_ppm; }
-        if (nlhs > 2) mxGetPr(plhs[2])[d] = res[d].n_pos_info;
-    }
-    if (nlhs > 3) {
-        size_t dims[3] = {6 * B, 2, D};
-        plhs[3] = mxCreateNumericArray(3, dims, mxDOUBLE_CLASS, mxREAL);
-        double *o = mxGetPr(plhs[3]);
-        for (size_t d = 0; d < D; ++d)
-            for (size_t i = 0; i < 6 * B; ++i)
-                for (int c = 0; c < 2; ++c)
-                    o[d * 12 * B + c * 6 * B + i] = ((int64_t)i < res[d].n_pos_info) ? pi[d * 12 * B + 2 * i + c] : mxGetNaN();
-    }
+    batch_outputs(nlhs, plhs, res, pi, D, B);
     if (nlhs > 4) {
         const char *f[] = {"demod_bits", "bits_to_decoder", "corr_val", "sch_ok", "flags"};
         plhs[4] = mxCreateStructMatrix(1, D, 5, f);
