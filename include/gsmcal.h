@@ -327,6 +327,63 @@ int gsmcal_calibrate_sch_timing_batch(const uint8_t *raw, int raw_mem, int64_t n
                                       gsmcal_sch_timing_result *timing /* [n_streams], required */,
                                       double *sch_tau, double *sch_x);
 
+/* gsmcal_calibrate_batch (every output as there, byte for byte) followed by a carrier estimate of every FCCH burst and a least-squares
+ * line through them over capture time: each dongle's carrier error without the about -1.07 ppm bias of total_carrier_ppm, and its drift
+ * over the capture.  Only oversampling_ratio 8 (osr below).  For stream d, with fs = 8 * 1625e3/6, f_nom = fs/32 = 1625e3/24 (the FCCH
+ * tone), e1 = sampling_ppm[0]*1e-6, e2 = sampling_ppm[1]*1e-6, r = r_correct (1-based, the samples gsmcal_calibrate_batch_r writes) and
+ * p_i the position of the i-th FCCH row (type 0) of pos_info.  A row is used when FCCH_demod's window r(p_i : p_i + 148*osr - 1) lies
+ * inside r (else GSMCAL_CARRIER_RANGE); the interior window below then always fits.  For a used row, all in fp64:
+ *   1. window: x(n) = r(p_i + 16*osr + n), n = 0..W-1, W = 116*osr = 928 (the burst without its edges and the inverted first
+ *      differential symbol).
+ *   2. y(n) = x(n) * exp(-i*pi*n/16) (f_nom removed; a 32-entry table), m = n - (W-1)/2.
+ *   3. coarse grid: P(w) = |sum_n y(n) exp(-i*w*m)|^2 (re^2 + im^2) at w_k = pi*k/(2W), k = -14..14: delta_k = k*fs/(4W), 583.7 Hz steps
+ *      over +-8172 Hz (the residual after the reference chain is about +1 kHz).  k* = the first maximum; k* = -14 or 14:
+ *      GSMCAL_CARRIER_EDGE, the row is excluded.
+ *   4. refine: 5 Newton steps on P'(w) = 0 from w_k*: with S_j = sum_n m^j y(n) exp(-i*w*m) (j = 0, 1, 2),
+ *      w <- w - Im(conj(S0)*S1) / (|S1|^2 - Re(conj(S0)*S2)).  |last step| * fs/(2*pi) > 1e-4 Hz (or NaN): GSMCAL_CARRIER_NOCONV, the
+ *      row is excluded.  f_i = f_nom + w * fs/(2*pi): the burst's tone in Hz, in r_correct's sample frame.
+ *   5. t_i = (((tau_c - 1)*(1 + e2))*(1 + e1)) / fs seconds of capture time, tau_c = p_i + 16*osr + (W-1)/2 the window centre in r
+ *      (r(j) sits at raw time (j-1)(1+e2)(1+e1)); every operation rounded on its own.
+ *   Fit over the n_fit used rows, in row order, every operation rounded on its own: t_mean = sum t / n_fit, a = sum f / n_fit,
+ *   b = sum (t - t_mean)(f - a) / sum (t - t_mean)^2, rms = sqrt(sum ((f - a) - b*(t - t_mean))^2 / n_fit): f = a + b*(t - t_mean).
+ *   residual_ppm = 1e6*(a - f_nom)/carrier_freq, carrier_fit_ppm = total_ppm_calculation([total_carrier_ppm, residual_ppm]),
+ *   drift_ppm_per_s = 1e6*b/carrier_freq.  n_fit < 3: GSMCAL_CARRIER_FEW and every fit field NaN.
+ * The tones are measured on r_correct's sample grid, whose rate is fs*(1+e1)(1+e2) in capture terms; that scale is not undone.  Over the
+ * +-50 ppm sampling range of SURVEY.md 8(d) it moves a 67.7 kHz tone by at most 67.7e3 * 50e-6 = 3.4 Hz, about 0.004 ppm of the carrier.
+ * The periodogram maximum is used rather than the lag-1 phase increment of FCCH_demod (angle(mean(u(n+1)/u(n)))): after the channel
+ * filter the noise is coloured, and the phase increment is pulled towards zero frequency.
+ * fcch_f, fcch_t [n_streams][B] (B as above; NULL = not copied): f_i and t_i by FCCH row, NaN where excluded; fcch_row_flags
+ * [n_streams][B] uint8 (NULL = not copied): 0 or the GSMCAL_CARRIER_RANGE / _EDGE / _NOCONV bit that excluded the row. */
+typedef struct gsmcal_carrier_fit_result {
+    int32_t n_fcch;            /* type-0 rows of pos_info; -1 when the step did not run (flags say why) */
+    int32_t n_fit;             /* rows with a finite f_i */
+    int32_t flags;             /* GSMCAL_CARRIER_* */
+    int32_t reserved;
+    double  t_mean;            /* mean capture time of the fitted rows, s */
+    double  freq_hz;           /* a: the fitted tone at t_mean, Hz in r_correct's frame (f_nom = 67708.33 Hz when nothing is left) */
+    double  drift_hz_per_s;    /* b */
+    double  rms_hz;            /* fit residual RMS, Hz */
+    double  residual_ppm;      /* the carrier error total_carrier_ppm left */
+    double  carrier_fit_ppm;   /* the dongle's carrier error at t_mean */
+    double  drift_ppm_per_s;
+} gsmcal_carrier_fit_result;   /* 72 bytes */
+
+#define GSMCAL_CARRIER_NO_POS_INFO  1  /* pos_info == -1: nothing to estimate */
+#define GSMCAL_CARRIER_NO_R_CORRECT 2  /* pos_info valid but results.r_len[2] == -1 */
+#define GSMCAL_CARRIER_RANGE        4  /* some row's FCCH window leaves r_correct (also a row flag) */
+#define GSMCAL_CARRIER_EDGE         8  /* some row's grid maximum sits on the first or last grid point (also a row flag) */
+#define GSMCAL_CARRIER_NOCONV      16  /* some row's last Newton step exceeds 1e-4 Hz (also a row flag) */
+#define GSMCAL_CARRIER_FEW         32  /* fewer than 3 used rows: every fit field NaN */
+
+int gsmcal_calibrate_carrier_fit_batch(const uint8_t *raw, int raw_mem, int64_t n_iq, int64_t n_streams,
+                                       double carrier_freq, const double *sch_training_sequence,
+                                       const double *coef, int n_taps, int oversampling_ratio, int coarse_decimation,
+                                       gsmcal_stream_result *results,
+                                       double *coarse_pos, double *coarse_snr, double *fcch_pos, double *pos_info,
+                                       void *cuda_stream,
+                                       gsmcal_carrier_fit_result *carrier /* [n_streams], required */,
+                                       double *fcch_f, double *fcch_t, uint8_t *fcch_row_flags);
+
 /* gsmcal_calibrate_demod_batch (every output as there, byte for byte; with normal_training_sequence and bcch, both set or both NULL,
  * gsmcal_calibrate_demod_bcch_batch's) followed by SCH channel decoding: the BSIC and the TDMA frame number (FN) each SCH burst carries,
  * and each dongle's capture start on the cell's frame clock.  Per type-1 row of pos_info, in row order (the rows SCH_demod
@@ -408,7 +465,9 @@ int gsmcal_calibrate_batch_cancel(int slot);
  * [0] uint8 column sums (+ H2D when raw is on the host) [1] coarse FCCH [2] fine FCCH sliding-DFT peak search
  * [3] fine ppm + tone estimate + gate [4] SCH correlation + pos_info [5] post-SCH tone estimate + result records
  * [6] (gsmcal_calibrate_demod_batch / _demod_bcch_batch / _sch_decode_batch only) SCH_demod (+ SCH decoding) + FCCH_demod (+ BCCH_demod);
- *     (gsmcal_calibrate_sch_timing_batch only) SCH row list, sub-sample SCH timing and the clock fit.  Returns the number of stages written. */
+ *     (gsmcal_calibrate_sch_timing_batch only) SCH row list, sub-sample SCH timing and the clock fit;
+ *     (gsmcal_calibrate_carrier_fit_batch only) FCCH row list, the tone of every FCCH burst and the carrier fit.  Returns the number of
+ *     stages written. */
 int gsmcal_last_batch_stage_ms(double *ms, int cap);
 
 /* FCCH scanner per-channel processing, multi_rtl_sdr_gsm_FCCH_scanner.m:132-135,163-186, for n_chan

@@ -36,6 +36,10 @@ static_assert(sizeof(gsmcal_sch_decode_result) == sizeof(SchDecodeResultDev) && 
 static_assert(GSMCAL_SCHDEC_NO_POS_INFO == SC_NO_POS_INFO && GSMCAL_SCHDEC_NO_R_CORRECT == SC_NO_R_CORRECT && GSMCAL_SCHDEC_NONE == SC_NONE &&
               GSMCAL_SCHDEC_DISAGREE == SC_DISAGREE && GSMCAL_SCHDEC_ROW_WINDOW == SC_ROW_WINDOW && GSMCAL_SCHDEC_ROW_ALIGN == SC_ROW_ALIGN &&
               GSMCAL_SCHDEC_ROW_CRC == SC_ROW_CRC && GSMCAL_SCHDEC_ROW_FIELD == SC_ROW_FIELD, "SCH decode flags");
+static_assert(sizeof(gsmcal_carrier_fit_result) == sizeof(CarrierFitDev) && sizeof(gsmcal_carrier_fit_result) == 72 &&
+              offsetof(gsmcal_carrier_fit_result, t_mean) == 16 && offsetof(gsmcal_carrier_fit_result, drift_ppm_per_s) == 64, "carrier fit record layout");
+static_assert(GSMCAL_CARRIER_NO_POS_INFO == CF_NO_POS_INFO && GSMCAL_CARRIER_NO_R_CORRECT == CF_NO_R_CORRECT && GSMCAL_CARRIER_RANGE == CF_RANGE &&
+              GSMCAL_CARRIER_EDGE == CF_EDGE && GSMCAL_CARRIER_NOCONV == CF_NOCONV && GSMCAL_CARRIER_FEW == CF_FEW, "carrier fit flags");
 
 namespace {
 
@@ -563,14 +567,16 @@ size_t sch_demod_smem(int osr);
 void gmsk_branch_table(int osr, double *W);
 void sch_training_pm(signed char *data_pm);
 
-// ---- the stage behind post-SCH ("tail") of gsmcal_calibrate_demod_batch, _demod_bcch_batch, _sch_decode_batch and _sch_timing_batch --
-// It is the SCH timing block when `timing` is set, else the demod block (batched SCH_demod / FCCH_demod) with the BCCH block when `nts`
-// is set and the SCH decoding block when `sdec` is set.
+// ---- the stage behind post-SCH ("tail") of gsmcal_calibrate_demod_batch, _demod_bcch_batch, _sch_decode_batch, _sch_timing_batch and
+// _carrier_fit_batch --
+// It is the SCH timing block when `timing` is set, the carrier fit block when `carrier` is set, else the demod block (batched SCH_demod /
+// FCCH_demod) with the BCCH block when `nts` is set and the SCH decoding block when `sdec` is set.
 struct TailOut {                     // the caller's host outputs; an array left NULL is not read back
     gsmcal_demod_result *demod; uint8_t *sch_ok, *bits, *dec; double *corr, *freq, *snr, *idx;
     const double *nts; gsmcal_bcch_result *bcch;
     gsmcal_sch_decode_result *sdec; int32_t *fn, *bsic; uint8_t *ham, *rflag;
     gsmcal_sch_timing_result *timing; double *tau, *x;
+    gsmcal_carrier_fit_result *carrier; double *cf_f, *cf_t; uint8_t *cf_flag;
 };
 struct TailDev {                     // device buffers of the same blocks
     DemodResultDev *rec; double *sch_pos, *fcch_pos; unsigned char *sch_ok, *fcch_ok;                       // the row lists
@@ -578,6 +584,7 @@ struct TailDev {                     // device buffers of the same blocks
     double2 *nts /* (26*osr) x 8 */; BcchResultDev *bcch;
     SchDecodeResultDev *sdec; int *key, *fn, *bsic; unsigned char *ham, *rflag;
     TimingResultDev *timing; double *tau, *x; unsigned char *row_flag;
+    CarrierFitDev *carrier; double *cf_f, *cf_t; unsigned char *cf_flag;
 };
 // every per-stream array ([D] records, [D][cap] rows) of the blocks `o` asks for: f(device pointer, bytes per stream, the caller's host
 // array or NULL).  Set-up, the slice of a stream group and the read-back all walk this one list.  The per-call constants (Ft, Wtab, dpm,
@@ -588,6 +595,10 @@ template <class F> void tail_arrays(TailDev &t, const TailOut &o, int cap, F &&f
     f(t.sch_ok, r, o.sch_ok); f(t.fcch_ok, r, nullptr);
     if (o.timing) {
         f(t.timing, sizeof(TimingResultDev), o.timing); f(t.tau, 8 * r, o.tau); f(t.x, 8 * r, o.x); f(t.row_flag, r, nullptr);
+        return;
+    }
+    if (o.carrier) {
+        f(t.carrier, sizeof(CarrierFitDev), o.carrier); f(t.cf_f, 8 * r, o.cf_f); f(t.cf_t, 8 * r, o.cf_t); f(t.cf_flag, r, o.cf_flag);
         return;
     }
     f(t.bits, 148 * r, o.bits); f(t.dec, 148 * r, o.dec); f(t.corr, 8 * 85 * r, o.corr); f(t.freq, 8 * r, o.freq); f(t.snr, 8 * r, o.snr);
@@ -610,13 +621,13 @@ int tail_setup(Ctx &c, i64 D, int cap, int osr, const double2 *tpl_dev, const Ta
         size_t off = 0;
         auto take = [&](auto *&p, size_t bytes) { place(p, base + off); off = align_up(off + bytes); };
         tail_arrays(*t, o, cap, [&](auto *&p, size_t per, const void *) { take(p, per * D); });
-        if (!o.timing) { take(t->Ft, sizeof(double2) * N); take(t->Wtab, sizeof(double2) * 16 * osr); take(t->dpm, 64); }
+        if (!o.timing && !o.carrier) { take(t->Ft, sizeof(double2) * N); take(t->Wtab, sizeof(double2) * 16 * osr); take(t->dpm, 64); }
         if (o.nts) take(t->nts, sizeof(double2) * 8 * 26 * osr);
         return off;
     };
     void *base; TRY(c.dem.get(layout(0), &base));
     layout((uintptr_t)base);
-    if (o.timing) return GSMCAL_OK;
+    if (o.timing || o.carrier) return GSMCAL_OK;
     if (o.nts) CU(cudaMemcpyAsync(t->nts, o.nts, sizeof(double2) * 8 * 26 * (size_t)osr, cudaMemcpyHostToDevice, st));
     W.assign(2 * 16 * (size_t)osr, 0.0);
     gmsk_branch_table(osr, W.data());
@@ -627,14 +638,21 @@ int tail_setup(Ctx &c, i64 D, int cap, int osr, const double2 *tpl_dev, const Ta
     LAUNCH(fde_template_kernel, 1, SD_THREADS, 3 * (size_t)N * sizeof(double2), st, tpl_dev, osr, tw, t->Ft);
     return GSMCAL_OK;
 }
-// one stream group: row lists + sentinels, then either the timing of every SCH row and the per-stream fit (osr 8), or SCH bursts, SCH
-// decoding and BCCH_demod when their outputs were asked for, FCCH bursts, FCCH means
+// one stream group: row lists + sentinels, then either the timing of every SCH row and the per-stream fit (osr 8), or the tone of every
+// FCCH row and the per-stream carrier fit (osr 8), or SCH bursts, SCH decoding and BCCH_demod when their outputs were asked for, FCCH
+// bursts, FCCH means
 int run_tail(Ctx &c, WinSrc src, const Work &ws, const TailDev &t, int osr, double carrier_freq, i64 nd, int cap, cudaStream_t st) {
     LAUNCH(demod_compact_kernel, (unsigned)nd, 32, 0, st, ws.ctl, ws.pos_info, cap, osr, t.rec, t.sch_pos, t.sch_ok, t.fcch_pos, t.fcch_ok);
     if (t.timing) {
         LAUNCH(sch_timing_batch_kernel, dim3((unsigned)cap, (unsigned)nd), SCH_THREADS, TM_SMEM, st, src, ws.ctl, t.rec, t.sch_pos, cap, ws.tpl,
                t.tau, t.row_flag);
         LAUNCH(sch_timing_fit_kernel, (unsigned)nd, 32, 0, st, ws.ctl, t.rec, t.sch_pos, t.row_flag, t.tau, cap, t.x, t.timing);
+        return GSMCAL_OK;
+    }
+    if (t.carrier) {
+        LAUNCH(carrier_fit_row_kernel, dim3((unsigned)cap, (unsigned)nd), CF_THREADS, CF_SMEM, st, with_cache(src, ws, cap), ws.ctl, t.rec, t.fcch_pos,
+               t.fcch_ok, cap, t.cf_f, t.cf_t, t.cf_flag);
+        LAUNCH(carrier_fit_stream_kernel, (unsigned)nd, 32, 0, st, ws.ctl, t.rec, t.cf_flag, t.cf_f, t.cf_t, cap, carrier_freq, t.carrier);
         return GSMCAL_OK;
     }
     const double2 *tw_s, *tw_f;                  // both built by the set-up: no launch here
@@ -1363,6 +1381,18 @@ int gsmcal_calibrate_sch_timing_batch(const uint8_t *raw, int raw_mem, int64_t n
     if (osr != 8) return fail(GSMCAL_ERR_ARG, "calibrate_sch_timing_batch: oversampling_ratio must be 8");
     TailOut o{};
     o.timing = timing; o.tau = sch_tau; o.x = sch_x;
+    return calibrate_batch_impl(raw, raw_mem, n_iq, D, carrier_freq, tpl, coef, n_taps, osr, coarse_dr, results, coarse_pos, coarse_snr, fcch_pos, pos_info,
+                                cuda_stream, nullptr, GSMCAL_MEM_DEVICE, 0, &o);
+}
+
+int gsmcal_calibrate_carrier_fit_batch(const uint8_t *raw, int raw_mem, int64_t n_iq, int64_t D, double carrier_freq, const double *tpl,
+                                       const double *coef, int n_taps, int osr, int coarse_dr, gsmcal_stream_result *results,
+                                       double *coarse_pos, double *coarse_snr, double *fcch_pos, double *pos_info, void *cuda_stream,
+                                       gsmcal_carrier_fit_result *carrier, double *fcch_f, double *fcch_t, uint8_t *fcch_row_flags) {
+    if (!carrier) return fail(GSMCAL_ERR_ARG, "calibrate_carrier_fit_batch: null carrier");
+    if (osr != 8) return fail(GSMCAL_ERR_ARG, "calibrate_carrier_fit_batch: oversampling_ratio must be 8");
+    TailOut o{};
+    o.carrier = carrier; o.cf_f = fcch_f; o.cf_t = fcch_t; o.cf_flag = fcch_row_flags;
     return calibrate_batch_impl(raw, raw_mem, n_iq, D, carrier_freq, tpl, coef, n_taps, osr, coarse_dr, results, coarse_pos, coarse_snr, fcch_pos, pos_info,
                                 cuda_stream, nullptr, GSMCAL_MEM_DEVICE, 0, &o);
 }

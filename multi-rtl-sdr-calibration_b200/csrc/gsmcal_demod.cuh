@@ -885,3 +885,177 @@ __global__ void __launch_bounds__(32) sch_decode_batch_kernel(const DemodResultD
     }
     if (lane == 0) out[stream] = o;
 }
+
+// ===================================================================================================
+// Carrier fit of gsmcal_calibrate_carrier_fit_batch (definition: include/gsmcal.h): the tone of every FCCH row of pos_info from the
+// periodogram maximum of the burst interior on r_correct, and the per-stream line through the tones over capture time.  The FCCH row
+// list and its fcch_ok (FCCH_demod's 148*osr-sample window inside r_correct, which holds the 116*osr-sample interior) are
+// demod_compact_kernel's.  osr 8 only.
+// ===================================================================================================
+struct CarrierFitDev {               // mirrors gsmcal_carrier_fit_result (include/gsmcal.h)
+    int n_fcch, n_fit, flags, reserved;
+    double t_mean, freq_hz, drift_hz_per_s, rms_hz, residual_ppm, carrier_fit_ppm, drift_ppm_per_s;
+};
+#define CF_NO_POS_INFO  1
+#define CF_NO_R_CORRECT 2
+#define CF_RANGE        4
+#define CF_EDGE         8
+#define CF_NOCONV      16
+#define CF_FEW         32
+#define CF_OFF    128                  // 16 symbols into the burst
+#define CF_W      928                  // 116 symbols: the interior without the edges and the first differential symbol
+#define CF_HALF   463.5                // m = n - (W-1)/2
+#define CF_K      14                   // grid delta_k = k*fs/(4W), k = -14..14: 583.7 Hz steps over +-8172 Hz
+#define CF_NGRID  (2 * CF_K + 1)
+#define CF_NEWTON 5
+#define CF_TOL_HZ 1e-4
+#define CF_THREADS 256
+#define CF_SMEM   ((size_t)(CF_W + GSMCAL_XCAP(CF_W) + CF_W + 8) * sizeof(double2))      // window | the loader's X, Y
+
+// One block per (FCCH row, stream).  The window comes through the fine search's filtered-window cache where it covers it (as in
+// fcch_demod_batch_kernel), then the dphi2 derotation and the nominal tone's removal.  Grid: warp w takes grid points w, w+8, ...; lane l
+// samples l, l+32, ... with a rotation recurrence seeded by an exact sincospi at its first sample.  Newton: thread t takes samples
+// t, t+256, ... seeded the same way; every thread gets the block sums and takes the same step.
+__global__ void __launch_bounds__(CF_THREADS) carrier_fit_row_kernel(WinSrc src, const StreamCtl *__restrict__ ctl, const DemodResultDev *__restrict__ rec,
+                                                                    const double *__restrict__ fcch_pos, const unsigned char *__restrict__ fcch_ok, int cap,
+                                                                    double *__restrict__ f_out, double *__restrict__ t_out,
+                                                                    unsigned char *__restrict__ row_flag) {
+    extern __shared__ double2 sm[];
+    __shared__ double2 ph0, tw32[32], gstep[CF_NGRID];
+    __shared__ double pgrid[CF_NGRID], red[8 * 6];
+    const int row = blockIdx.x, stream = blockIdx.y, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    if (row >= rec[stream].n_fcch) return;                     // also n_fcch = -1: the step does not run for this stream
+    const i64 o = (i64)stream * cap + row;
+    if (!fcch_ok[o]) {
+        if (tid == 0) { f_out[o] = NAN; t_out[o] = NAN; row_flag[o] = CF_RANGE; }
+        return;
+    }
+    const StreamCtl c = ctl[stream];
+    const double p = fcch_pos[o];
+    const i64 j0 = (i64)p - 1 + CF_OFF;                        // 0-based first sample of r_correct(p + 128 : p + 128 + 927)
+    double2 *y = sm, *X = y + CF_W, *Y = X + GSMCAL_XCAP(CF_W);
+    if (tid == 0) { double sn, cs; sincos((double)j0 * c.dphi2, &sn, &cs); ph0 = make_double2(cs, sn); }
+    if (tid >= 32 && tid < 64) { double sn, cs; sincospi(-(double)(tid - 32) / 16.0, &sn, &cs); tw32[tid - 32] = make_double2(cs, sn); }
+    if (tid >= 64 && tid < 64 + CF_NGRID) {                    // exp(-i*omega_k*32), omega_k = pi*k/(2W)
+        double sn, cs; sincospi(-32.0 * (double)(tid - 64 - CF_K) / (2.0 * CF_W), &sn, &cs); gstep[tid - 64] = make_double2(cs, sn);
+    }
+    load_window(src, c, stream, j0, CF_W, y, X, Y, row);       // level 3; ends with a barrier
+    derotate_post(y, CF_W, c.dphi2, ph0);                      // r_correct (carrier_correct_post_SCH.m:83)
+    for (int i = tid; i < CF_W; i += CF_THREADS) y[i] = cmul(y[i], tw32[i & 31]);     // the same samples derotate_post gave this thread
+    __syncthreads();
+    // coarse grid
+    for (int g = warp; g < CF_NGRID; g += CF_THREADS / 32) {
+        double sn, cs; sincospi(-(double)(g - CF_K) * ((double)lane - CF_HALF) / (2.0 * CF_W), &sn, &cs);
+        double2 z = make_double2(cs, sn);
+        const double2 st = gstep[g];
+        double ar = 0.0, ai = 0.0;
+#pragma unroll 4
+        for (int n = lane; n < CF_W; n += 32) {
+            const double2 v = y[n];
+            ar = fma(v.x, z.x, fma(-v.y, z.y, ar));
+            ai = fma(v.x, z.y, fma(v.y, z.x, ai));
+            z = cmul(z, st);
+        }
+        ar = warp_sum(ar); ai = warp_sum(ai);
+        if (lane == 0) pgrid[g] = __dadd_rn(__dmul_rn(ar, ar), __dmul_rn(ai, ai));
+    }
+    __syncthreads();
+    int kb = 0;
+    for (int g = 1; g < CF_NGRID; ++g) if (pgrid[g] > pgrid[kb]) kb = g;                // first maximum
+    if (kb == 0 || kb == CF_NGRID - 1) {
+        if (tid == 0) { f_out[o] = NAN; t_out[o] = NAN; row_flag[o] = CF_EDGE; }
+        return;
+    }
+    // Newton on P'(omega) = 0: P' = 2 Im(conj(S0) S1), P'' = 2 (|S1|^2 - Re(conj(S0) S2)), S_j = sum m^j y exp(-i omega m)
+    double omega = GSMCAL_PI * (double)(kb - CF_K) / (2.0 * CF_W), step = 0.0;
+    for (int it = 0; it < CF_NEWTON; ++it) {
+        double sn, cs;
+        sincos(-omega * ((double)tid - CF_HALF), &sn, &cs);
+        double2 z = make_double2(cs, sn);
+        sincos(-omega * (double)CF_THREADS, &sn, &cs);
+        const double2 st = make_double2(cs, sn);
+        double s[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};          // S0, S1, S2 (re, im)
+        for (int n = tid; n < CF_W; n += CF_THREADS) {
+            const double m = (double)n - CF_HALF;
+            const double2 v = cmul(y[n], z);
+            s[0] += v.x; s[1] += v.y;
+            s[2] = fma(m, v.x, s[2]); s[3] = fma(m, v.y, s[3]);
+            s[4] = fma(m * m, v.x, s[4]); s[5] = fma(m * m, v.y, s[5]);
+            z = cmul(z, st);
+        }
+        block_sum_n<6, true>(s, red);
+        const double num = s[0] * s[3] - s[1] * s[2];
+        const double den = (s[2] * s[2] + s[3] * s[3]) - (s[0] * s[4] + s[1] * s[5]);
+        step = -num / den;
+        omega += step;
+    }
+    if (tid != 0) return;
+    const double hz_per_rad = (((1625.0 / 6.0) * 1e3) * 8.0) / (2.0 * GSMCAL_PI);
+    if (!(fabs(step) * hz_per_rad <= CF_TOL_HZ)) { f_out[o] = NAN; t_out[o] = NAN; row_flag[o] = CF_NOCONV; return; }
+    f_out[o] = __dadd_rn(((1625.0 / 6.0) * 1e3) / 4.0, __dmul_rn(omega, hz_per_rad));
+    const double s1 = __dadd_rn(1.0, __dmul_rn(c.sppm1, 1e-6)), s2 = __dadd_rn(1.0, __dmul_rn(c.sppm2, 1e-6));   // sampling_ppm[0], [1] of the record
+    const double tau_c = p + (double)CF_OFF + CF_HALF;                                  // exact
+    t_out[o] = __ddiv_rn(__dmul_rn(__dmul_rn(tau_c - 1.0, s2), s1), ((1625.0 / 6.0) * 1e3) * 8.0);
+    row_flag[o] = 0;
+}
+
+// One warp per stream: the lanes gather the row flags and count the fitted rows, lane 0 fits f = a + b (t - t_mean) in row order
+// (the sums as include/gsmcal.h states them, every product and sum rounded on its own) and composes the ppm figures.
+__global__ void __launch_bounds__(32) carrier_fit_stream_kernel(const StreamCtl *__restrict__ ctl, const DemodResultDev *__restrict__ rec,
+                                                                const unsigned char *__restrict__ row_flag, const double *__restrict__ f,
+                                                                const double *__restrict__ t, int cap, double carrier_freq,
+                                                                CarrierFitDev *__restrict__ out) {
+    const int stream = blockIdx.x, lane = threadIdx.x;
+    const DemodResultDev r = rec[stream];
+    CarrierFitDev q;
+    q.n_fcch = -1; q.n_fit = 0; q.flags = 0; q.reserved = 0;
+    q.t_mean = q.freq_hz = q.drift_hz_per_s = q.rms_hz = q.residual_ppm = q.carrier_fit_ppm = q.drift_ppm_per_s = NAN;
+    if (r.flags & (DM_NO_POS_INFO | DM_NO_R_CORRECT)) {
+        q.flags = (r.flags & DM_NO_POS_INFO) ? CF_NO_POS_INFO : CF_NO_R_CORRECT;
+        if (lane == 0) out[stream] = q;
+        return;
+    }
+    const i64 base = (i64)stream * cap;
+    const int n = r.n_fcch;
+    unsigned fl = 0, nf = 0;
+    for (int i = lane; i < n; i += 32) {
+        fl |= row_flag[base + i];
+        nf += isfinite(f[base + i]) ? 1u : 0u;
+    }
+    fl = __reduce_or_sync(0xffffffffu, fl);
+    nf = __reduce_add_sync(0xffffffffu, nf);
+    if (lane != 0) return;
+    q.n_fcch = n; q.n_fit = (int)nf; q.flags = (int)fl;
+    if (nf < 3) {
+        q.flags |= CF_FEW;
+        out[stream] = q;
+        return;
+    }
+    double st = 0.0, sf = 0.0;
+    for (int i = 0; i < n; ++i) {
+        if (!isfinite(f[base + i])) continue;
+        st = __dadd_rn(st, t[base + i]);
+        sf = __dadd_rn(sf, f[base + i]);
+    }
+    const double t_bar = st / (double)nf, a = sf / (double)nf;
+    double stt = 0.0, stf = 0.0;
+    for (int i = 0; i < n; ++i) {
+        if (!isfinite(f[base + i])) continue;
+        const double dt = __dsub_rn(t[base + i], t_bar);
+        stt = __dadd_rn(stt, __dmul_rn(dt, dt));
+        stf = __dadd_rn(stf, __dmul_rn(dt, __dsub_rn(f[base + i], a)));
+    }
+    const double b = stf / stt;
+    double ss = 0.0;
+    for (int i = 0; i < n; ++i) {
+        if (!isfinite(f[base + i])) continue;
+        const double e = __dsub_rn(__dsub_rn(f[base + i], a), __dmul_rn(b, __dsub_rn(t[base + i], t_bar)));
+        ss = __dadd_rn(ss, __dmul_rn(e, e));
+    }
+    const StreamCtl c = ctl[stream];
+    q.t_mean = t_bar; q.freq_hz = a; q.drift_hz_per_s = b; q.rms_hz = sqrt(ss / (double)nf);
+    q.residual_ppm = __dmul_rn(1e6, __dsub_rn(a, ((1625.0 / 6.0) * 1e3) / 4.0)) / carrier_freq;
+    q.carrier_fit_ppm = total_ppm2(total_ppm2(c.cppm1, c.cppm2), q.residual_ppm);         // total_carrier_ppm of the record, then the residual
+    q.drift_ppm_per_s = __dmul_rn(1e6, b) / carrier_freq;
+    out[stream] = q;
+}

@@ -38,6 +38,12 @@ class SchDecodeResult(C.Structure):
                 ("fn_first", C.c_int32), ("frame_clock_start", C.c_double)]
 
 
+class CarrierFitResult(C.Structure):
+    _fields_ = [("n_fcch", C.c_int32), ("n_fit", C.c_int32), ("flags", C.c_int32), ("reserved", C.c_int32),
+                ("t_mean", C.c_double), ("freq_hz", C.c_double), ("drift_hz_per_s", C.c_double), ("rms_hz", C.c_double),
+                ("residual_ppm", C.c_double), ("carrier_fit_ppm", C.c_double), ("drift_ppm_per_s", C.c_double)]
+
+
 # the leading arguments of gsmcal_calibrate_batch and its variants: raw, raw_mem, n_iq, D, carrier_freq, tpl, coef, n_taps, osr,
 # coarse_dr, results, coarse_pos, coarse_snr, fcch_pos, pos_info, cuda_stream
 _BATCH = [C.c_void_p, C.c_int, c_i64, c_i64, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 6
@@ -84,6 +90,7 @@ SIGNATURES = {
     "gsmcal_calibrate_demod_bcch_batch": (C.c_int, _BATCH + [C.c_void_p] * 10),
     "gsmcal_calibrate_sch_decode_batch": (C.c_int, _BATCH + [C.c_void_p] * 15),
     "gsmcal_calibrate_sch_timing_batch": (C.c_int, _BATCH + [C.c_void_p] * 3),
+    "gsmcal_calibrate_carrier_fit_batch": (C.c_int, _BATCH + [C.c_void_p] * 4),
     "gsmcal_calibrate_batch_submit": (C.c_int, [C.c_int, C.c_void_p, c_i64, c_i64, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "gsmcal_calibrate_batch_collect": (C.c_int, [C.c_int]),

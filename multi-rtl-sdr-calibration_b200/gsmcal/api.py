@@ -11,7 +11,7 @@ import ctypes as C
 
 import numpy as np
 
-from ._lib import BcchResult, DemodResult, GsmcalError, SchDecodeResult, SchTimingResult, StreamResult, check, lib  # noqa: F401
+from ._lib import BcchResult, CarrierFitResult, DemodResult, GsmcalError, SchDecodeResult, SchTimingResult, StreamResult, check, lib  # noqa: F401
 
 SYMBOL_RATE = (1625.0 / 6.0) * 1e3
 
@@ -330,7 +330,7 @@ def _batch_args(raw, carrier_freq, sch_training_sequence, coef, osr, coarse_dr, 
 def calibrate_batch(raw, carrier_freq: float, sch_training_sequence, coef, osr: int = 8, coarse_dr: int = 8,
                     device_ptr: int | None = None, n_iq: int | None = None, n_streams: int | None = None,
                     cuda_stream: int = 0, details: bool = True, r_correct=None, r_device_ptr: int | None = None,
-                    sch_timing: bool = False):
+                    sch_timing: bool = False, carrier_fit: bool = False):
     """gsm_sync_demod.m:107-124 for every row of `raw` ([D, 2N] uint8, row d == dongle d's fread column).
 
     `raw` is a host NumPy array, or pass device_ptr/n_iq/n_streams for a capture already resident in HBM.
@@ -341,16 +341,30 @@ def calibrate_batch(raw, carrier_freq: float, sch_training_sequence, coef, osr: 
     gains timing: dict(t0, fit_ppm, rms, n_fit, flags, tau, x): t0 the raw-capture time (0-based samples) of the first fitted burst's
     training start, fit_ppm the sample clock error of the fit, rms its residual (samples), flags TIMING_* bits, and per SCH row tau (time
     in r_correct, 1-based) and x (time in the uint8 capture, 0-based), NaN where excluded; tau and x are None when the step did not
-    run (TIMING_NO_POS_INFO / TIMING_NO_R_CORRECT)."""
-    if sch_timing and (r_correct is not None or r_device_ptr is not None):
-        raise ValueError("sch_timing does not combine with r_correct / r_device_ptr")
-    details = details or sch_timing
+    run (TIMING_NO_POS_INFO / TIMING_NO_R_CORRECT).
+
+    carrier_fit=True (osr 8, not with r_correct / r_device_ptr or sch_timing, implies details) also estimates the tone of every FCCH
+    burst of pos_info on r_correct from the periodogram maximum of its interior and fits a line through the tones over capture time
+    (gsmcal_calibrate_carrier_fit_batch, include/gsmcal.h); each dict gains carrier: dict(carrier_fit_ppm, drift_ppm_per_s, t_mean,
+    freq_hz, drift_hz_per_s, rms_hz, residual_ppm, n_fit, flags, f, t, row_flags): carrier_fit_ppm the dongle's carrier error at t_mean
+    (seconds of capture time), drift_ppm_per_s its drift, freq_hz / drift_hz_per_s / rms_hz the line through the tones in r_correct's
+    frame, residual_ppm what total_carrier_ppm left, flags CARRIER_* bits, and per FCCH row f (Hz), t (s) and row_flags, f and t NaN
+    where excluded; f, t and row_flags are None when the step did not run (CARRIER_NO_POS_INFO / CARRIER_NO_R_CORRECT)."""
+    if (sch_timing or carrier_fit) and (r_correct is not None or r_device_ptr is not None):
+        raise ValueError("sch_timing / carrier_fit do not combine with r_correct / r_device_ptr")
+    if sch_timing and carrier_fit:
+        raise ValueError("sch_timing and carrier_fit are separate calls")
+    details = details or sch_timing or carrier_fit
     args, keep, D, n_iq, cap, res, arrays = _batch_args(raw, carrier_freq, sch_training_sequence, coef, osr, coarse_dr, device_ptr, n_iq,
                                                         n_streams, cuda_stream, details)
     if sch_timing:
         tm = (SchTimingResult * D)()
         tau, x = np.empty((D, cap)), np.empty((D, cap))
         check(lib().gsmcal_calibrate_sch_timing_batch(*args, C.cast(tm, C.c_void_p), _ptr(tau), _ptr(x)))
+    elif carrier_fit:
+        cf = (CarrierFitResult * D)()
+        f, t, rf = np.empty((D, cap)), np.empty((D, cap)), np.empty((D, cap), dtype=np.uint8)
+        check(lib().gsmcal_calibrate_carrier_fit_batch(*args, C.cast(cf, C.c_void_p), _ptr(f), _ptr(t), _ptr(rf)))
     elif r_correct is None and r_device_ptr is None:
         check(lib().gsmcal_calibrate_batch(*args))
     else:
@@ -370,10 +384,19 @@ def calibrate_batch(raw, carrier_freq: float, sch_training_sequence, coef, osr: 
             n = t.n_sch
             item["timing"] = dict(t0=t.t0, fit_ppm=t.fit_ppm, rms=t.rms, n_fit=t.n_fit, flags=t.flags,
                                   tau=None if n < 0 else tau[d, :n].copy(), x=None if n < 0 else x[d, :n].copy())
+    if carrier_fit:
+        for d, item in enumerate(out):
+            c = cf[d]
+            n = c.n_fcch
+            item["carrier"] = dict(carrier_fit_ppm=c.carrier_fit_ppm, drift_ppm_per_s=c.drift_ppm_per_s, t_mean=c.t_mean, freq_hz=c.freq_hz,
+                                   drift_hz_per_s=c.drift_hz_per_s, rms_hz=c.rms_hz, residual_ppm=c.residual_ppm, n_fit=c.n_fit,
+                                   flags=c.flags, f=None if n < 0 else f[d, :n].copy(), t=None if n < 0 else t[d, :n].copy(),
+                                   row_flags=None if n < 0 else rf[d, :n].astype(np.int64))
     return out
 
 
 TIMING_NO_POS_INFO, TIMING_NO_R_CORRECT, TIMING_RANGE, TIMING_EDGE, TIMING_FEW = 1, 2, 4, 8, 16
+CARRIER_NO_POS_INFO, CARRIER_NO_R_CORRECT, CARRIER_RANGE, CARRIER_EDGE, CARRIER_NOCONV, CARRIER_FEW = 1, 2, 4, 8, 16, 32
 DEMOD_NO_POS_INFO, DEMOD_NO_R_CORRECT, DEMOD_SCH_RANGE, DEMOD_FCCH_RANGE = 1, 2, 4, 8
 BCCH_NO_POS_INFO, BCCH_FEW_BCCH, BCCH_FCCH_RANGE, BCCH_TRAIN_RANGE = 1, 2, 4, 8
 SCHDEC_NO_POS_INFO, SCHDEC_NO_R_CORRECT, SCHDEC_NONE, SCHDEC_DISAGREE = 1, 2, 4, 8

@@ -65,6 +65,7 @@ class StreamSpec:
     tsc: int | None = None          # normal training sequence code (0..7) put at bits 61..86 of every normal burst; None = random bits
     bsic: int | None = None         # 0..63: every SCH burst carries the coded (BSIC, FN) of TS 45.003 4.7; None = random coded bits
     fn0: int = 0                    # TDMA frame number of slot 0's frame (a multiple of 51, below FN_MOD)
+    carrier_drift_ppm_per_s: float = 0.0   # the carrier error grows by this much per second of receiver time (a warming crystal)
 
 
 def random_spec(seed: int, n_samples: int, carrier_freq: float = 957.4e6) -> StreamSpec:
@@ -174,6 +175,11 @@ def true_frame_clock_start(spec: StreamSpec) -> float:
     return spec.fn0 * FRAME + spec.start_offset
 
 
+def true_carrier_ppm(spec: StreamSpec, t_seconds):
+    """the carrier error (ppm) at receiver time t_seconds (capture sample t * 8 * SYMBOL_RATE, 0-based)"""
+    return spec.carrier_ppm + spec.carrier_drift_ppm_per_s * np.asarray(t_seconds, dtype=np.float64)
+
+
 def generate_stream(spec: StreamSpec, device="cpu", out: torch.Tensor | None = None) -> torch.Tensor:
     """Returns 2*n_samples uint8 (I,Q interleaved).  `out` may be a preallocated uint8 view to fill."""
     dev = torch.device(device)
@@ -190,6 +196,7 @@ def generate_stream(spec: StreamSpec, device="cpu", out: torch.Tensor | None = N
     result = out if out is not None else torch.empty(2 * n, dtype=torch.uint8, device=dev)
     noise_sigma = spec.amplitude / math.sqrt(2.0) * 10.0 ** (-spec.snr_db / 20.0)
     w_off = 2.0 * math.pi * (spec.carrier_ppm * 1e-6 * spec.carrier_freq) / (SYMBOL_RATE * 8)
+    w_drift = 2.0 * math.pi * (spec.carrier_drift_ppm_per_s * 1e-6 * spec.carrier_freq) / (SYMBOL_RATE * 8) ** 2
     chunk = 1 << 22
     for c0 in range(0, n, chunk):
         c1 = min(n, c0 + chunk)
@@ -208,7 +215,10 @@ def generate_stream(spec: StreamSpec, device="cpu", out: torch.Tensor | None = N
             gjc = gj.clamp(min=0)
             tj = (gjc // SYM_PER_SLOT).to(f64) * SLOT + (gjc % SYM_PER_SLOT).to(f64) * 8.0
             phase = phase + torch.where(valid, a[gjc].to(f64) * gmsk_q((t - tj) / 8.0), torch.zeros_like(t))
-        theta = (math.pi / 2.0) * phase + (idx * w_off + spec.phase0)
+        off = idx * w_off
+        if spec.carrier_drift_ppm_per_s:
+            off = off + 0.5 * w_drift * idx * idx
+        theta = (math.pi / 2.0) * phase + (off + spec.phase0)
         amp = 0.0 if spec.noise_only else spec.amplitude
         re = amp * torch.cos(theta) + noise_sigma * torch.randn(c1 - c0, generator=gen, device=dev, dtype=f64)
         im = amp * torch.sin(theta) + noise_sigma * torch.randn(c1 - c0, generator=gen, device=dev, dtype=f64)

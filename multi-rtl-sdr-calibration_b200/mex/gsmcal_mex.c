@@ -334,6 +334,53 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
     mxFree(res); mxFree(pi); if (own) mxFree((void *)tpl);
 }
 
+#elif defined(GSMCAL_MEX_gsm_calibrate_carrier_batch)
+/* [sampling_ppm, carrier_ppm, n_pos_info, pos_info, carrier] = gsm_calibrate_carrier_batch(raw_uint8, carrier_freq, sch_training_sequence, coef)
+ * Outputs 1-4 are gsm_calibrate_batch's.  carrier: 1 x D struct array of the carrier fit of gsmcal_calibrate_carrier_fit_batch:
+ * carrier_fit_ppm (the dongle's carrier error at t_mean, without total_carrier_ppm's bias), drift_ppm_per_s, t_mean (s of capture
+ * time), freq_hz, drift_hz_per_s, rms_hz (the line through the FCCH tones in r_correct's frame), residual_ppm, n_fit, flags (1 pos_info
+ * == -1, 2 r_correct == -1, 4 an FCCH window leaves r_correct, 8 a grid maximum on the edge, 16 Newton did not converge, 32 fewer than
+ * 3 fitted bursts), f, t and row_flags (1 x n_fcch: each FCCH burst's tone in Hz, its capture time in s, NaN where excluded, and the
+ * flag that excluded it; empty when the step did not run).  See include/gsmcal.h. */
+void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
+    init_once();
+    if (nrhs != 4 || nlhs > 5)
+        mexErrMsgIdAndTxt("gsmcal:nargin", "usage: [sampling_ppm,carrier_ppm,n_pos_info,pos_info,carrier] = "
+                          "gsm_calibrate_carrier_batch(raw_uint8,carrier_freq,sch_training_sequence,coef)");
+    if (!mxIsUint8(prhs[0])) mexErrMsgIdAndTxt("gsmcal:type", "raw must be uint8");
+    size_t rows = mxGetM(prhs[0]), D = mxGetN(prhs[0]);
+    int own; const double *tpl = get_c128(prhs[2], &own);
+    size_t nt; const double *coef = real_vector(prhs[3], &nt);
+    int64_t n_iq = (int64_t)(rows / 2);
+    int64_t B = gsmcal_max_bursts((n_iq + 63) / 64, 8);
+    gsmcal_stream_result *res = (gsmcal_stream_result *)mxMalloc(D * sizeof(*res));
+    double *pi = (double *)mxMalloc(D * 12 * (size_t)B * sizeof(double));
+    gsmcal_carrier_fit_result *cf = (gsmcal_carrier_fit_result *)mxMalloc(D * sizeof(*cf));
+    double *fr = (double *)mxMalloc(2 * D * (size_t)B * sizeof(double)), *tr = fr + D * (size_t)B;
+    uint8_t *rf = (uint8_t *)mxMalloc(D * (size_t)B);
+    fail_on(gsmcal_calibrate_carrier_fit_batch((const uint8_t *)mxGetData(prhs[0]), GSMCAL_MEM_HOST, n_iq, (int64_t)D, mxGetScalar(prhs[1]), tpl, coef,
+                                               (int)nt, 8, 8, res, NULL, NULL, NULL, pi, NULL, cf, fr, tr, rf), "gsm_calibrate_carrier_batch");
+    batch_outputs(nlhs, plhs, res, pi, D, (size_t)B);
+    if (nlhs > 4) {
+        const char *f[] = {"carrier_fit_ppm", "drift_ppm_per_s", "t_mean", "freq_hz", "drift_hz_per_s", "rms_hz", "residual_ppm", "n_fit", "flags",
+                           "f", "t", "row_flags"};
+        plhs[4] = mxCreateStructMatrix(1, D, 12, f);
+        for (size_t d = 0; d < D; ++d) {
+            const size_t n = cf[d].n_fcch > 0 ? (size_t)cf[d].n_fcch : 0;
+            mxArray *fa = mxCreateDoubleMatrix(1, n, mxREAL), *ta = mxCreateDoubleMatrix(1, n, mxREAL), *ra = mxCreateDoubleMatrix(1, n, mxREAL);
+            if (n) { memcpy(mxGetPr(fa), fr + d * B, n * sizeof(double)); memcpy(mxGetPr(ta), tr + d * B, n * sizeof(double)); }
+            for (size_t i = 0; i < n; ++i) mxGetPr(ra)[i] = rf[d * B + i];
+            mxSetField(plhs[4], d, "carrier_fit_ppm", scalar(cf[d].carrier_fit_ppm)); mxSetField(plhs[4], d, "drift_ppm_per_s", scalar(cf[d].drift_ppm_per_s));
+            mxSetField(plhs[4], d, "t_mean", scalar(cf[d].t_mean)); mxSetField(plhs[4], d, "freq_hz", scalar(cf[d].freq_hz));
+            mxSetField(plhs[4], d, "drift_hz_per_s", scalar(cf[d].drift_hz_per_s)); mxSetField(plhs[4], d, "rms_hz", scalar(cf[d].rms_hz));
+            mxSetField(plhs[4], d, "residual_ppm", scalar(cf[d].residual_ppm)); mxSetField(plhs[4], d, "n_fit", scalar(cf[d].n_fit));
+            mxSetField(plhs[4], d, "flags", scalar(cf[d].flags)); mxSetField(plhs[4], d, "f", fa); mxSetField(plhs[4], d, "t", ta);
+            mxSetField(plhs[4], d, "row_flags", ra);
+        }
+    }
+    mxFree(cf); mxFree(fr); mxFree(rf); mxFree(res); mxFree(pi); if (own) mxFree((void *)tpl);
+}
+
 #elif defined(GSMCAL_MEX_gsm_calibrate_demod_batch) || defined(GSMCAL_MEX_gsm_calibrate_sch_decode_batch)
 /* [sampling_ppm, carrier_ppm, n_pos_info, pos_info, sch, fcch, bcch] =
  *     gsm_calibrate_demod_batch(raw_uint8, carrier_freq, sch_training_sequence, coef [, normal_training_sequence])
