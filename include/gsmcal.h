@@ -443,6 +443,40 @@ int gsmcal_calibrate_sch_decode_batch(const uint8_t *raw, int raw_mem, int64_t n
                                       gsmcal_sch_decode_result *dec /* [n_streams], required */,
                                       int32_t *sch_fn, int32_t *sch_bsic, uint8_t *sch_hamming, uint8_t *sch_row_flags);
 
+/* gsmcal_calibrate_carrier_fit_batch (every output as there, byte for byte) followed by SCH_demod of every SCH row of pos_info on
+ * r_correct with the carrier fit's residual removed, then the SCH decoding above: each dongle's cell and frame clock from a short capture.
+ * r_correct keeps the about +1 kHz that total_carrier_ppm leaves (residual_ppm); SCH_demod's channel estimate has no phase tracking, so
+ * at 1 kHz the outermost coded bits, about 70 symbols (258 us) from the training centre, see up to 1.6 rad of phase error and most rows
+ * fail the CRC.  Only oversampling_ratio 8 (osr).  For stream d, with a = freq_hz, b = drift_hz_per_s, t_mean of its carrier record,
+ * fs = 8 * 1625e3/6, f_nom = fs/32, e1 = sampling_ppm[0]*1e-6, e2 = sampling_ppm[1]*1e-6, r = r_correct (1-based) and p_i the position of
+ * the i-th SCH row (type 1) of pos_info:
+ *   1. t_i = (((p_i + 74*osr - 1)*(1 + e2))*(1 + e1))/fs: the capture time of the training centre, mapped as step 5 of the carrier fit.
+ *   2. df_i = (a - f_nom) + b*(t_i - t_mean) Hz, in r_correct's frame.  Steps 1 and 2 round every operation on its own.
+ *   3. x(n) = r(p_i - 8*osr + n) * exp(-i*2*pi*df_i*n/fs), n = 0..194*osr-1 (SCH_demod.m:79-81's window; a constant phase cancels in
+ *      the FDE channel estimate, so the window start is the phase reference), then SCH_demod.m:83-110 unchanged: demod_bits, corr_val
+ *      (bits_to_decoder is not returned).  A window outside r: sch_ok = 0 and zeros, as in gsmcal_calibrate_demod_batch.
+ *   4. steps 1-7 of the SCH decoding above on these rows: the same row flags, vote and frame_clock_start.
+ *   5. a stream with r_correct but no fit (GSMCAL_CARRIER_FEW): df_i = 0, so its rows are gsmcal_calibrate_demod_batch's; its decode
+ *      record gets GSMCAL_SCHDEC_UNCORRECTED (never set by gsmcal_calibrate_sch_decode_batch) and sch_df is NaN.  NO_POS_INFO and
+ *      NO_R_CORRECT as in gsmcal_calibrate_sch_decode_batch.
+ * Per-row arrays [n_streams][B] (B as above), each may be NULL (not copied back): the carrier fit's fcch_f, fcch_t, fcch_row_flags; sch_ok,
+ * demod_bits [..][148], corr_val [..][85] and sch_df (df_i; NaN beyond the record's n_sch) of the corrected SCH rows; sch_fn, sch_bsic,
+ * sch_hamming, sch_row_flags as in gsmcal_calibrate_sch_decode_batch.  The rows of sch_ok, demod_bits and corr_val beyond n_sch are not
+ * written. */
+#define GSMCAL_SCHDEC_UNCORRECTED  16  /* gsmcal_calibrate_cell_batch: no carrier fit, the rows were demodulated without a correction */
+
+int gsmcal_calibrate_cell_batch(const uint8_t *raw, int raw_mem, int64_t n_iq, int64_t n_streams,
+                                double carrier_freq, const double *sch_training_sequence,
+                                const double *coef, int n_taps, int oversampling_ratio, int coarse_decimation,
+                                gsmcal_stream_result *results,
+                                double *coarse_pos, double *coarse_snr, double *fcch_pos, double *pos_info,
+                                void *cuda_stream,
+                                gsmcal_carrier_fit_result *carrier /* [n_streams], required */,
+                                double *fcch_f, double *fcch_t, uint8_t *fcch_row_flags,
+                                gsmcal_sch_decode_result *dec /* [n_streams], required */, uint8_t *sch_ok, uint8_t *demod_bits,
+                                double *corr_val, double *sch_df, int32_t *sch_fn, int32_t *sch_bsic, uint8_t *sch_hamming,
+                                uint8_t *sch_row_flags);
+
 /* The same pipeline with several batches in flight (continuous captures): _submit enqueues batch `slot` (0..3) on the library's
  * own streams once the caller's `cuda_stream` has produced the DEVICE-resident capture, and returns; _collect waits for that batch
  * and fills the result pointers given to _submit (they must stay valid until then).  Batches are staggered on the device: the
@@ -466,8 +500,9 @@ int gsmcal_calibrate_batch_cancel(int slot);
  * [3] fine ppm + tone estimate + gate [4] SCH correlation + pos_info [5] post-SCH tone estimate + result records
  * [6] (gsmcal_calibrate_demod_batch / _demod_bcch_batch / _sch_decode_batch only) SCH_demod (+ SCH decoding) + FCCH_demod (+ BCCH_demod);
  *     (gsmcal_calibrate_sch_timing_batch only) SCH row list, sub-sample SCH timing and the clock fit;
- *     (gsmcal_calibrate_carrier_fit_batch only) FCCH row list, the tone of every FCCH burst and the carrier fit.  Returns the number of
- *     stages written. */
+ *     (gsmcal_calibrate_carrier_fit_batch only) FCCH row list, the tone of every FCCH burst and the carrier fit;
+ *     (gsmcal_calibrate_cell_batch only) the row lists, the carrier fit, SCH_demod less the residual and SCH decoding.  Returns the number
+ *     of stages written. */
 int gsmcal_last_batch_stage_ms(double *ms, int cap);
 
 /* FCCH scanner per-channel processing, multi_rtl_sdr_gsm_FCCH_scanner.m:132-135,163-186, for n_chan

@@ -212,6 +212,7 @@ int get_ctx(Ctx **out) {
         CU(cudaFuncSetAttribute(fde_template_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 120 * 1024));    //  all of them live here, keyed by
         CU(cudaFuncSetAttribute(sch_demod_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 120 * 1024));       //  the device's Ctx)
         CU(cudaFuncSetAttribute(sch_demod_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
+        CU(cudaFuncSetAttribute(sch_demod_resid_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
         CU(cudaFuncSetAttribute(fcch_demod_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
         c.attrs = true;
     }
@@ -567,16 +568,18 @@ size_t sch_demod_smem(int osr);
 void gmsk_branch_table(int osr, double *W);
 void sch_training_pm(signed char *data_pm);
 
-// ---- the stage behind post-SCH ("tail") of gsmcal_calibrate_demod_batch, _demod_bcch_batch, _sch_decode_batch, _sch_timing_batch and
-// _carrier_fit_batch --
-// It is the SCH timing block when `timing` is set, the carrier fit block when `carrier` is set, else the demod block (batched SCH_demod /
-// FCCH_demod) with the BCCH block when `nts` is set and the SCH decoding block when `sdec` is set.
+// ---- the stage behind post-SCH ("tail") of gsmcal_calibrate_demod_batch, _demod_bcch_batch, _sch_decode_batch, _sch_timing_batch,
+// _carrier_fit_batch and _cell_batch --
+// It is the SCH timing block when `timing` is set, the carrier fit block when `carrier` is set (with `sdec`: then the residual-corrected
+// SCH_demod and the SCH decoding block), else the demod block (batched SCH_demod / FCCH_demod) with the BCCH block when `nts` is set and
+// the SCH decoding block when `sdec` is set.
 struct TailOut {                     // the caller's host outputs; an array left NULL is not read back
     gsmcal_demod_result *demod; uint8_t *sch_ok, *bits, *dec; double *corr, *freq, *snr, *idx;
     const double *nts; gsmcal_bcch_result *bcch;
     gsmcal_sch_decode_result *sdec; int32_t *fn, *bsic; uint8_t *ham, *rflag;
     gsmcal_sch_timing_result *timing; double *tau, *x;
     gsmcal_carrier_fit_result *carrier; double *cf_f, *cf_t; uint8_t *cf_flag;
+    double *sch_df;
 };
 struct TailDev {                     // device buffers of the same blocks
     DemodResultDev *rec; double *sch_pos, *fcch_pos; unsigned char *sch_ok, *fcch_ok;                       // the row lists
@@ -585,6 +588,7 @@ struct TailDev {                     // device buffers of the same blocks
     SchDecodeResultDev *sdec; int *key, *fn, *bsic; unsigned char *ham, *rflag;
     TimingResultDev *timing; double *tau, *x; unsigned char *row_flag;
     CarrierFitDev *carrier; double *cf_f, *cf_t; unsigned char *cf_flag;
+    double *sch_df;
 };
 // every per-stream array ([D] records, [D][cap] rows) of the blocks `o` asks for: f(device pointer, bytes per stream, the caller's host
 // array or NULL).  Set-up, the slice of a stream group and the read-back all walk this one list.  The per-call constants (Ft, Wtab, dpm,
@@ -599,6 +603,11 @@ template <class F> void tail_arrays(TailDev &t, const TailOut &o, int cap, F &&f
     }
     if (o.carrier) {
         f(t.carrier, sizeof(CarrierFitDev), o.carrier); f(t.cf_f, 8 * r, o.cf_f); f(t.cf_t, 8 * r, o.cf_t); f(t.cf_flag, r, o.cf_flag);
+        if (o.sdec) {                // the corrected SCH rows (bits_to_decoder is written, not returned) and their decoding
+            f(t.bits, 148 * r, o.bits); f(t.dec, 148 * r, nullptr); f(t.corr, 8 * 85 * r, o.corr); f(t.sch_df, 8 * r, o.sch_df);
+            f(t.sdec, sizeof(SchDecodeResultDev), o.sdec); f(t.key, 4 * r, nullptr); f(t.fn, 4 * r, o.fn); f(t.bsic, 4 * r, o.bsic);
+            f(t.ham, r, o.ham); f(t.rflag, r, o.rflag);
+        }
         return;
     }
     f(t.bits, 148 * r, o.bits); f(t.dec, 148 * r, o.dec); f(t.corr, 8 * 85 * r, o.corr); f(t.freq, 8 * r, o.freq); f(t.snr, 8 * r, o.snr);
@@ -616,18 +625,19 @@ template <class T> void place(T *&p, uintptr_t a) { p = (T *)a; }
 int tail_setup(Ctx &c, i64 D, int cap, int osr, const double2 *tpl_dev, const TailOut &o, std::vector<double> &W, signed char *data_pm,
                cudaStream_t st, TailDev *t) {
     const int N = SD_NSYM * osr;
+    const bool sch = !o.timing && (!o.carrier || o.sdec);        // SCH rows are demodulated
     *t = TailDev{};
     auto layout = [&](uintptr_t base) {          // points every buffer into [base, base + the size it returns)
         size_t off = 0;
         auto take = [&](auto *&p, size_t bytes) { place(p, base + off); off = align_up(off + bytes); };
         tail_arrays(*t, o, cap, [&](auto *&p, size_t per, const void *) { take(p, per * D); });
-        if (!o.timing && !o.carrier) { take(t->Ft, sizeof(double2) * N); take(t->Wtab, sizeof(double2) * 16 * osr); take(t->dpm, 64); }
+        if (sch) { take(t->Ft, sizeof(double2) * N); take(t->Wtab, sizeof(double2) * 16 * osr); take(t->dpm, 64); }
         if (o.nts) take(t->nts, sizeof(double2) * 8 * 26 * osr);
         return off;
     };
     void *base; TRY(c.dem.get(layout(0), &base));
     layout((uintptr_t)base);
-    if (o.timing || o.carrier) return GSMCAL_OK;
+    if (!sch) return GSMCAL_OK;
     if (o.nts) CU(cudaMemcpyAsync(t->nts, o.nts, sizeof(double2) * 8 * 26 * (size_t)osr, cudaMemcpyHostToDevice, st));
     W.assign(2 * 16 * (size_t)osr, 0.0);
     gmsk_branch_table(osr, W.data());
@@ -639,7 +649,8 @@ int tail_setup(Ctx &c, i64 D, int cap, int osr, const double2 *tpl_dev, const Ta
     return GSMCAL_OK;
 }
 // one stream group: row lists + sentinels, then either the timing of every SCH row and the per-stream fit (osr 8), or the tone of every
-// FCCH row and the per-stream carrier fit (osr 8), or SCH bursts, SCH decoding and BCCH_demod when their outputs were asked for, FCCH
+// FCCH row and the per-stream carrier fit (osr 8) with, for _cell_batch, the SCH bursts less the fitted residual and their decoding, or
+// SCH bursts, SCH decoding and BCCH_demod when their outputs were asked for, FCCH
 // bursts, FCCH means
 int run_tail(Ctx &c, WinSrc src, const Work &ws, const TailDev &t, int osr, double carrier_freq, i64 nd, int cap, cudaStream_t st) {
     LAUNCH(demod_compact_kernel, (unsigned)nd, 32, 0, st, ws.ctl, ws.pos_info, cap, osr, t.rec, t.sch_pos, t.sch_ok, t.fcch_pos, t.fcch_ok);
@@ -653,6 +664,12 @@ int run_tail(Ctx &c, WinSrc src, const Work &ws, const TailDev &t, int osr, doub
         LAUNCH(carrier_fit_row_kernel, dim3((unsigned)cap, (unsigned)nd), CF_THREADS, CF_SMEM, st, with_cache(src, ws, cap), ws.ctl, t.rec, t.fcch_pos,
                t.fcch_ok, cap, t.cf_f, t.cf_t, t.cf_flag);
         LAUNCH(carrier_fit_stream_kernel, (unsigned)nd, 32, 0, st, ws.ctl, t.rec, t.cf_flag, t.cf_f, t.cf_t, cap, carrier_freq, t.carrier);
+        if (!t.sdec) return GSMCAL_OK;
+        const double2 *tw_s; TRY(get_twiddle(c, SD_NSYM * osr, st, &tw_s));        // built by the set-up: no launch here
+        LAUNCH(sch_demod_resid_kernel, dim3((unsigned)cap, (unsigned)nd), SDB_THREADS, sch_demod_smem(osr), st, src, ws.ctl, t.rec, t.sch_pos, t.sch_ok,
+               cap, tw_s, t.Ft, t.Wtab, t.dpm, t.carrier, t.bits, t.dec, t.corr, t.sch_df);
+        LAUNCH(sch_decode_batch_kernel, (unsigned)nd, 32, 0, st, t.rec, t.sch_pos, t.sch_ok, t.bits, t.corr, cap, osr, t.key, t.fn, t.bsic,
+               t.ham, t.rflag, t.sdec);
         return GSMCAL_OK;
     }
     const double2 *tw_s, *tw_f;                  // both built by the set-up: no launch here
@@ -1395,6 +1412,25 @@ int gsmcal_calibrate_carrier_fit_batch(const uint8_t *raw, int raw_mem, int64_t 
     o.carrier = carrier; o.cf_f = fcch_f; o.cf_t = fcch_t; o.cf_flag = fcch_row_flags;
     return calibrate_batch_impl(raw, raw_mem, n_iq, D, carrier_freq, tpl, coef, n_taps, osr, coarse_dr, results, coarse_pos, coarse_snr, fcch_pos, pos_info,
                                 cuda_stream, nullptr, GSMCAL_MEM_DEVICE, 0, &o);
+}
+
+int gsmcal_calibrate_cell_batch(const uint8_t *raw, int raw_mem, int64_t n_iq, int64_t D, double carrier_freq, const double *tpl,
+                                const double *coef, int n_taps, int osr, int coarse_dr, gsmcal_stream_result *results,
+                                double *coarse_pos, double *coarse_snr, double *fcch_pos, double *pos_info, void *cuda_stream,
+                                gsmcal_carrier_fit_result *carrier, double *fcch_f, double *fcch_t, uint8_t *fcch_row_flags,
+                                gsmcal_sch_decode_result *dec, uint8_t *sch_ok, uint8_t *demod_bits, double *corr_val,
+                                double *sch_df, int32_t *sch_fn, int32_t *sch_bsic, uint8_t *sch_hamming, uint8_t *sch_row_flags) {
+    if (!carrier || !dec) return fail(GSMCAL_ERR_ARG, "calibrate_cell_batch: null carrier or dec");
+    if (osr != 8) return fail(GSMCAL_ERR_ARG, "calibrate_cell_batch: oversampling_ratio must be 8");
+    TailOut o{};
+    o.carrier = carrier; o.cf_f = fcch_f; o.cf_t = fcch_t; o.cf_flag = fcch_row_flags;
+    o.sdec = dec; o.sch_ok = sch_ok; o.bits = demod_bits; o.corr = corr_val; o.sch_df = sch_df;
+    o.fn = sch_fn; o.bsic = sch_bsic; o.ham = sch_hamming; o.rflag = sch_row_flags;
+    TRY(calibrate_batch_impl(raw, raw_mem, n_iq, D, carrier_freq, tpl, coef, n_taps, osr, coarse_dr, results, coarse_pos, coarse_snr, fcch_pos, pos_info,
+                             cuda_stream, nullptr, GSMCAL_MEM_DEVICE, 0, &o));
+    for (int64_t d = 0; d < D; ++d)                              // SCH_demod ran on r_correct as it is: the rows of _demod_batch
+        if (dec[d].n_sch >= 0 && (carrier[d].flags & GSMCAL_CARRIER_FEW)) dec[d].flags |= GSMCAL_SCHDEC_UNCORRECTED;
+    return GSMCAL_OK;
 }
 
 // ---- submit / collect: the same pipeline, several batches in flight -----------------------------------------------------------

@@ -413,13 +413,15 @@ __device__ __forceinline__ void derotate_post(double2 *dst, int count, double dp
 
 // SCH_demod.m:65-110 for one (SCH row, stream).  320 threads: the 1552-sample level-0 window of the loader is filtered by its unrolled
 // 5-outputs-per-thread path.  Shared: x[N] | b1[N] | b2[N] | b3[N] (the loader's scratch and the branch correlations alias b1..b3).
+// RESID (sch_demod_resid_kernel): the derotation step is dphi2 - resid, which also rotates the window by exp(-i*resid*n) from its start.
 #define SDB_THREADS 320
-__global__ void __launch_bounds__(SDB_THREADS, 2) sch_demod_batch_kernel(WinSrc src, const StreamCtl *__restrict__ ctl, const DemodResultDev *__restrict__ rec,
-                                                                        const double *__restrict__ sch_pos, const unsigned char *__restrict__ sch_ok, int cap, int osr,
-                                                                        const double2 *__restrict__ tw, const double2 *__restrict__ Ft,
-                                                                        const double2 *__restrict__ Wtab, const signed char *__restrict__ data_pm,
-                                                                        unsigned char *__restrict__ demod_bits, unsigned char *__restrict__ dec_bits,
-                                                                        double *__restrict__ corr_val) {
+template <bool RESID>
+__device__ __forceinline__ void sch_demod_body(WinSrc src, const StreamCtl *__restrict__ ctl, const DemodResultDev *__restrict__ rec,
+                                               const double *__restrict__ sch_pos, const unsigned char *__restrict__ sch_ok, int cap, int osr,
+                                               const double2 *__restrict__ tw, const double2 *__restrict__ Ft,
+                                               const double2 *__restrict__ Wtab, const signed char *__restrict__ data_pm,
+                                               unsigned char *__restrict__ demod_bits, unsigned char *__restrict__ dec_bits,
+                                               double *__restrict__ corr_val, double resid) {
     extern __shared__ double2 sm[];
     __shared__ unsigned char bits[SD_NSYM + 2];
     __shared__ signed char dpm[64];
@@ -442,7 +444,7 @@ __global__ void __launch_bounds__(SDB_THREADS, 2) sch_demod_batch_kernel(WinSrc 
     if (tid < M / 2) wm[tid] = tw[97 * tid];
     if (tid == 0) { double sn, cs; sincos((double)j0 * c.dphi2, &sn, &cs); ph0 = make_double2(cs, sn); }
     load_window(src, c, stream, j0, N, x, b1, b1 + GSMCAL_XCAP(N));          // ends with a barrier
-    derotate_post(x, N, c.dphi2, ph0);
+    derotate_post(x, N, RESID ? c.dphi2 - resid : c.dphi2, ph0);
     __syncthreads();
     for (int n = tid; n < N; n += SDB_THREADS) b1[n] = (n >= sp_tr && n < sp_tr + L) ? x[n] : make_double2(0.0, 0.0);     // :83-84
     __syncthreads();
@@ -454,6 +456,14 @@ __global__ void __launch_bounds__(SDB_THREADS, 2) sch_demod_batch_kernel(WinSrc 
     __syncthreads();
     dft97<true>(x, b2, b3, x, M, 1, tw, w97, wm);                            // x = ifft(fd_x) (:90)
     sch_bits_body(x, b1, osr, Wtab, dpm, bits, demod_bits + o * 148, dec_bits + o * 148, corr_val + o * 85);
+}
+__global__ void __launch_bounds__(SDB_THREADS, 2) sch_demod_batch_kernel(WinSrc src, const StreamCtl *__restrict__ ctl, const DemodResultDev *__restrict__ rec,
+                                                                        const double *__restrict__ sch_pos, const unsigned char *__restrict__ sch_ok, int cap, int osr,
+                                                                        const double2 *__restrict__ tw, const double2 *__restrict__ Ft,
+                                                                        const double2 *__restrict__ Wtab, const signed char *__restrict__ data_pm,
+                                                                        unsigned char *__restrict__ demod_bits, unsigned char *__restrict__ dec_bits,
+                                                                        double *__restrict__ corr_val) {
+    sch_demod_body<false>(src, ctl, rec, sch_pos, sch_ok, cap, osr, tw, Ft, Wtab, data_pm, demod_bits, dec_bits, corr_val, 0.0);
 }
 
 // FCCH_demod.m:21-66 for one (FCCH row, stream): the window comes through the fine search's filtered-window cache where it covers it
@@ -1058,4 +1068,38 @@ __global__ void __launch_bounds__(32) carrier_fit_stream_kernel(const StreamCtl 
     q.carrier_fit_ppm = total_ppm2(total_ppm2(c.cppm1, c.cppm2), q.residual_ppm);         // total_carrier_ppm of the record, then the residual
     q.drift_ppm_per_s = __dmul_rn(1e6, b) / carrier_freq;
     out[stream] = q;
+}
+
+// ===================================================================================================
+// SCH_demod of gsmcal_calibrate_cell_batch (definition: include/gsmcal.h): every SCH row of pos_info on r_correct with the stream's
+// carrier-fit line removed from its equaliser window, on what carrier_fit_stream_kernel wrote.  osr 8 only.
+// ===================================================================================================
+// df_i (Hz, r_correct's frame) of the SCH row at p: the fitted line at the capture time of the training centre r(p + 74*osr), mapped as
+// carrier_fit_row_kernel maps its window centre; every operation rounded on its own.  NaN without a fit.
+__device__ __forceinline__ double sch_resid_hz(const CarrierFitDev &q, const StreamCtl &c, double p) {
+    if (q.flags & CF_FEW) return NAN;
+    const double s1 = __dadd_rn(1.0, __dmul_rn(c.sppm1, 1e-6)), s2 = __dadd_rn(1.0, __dmul_rn(c.sppm2, 1e-6));
+    const double t = __ddiv_rn(__dmul_rn(__dmul_rn(p + (double)(74 * 8 - 1), s2), s1), ((1625.0 / 6.0) * 1e3) * 8.0);   // p + 591: exact
+    return __dadd_rn(__dsub_rn(q.freq_hz, ((1625.0 / 6.0) * 1e3) / 4.0), __dmul_rn(q.drift_hz_per_s, __dsub_rn(t, q.t_mean)));
+}
+
+// sch_demod_batch_kernel's body with the residual folded into the derotation it already does: no extra pass over the window.  df_out
+// [stream][cap]: df_i, NaN without a fit and for rows beyond n_sch.
+__global__ void __launch_bounds__(SDB_THREADS, 2) sch_demod_resid_kernel(WinSrc src, const StreamCtl *__restrict__ ctl, const DemodResultDev *__restrict__ rec,
+                                                                        const double *__restrict__ sch_pos, const unsigned char *__restrict__ sch_ok, int cap,
+                                                                        const double2 *__restrict__ tw, const double2 *__restrict__ Ft,
+                                                                        const double2 *__restrict__ Wtab, const signed char *__restrict__ data_pm,
+                                                                        const CarrierFitDev *__restrict__ carrier, unsigned char *__restrict__ demod_bits,
+                                                                        unsigned char *__restrict__ dec_bits, double *__restrict__ corr_val,
+                                                                        double *__restrict__ df_out) {
+    const int row = blockIdx.x, stream = blockIdx.y;
+    const i64 o = (i64)stream * cap + row;
+    if (row >= rec[stream].n_sch) {
+        if (threadIdx.x == 0) df_out[o] = NAN;
+        return;
+    }
+    const double df = sch_resid_hz(carrier[stream], ctl[stream], sch_pos[o]);
+    if (threadIdx.x == 0) df_out[o] = df;
+    const double resid = isnan(df) ? 0.0 : __ddiv_rn(__dmul_rn(2.0 * GSMCAL_PI, df), ((1625.0 / 6.0) * 1e3) * 8.0);      // rad per sample
+    sch_demod_body<true>(src, ctl, rec, sch_pos, sch_ok, cap, 8, tw, Ft, Wtab, data_pm, demod_bits, dec_bits, corr_val, resid);
 }

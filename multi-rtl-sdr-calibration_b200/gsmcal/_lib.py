@@ -91,6 +91,7 @@ SIGNATURES = {
     "gsmcal_calibrate_sch_decode_batch": (C.c_int, _BATCH + [C.c_void_p] * 15),
     "gsmcal_calibrate_sch_timing_batch": (C.c_int, _BATCH + [C.c_void_p] * 3),
     "gsmcal_calibrate_carrier_fit_batch": (C.c_int, _BATCH + [C.c_void_p] * 4),
+    "gsmcal_calibrate_cell_batch": (C.c_int, _BATCH + [C.c_void_p] * 13),
     "gsmcal_calibrate_batch_submit": (C.c_int, [C.c_int, C.c_void_p, c_i64, c_i64, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "gsmcal_calibrate_batch_collect": (C.c_int, [C.c_int]),

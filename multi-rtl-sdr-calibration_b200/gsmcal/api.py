@@ -330,7 +330,7 @@ def _batch_args(raw, carrier_freq, sch_training_sequence, coef, osr, coarse_dr, 
 def calibrate_batch(raw, carrier_freq: float, sch_training_sequence, coef, osr: int = 8, coarse_dr: int = 8,
                     device_ptr: int | None = None, n_iq: int | None = None, n_streams: int | None = None,
                     cuda_stream: int = 0, details: bool = True, r_correct=None, r_device_ptr: int | None = None,
-                    sch_timing: bool = False, carrier_fit: bool = False):
+                    sch_timing: bool = False, carrier_fit: bool = False, sch_decode: bool = False):
     """gsm_sync_demod.m:107-124 for every row of `raw` ([D, 2N] uint8, row d == dongle d's fread column).
 
     `raw` is a host NumPy array, or pass device_ptr/n_iq/n_streams for a capture already resident in HBM.
@@ -349,11 +349,20 @@ def calibrate_batch(raw, carrier_freq: float, sch_training_sequence, coef, osr: 
     freq_hz, drift_hz_per_s, rms_hz, residual_ppm, n_fit, flags, f, t, row_flags): carrier_fit_ppm the dongle's carrier error at t_mean
     (seconds of capture time), drift_ppm_per_s its drift, freq_hz / drift_hz_per_s / rms_hz the line through the tones in r_correct's
     frame, residual_ppm what total_carrier_ppm left, flags CARRIER_* bits, and per FCCH row f (Hz), t (s) and row_flags, f and t NaN
-    where excluded; f, t and row_flags are None when the step did not run (CARRIER_NO_POS_INFO / CARRIER_NO_R_CORRECT)."""
+    where excluded; f, t and row_flags are None when the step did not run (CARRIER_NO_POS_INFO / CARRIER_NO_R_CORRECT).
+
+    sch_decode=True (only with carrier_fit=True) then demodulates every SCH burst of pos_info on r_correct with the fitted residual
+    removed and decodes it (gsmcal_calibrate_cell_batch, include/gsmcal.h); each dict also gains
+      cell: calibrate_demod_batch(..., sch_decode=True)'s cell dict plus df, the residual removed from each SCH row (Hz; NaN without a
+            fit, where flags has SCHDEC_UNCORRECTED and the rows are demodulated as calibrate_demod_batch does);
+      sch:  dict(demod_bits [n x 148], corr_val [n x 85], sch_ok [n] bool) of the corrected rows, n = SCH rows of pos_info.
+    cell's per-row arrays and sch are None where SCH_demod did not run.  frame_clock_offsets takes these results as they are."""
     if (sch_timing or carrier_fit) and (r_correct is not None or r_device_ptr is not None):
         raise ValueError("sch_timing / carrier_fit do not combine with r_correct / r_device_ptr")
     if sch_timing and carrier_fit:
         raise ValueError("sch_timing and carrier_fit are separate calls")
+    if sch_decode and (sch_timing or not carrier_fit):
+        raise ValueError("calibrate_batch decodes SCH bursts only with carrier_fit=True and without sch_timing")
     details = details or sch_timing or carrier_fit
     args, keep, D, n_iq, cap, res, arrays = _batch_args(raw, carrier_freq, sch_training_sequence, coef, osr, coarse_dr, device_ptr, n_iq,
                                                         n_streams, cuda_stream, details)
@@ -364,7 +373,16 @@ def calibrate_batch(raw, carrier_freq: float, sch_training_sequence, coef, osr: 
     elif carrier_fit:
         cf = (CarrierFitResult * D)()
         f, t, rf = np.empty((D, cap)), np.empty((D, cap)), np.empty((D, cap), dtype=np.uint8)
-        check(lib().gsmcal_calibrate_carrier_fit_batch(*args, C.cast(cf, C.c_void_p), _ptr(f), _ptr(t), _ptr(rf)))
+        cf_args = [C.cast(cf, C.c_void_p), _ptr(f), _ptr(t), _ptr(rf)]
+        if sch_decode:
+            sd = (SchDecodeResult * D)()
+            sch_ok, bits, corr = np.zeros((D, cap), dtype=np.uint8), np.zeros((D, cap, 148), dtype=np.uint8), np.zeros((D, cap, 85))
+            df, fn, bsic = np.empty((D, cap)), np.empty((D, cap), dtype=np.int32), np.empty((D, cap), dtype=np.int32)
+            ham, rfl = np.empty((D, cap), dtype=np.uint8), np.empty((D, cap), dtype=np.uint8)
+            check(lib().gsmcal_calibrate_cell_batch(*args, *cf_args, C.cast(sd, C.c_void_p), _ptr(sch_ok), _ptr(bits), _ptr(corr), _ptr(df),
+                                                    _ptr(fn), _ptr(bsic), _ptr(ham), _ptr(rfl)))
+        else:
+            check(lib().gsmcal_calibrate_carrier_fit_batch(*args, *cf_args))
     elif r_correct is None and r_device_ptr is None:
         check(lib().gsmcal_calibrate_batch(*args))
     else:
@@ -392,7 +410,23 @@ def calibrate_batch(raw, carrier_freq: float, sch_training_sequence, coef, osr: 
                                    drift_hz_per_s=c.drift_hz_per_s, rms_hz=c.rms_hz, residual_ppm=c.residual_ppm, n_fit=c.n_fit,
                                    flags=c.flags, f=None if n < 0 else f[d, :n].copy(), t=None if n < 0 else t[d, :n].copy(),
                                    row_flags=None if n < 0 else rf[d, :n].astype(np.int64))
+    if sch_decode:
+        for d, item in enumerate(out):
+            item["cell"] = _cell_dict(sd[d], d, fn, bsic, ham, rfl)
+            n = sd[d].n_sch
+            item["cell"]["df"] = None if n < 0 else df[d, :n].copy()
+            item["sch"] = None if n < 0 else dict(demod_bits=bits[d, :n].astype(np.int64), corr_val=corr[d, :n].copy(),
+                                                  sch_ok=sch_ok[d, :n].astype(bool))
     return out
+
+
+def _cell_dict(c, d, fn, bsic, ham, rfl):
+    """the cell dict of stream d from its gsmcal_sch_decode_result and the per-row arrays"""
+    n = c.n_sch
+    rows = lambda a: None if n < 0 else a[d, :n].astype(np.int64)          # noqa: E731
+    return dict(bsic=c.bsic, ncc=c.bsic >> 3 if c.bsic >= 0 else -1, bcc=c.bsic & 7 if c.bsic >= 0 else -1, fn_first=c.fn_first,
+                frame_clock_start=c.frame_clock_start, n_crc_ok=c.n_crc_ok, n_agree=c.n_agree, flags=c.flags, fn=rows(fn),
+                bsic_rows=rows(bsic), hamming=rows(ham), row_flags=rows(rfl))
 
 
 TIMING_NO_POS_INFO, TIMING_NO_R_CORRECT, TIMING_RANGE, TIMING_EDGE, TIMING_FEW = 1, 2, 4, 8, 16
@@ -401,6 +435,7 @@ DEMOD_NO_POS_INFO, DEMOD_NO_R_CORRECT, DEMOD_SCH_RANGE, DEMOD_FCCH_RANGE = 1, 2,
 BCCH_NO_POS_INFO, BCCH_FEW_BCCH, BCCH_FCCH_RANGE, BCCH_TRAIN_RANGE = 1, 2, 4, 8
 SCHDEC_NO_POS_INFO, SCHDEC_NO_R_CORRECT, SCHDEC_NONE, SCHDEC_DISAGREE = 1, 2, 4, 8
 SCHDEC_ROW_WINDOW, SCHDEC_ROW_ALIGN, SCHDEC_ROW_CRC, SCHDEC_ROW_FIELD = 1, 2, 4, 8
+SCHDEC_UNCORRECTED = 16                            # calibrate_batch(..., carrier_fit=True, sch_decode=True): no fit, rows not corrected
 FN_MOD = 2715648                                   # TDMA frames in a hyperframe
 
 
@@ -469,16 +504,13 @@ def calibrate_demod_batch(raw, carrier_freq: float, sch_training_sequence, coef,
             item["bcch"] = dict(carrier_ppm=b.carrier_ppm, nts_idx=b.nts_idx, flags=b.flags,
                                 corr_abs=None if none else np.array(b.corr_abs).reshape(4, 8).T.copy())
         if sch_decode:
-            c, n = sd[d], sd[d].n_sch
-            rows = lambda a: None if n < 0 else a[d, :n].astype(np.int64)      # noqa: E731
-            item["cell"] = dict(bsic=c.bsic, ncc=c.bsic >> 3 if c.bsic >= 0 else -1, bcc=c.bsic & 7 if c.bsic >= 0 else -1,
-                                fn_first=c.fn_first, frame_clock_start=c.frame_clock_start, n_crc_ok=c.n_crc_ok, n_agree=c.n_agree,
-                                flags=c.flags, fn=rows(fn), bsic_rows=rows(bsic), hamming=rows(ham), row_flags=rows(rfl))
+            item["cell"] = _cell_dict(sd[d], d, fn, bsic, ham, rfl)
     return out
 
 
 def frame_clock_offsets(results, ref: int = 0, osr: int = 8) -> np.ndarray:
-    """Capture-start offsets on the cell's frame clock, from calibrate_demod_batch(..., sch_decode=True) results: for every stream that
+    """Capture-start offsets on the cell's frame clock, from calibrate_demod_batch(..., sch_decode=True) or calibrate_batch(...,
+    carrier_fit=True, sch_decode=True) results: for every stream that
     decoded the same BSIC as stream `ref` (both with a winner), frame_clock_start[d] - frame_clock_start[ref] wrapped into (-H/2, H/2],
     H = one hyperframe = 2,715,648 * 1250 * osr nominal samples; NaN for every other stream.  Positive: stream d started later."""
     h = float(FN_MOD * 1250 * int(osr))

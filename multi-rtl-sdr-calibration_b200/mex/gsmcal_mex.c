@@ -111,6 +111,58 @@ static void batch_outputs(int nlhs, mxArray *plhs[], const gsmcal_stream_result 
 }
 
 /* ------------------------------------------------------------------------------------------------ */
+#if defined(GSMCAL_MEX_gsm_calibrate_carrier_batch) || defined(GSMCAL_MEX_gsm_calibrate_cell_batch)
+/* 1 x D struct array of the carrier fit: the records and the per-FCCH-row f, t, row_flags ([D][B]) */
+static mxArray *carrier_struct(const gsmcal_carrier_fit_result *cf, const double *fr, const double *tr, const uint8_t *rf, size_t D, size_t B) {
+    const char *f[] = {"carrier_fit_ppm", "drift_ppm_per_s", "t_mean", "freq_hz", "drift_hz_per_s", "rms_hz", "residual_ppm", "n_fit", "flags",
+                       "f", "t", "row_flags"};
+    mxArray *s = mxCreateStructMatrix(1, D, 12, f);
+    for (size_t d = 0; d < D; ++d) {
+        const size_t n = cf[d].n_fcch > 0 ? (size_t)cf[d].n_fcch : 0;
+        mxArray *fa = mxCreateDoubleMatrix(1, n, mxREAL), *ta = mxCreateDoubleMatrix(1, n, mxREAL), *ra = mxCreateDoubleMatrix(1, n, mxREAL);
+        if (n) { memcpy(mxGetPr(fa), fr + d * B, n * sizeof(double)); memcpy(mxGetPr(ta), tr + d * B, n * sizeof(double)); }
+        for (size_t i = 0; i < n; ++i) mxGetPr(ra)[i] = rf[d * B + i];
+        mxSetField(s, d, "carrier_fit_ppm", scalar(cf[d].carrier_fit_ppm)); mxSetField(s, d, "drift_ppm_per_s", scalar(cf[d].drift_ppm_per_s));
+        mxSetField(s, d, "t_mean", scalar(cf[d].t_mean)); mxSetField(s, d, "freq_hz", scalar(cf[d].freq_hz));
+        mxSetField(s, d, "drift_hz_per_s", scalar(cf[d].drift_hz_per_s)); mxSetField(s, d, "rms_hz", scalar(cf[d].rms_hz));
+        mxSetField(s, d, "residual_ppm", scalar(cf[d].residual_ppm)); mxSetField(s, d, "n_fit", scalar(cf[d].n_fit));
+        mxSetField(s, d, "flags", scalar(cf[d].flags)); mxSetField(s, d, "f", fa); mxSetField(s, d, "t", ta);
+        mxSetField(s, d, "row_flags", ra);
+    }
+    return s;
+}
+#endif
+
+#if defined(GSMCAL_MEX_gsm_calibrate_sch_decode_batch) || defined(GSMCAL_MEX_gsm_calibrate_cell_batch)
+/* 1 x D struct array of the SCH decoding: the records and the per-SCH-row fn, bsic, hamming, row_flags ([D][B]); with df ([D][B], or
+ * NULL) also the residual removed from each row */
+static mxArray *cell_struct(const gsmcal_sch_decode_result *sd, const int32_t *sfn, const int32_t *sbs, const uint8_t *sham, const uint8_t *srf,
+                            const double *df, size_t D, size_t B) {
+    const char *f[] = {"bsic", "ncc", "bcc", "fn_first", "frame_clock_start", "n_crc_ok", "n_agree", "flags", "fn", "bsic_rows", "hamming", "row_flags",
+                       "df"};
+    mxArray *s = mxCreateStructMatrix(1, D, df ? 13 : 12, f);
+    for (size_t d = 0; d < D; ++d) {
+        const gsmcal_sch_decode_result *c = sd + d;
+        const size_t k = c->n_sch < 0 ? 0 : (size_t)c->n_sch;
+        mxArray *a[5];
+        for (int j = 0; j < 5; ++j) a[j] = mxCreateDoubleMatrix(1, k, mxREAL);
+        for (size_t i = 0; i < k; ++i) {
+            mxGetPr(a[0])[i] = sfn[d * B + i]; mxGetPr(a[1])[i] = sbs[d * B + i];
+            mxGetPr(a[2])[i] = sham[d * B + i]; mxGetPr(a[3])[i] = srf[d * B + i];
+            if (df) mxGetPr(a[4])[i] = df[d * B + i];
+        }
+        mxSetField(s, d, "bsic", scalar(c->bsic)); mxSetField(s, d, "ncc", scalar(c->bsic < 0 ? -1 : c->bsic >> 3));
+        mxSetField(s, d, "bcc", scalar(c->bsic < 0 ? -1 : c->bsic & 7)); mxSetField(s, d, "fn_first", scalar(c->fn_first));
+        mxSetField(s, d, "frame_clock_start", scalar(c->frame_clock_start)); mxSetField(s, d, "n_crc_ok", scalar(c->n_crc_ok));
+        mxSetField(s, d, "n_agree", scalar(c->n_agree)); mxSetField(s, d, "flags", scalar(c->flags));
+        mxSetField(s, d, "fn", a[0]); mxSetField(s, d, "bsic_rows", a[1]);
+        mxSetField(s, d, "hamming", a[2]); mxSetField(s, d, "row_flags", a[3]);
+        if (df) mxSetField(s, d, "df", a[4]); else mxDestroyArray(a[4]);
+    }
+    return s;
+}
+#endif
+
 #if defined(GSMCAL_MEX_raw2iq)
 /* b = raw2iq(a)                                                                        raw2iq.m:5 */
 void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
@@ -362,23 +414,42 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
                                                (int)nt, 8, 8, res, NULL, NULL, NULL, pi, NULL, cf, fr, tr, rf), "gsm_calibrate_carrier_batch");
     batch_outputs(nlhs, plhs, res, pi, D, (size_t)B);
     if (nlhs > 4) {
-        const char *f[] = {"carrier_fit_ppm", "drift_ppm_per_s", "t_mean", "freq_hz", "drift_hz_per_s", "rms_hz", "residual_ppm", "n_fit", "flags",
-                           "f", "t", "row_flags"};
-        plhs[4] = mxCreateStructMatrix(1, D, 12, f);
-        for (size_t d = 0; d < D; ++d) {
-            const size_t n = cf[d].n_fcch > 0 ? (size_t)cf[d].n_fcch : 0;
-            mxArray *fa = mxCreateDoubleMatrix(1, n, mxREAL), *ta = mxCreateDoubleMatrix(1, n, mxREAL), *ra = mxCreateDoubleMatrix(1, n, mxREAL);
-            if (n) { memcpy(mxGetPr(fa), fr + d * B, n * sizeof(double)); memcpy(mxGetPr(ta), tr + d * B, n * sizeof(double)); }
-            for (size_t i = 0; i < n; ++i) mxGetPr(ra)[i] = rf[d * B + i];
-            mxSetField(plhs[4], d, "carrier_fit_ppm", scalar(cf[d].carrier_fit_ppm)); mxSetField(plhs[4], d, "drift_ppm_per_s", scalar(cf[d].drift_ppm_per_s));
-            mxSetField(plhs[4], d, "t_mean", scalar(cf[d].t_mean)); mxSetField(plhs[4], d, "freq_hz", scalar(cf[d].freq_hz));
-            mxSetField(plhs[4], d, "drift_hz_per_s", scalar(cf[d].drift_hz_per_s)); mxSetField(plhs[4], d, "rms_hz", scalar(cf[d].rms_hz));
-            mxSetField(plhs[4], d, "residual_ppm", scalar(cf[d].residual_ppm)); mxSetField(plhs[4], d, "n_fit", scalar(cf[d].n_fit));
-            mxSetField(plhs[4], d, "flags", scalar(cf[d].flags)); mxSetField(plhs[4], d, "f", fa); mxSetField(plhs[4], d, "t", ta);
-            mxSetField(plhs[4], d, "row_flags", ra);
-        }
+        plhs[4] = carrier_struct(cf, fr, tr, rf, D, (size_t)B);
     }
     mxFree(cf); mxFree(fr); mxFree(rf); mxFree(res); mxFree(pi); if (own) mxFree((void *)tpl);
+}
+
+#elif defined(GSMCAL_MEX_gsm_calibrate_cell_batch)
+/* [sampling_ppm, carrier_ppm, n_pos_info, pos_info, carrier, cell] = gsm_calibrate_cell_batch(raw_uint8, carrier_freq, sch_training_sequence, coef)
+ * gsmcal_calibrate_cell_batch: gsm_calibrate_carrier_batch (outputs 1-5 as there), then SCH_demod of every SCH burst with the fitted
+ * carrier residual removed and the SCH decoding, so a short capture gives each dongle its cell and frame clock.  cell: 1 x D struct
+ * array with gsm_calibrate_sch_decode_batch's fields (flags also 16: no carrier fit, the rows were not corrected) and df (1 x n_sch: the
+ * residual removed from each SCH burst in Hz, NaN without a fit).  See include/gsmcal.h. */
+void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
+    init_once();
+    if (nrhs != 4 || nlhs > 6)
+        mexErrMsgIdAndTxt("gsmcal:nargin", "usage: [sampling_ppm,carrier_ppm,n_pos_info,pos_info,carrier,cell] = "
+                          "gsm_calibrate_cell_batch(raw_uint8,carrier_freq,sch_training_sequence,coef)");
+    if (!mxIsUint8(prhs[0])) mexErrMsgIdAndTxt("gsmcal:type", "raw must be uint8");
+    size_t rows = mxGetM(prhs[0]), D = mxGetN(prhs[0]);
+    int own; const double *tpl = get_c128(prhs[2], &own);
+    size_t nt; const double *coef = real_vector(prhs[3], &nt);
+    int64_t n_iq = (int64_t)(rows / 2);
+    size_t B = (size_t)gsmcal_max_bursts((n_iq + 63) / 64, 8), R = D * B;
+    gsmcal_stream_result *res = (gsmcal_stream_result *)mxMalloc(D * sizeof(*res));
+    double *pi = (double *)mxMalloc(D * 12 * B * sizeof(double));
+    gsmcal_carrier_fit_result *cf = (gsmcal_carrier_fit_result *)mxMalloc(D * sizeof(*cf));
+    gsmcal_sch_decode_result *sd = (gsmcal_sch_decode_result *)mxMalloc(D * sizeof(*sd));
+    double *fr = (double *)mxMalloc(R * 3 * sizeof(double)), *tr = fr + R, *df = tr + R;
+    int32_t *sfn = (int32_t *)mxMalloc(R * 2 * sizeof(int32_t)), *sbs = sfn + R;
+    uint8_t *rf = (uint8_t *)mxMalloc(R * 3), *sham = rf + R, *srf = sham + R;
+    fail_on(gsmcal_calibrate_cell_batch((const uint8_t *)mxGetData(prhs[0]), GSMCAL_MEM_HOST, n_iq, (int64_t)D, mxGetScalar(prhs[1]), tpl, coef, (int)nt,
+                                        8, 8, res, NULL, NULL, NULL, pi, NULL, cf, fr, tr, rf, sd, NULL, NULL, NULL, df, sfn, sbs, sham, srf),
+            "gsm_calibrate_cell_batch");
+    batch_outputs(nlhs, plhs, res, pi, D, B);
+    if (nlhs > 4) plhs[4] = carrier_struct(cf, fr, tr, rf, D, B);
+    if (nlhs > 5) plhs[5] = cell_struct(sd, sfn, sbs, sham, srf, df, D, B);
+    mxFree(cf); mxFree(sd); mxFree(fr); mxFree(sfn); mxFree(rf); mxFree(res); mxFree(pi); if (own) mxFree((void *)tpl);
 }
 
 #elif defined(GSMCAL_MEX_gsm_calibrate_demod_batch) || defined(GSMCAL_MEX_gsm_calibrate_sch_decode_batch)
@@ -471,24 +542,7 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
     }
 #if defined(GSMCAL_MEX_gsm_calibrate_sch_decode_batch)
     if (nlhs > 6) {
-        const char *f[] = {"bsic", "ncc", "bcc", "fn_first", "frame_clock_start", "n_crc_ok", "n_agree", "flags", "fn", "bsic_rows", "hamming", "row_flags"};
-        plhs[6] = mxCreateStructMatrix(1, D, 12, f);
-        for (size_t d = 0; d < D; ++d) {
-            const gsmcal_sch_decode_result *c = sd + d;
-            const size_t k = c->n_sch < 0 ? 0 : (size_t)c->n_sch;
-            mxArray *a[4];
-            for (int j = 0; j < 4; ++j) a[j] = mxCreateDoubleMatrix(1, k, mxREAL);
-            for (size_t i = 0; i < k; ++i) {
-                mxGetPr(a[0])[i] = sfn[d * B + i]; mxGetPr(a[1])[i] = sbs[d * B + i];
-                mxGetPr(a[2])[i] = sham[d * B + i]; mxGetPr(a[3])[i] = srf[d * B + i];
-            }
-            mxSetField(plhs[6], d, "bsic", scalar(c->bsic)); mxSetField(plhs[6], d, "ncc", scalar(c->bsic < 0 ? -1 : c->bsic >> 3));
-            mxSetField(plhs[6], d, "bcc", scalar(c->bsic < 0 ? -1 : c->bsic & 7)); mxSetField(plhs[6], d, "fn_first", scalar(c->fn_first));
-            mxSetField(plhs[6], d, "frame_clock_start", scalar(c->frame_clock_start)); mxSetField(plhs[6], d, "n_crc_ok", scalar(c->n_crc_ok));
-            mxSetField(plhs[6], d, "n_agree", scalar(c->n_agree)); mxSetField(plhs[6], d, "flags", scalar(c->flags));
-            mxSetField(plhs[6], d, "fn", a[0]); mxSetField(plhs[6], d, "bsic_rows", a[1]);
-            mxSetField(plhs[6], d, "hamming", a[2]); mxSetField(plhs[6], d, "row_flags", a[3]);
-        }
+        plhs[6] = cell_struct(sd, sfn, sbs, sham, srf, NULL, D, B);
     }
     mxFree(sd); mxFree(sfn); mxFree(sham);
 #else
