@@ -477,6 +477,97 @@ int gsmcal_calibrate_cell_batch(const uint8_t *raw, int raw_mem, int64_t n_iq, i
                                 double *corr_val, double *sch_df, int32_t *sch_fn, int32_t *sch_bsic, uint8_t *sch_hamming,
                                 uint8_t *sch_row_flags);
 
+/* gsmcal_calibrate_cell_batch (every output as there, byte for byte) followed by decoding every BCCH block of pos_info: the System
+ * Information the cell broadcasts, and from its SI3 the Cell Global Identity (MCC, MNC, LAC, Cell Identity).  A BSIC does not name a
+ * cell (neighbours reuse it); the CGI does, so dongles that report the same CGI are on the same cell.  Only oversampling_ratio 8 (osr).
+ * fs = 8 * 1625e3/6, F = 1250*osr = 10,000 samples per frame, N = 194*osr = 1552, r = r_correct (1-based).  For stream d:
+ *   TSC = bsic & 7 of its gsmcal_sch_decode_result (the BCC), t_n (n = 0..207) that column of normal_training_sequence ((26*osr) x 8
+ *   complex, column-major, as gsmcal_calibrate_demod_bcch_batch takes it).  A stream without a winning BSIC: GSMCAL_SI_NO_CELL and no
+ *   block is decoded.  GSMCAL_SI_NO_POS_INFO and _NO_R_CORRECT as in the SCH decoding (n_blocks = -1).
+ *   1. blocks: block b is the type-2 rows that directly follow a type-1 row in pos_info order (SCH_corr_rate_correction.m:138-181 puts
+ *      four, at p_sch + k*F, k = 1..4, behind every SCH row it flags); a type-1 row with none is no block, one with fewer than four
+ *      (the capture ended) is a block with GSMCAL_SI_BLK_SHORT, not decoded.  At most B blocks (B as above).  With p_b1 its first row and
+ *      p_first the record's first SCH row: FN_b = (fn_first + (p_b1 - p_first)/F) mod 2,715,648 (exact integers); FN_b mod 51 != 2:
+ *      GSMCAL_SI_BLK_FN, not decoded.  TC = (FN_b div 51) mod 8 (TS 45.002 6.3.1.3: which SI type the block carries).
+ *   2. every row at p of every block, GSMCAL_SI_BLK_FN and _SHORT blocks included:
+ *      df = the carrier fit's line at t = (((p + 74*osr - 1)(1 + e2))(1 + e1))/fs, gsmcal_calibrate_cell_batch's steps 1-2 (bit 74 is also
+ *      the centre of the normal burst's training sequence); a stream without a fit: df = 0 and GSMCAL_SI_UNCORRECTED.
+ *      g = p + 61*osr (BCCH_demod.m:85's training start), s0 = g - 64 - 69*osr, y(j) = r(s0 + j) * exp(-i*2*pi*df*j/fs), j = 0..N+158
+ *      (1711 samples).  A range that leaves r (or a non-integer p): GSMCAL_SI_ROW_RANGE.
+ *      c(l) = sum_n conj(t_n) * y(l + 64 + 69*osr + n) for l = -64..+95 (l = 0: the training where pos_info puts it; the lags past +64
+ *      recover streams whose pos_info locked early).  l* = the first maximum of re^2 + im^2; l* = -64 or +95: GSMCAL_SI_ROW_EDGE.
+ *      h = c(l*) / sum_n |t_n|^2 (the one-tap channel), w = conj(h) / (re(h)^2 + im(h)^2), x(n) = y(l* + 64 + n) * w, n = 0..N-1.
+ *      m = the 32-state GMSK MLSE of SCH_demod.m:92-95 on x (traceback 30, gsmcal_calibrate_demod_batch's arithmetic), symbols 38..185.
+ *      burst bits: b(61 + j) = TSC bit j (j = 0..25), b_i = b_(i+1) xor (1 - m_(i+1)) for i = 60..0, b_i = b_(i-1) xor (1 - m_i) for
+ *      i = 87..147.  i(0..56) = b(3..59), i(57..113) = b(88..144); the stealing bits b(60), b(87) are reported (TS 45.003 4.1.5).
+ *      The frequency-domain equaliser of SCH_demod with the 26-symbol training as its template is NOT used: 208 of 1552 samples give a
+ *      channel estimate too noisy for it (23 % bit errors on the synthetic captures).
+ *   3. block decode (TS 45.003 4.1), only when no row has a flag: c(k) = i_(k mod 4)(2*((49k) mod 57) + ((k mod 8) div 4)), k = 0..455;
+ *      the hard-decision Viterbi of the SCH decoding (same code, states, tie rule) over 228 steps from and back to state 0, u(224..227) = 0
+ *      the tail; hamming = the final metric.  Fire code: d(0)D^223 + ... + d(183)D^40 + p(0)D^39 + ... + p(39), u(0..183) = d,
+ *      u(184..223) = p, divided by D^40 + D^26 + D^23 + D^17 + D^3 + 1 must leave 1 + D + ... + D^39, else GSMCAL_SI_BLK_FIRE
+ *      (detection only, no error trapping).  A block with a row flag: GSMCAL_SI_BLK_ROW, not decoded.
+ *   4. payload: 23 octets, d(8m + q) = bit q (LSB = 0) of octet m: OsmocomBB's LSB-first packing, like the SCH's field order unverified
+ *      against a live cell.  Octet 0 is the L2 pseudo length; the message type is octet 2 when octet 1 is 0x06 (RR).  SI3 (0x1B, TS 44.018
+ *      9.1.35): Cell Identity = octets 3-4 big-endian; the LAI is octets 5-9: MCC digits 1, 2 = low, high nibble of octet 5, MCC digit 3 =
+ *      low nibble of octet 6, MNC digit 3 = its high nibble (0xF: a 2-digit MNC), MNC digits 1, 2 = low, high nibble of octet 7, LAC =
+ *      octets 8-9 big-endian.  MCC = 100*d1 + 10*d2 + d3, MNC = 10*d1 + d2 or 100*d1 + 10*d2 + d3 (nibbles as they are, not checked).
+ *   5. per stream: si_mask = one GSMCAL_SI_HAS_* bit per message type seen in a block that passed the Fire check; a vote over those SI3
+ *      blocks on their octets 3-9: most votes wins, equal votes the earliest block; n_si3_agree = its votes, GSMCAL_SI_SI3_DISAGREE when
+ *      another SI3 block voted otherwise, GSMCAL_SI_NO_SI3 (fields -1) when there is none.
+ * Per-row arrays [n_streams][B][4] (row k of block b), each may be NULL (not copied back): bcch_lag int8 (l*; -128 where not
+ * correlated), bcch_row_flags uint8 (GSMCAL_SI_ROW_*), bcch_steal uint8 (bit 0 = b(60), bit 1 = b(87)).  Per-block arrays [n_streams][B]:
+ * blk_fn int32 (FN_b; -1 without a cell), blk_tc uint8 (TC; 255 without a cell), blk_flags uint8 (GSMCAL_SI_BLK_*), blk_hamming uint16,
+ * blk_payload [..][23] (the decoded octets, Fire check passed or not; zeros where not decoded).  Entries beyond the record's n_blocks are unspecified. */
+typedef struct gsmcal_sysinfo_result {
+    int32_t n_blocks;          /* BCCH blocks; -1: not run (flags say why) */
+    int32_t n_fire_ok;         /* blocks that passed the Fire check */
+    int32_t n_si3;             /* of those, SI3 messages */
+    int32_t n_si3_agree;       /* SI3 blocks that voted for the reported CGI */
+    int32_t flags;             /* GSMCAL_SI_* */
+    int32_t si_mask;           /* GSMCAL_SI_HAS_* */
+    int32_t mcc, mnc, mnc_digits, lac, ci;   /* from the winning SI3, or -1 */
+    int32_t reserved;
+} gsmcal_sysinfo_result;       /* 48 bytes */
+
+#define GSMCAL_SI_NO_POS_INFO    1   /* as GSMCAL_SCHDEC_NO_POS_INFO */
+#define GSMCAL_SI_NO_R_CORRECT   2   /* as GSMCAL_SCHDEC_NO_R_CORRECT */
+#define GSMCAL_SI_NO_CELL        4   /* no winning BSIC: no TSC and no frame number, nothing decoded */
+#define GSMCAL_SI_UNCORRECTED    8   /* no carrier fit: df = 0 */
+#define GSMCAL_SI_NO_SI3        16   /* no SI3 block passed the Fire check: the CGI fields are -1 */
+#define GSMCAL_SI_SI3_DISAGREE  32   /* some SI3 block voted for another CGI */
+#define GSMCAL_SI_ROW_RANGE      1   /* row flags: the 1711-sample window leaves r_correct */
+#define GSMCAL_SI_ROW_EDGE       2   /* l* on -64 or +95 */
+#define GSMCAL_SI_BLK_FN         1   /* block flags: FN_b mod 51 != 2 */
+#define GSMCAL_SI_BLK_ROW        2   /* a row of the block has a flag */
+#define GSMCAL_SI_BLK_FIRE       4   /* Fire check failed */
+#define GSMCAL_SI_BLK_SHORT      8   /* fewer than four BCCH rows: the capture ended */
+#define GSMCAL_SI_HAS_SI1        1   /* si_mask bits: message type 0x19 */
+#define GSMCAL_SI_HAS_SI2        2   /* 0x1A */
+#define GSMCAL_SI_HAS_SI2BIS     4   /* 0x02 */
+#define GSMCAL_SI_HAS_SI2TER     8   /* 0x03 */
+#define GSMCAL_SI_HAS_SI2QUATER 16   /* 0x07 */
+#define GSMCAL_SI_HAS_SI3       32   /* 0x1B */
+#define GSMCAL_SI_HAS_SI4       64   /* 0x1C */
+#define GSMCAL_SI_HAS_SI13     128   /* 0x00 */
+#define GSMCAL_SI_HAS_OTHER    256   /* any other type, or octet 1 != 0x06 */
+
+int gsmcal_calibrate_sysinfo_batch(const uint8_t *raw, int raw_mem, int64_t n_iq, int64_t n_streams,
+                                   double carrier_freq, const double *sch_training_sequence,
+                                   const double *coef, int n_taps, int oversampling_ratio, int coarse_decimation,
+                                   gsmcal_stream_result *results,
+                                   double *coarse_pos, double *coarse_snr, double *fcch_pos, double *pos_info,
+                                   void *cuda_stream,
+                                   gsmcal_carrier_fit_result *carrier /* [n_streams], required */,
+                                   double *fcch_f, double *fcch_t, uint8_t *fcch_row_flags,
+                                   gsmcal_sch_decode_result *dec /* [n_streams], required */, uint8_t *sch_ok, uint8_t *demod_bits,
+                                   double *corr_val, double *sch_df, int32_t *sch_fn, int32_t *sch_bsic, uint8_t *sch_hamming,
+                                   uint8_t *sch_row_flags,
+                                   const double *normal_training_sequence /* required */,
+                                   gsmcal_sysinfo_result *sysinfo /* [n_streams], required */,
+                                   int8_t *bcch_lag, uint8_t *bcch_row_flags, uint8_t *bcch_steal,
+                                   int32_t *blk_fn, uint8_t *blk_tc, uint8_t *blk_flags, uint16_t *blk_hamming, uint8_t *blk_payload);
+
 /* The same pipeline with several batches in flight (continuous captures): _submit enqueues batch `slot` (0..3) on the library's
  * own streams once the caller's `cuda_stream` has produced the DEVICE-resident capture, and returns; _collect waits for that batch
  * and fills the result pointers given to _submit (they must stay valid until then).  Batches are staggered on the device: the
@@ -501,7 +592,8 @@ int gsmcal_calibrate_batch_cancel(int slot);
  * [6] (gsmcal_calibrate_demod_batch / _demod_bcch_batch / _sch_decode_batch only) SCH_demod (+ SCH decoding) + FCCH_demod (+ BCCH_demod);
  *     (gsmcal_calibrate_sch_timing_batch only) SCH row list, sub-sample SCH timing and the clock fit;
  *     (gsmcal_calibrate_carrier_fit_batch only) FCCH row list, the tone of every FCCH burst and the carrier fit;
- *     (gsmcal_calibrate_cell_batch only) the row lists, the carrier fit, SCH_demod less the residual and SCH decoding.  Returns the number
+ *     (gsmcal_calibrate_cell_batch only) the row lists, the carrier fit, SCH_demod less the residual and SCH decoding;
+ *     (gsmcal_calibrate_sysinfo_batch only) those, then the BCCH block list, every BCCH burst and the block decoding.  Returns the number
  *     of stages written. */
 int gsmcal_last_batch_stage_ms(double *ms, int cap);
 

@@ -213,6 +213,7 @@ int get_ctx(Ctx **out) {
         CU(cudaFuncSetAttribute(sch_demod_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 120 * 1024));       //  the device's Ctx)
         CU(cudaFuncSetAttribute(sch_demod_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
         CU(cudaFuncSetAttribute(sch_demod_resid_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
+        CU(cudaFuncSetAttribute(bcch_burst_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BB_SMEM));
         CU(cudaFuncSetAttribute(fcch_demod_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
         c.attrs = true;
     }
@@ -569,9 +570,9 @@ void gmsk_branch_table(int osr, double *W);
 void sch_training_pm(signed char *data_pm);
 
 // ---- the stage behind post-SCH ("tail") of gsmcal_calibrate_demod_batch, _demod_bcch_batch, _sch_decode_batch, _sch_timing_batch,
-// _carrier_fit_batch and _cell_batch --
+// _carrier_fit_batch, _cell_batch and _sysinfo_batch --
 // It is the SCH timing block when `timing` is set, the carrier fit block when `carrier` is set (with `sdec`: then the residual-corrected
-// SCH_demod and the SCH decoding block), else the demod block (batched SCH_demod / FCCH_demod) with the BCCH block when `nts` is set and
+// SCH_demod and the SCH decoding block, and with `si` as well the BCCH decoding block), else the demod block (batched SCH_demod / FCCH_demod) with the BCCH block when `nts` is set and
 // the SCH decoding block when `sdec` is set.
 struct TailOut {                     // the caller's host outputs; an array left NULL is not read back
     gsmcal_demod_result *demod; uint8_t *sch_ok, *bits, *dec; double *corr, *freq, *snr, *idx;
@@ -580,6 +581,7 @@ struct TailOut {                     // the caller's host outputs; an array left
     gsmcal_sch_timing_result *timing; double *tau, *x;
     gsmcal_carrier_fit_result *carrier; double *cf_f, *cf_t; uint8_t *cf_flag;
     double *sch_df;
+    gsmcal_sysinfo_result *si; int8_t *lag; uint8_t *bflag, *steal; int32_t *bfn; uint8_t *btc, *bblk; uint16_t *bham; uint8_t *pay;
 };
 struct TailDev {                     // device buffers of the same blocks
     DemodResultDev *rec; double *sch_pos, *fcch_pos; unsigned char *sch_ok, *fcch_ok;                       // the row lists
@@ -589,6 +591,8 @@ struct TailDev {                     // device buffers of the same blocks
     TimingResultDev *timing; double *tau, *x; unsigned char *row_flag;
     CarrierFitDev *carrier; double *cf_f, *cf_t; unsigned char *cf_flag;
     double *sch_df;
+    SysinfoDev *si; int *blk_n; double *blk_pos; unsigned char *blk_nrow; signed char *lag; unsigned char *bflag, *steal;
+    unsigned long long *ibits, *skey; int *bfn; unsigned char *btc, *bblk; unsigned short *bham; unsigned char *pay;
 };
 // every per-stream array ([D] records, [D][cap] rows) of the blocks `o` asks for: f(device pointer, bytes per stream, the caller's host
 // array or NULL).  Set-up, the slice of a stream group and the read-back all walk this one list.  The per-call constants (Ft, Wtab, dpm,
@@ -607,6 +611,12 @@ template <class F> void tail_arrays(TailDev &t, const TailOut &o, int cap, F &&f
             f(t.bits, 148 * r, o.bits); f(t.dec, 148 * r, nullptr); f(t.corr, 8 * 85 * r, o.corr); f(t.sch_df, 8 * r, o.sch_df);
             f(t.sdec, sizeof(SchDecodeResultDev), o.sdec); f(t.key, 4 * r, nullptr); f(t.fn, 4 * r, o.fn); f(t.bsic, 4 * r, o.bsic);
             f(t.ham, r, o.ham); f(t.rflag, r, o.rflag);
+        }
+        if (o.si) {                  // the block list, the BCCH rows ([cap][4] per stream) and the blocks
+            f(t.si, sizeof(SysinfoDev), o.si); f(t.blk_n, 4, nullptr); f(t.blk_pos, 8 * 4 * r, nullptr); f(t.blk_nrow, r, nullptr);
+            f(t.lag, 4 * r, o.lag); f(t.bflag, 4 * r, o.bflag); f(t.steal, 4 * r, o.steal); f(t.ibits, 8 * 8 * r, nullptr);
+            f(t.skey, 8 * r, nullptr); f(t.bfn, 4 * r, o.bfn); f(t.btc, r, o.btc); f(t.bblk, r, o.bblk); f(t.bham, 2 * r, o.bham);
+            f(t.pay, 23 * r, o.pay);
         }
         return;
     }
@@ -649,7 +659,8 @@ int tail_setup(Ctx &c, i64 D, int cap, int osr, const double2 *tpl_dev, const Ta
     return GSMCAL_OK;
 }
 // one stream group: row lists + sentinels, then either the timing of every SCH row and the per-stream fit (osr 8), or the tone of every
-// FCCH row and the per-stream carrier fit (osr 8) with, for _cell_batch, the SCH bursts less the fitted residual and their decoding, or
+// FCCH row and the per-stream carrier fit (osr 8) with, for _cell_batch, the SCH bursts less the fitted residual and their decoding (and
+// for _sysinfo_batch the BCCH blocks behind them), or
 // SCH bursts, SCH decoding and BCCH_demod when their outputs were asked for, FCCH
 // bursts, FCCH means
 int run_tail(Ctx &c, WinSrc src, const Work &ws, const TailDev &t, int osr, double carrier_freq, i64 nd, int cap, cudaStream_t st) {
@@ -670,6 +681,12 @@ int run_tail(Ctx &c, WinSrc src, const Work &ws, const TailDev &t, int osr, doub
                cap, tw_s, t.Ft, t.Wtab, t.dpm, t.carrier, t.bits, t.dec, t.corr, t.sch_df);
         LAUNCH(sch_decode_batch_kernel, (unsigned)nd, 32, 0, st, t.rec, t.sch_pos, t.sch_ok, t.bits, t.corr, cap, osr, t.key, t.fn, t.bsic,
                t.ham, t.rflag, t.sdec);
+        if (!t.si) return GSMCAL_OK;
+        LAUNCH(bcch_block_kernel, (unsigned)((nd + 127) / 128), 128, 0, st, ws.ctl, ws.pos_info, t.rec, (int)nd, cap, t.blk_n, t.blk_pos, t.blk_nrow);
+        LAUNCH(bcch_burst_kernel, dim3(4 * (unsigned)cap, (unsigned)nd), BB_THREADS, BB_SMEM, st, src, ws.ctl, t.blk_n, t.blk_pos, t.blk_nrow, t.sdec,
+               t.carrier, t.nts, t.Wtab, cap, t.lag, t.bflag, t.steal, t.ibits);
+        LAUNCH(bcch_decode_kernel, (unsigned)nd, 32, 0, st, t.rec, t.sdec, t.carrier, t.sch_pos, t.blk_n, t.blk_pos, t.blk_nrow, t.bflag, t.ibits, cap,
+               t.skey, t.bfn, t.btc, t.bblk, t.bham, t.pay, t.si);
         return GSMCAL_OK;
     }
     const double2 *tw_s, *tw_f;                  // both built by the set-up: no launch here
@@ -1429,6 +1446,30 @@ int gsmcal_calibrate_cell_batch(const uint8_t *raw, int raw_mem, int64_t n_iq, i
     TRY(calibrate_batch_impl(raw, raw_mem, n_iq, D, carrier_freq, tpl, coef, n_taps, osr, coarse_dr, results, coarse_pos, coarse_snr, fcch_pos, pos_info,
                              cuda_stream, nullptr, GSMCAL_MEM_DEVICE, 0, &o));
     for (int64_t d = 0; d < D; ++d)                              // SCH_demod ran on r_correct as it is: the rows of _demod_batch
+        if (dec[d].n_sch >= 0 && (carrier[d].flags & GSMCAL_CARRIER_FEW)) dec[d].flags |= GSMCAL_SCHDEC_UNCORRECTED;
+    return GSMCAL_OK;
+}
+
+int gsmcal_calibrate_sysinfo_batch(const uint8_t *raw, int raw_mem, int64_t n_iq, int64_t D, double carrier_freq, const double *tpl,
+                                   const double *coef, int n_taps, int osr, int coarse_dr, gsmcal_stream_result *results,
+                                   double *coarse_pos, double *coarse_snr, double *fcch_pos, double *pos_info, void *cuda_stream,
+                                   gsmcal_carrier_fit_result *carrier, double *fcch_f, double *fcch_t, uint8_t *fcch_row_flags,
+                                   gsmcal_sch_decode_result *dec, uint8_t *sch_ok, uint8_t *demod_bits, double *corr_val,
+                                   double *sch_df, int32_t *sch_fn, int32_t *sch_bsic, uint8_t *sch_hamming, uint8_t *sch_row_flags,
+                                   const double *nts, gsmcal_sysinfo_result *sysinfo, int8_t *bcch_lag, uint8_t *bcch_row_flags,
+                                   uint8_t *bcch_steal, int32_t *blk_fn, uint8_t *blk_tc, uint8_t *blk_flags, uint16_t *blk_hamming,
+                                   uint8_t *blk_payload) {
+    if (!carrier || !dec || !nts || !sysinfo) return fail(GSMCAL_ERR_ARG, "calibrate_sysinfo_batch: null carrier, dec, normal_training_sequence or sysinfo");
+    if (osr != 8) return fail(GSMCAL_ERR_ARG, "calibrate_sysinfo_batch: oversampling_ratio must be 8");
+    TailOut o{};
+    o.carrier = carrier; o.cf_f = fcch_f; o.cf_t = fcch_t; o.cf_flag = fcch_row_flags;
+    o.sdec = dec; o.sch_ok = sch_ok; o.bits = demod_bits; o.corr = corr_val; o.sch_df = sch_df;
+    o.fn = sch_fn; o.bsic = sch_bsic; o.ham = sch_hamming; o.rflag = sch_row_flags;
+    o.nts = nts; o.si = sysinfo; o.lag = bcch_lag; o.bflag = bcch_row_flags; o.steal = bcch_steal;
+    o.bfn = blk_fn; o.btc = blk_tc; o.bblk = blk_flags; o.bham = blk_hamming; o.pay = blk_payload;
+    TRY(calibrate_batch_impl(raw, raw_mem, n_iq, D, carrier_freq, tpl, coef, n_taps, osr, coarse_dr, results, coarse_pos, coarse_snr, fcch_pos, pos_info,
+                             cuda_stream, nullptr, GSMCAL_MEM_DEVICE, 0, &o));
+    for (int64_t d = 0; d < D; ++d)                              // as gsmcal_calibrate_cell_batch
         if (dec[d].n_sch >= 0 && (carrier[d].flags & GSMCAL_CARRIER_FEW)) dec[d].flags |= GSMCAL_SCHDEC_UNCORRECTED;
     return GSMCAL_OK;
 }

@@ -1103,3 +1103,328 @@ __global__ void __launch_bounds__(SDB_THREADS, 2) sch_demod_resid_kernel(WinSrc 
     const double resid = isnan(df) ? 0.0 : __ddiv_rn(__dmul_rn(2.0 * GSMCAL_PI, df), ((1625.0 / 6.0) * 1e3) * 8.0);      // rad per sample
     sch_demod_body<true>(src, ctl, rec, sch_pos, sch_ok, cap, 8, tw, Ft, Wtab, data_pm, demod_bits, dec_bits, corr_val, resid);
 }
+
+// ===================================================================================================
+// BCCH decoding of gsmcal_calibrate_sysinfo_batch (definition: include/gsmcal.h), behind sch_decode_batch_kernel on what the cell
+// call wrote: the block list, every BCCH burst (one-tap equaliser on the normal training sequence of the cell's BCC, MLSE) and the
+// block decoding (deinterleaver, Viterbi, Fire code, payload), the per-stream SI mask and the SI3 vote.  osr 8 only.
+// ===================================================================================================
+struct SysinfoDev {                  // mirrors gsmcal_sysinfo_result (include/gsmcal.h)
+    int n_blocks, n_fire_ok, n_si3, n_si3_agree, flags, si_mask, mcc, mnc, mnc_digits, lac, ci, reserved;
+};
+#define SI_NO_POS_INFO   1
+#define SI_NO_R_CORRECT  2
+#define SI_NO_CELL       4
+#define SI_UNCORRECTED   8
+#define SI_NO_SI3       16
+#define SI_SI3_DISAGREE 32
+#define SI_ROW_RANGE     1
+#define SI_ROW_EDGE      2
+#define SI_BLK_FN        1
+#define SI_BLK_ROW       2
+#define SI_BLK_FIRE      4
+#define SI_BLK_SHORT     8
+#define SI_NO_LAG     (-128)
+#define BB_N      1552                 // 194*osr: the equaliser window of SCH_demod
+#define BB_L      208                  // 26*osr template samples
+#define BB_LAG0   64                   // lags -64..+95
+#define BB_NLAG   160
+#define BB_NY     (BB_N + BB_NLAG - 1) // 1711 samples of y
+#define BB_TR     552                  // 69*osr: the training start in x
+#define BB_THREADS 384                 // the loader's unrolled FIR path covers ceil(1714 / 5) level-0 groups
+#define BB_S ((GSMCAL_XCAP(BB_NY) + BB_NY + 8) > (BB_N + SD_NSYM * 16) ? (GSMCAL_XCAP(BB_NY) + BB_NY + 8) : (BB_N + SD_NSYM * 16))
+#define BB_SMEM ((size_t)(BB_NY + 1 + BB_S) * sizeof(double2))      // y | the loader's X, Y, later x | branch correlations
+#define SI_FIRE_G 0x10004820009ull       // D^40 + D^26 + D^23 + D^17 + D^3 + 1
+__constant__ unsigned c_nts_bits[8] = {0x970897u, 0xb778b7u, 0x10ee90eu, 0x11ed11eu, 0x6b906bu, 0x13ac13au, 0x29f629fu, 0x3bc4bbcu};  // bit j at 25 - j
+
+// One thread per stream: the blocks of pos_info (type-2 rows directly behind a type-1 row, pos_info order), at most cap; blk_n = -1 when
+// the cell call's SCH stage did not run.
+__global__ void bcch_block_kernel(const StreamCtl *__restrict__ ctl, const double *__restrict__ pos_info, const DemodResultDev *__restrict__ rec,
+                                  int n_streams, int cap, int *__restrict__ blk_n, double *__restrict__ blk_pos, unsigned char *__restrict__ blk_nrow) {
+    const int stream = blockIdx.x * blockDim.x + threadIdx.x;
+    if (stream >= n_streams) return;
+    if (rec[stream].n_sch < 0) { blk_n[stream] = -1; return; }
+    const double *pi = pos_info + (i64)stream * 6 * cap * 2;
+    const int rows = ctl[stream].n_pos_info;
+    const i64 base = (i64)stream * cap;
+    int n = 0, k = -1;                                             // k: rows of the open block, -1 = none open
+    bool after_sch = false;
+    for (int i = 0; i < rows; ++i) {
+        const double t = pi[2 * i + 1];
+        if (t == 2.0 && after_sch) {
+            if (k < 0) { if (n >= cap) break; k = 0; ++n; }
+            if (k < 4) { blk_pos[(base + n - 1) * 4 + k] = pi[2 * i]; ++k; blk_nrow[base + n - 1] = (unsigned char)k; }
+            continue;
+        }
+        after_sch = (t == 1.0);
+        k = -1;
+    }
+    blk_n[stream] = n;
+}
+
+// One block per (BCCH row, stream), row 4b + k = row k of block b: the 1711-sample window through the level-3 loader with
+// dphi2 - 2*pi*df/fs folded into the derotation step (as sch_demod_resid_kernel), the 160-lag x 208-tap training correlation in fp64,
+// the one-tap division, gmsk_viterbi_warp, and the 114 coded bits (two 57-bit words) and stealing bits of the burst.
+__global__ void __launch_bounds__(BB_THREADS, 2) bcch_burst_kernel(WinSrc src, const StreamCtl *__restrict__ ctl, const int *__restrict__ blk_n,
+                                                                   const double *__restrict__ blk_pos, const unsigned char *__restrict__ blk_nrow,
+                                                                   const SchDecodeResultDev *__restrict__ sdec, const CarrierFitDev *__restrict__ carrier,
+                                                                   const double2 *__restrict__ nts, const double2 *__restrict__ Wtab, int cap,
+                                                                   signed char *__restrict__ lag_out, unsigned char *__restrict__ rflag_out,
+                                                                   unsigned char *__restrict__ steal_out, unsigned long long *__restrict__ ibits) {
+    extern __shared__ double2 sm[];
+    __shared__ double2 tpl[BB_L], cr[BB_NLAG], wsh, ph0;
+    __shared__ double pw[BB_NLAG], energy;
+    __shared__ int lstar;
+    __shared__ unsigned char bits[SD_NSYM + 2];
+    const int j = blockIdx.x, stream = blockIdx.y, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int b = j >> 2, k = j & 3;
+    if (b >= blk_n[stream]) return;
+    const i64 o = (i64)stream * cap * 4 + j;
+    const int bsic = sdec[stream].bsic;
+    const double p = blk_pos[o];
+    const StreamCtl c = ctl[stream];
+    const double s0 = p - 128.0;                                   // g - 64 - 69*osr, g = p + 61*osr
+    const bool run = bsic >= 0 && k < blk_nrow[(i64)stream * cap + b];
+    const bool in_range = p == floor(p) && s0 >= 1.0 && s0 + (double)(BB_NY - 1) <= (double)c.len3;
+    if (!run || !in_range) {
+        if (tid == 0) {
+            lag_out[o] = SI_NO_LAG; rflag_out[o] = run ? SI_ROW_RANGE : 0; steal_out[o] = 0;
+            ibits[2 * o] = 0ull; ibits[2 * o + 1] = 0ull;
+        }
+        return;
+    }
+    double2 *y = sm, *S = y + BB_NY + 1, *x = S, *cb = S + BB_N;
+    const i64 j0 = (i64)s0 - 1;
+    const double df = sch_resid_hz(carrier[stream], c, p);
+    const double resid = isnan(df) ? 0.0 : __ddiv_rn(__dmul_rn(2.0 * GSMCAL_PI, df), ((1625.0 / 6.0) * 1e3) * 8.0);     // rad per sample
+    const double2 *t_col = nts + (i64)(bsic & 7) * BB_L;
+    for (int n = tid; n < BB_L; n += BB_THREADS) tpl[n] = t_col[n];
+    if (tid == 0) { double sn, cs; sincos((double)j0 * c.dphi2, &sn, &cs); ph0 = make_double2(cs, sn); }
+    load_window(src, c, stream, j0, BB_NY, y, S, S + GSMCAL_XCAP(BB_NY));  // ends with a barrier
+    derotate_post(y, BB_NY, c.dphi2 - resid, ph0);
+    __syncthreads();
+    if (tid == 0) {                                                // sum |t_n|^2 in n order
+        double e = 0.0;
+        for (int n = 0; n < BB_L; ++n) e += tpl[n].x * tpl[n].x + tpl[n].y * tpl[n].y;
+        energy = e;
+    }
+    for (int li = warp; li < BB_NLAG; li += BB_THREADS / 32) {     // c(l), l = li - 64, over y(li + 552 + n)
+        double ar = 0.0, ai = 0.0;
+        for (int n = lane; n < BB_L; n += 32) {
+            const double2 t = tpl[n], v = y[li + BB_TR + n];
+            ar += t.x * v.x + t.y * v.y;                           // conj(t) * v
+            ai += t.x * v.y - t.y * v.x;
+        }
+        ar = warp_sum(ar); ai = warp_sum(ai);
+        if (lane == 0) { cr[li] = make_double2(ar, ai); pw[li] = ar * ar + ai * ai; }
+    }
+    __syncthreads();
+    if (warp == 0) {                                               // first maximum
+        double bv = -1.0; int bi = BB_NLAG;
+        for (int li = lane; li < BB_NLAG; li += 32) if (pw[li] > bv) { bv = pw[li]; bi = li; }
+        for (int s = 16; s > 0; s >>= 1) {
+            const double v2 = __shfl_xor_sync(0xffffffffu, bv, s);
+            const int i2 = __shfl_xor_sync(0xffffffffu, bi, s);
+            if (v2 > bv || (v2 == bv && i2 < bi)) { bv = v2; bi = i2; }
+        }
+        if (lane == 0) {
+            lstar = bi;
+            const double2 h = make_double2(cr[bi].x / energy, cr[bi].y / energy);
+            const double q = h.x * h.x + h.y * h.y;
+            wsh = make_double2(h.x / q, -h.y / q);                 // 1/h = conj(h) / |h|^2
+        }
+    }
+    __syncthreads();
+    const int ls = lstar;
+    const double2 w = wsh;
+    for (int n = tid; n < BB_N; n += BB_THREADS) x[n] = cmul(y[ls + n], w);     // x(n) = y(l* + 64 + n) / h
+    __syncthreads();
+    for (int i = tid; i < SD_NSYM * 16; i += BB_THREADS) {         // sch_bits_body's branch correlations
+        const int m = i >> 4, combo = i & 15;
+        double ar = 0.0, ai = 0.0;
+        for (int q = 0; q < 8; ++q) {
+            const double2 v = x[m * 8 + q], wt = Wtab[combo * 8 + q];
+            ar += v.x * wt.x + v.y * wt.y;                         // v * conj(w)
+            ai += v.y * wt.x - v.x * wt.y;
+        }
+        cb[i] = make_double2(ar, ai);
+    }
+    __syncthreads();
+    if (tid < 32) gmsk_viterbi_warp(cb, SD_NSYM, bits);
+    __syncthreads();
+    if (tid == 0) {
+        const unsigned char *m = bits + SD_TB + SD_EX;             // burst symbols 0..147
+        const unsigned tsc = c_nts_bits[bsic & 7];
+        unsigned long long w0 = 0ull, w1 = 0ull;
+        int bb = (int)(tsc >> 25) & 1;                             // b(61) = TSC bit 0, then backwards
+        int steal = 0;
+        for (int i = 60; i >= 0; --i) {
+            bb ^= 1 - m[i + 1];
+            if (i == 60) steal |= bb;
+            else if (i >= 3) w0 |= (unsigned long long)bb << (i - 3);      // i(0..56) = b(3..59)
+        }
+        bb = (int)tsc & 1;                                         // b(86) = TSC bit 25, then forwards
+        for (int i = 87; i <= 147; ++i) {
+            bb ^= 1 - m[i];
+            if (i == 87) steal |= bb << 1;
+            else if (i <= 144) w1 |= (unsigned long long)bb << (i - 88);   // i(57..113) = b(88..144)
+        }
+        const int l = ls - BB_LAG0;
+        lag_out[o] = (signed char)l;
+        rflag_out[o] = (l == -BB_LAG0 || l == BB_NLAG - 1 - BB_LAG0) ? SI_ROW_EDGE : 0;
+        steal_out[o] = (unsigned char)steal;
+        ibits[2 * o] = w0; ibits[2 * o + 1] = w1;
+    }
+}
+
+// One warp per stream, one lane per block (b = lane, lane + 32, ...): FN and TC, the deinterleaver, the 16-state hard-decision Viterbi
+// over 228 steps with one 16-bit decision word per step in shared memory, the Fire check on 64-bit shift registers during the traceback,
+// the payload; then the warp's SI mask and SI3 vote (keys: octets 3..9 of the SI3 blocks, ~0 for blocks that do not vote).
+#define BD_STEPS 228
+__global__ void __launch_bounds__(32) bcch_decode_kernel(const DemodResultDev *__restrict__ rec, const SchDecodeResultDev *__restrict__ sdec,
+                                                         const CarrierFitDev *__restrict__ carrier, const double *__restrict__ sch_pos,
+                                                         const int *__restrict__ blk_n, const double *__restrict__ blk_pos,
+                                                         const unsigned char *__restrict__ blk_nrow, const unsigned char *__restrict__ rflag,
+                                                         const unsigned long long *__restrict__ ibits, int cap, unsigned long long *__restrict__ key,
+                                                         int *__restrict__ fn_out, unsigned char *__restrict__ tc_out, unsigned char *__restrict__ flag_out,
+                                                         unsigned short *__restrict__ ham_out, unsigned char *__restrict__ payload,
+                                                         SysinfoDev *__restrict__ out) {
+    __shared__ unsigned short dec[32][BD_STEPS];
+    __shared__ unsigned long long ib[32][8];
+    const int stream = blockIdx.x, lane = threadIdx.x;
+    const i64 base = (i64)stream * cap;
+    const int n = blk_n[stream];
+    const SchDecodeResultDev sd = sdec[stream];
+    const bool cell = sd.bsic >= 0;
+    const double p_first = (rec[stream].n_sch > 0) ? sch_pos[base] : 0.0;
+    int n_fire = 0, n_si3 = 0, mask = 0;
+    for (int b = lane; b < n; b += 32) {
+        const i64 ob = base + b;
+        int fn = -1, tc = 255, fl = 0, ham = 0;
+        unsigned long long kv = ~0ull;
+        unsigned char pay[23];
+        for (int m = 0; m < 23; ++m) pay[m] = 0;
+        if (cell) {
+            const i64 f = (i64)(blk_pos[ob * 4] - p_first) / 10000;
+            fn = (int)(((i64)sd.fn_first + f) % SC_FN_MOD);
+            tc = (fn / 51) % 8;
+            const int nr = blk_nrow[ob];
+            if (nr < 4) fl |= SI_BLK_SHORT;
+            if (fn % 51 != 2) fl |= SI_BLK_FN;
+            for (int r = 0; r < nr; ++r) if (rflag[ob * 4 + r]) fl |= SI_BLK_ROW;
+        }
+        if (cell && !fl) {
+            for (int q = 0; q < 8; ++q) ib[lane][q] = ibits[ob * 8 + q];     // row r's words at 2r, 2r + 1
+            int metric[16];
+#pragma unroll
+            for (int s = 0; s < 16; ++s) metric[s] = (s == 0) ? 0 : 1 << 20;
+            for (int t = 0; t < BD_STEPS; ++t) {
+                int cc[2];
+#pragma unroll
+                for (int h = 0; h < 2; ++h) {                      // c(k) = i_(k mod 4)(2*((49k) mod 57) + ((k mod 8) div 4))
+                    const int kk = 2 * t + h, jj = 2 * ((49 * kk) % 57) + ((kk & 7) >> 2);
+                    const unsigned long long wd = ib[lane][2 * (kk & 3) + (jj >= 57)];
+                    cc[h] = (int)(wd >> (jj >= 57 ? jj - 57 : jj)) & 1;
+                }
+                int nm[16];
+                unsigned dw = 0u;
+#pragma unroll
+                for (int s = 0; s < 16; ++s) {                     // sch_decode_row's step
+                    const int u = s & 1, p0 = s >> 1, p1 = p0 | 8;
+                    const int a0 = u ^ ((p0 >> 2) & 1), a1 = u ^ (p0 & 1) ^ ((p0 >> 2) & 1);
+                    const int m0 = metric[p0] + (a0 ^ cc[0]) + (a1 ^ cc[1]);
+                    const int m1 = metric[p1] + (a0 ^ 1 ^ cc[0]) + (a1 ^ 1 ^ cc[1]);
+                    const bool take1 = m1 < m0;                    // a tie keeps dropped bit 0
+                    nm[s] = take1 ? m1 : m0;
+                    dw |= (unsigned)take1 << s;
+                }
+#pragma unroll
+                for (int s = 0; s < 16; ++s) metric[s] = nm[s];
+                dec[lane][t] = (unsigned short)dw;
+            }
+            ham = metric[0];
+            // traceback from state 0: u(t) = s & 1.  Fire: rem = sum u(t) D^(223-t) mod g, built from the low powers up.
+            unsigned long long rem = 0ull, pwr = 1ull;
+            int s = 0, acc = 0;
+            for (int t = BD_STEPS - 1; t >= 0; --t) {
+                const int u = s & 1;
+                s = (s >> 1) | ((((int)dec[lane][t] >> s) & 1) << 3);
+                if (t < 224) {
+                    if (u) rem ^= pwr;
+                    pwr <<= 1;
+                    if (pwr >> 40) pwr ^= SI_FIRE_G;
+                }
+                if (t < 184) {
+                    acc |= u << (t & 7);
+                    if ((t & 7) == 0) { pay[t >> 3] = (unsigned char)acc; acc = 0; }
+                }
+            }
+            if (rem != 0xFFFFFFFFFFull) fl |= SI_BLK_FIRE;
+            else {
+                ++n_fire;
+                const int mt = pay[2];
+                int bit = 256;
+                if (pay[1] == 0x06) {
+                    switch (mt) {
+                        case 0x19: bit = 1; break;   case 0x1A: bit = 2; break;   case 0x02: bit = 4; break;
+                        case 0x03: bit = 8; break;   case 0x07: bit = 16; break;  case 0x1B: bit = 32; break;
+                        case 0x1C: bit = 64; break;  case 0x00: bit = 128; break; default: break;
+                    }
+                }
+                mask |= bit;
+                if (bit == 32) {
+                    ++n_si3;
+                    kv = 0ull;
+                    for (int m = 0; m < 7; ++m) kv |= (unsigned long long)pay[3 + m] << (8 * m);
+                }
+            }
+        }
+        fn_out[ob] = fn; tc_out[ob] = (unsigned char)tc; flag_out[ob] = (unsigned char)fl; ham_out[ob] = (unsigned short)ham;
+        for (int m = 0; m < 23; ++m) payload[ob * 23 + m] = pay[m];
+        key[ob] = kv;
+    }
+    n_fire = __reduce_add_sync(0xffffffffu, n_fire);
+    n_si3 = __reduce_add_sync(0xffffffffu, n_si3);
+    mask = (int)__reduce_or_sync(0xffffffffu, (unsigned)mask);
+    __syncwarp();                                                  // every lane's keys are visible to the warp
+    SysinfoDev o;
+    o.n_blocks = n; o.n_fire_ok = n_fire; o.n_si3 = n_si3; o.n_si3_agree = 0; o.flags = 0; o.si_mask = mask;
+    o.mcc = o.mnc = o.mnc_digits = o.lac = o.ci = -1; o.reserved = 0;
+    const int rf = rec[stream].flags;
+    if (n < 0) o.flags = (rf & DM_NO_POS_INFO) ? SI_NO_POS_INFO : SI_NO_R_CORRECT;
+    else {
+        if (!cell) o.flags |= SI_NO_CELL;
+        if (carrier[stream].flags & CF_FEW) o.flags |= SI_UNCORRECTED;
+        if (n_si3 == 0) o.flags |= SI_NO_SI3;
+        else {
+            int best_cnt = 0, best_first = 0x7fffffff;
+            unsigned long long best_key = ~0ull;
+            for (int i = lane; i < n; i += 32) {
+                const unsigned long long ki = key[base + i];
+                if (ki == ~0ull) continue;
+                int cnt = 0, first = i;
+                for (int j = 0; j < n; ++j) {
+                    if (key[base + j] != ki) continue;
+                    ++cnt;
+                    if (j < first) first = j;
+                }
+                if (cnt > best_cnt || (cnt == best_cnt && first < best_first)) { best_cnt = cnt; best_first = first; best_key = ki; }
+            }
+            for (int s = 16; s > 0; s >>= 1) {
+                const int c2 = __shfl_xor_sync(0xffffffffu, best_cnt, s), f2 = __shfl_xor_sync(0xffffffffu, best_first, s);
+                const unsigned long long k2 = __shfl_xor_sync(0xffffffffu, best_key, s);
+                if (c2 > best_cnt || (c2 == best_cnt && f2 < best_first)) { best_cnt = c2; best_first = f2; best_key = k2; }
+            }
+            auto oct = [&](int m) { return (int)(best_key >> (8 * (m - 3))) & 0xFF; };     // octets 3..9
+            o.n_si3_agree = best_cnt;
+            if (best_cnt < n_si3) o.flags |= SI_SI3_DISAGREE;
+            o.ci = (oct(3) << 8) | oct(4);
+            o.mcc = 100 * (oct(5) & 15) + 10 * (oct(5) >> 4) + (oct(6) & 15);
+            const int d3 = oct(6) >> 4, m1 = oct(7) & 15, m2 = oct(7) >> 4;
+            o.mnc_digits = (d3 == 15) ? 2 : 3;
+            o.mnc = (d3 == 15) ? 10 * m1 + m2 : 100 * m1 + 10 * m2 + d3;
+            o.lac = (oct(8) << 8) | oct(9);
+        }
+    }
+    if (lane == 0) out[stream] = o;
+}

@@ -44,6 +44,11 @@ class CarrierFitResult(C.Structure):
                 ("residual_ppm", C.c_double), ("carrier_fit_ppm", C.c_double), ("drift_ppm_per_s", C.c_double)]
 
 
+class SysinfoResult(C.Structure):
+    _fields_ = [(n, C.c_int32) for n in ("n_blocks", "n_fire_ok", "n_si3", "n_si3_agree", "flags", "si_mask", "mcc", "mnc", "mnc_digits",
+                                         "lac", "ci", "reserved")]
+
+
 # the leading arguments of gsmcal_calibrate_batch and its variants: raw, raw_mem, n_iq, D, carrier_freq, tpl, coef, n_taps, osr,
 # coarse_dr, results, coarse_pos, coarse_snr, fcch_pos, pos_info, cuda_stream
 _BATCH = [C.c_void_p, C.c_int, c_i64, c_i64, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 6
@@ -92,6 +97,7 @@ SIGNATURES = {
     "gsmcal_calibrate_sch_timing_batch": (C.c_int, _BATCH + [C.c_void_p] * 3),
     "gsmcal_calibrate_carrier_fit_batch": (C.c_int, _BATCH + [C.c_void_p] * 4),
     "gsmcal_calibrate_cell_batch": (C.c_int, _BATCH + [C.c_void_p] * 13),
+    "gsmcal_calibrate_sysinfo_batch": (C.c_int, _BATCH + [C.c_void_p] * 23),
     "gsmcal_calibrate_batch_submit": (C.c_int, [C.c_int, C.c_void_p, c_i64, c_i64, C.c_double, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "gsmcal_calibrate_batch_collect": (C.c_int, [C.c_int]),

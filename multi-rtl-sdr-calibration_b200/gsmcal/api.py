@@ -11,7 +11,8 @@ import ctypes as C
 
 import numpy as np
 
-from ._lib import BcchResult, CarrierFitResult, DemodResult, GsmcalError, SchDecodeResult, SchTimingResult, StreamResult, check, lib  # noqa: F401
+from ._lib import (BcchResult, CarrierFitResult, DemodResult, GsmcalError, SchDecodeResult, SchTimingResult, StreamResult,  # noqa: F401
+                   SysinfoResult, check, lib)
 
 SYMBOL_RATE = (1625.0 / 6.0) * 1e3
 
@@ -330,7 +331,7 @@ def _batch_args(raw, carrier_freq, sch_training_sequence, coef, osr, coarse_dr, 
 def calibrate_batch(raw, carrier_freq: float, sch_training_sequence, coef, osr: int = 8, coarse_dr: int = 8,
                     device_ptr: int | None = None, n_iq: int | None = None, n_streams: int | None = None,
                     cuda_stream: int = 0, details: bool = True, r_correct=None, r_device_ptr: int | None = None,
-                    sch_timing: bool = False, carrier_fit: bool = False, sch_decode: bool = False):
+                    sch_timing: bool = False, carrier_fit: bool = False, sch_decode: bool = False, sysinfo: bool = False):
     """gsm_sync_demod.m:107-124 for every row of `raw` ([D, 2N] uint8, row d == dongle d's fread column).
 
     `raw` is a host NumPy array, or pass device_ptr/n_iq/n_streams for a capture already resident in HBM.
@@ -356,13 +357,22 @@ def calibrate_batch(raw, carrier_freq: float, sch_training_sequence, coef, osr: 
       cell: calibrate_demod_batch(..., sch_decode=True)'s cell dict plus df, the residual removed from each SCH row (Hz; NaN without a
             fit, where flags has SCHDEC_UNCORRECTED and the rows are demodulated as calibrate_demod_batch does);
       sch:  dict(demod_bits [n x 148], corr_val [n x 85], sch_ok [n] bool) of the corrected rows, n = SCH rows of pos_info.
-    cell's per-row arrays and sch are None where SCH_demod did not run.  frame_clock_offsets takes these results as they are."""
+    cell's per-row arrays and sch are None where SCH_demod did not run.  frame_clock_offsets takes these results as they are.
+
+    sysinfo=True (only with carrier_fit=True and sch_decode=True) then decodes every BCCH block of pos_info with the training sequence of
+    the cell's BCC (gsmcal_calibrate_sysinfo_batch, include/gsmcal.h); each dict also gains
+      sysinfo: dict(n_blocks, n_fire_ok, n_si3, n_si3_agree, flags, si_mask, mcc, mnc, mnc_digits, lac, ci, cgi, fn, tc, block_flags,
+               hamming, payload, lag, row_flags, steal): flags SI_* bits, si_mask SI_HAS_* bits, the SI3 fields (-1 without an SI3) and
+               cgi = (mcc, mnc, mnc_digits, lac, ci) or None; per block fn, tc, block_flags, hamming [n] and payload [n x 23] uint8; per
+               BCCH row lag, row_flags, steal [n x 4] (lag -128 where the row was not correlated).  The arrays are None when n_blocks < 0."""
     if (sch_timing or carrier_fit) and (r_correct is not None or r_device_ptr is not None):
         raise ValueError("sch_timing / carrier_fit do not combine with r_correct / r_device_ptr")
     if sch_timing and carrier_fit:
         raise ValueError("sch_timing and carrier_fit are separate calls")
     if sch_decode and (sch_timing or not carrier_fit):
         raise ValueError("calibrate_batch decodes SCH bursts only with carrier_fit=True and without sch_timing")
+    if sysinfo and not (carrier_fit and sch_decode):
+        raise ValueError("calibrate_batch decodes BCCH blocks only with carrier_fit=True and sch_decode=True")
     details = details or sch_timing or carrier_fit
     args, keep, D, n_iq, cap, res, arrays = _batch_args(raw, carrier_freq, sch_training_sequence, coef, osr, coarse_dr, device_ptr, n_iq,
                                                         n_streams, cuda_stream, details)
@@ -379,8 +389,17 @@ def calibrate_batch(raw, carrier_freq: float, sch_training_sequence, coef, osr: 
             sch_ok, bits, corr = np.zeros((D, cap), dtype=np.uint8), np.zeros((D, cap, 148), dtype=np.uint8), np.zeros((D, cap, 85))
             df, fn, bsic = np.empty((D, cap)), np.empty((D, cap), dtype=np.int32), np.empty((D, cap), dtype=np.int32)
             ham, rfl = np.empty((D, cap), dtype=np.uint8), np.empty((D, cap), dtype=np.uint8)
-            check(lib().gsmcal_calibrate_cell_batch(*args, *cf_args, C.cast(sd, C.c_void_p), _ptr(sch_ok), _ptr(bits), _ptr(corr), _ptr(df),
-                                                    _ptr(fn), _ptr(bsic), _ptr(ham), _ptr(rfl)))
+            cell_args = [C.cast(sd, C.c_void_p), _ptr(sch_ok), _ptr(bits), _ptr(corr), _ptr(df), _ptr(fn), _ptr(bsic), _ptr(ham), _ptr(rfl)]
+            if sysinfo:
+                nts = np.ascontiguousarray(gsm_normal_training_sequence_gen(osr).T)          # column-major (26*osr) x 8
+                si = (SysinfoResult * D)()
+                lag, brf, steal = (np.empty((D, cap, 4), dtype=t) for t in (np.int8, np.uint8, np.uint8))
+                bfn, btc, bfl = np.empty((D, cap), dtype=np.int32), np.empty((D, cap), dtype=np.uint8), np.empty((D, cap), dtype=np.uint8)
+                bham, pay = np.empty((D, cap), dtype=np.uint16), np.empty((D, cap, 23), dtype=np.uint8)
+                check(lib().gsmcal_calibrate_sysinfo_batch(*args, *cf_args, *cell_args, _ptr(nts), C.cast(si, C.c_void_p), _ptr(lag), _ptr(brf),
+                                                           _ptr(steal), _ptr(bfn), _ptr(btc), _ptr(bfl), _ptr(bham), _ptr(pay)))
+            else:
+                check(lib().gsmcal_calibrate_cell_batch(*args, *cf_args, *cell_args))
         else:
             check(lib().gsmcal_calibrate_carrier_fit_batch(*args, *cf_args))
     elif r_correct is None and r_device_ptr is None:
@@ -417,6 +436,15 @@ def calibrate_batch(raw, carrier_freq: float, sch_training_sequence, coef, osr: 
             item["cell"]["df"] = None if n < 0 else df[d, :n].copy()
             item["sch"] = None if n < 0 else dict(demod_bits=bits[d, :n].astype(np.int64), corr_val=corr[d, :n].copy(),
                                                   sch_ok=sch_ok[d, :n].astype(bool))
+    if sysinfo:
+        for d, item in enumerate(out):
+            r, n = si[d], si[d].n_blocks
+            rows = lambda a: None if n < 0 else a[d, :n].astype(np.int64)          # noqa: E731
+            item["sysinfo"] = dict(n_blocks=n, n_fire_ok=r.n_fire_ok, n_si3=r.n_si3, n_si3_agree=r.n_si3_agree, flags=r.flags,
+                                   si_mask=r.si_mask, mcc=r.mcc, mnc=r.mnc, mnc_digits=r.mnc_digits, lac=r.lac, ci=r.ci,
+                                   cgi=None if r.flags & SI_NO_SI3 or n < 0 else (r.mcc, r.mnc, r.mnc_digits, r.lac, r.ci),
+                                   fn=rows(bfn), tc=rows(btc), block_flags=rows(bfl), hamming=rows(bham),
+                                   payload=None if n < 0 else pay[d, :n].copy(), lag=rows(lag), row_flags=rows(brf), steal=rows(steal))
     return out
 
 
@@ -436,6 +464,11 @@ BCCH_NO_POS_INFO, BCCH_FEW_BCCH, BCCH_FCCH_RANGE, BCCH_TRAIN_RANGE = 1, 2, 4, 8
 SCHDEC_NO_POS_INFO, SCHDEC_NO_R_CORRECT, SCHDEC_NONE, SCHDEC_DISAGREE = 1, 2, 4, 8
 SCHDEC_ROW_WINDOW, SCHDEC_ROW_ALIGN, SCHDEC_ROW_CRC, SCHDEC_ROW_FIELD = 1, 2, 4, 8
 SCHDEC_UNCORRECTED = 16                            # calibrate_batch(..., carrier_fit=True, sch_decode=True): no fit, rows not corrected
+SI_NO_POS_INFO, SI_NO_R_CORRECT, SI_NO_CELL, SI_UNCORRECTED, SI_NO_SI3, SI_SI3_DISAGREE = 1, 2, 4, 8, 16, 32
+SI_ROW_RANGE, SI_ROW_EDGE = 1, 2
+SI_BLK_FN, SI_BLK_ROW, SI_BLK_FIRE, SI_BLK_SHORT = 1, 2, 4, 8
+SI_HAS = {0x19: 1, 0x1A: 2, 0x02: 4, 0x03: 8, 0x07: 16, 0x1B: 32, 0x1C: 64, 0x00: 128}     # message type -> si_mask bit
+SI_HAS_OTHER = 256
 FN_MOD = 2715648                                   # TDMA frames in a hyperframe
 
 

@@ -204,7 +204,8 @@ class DongleIngest:
 
 def calibrate_from_dongles(endpoints, num_sample: int, freq: float, n_captures: int = 1, osr: int = 8,
                            coarse_dr: int = 8, gain: float = 0, details: bool = True, demod: bool = False,
-                           sch_timing: bool = False, carrier_fit: bool = False, sch_decode: bool = False, **kw):
+                           sch_timing: bool = False, carrier_fit: bool = False, sch_decode: bool = False,
+                           sysinfo: bool = False, **kw):
     """gsm_sync_demod.m:57-124 with every dongle of `endpoints` in one batched library call per capture.
 
     Returns a list (one entry per capture) of the per-dongle result lists of `calibrate_batch`.  With demod=True the call is
@@ -215,7 +216,9 @@ def calibrate_from_dongles(endpoints, num_sample: int, freq: float, n_captures: 
     carrier_fit=True (and demod False) the call is `calibrate_batch(..., carrier_fit=True)`: each per-dongle dict carries its carrier
     entry, the unbiased carrier ppm of the dongle and its drift over the capture; with sch_decode=True as well it is
     `calibrate_batch(..., carrier_fit=True, sch_decode=True)` and each dict also carries its cell: BSIC, frame number and capture start on
-    the cell's frame clock from SCH bursts with the fitted residual removed (frame_clock_offsets aligns the dongles)."""
+    the cell's frame clock from SCH bursts with the fitted residual removed (frame_clock_offsets aligns the dongles); with sysinfo=True as
+    well each dict also carries its sysinfo: the decoded BCCH blocks and the cell's CGI from SI3, so dongles on the same cell can be told
+    from dongles on cells that share a BSIC."""
     from . import api
     fs = (1625.0 / 6.0) * 1e3 * osr
     coef = api.fir1(46, 200e3 / fs)                                 # gsm_sync_demod.m:34
@@ -228,5 +231,5 @@ def calibrate_from_dongles(endpoints, num_sample: int, freq: float, n_captures: 
                 out.append(api.calibrate_demod_batch(buf, freq, tpl, coef, osr, coarse_dr, normal_training_sequence=nts))
             else:
                 out.append(api.calibrate_batch(buf, freq, tpl, coef, osr, coarse_dr, details=details, sch_timing=sch_timing,
-                                               carrier_fit=carrier_fit, sch_decode=sch_decode))
+                                               carrier_fit=carrier_fit, sch_decode=sch_decode, sysinfo=sysinfo))
     return out

@@ -66,6 +66,8 @@ class StreamSpec:
     bsic: int | None = None         # 0..63: every SCH burst carries the coded (BSIC, FN) of TS 45.003 4.7; None = random coded bits
     fn0: int = 0                    # TDMA frame number of slot 0's frame (a multiple of 51, below FN_MOD)
     carrier_drift_ppm_per_s: float = 0.0   # the carrier error grows by this much per second of receiver time (a warming crystal)
+    sysinfo: tuple | None = None    # eight 23-octet BCCH messages indexed by TC = (FN div 51) mod 8 (needs bsic and tsc == bsic & 7);
+                                    # None = random bits in frames 2..5
 
 
 def random_spec(seed: int, n_samples: int, carrier_freq: float = 957.4e6) -> StreamSpec:
@@ -122,6 +124,62 @@ def sch_encode(bsic: int, fn: int) -> np.ndarray:
     return np.array(c, dtype=np.int64)
 
 
+FIRE_G = (1 << 40) | (1 << 26) | (1 << 23) | (1 << 17) | (1 << 3) | 1     # TS 45.003 4.1.2
+
+
+def bcch_encode(msg) -> np.ndarray:
+    """[4, 114] coded bits of one BCCH block (TS 45.003 4.1): the 184 data bits d(8m + q) = bit q of octet m (OsmocomBB's LSB-first
+    packing), the 40 Fire parity bits that leave the remainder 1 + D + ... + D^39, four tail bits, the rate-1/2 code of the SCH, and the
+    block-diagonal interleaver over four bursts.  Row B holds i(B, 0..113); parity with a live cell is unverified (no recorded capture)."""
+    msg = bytes(msg)
+    assert len(msg) == 23
+    d = [(msg[m] >> q) & 1 for m in range(23) for q in range(8)]
+    rem = 0
+    for b in d + [0] * 40:                                              # d(D) * D^40 mod g(D)
+        rem = (rem << 1) | b
+        if rem >> 40:
+            rem ^= FIRE_G
+    u = d + [((rem ^ ((1 << 40) - 1)) >> (39 - i)) & 1 for i in range(40)] + [0, 0, 0, 0]
+    c = []
+    for k in range(228):
+        v = lambda j: u[k - j] if k >= j else 0                         # noqa: E731
+        c += [v(0) ^ v(3) ^ v(4), v(0) ^ v(1) ^ v(3) ^ v(4)]
+    out = np.zeros((4, 114), dtype=np.int64)
+    for k in range(456):
+        out[k % 4, 2 * ((49 * k) % 57) + ((k % 8) // 4)] = c[k]
+    return out
+
+
+def _lai(mcc: int, mnc: int, mnc_digits: int, lac: int) -> list:
+    """the 5-octet Location Area Identification (TS 24.008 10.5.1.3): MCC / MNC as BCD nibbles, MNC digit 3 = 0xF for 2 digits"""
+    assert 0 <= mcc <= 999 and mnc_digits in (2, 3) and 0 <= mnc < 10 ** mnc_digits and 0 <= lac <= 0xFFFF
+    d1, d2, d3 = mcc // 100, mcc // 10 % 10, mcc % 10
+    m1, m2, m3 = (mnc // 10, mnc % 10, 0xF) if mnc_digits == 2 else (mnc // 100, mnc // 10 % 10, mnc % 10)
+    return [(d2 << 4) | d1, (m3 << 4) | d3, (m2 << 4) | m1, lac >> 8, lac & 0xFF]
+
+
+def si3_message(ci: int, mcc: int, mnc: int, lac: int, mnc_digits: int = 2) -> bytes:
+    """a well-formed System Information type 3 (TS 44.018 9.1.35): L2 pseudo length, RR, 0x1B, Cell Identity, LAI, control channel
+    description, cell options, cell selection parameters, RACH control, rest octets padded with 0x2B"""
+    assert 0 <= ci <= 0xFFFF
+    m = [0x49, 0x06, 0x1B, ci >> 8, ci & 0xFF] + _lai(mcc, mnc, mnc_digits, lac) + [0x49, 0x03, 0x05, 0x27, 0x47, 0x40, 0xE5, 0x04, 0x00]
+    return bytes(m + [0x2B] * (23 - len(m)))
+
+
+def si4_message(mcc: int, mnc: int, lac: int, mnc_digits: int = 2) -> bytes:
+    """a well-formed System Information type 4 (TS 44.018 9.1.36): LAI, cell selection parameters, RACH control, padding"""
+    m = [0x31, 0x06, 0x1C] + _lai(mcc, mnc, mnc_digits, lac) + [0x47, 0x40, 0xE5, 0x04, 0x00]
+    return bytes(m + [0x2B] * (23 - len(m)))
+
+
+def cell_sysinfo(ci: int, mcc: int, mnc: int, lac: int, mnc_digits: int = 2) -> tuple:
+    """StreamSpec.sysinfo of a cell: SI1, SI2, SI3, SI4, SI2quater, SI13, SI3, SI4 on TC 0..7 (TS 45.002 6.3.1.3's usual plan); the
+    messages other than SI3 / SI4 carry their message type and a fixed filler"""
+    other = lambda mt: bytes([0x59, 0x06, mt] + [(mt * 37 + 11 * i) & 0xFF for i in range(20)])      # noqa: E731
+    si3, si4 = si3_message(ci, mcc, mnc, lac, mnc_digits), si4_message(mcc, mnc, lac, mnc_digits)
+    return (other(0x19), other(0x1A), si3, si4, other(0x07), other(0x00), si3, si4)
+
+
 def _slot_bits(n_slots: int, gen: torch.Generator, device, drop_fcch=(), tsc=None) -> torch.Tensor:
     """[n_slots, 156] bits: TS0 of frames 0/10/20/30/40 (mod 51) FCCH, 1/11/21/31/41 SCH, else random."""
     bits = torch.randint(0, 2, (n_slots, SYM_PER_SLOT), generator=gen, device=device, dtype=torch.int64)
@@ -151,7 +209,8 @@ def _slot_bits(n_slots: int, gen: torch.Generator, device, drop_fcch=(), tsc=Non
 def stream_bits(spec: StreamSpec, gen: torch.Generator | None = None, device="cpu") -> torch.Tensor:
     """[n_slots, 156] burst bits of the stream (what generate_stream modulates); gen: the stream's generator, seeded here when None.
     With spec.bsic set, the coded SCH bits are written over bits 3..41 and 106..144 of every SCH burst after the random draws, so the
-    generator's later draws (the noise) and every other bit are those of bsic=None."""
+    generator's later draws (the noise) and every other bit are those of bsic=None; spec.sysinfo likewise writes the coded BCCH block
+    of message[TC] and stealing bits 1, 1 over TS0 of frames 2..5 of every multiframe."""
     dev = torch.device(device)
     if gen is None:
         gen = torch.Generator(device=dev)
@@ -167,6 +226,17 @@ def stream_bits(spec: StreamSpec, gen: torch.Generator | None = None, device="cp
                 c = torch.from_numpy(sch_encode(spec.bsic, (spec.fn0 + s // 8) % FN_MOD)).to(dev)
                 bits[s, 3:42] = c[:39]
                 bits[s, 106:145] = c[39:]
+    if spec.sysinfo is not None:
+        assert spec.bsic is not None and spec.tsc == spec.bsic & 7 and len(spec.sysinfo) == 8
+        coded = [torch.from_numpy(bcch_encode(m)).to(dev) for m in spec.sysinfo]
+        for s in range(0, n_slots, 8):
+            f = (s // 8) % 51
+            if 2 <= f <= 5:
+                i = coded[((spec.fn0 + s // 8) % FN_MOD) // 51 % 8][f - 2]
+                bits[s, 3:60] = i[:57]
+                bits[s, 88:145] = i[57:]
+                bits[s, 60] = 1                                         # stealing bits: a control channel block
+                bits[s, 87] = 1
     return bits
 
 

@@ -111,7 +111,7 @@ static void batch_outputs(int nlhs, mxArray *plhs[], const gsmcal_stream_result 
 }
 
 /* ------------------------------------------------------------------------------------------------ */
-#if defined(GSMCAL_MEX_gsm_calibrate_carrier_batch) || defined(GSMCAL_MEX_gsm_calibrate_cell_batch)
+#if defined(GSMCAL_MEX_gsm_calibrate_carrier_batch) || defined(GSMCAL_MEX_gsm_calibrate_cell_batch) || defined(GSMCAL_MEX_gsm_calibrate_sysinfo_batch)
 /* 1 x D struct array of the carrier fit: the records and the per-FCCH-row f, t, row_flags ([D][B]) */
 static mxArray *carrier_struct(const gsmcal_carrier_fit_result *cf, const double *fr, const double *tr, const uint8_t *rf, size_t D, size_t B) {
     const char *f[] = {"carrier_fit_ppm", "drift_ppm_per_s", "t_mean", "freq_hz", "drift_hz_per_s", "rms_hz", "residual_ppm", "n_fit", "flags",
@@ -133,7 +133,7 @@ static mxArray *carrier_struct(const gsmcal_carrier_fit_result *cf, const double
 }
 #endif
 
-#if defined(GSMCAL_MEX_gsm_calibrate_sch_decode_batch) || defined(GSMCAL_MEX_gsm_calibrate_cell_batch)
+#if defined(GSMCAL_MEX_gsm_calibrate_sch_decode_batch) || defined(GSMCAL_MEX_gsm_calibrate_cell_batch) || defined(GSMCAL_MEX_gsm_calibrate_sysinfo_batch)
 /* 1 x D struct array of the SCH decoding: the records and the per-SCH-row fn, bsic, hamming, row_flags ([D][B]); with df ([D][B], or
  * NULL) also the residual removed from each row */
 static mxArray *cell_struct(const gsmcal_sch_decode_result *sd, const int32_t *sfn, const int32_t *sbs, const uint8_t *sham, const uint8_t *srf,
@@ -450,6 +450,77 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
     if (nlhs > 4) plhs[4] = carrier_struct(cf, fr, tr, rf, D, B);
     if (nlhs > 5) plhs[5] = cell_struct(sd, sfn, sbs, sham, srf, df, D, B);
     mxFree(cf); mxFree(sd); mxFree(fr); mxFree(sfn); mxFree(rf); mxFree(res); mxFree(pi); if (own) mxFree((void *)tpl);
+}
+
+#elif defined(GSMCAL_MEX_gsm_calibrate_sysinfo_batch)
+/* [sampling_ppm, carrier_ppm, n_pos_info, pos_info, carrier, cell, sysinfo] = gsm_calibrate_sysinfo_batch(raw_uint8, carrier_freq,
+ *                                                                           sch_training_sequence, coef, normal_training_sequence)
+ * gsmcal_calibrate_sysinfo_batch: gsm_calibrate_cell_batch (outputs 1-6 as there), then every BCCH block of pos_info decoded with the
+ * training sequence of the cell's BCC.  sysinfo: 1 x D struct array with the record's fields (n_blocks, n_fire_ok, n_si3, n_si3_agree,
+ * flags, si_mask, mcc, mnc, mnc_digits, lac, ci) and per block fn, tc, block_flags, hamming (1 x n_blocks), payload (23 x n_blocks uint8)
+ * and per BCCH row lag, row_flags, steal (4 x n_blocks).  normal_training_sequence: (26*8) x 8 complex, gsm_normal_training_sequence_gen(8).
+ * See include/gsmcal.h. */
+void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
+    init_once();
+    if (nrhs != 5 || nlhs > 7)
+        mexErrMsgIdAndTxt("gsmcal:nargin", "usage: [sampling_ppm,carrier_ppm,n_pos_info,pos_info,carrier,cell,sysinfo] = "
+                          "gsm_calibrate_sysinfo_batch(raw_uint8,carrier_freq,sch_training_sequence,coef,normal_training_sequence)");
+    if (!mxIsUint8(prhs[0])) mexErrMsgIdAndTxt("gsmcal:type", "raw must be uint8");
+    if (mxGetM(prhs[4]) != 26 * 8 || mxGetN(prhs[4]) != 8) mexErrMsgIdAndTxt("gsmcal:size", "normal_training_sequence must be 208 x 8");
+    size_t rows = mxGetM(prhs[0]), D = mxGetN(prhs[0]);
+    int own, own_n; const double *tpl = get_c128(prhs[2], &own), *nts = get_c128(prhs[4], &own_n);
+    size_t nt; const double *coef = real_vector(prhs[3], &nt);
+    int64_t n_iq = (int64_t)(rows / 2);
+    size_t B = (size_t)gsmcal_max_bursts((n_iq + 63) / 64, 8), R = D * B;
+    gsmcal_stream_result *res = (gsmcal_stream_result *)mxMalloc(D * sizeof(*res));
+    double *pi = (double *)mxMalloc(D * 12 * B * sizeof(double));
+    gsmcal_carrier_fit_result *cf = (gsmcal_carrier_fit_result *)mxMalloc(D * sizeof(*cf));
+    gsmcal_sch_decode_result *sd = (gsmcal_sch_decode_result *)mxMalloc(D * sizeof(*sd));
+    gsmcal_sysinfo_result *si = (gsmcal_sysinfo_result *)mxMalloc(D * sizeof(*si));
+    double *fr = (double *)mxMalloc(R * 3 * sizeof(double)), *tr = fr + R, *df = tr + R;
+    int32_t *sfn = (int32_t *)mxMalloc(R * 3 * sizeof(int32_t)), *sbs = sfn + R, *bfn = sbs + R;
+    uint8_t *rf = (uint8_t *)mxMalloc(R * (5 + 23 + 3 * 4)), *sham = rf + R, *srf = sham + R, *btc = srf + R, *bfl = btc + R, *pay = bfl + R;
+    uint8_t *brf = pay + 23 * R, *steal = brf + 4 * R;
+    int8_t *lag = (int8_t *)(steal + 4 * R);
+    uint16_t *bham = (uint16_t *)mxMalloc(R * sizeof(uint16_t));
+    fail_on(gsmcal_calibrate_sysinfo_batch((const uint8_t *)mxGetData(prhs[0]), GSMCAL_MEM_HOST, n_iq, (int64_t)D, mxGetScalar(prhs[1]), tpl, coef,
+                                           (int)nt, 8, 8, res, NULL, NULL, NULL, pi, NULL, cf, fr, tr, rf, sd, NULL, NULL, NULL, df, sfn, sbs, sham, srf,
+                                           nts, si, lag, brf, steal, bfn, btc, bfl, bham, pay),
+            "gsm_calibrate_sysinfo_batch");
+    batch_outputs(nlhs, plhs, res, pi, D, B);
+    if (nlhs > 4) plhs[4] = carrier_struct(cf, fr, tr, rf, D, B);
+    if (nlhs > 5) plhs[5] = cell_struct(sd, sfn, sbs, sham, srf, df, D, B);
+    if (nlhs > 6) {
+        const char *f[] = {"n_blocks", "n_fire_ok", "n_si3", "n_si3_agree", "flags", "si_mask", "mcc", "mnc", "mnc_digits", "lac", "ci", "fn", "tc",
+                           "block_flags", "hamming", "payload", "lag", "row_flags", "steal"};
+        mxArray *s = mxCreateStructMatrix(1, D, 19, f);
+        for (size_t d = 0; d < D; ++d) {
+            const gsmcal_sysinfo_result *c = si + d;
+            const int32_t v[11] = {c->n_blocks, c->n_fire_ok, c->n_si3, c->n_si3_agree, c->flags, c->si_mask, c->mcc, c->mnc, c->mnc_digits, c->lac, c->ci};
+            for (int j = 0; j < 11; ++j) mxSetField(s, d, f[j], scalar(v[j]));
+            const size_t k = c->n_blocks < 0 ? 0 : (size_t)c->n_blocks;
+            mxArray *a[4], *r[3];
+            for (int j = 0; j < 4; ++j) a[j] = mxCreateDoubleMatrix(1, k, mxREAL);
+            for (int j = 0; j < 3; ++j) r[j] = mxCreateDoubleMatrix(4, k, mxREAL);
+            size_t pd[2] = {23, k};
+            mxArray *p = mxCreateNumericArray(2, pd, mxUINT8_CLASS, mxREAL);
+            for (size_t i = 0; i < k; ++i) {
+                const size_t o = d * B + i;
+                mxGetPr(a[0])[i] = bfn[o]; mxGetPr(a[1])[i] = btc[o]; mxGetPr(a[2])[i] = bfl[o]; mxGetPr(a[3])[i] = bham[o];
+                for (int q = 0; q < 23; ++q) ((uint8_t *)mxGetData(p))[23 * i + q] = pay[23 * o + q];
+                for (int q = 0; q < 4; ++q) {
+                    mxGetPr(r[0])[4 * i + q] = lag[4 * o + q]; mxGetPr(r[1])[4 * i + q] = brf[4 * o + q]; mxGetPr(r[2])[4 * i + q] = steal[4 * o + q];
+                }
+            }
+            for (int j = 0; j < 4; ++j) mxSetField(s, d, f[11 + j], a[j]);
+            mxSetField(s, d, "payload", p);
+            for (int j = 0; j < 3; ++j) mxSetField(s, d, f[16 + j], r[j]);
+        }
+        plhs[6] = s;
+    }
+    mxFree(cf); mxFree(sd); mxFree(si); mxFree(fr); mxFree(sfn); mxFree(rf); mxFree(bham); mxFree(res); mxFree(pi);
+    if (own) mxFree((void *)tpl);
+    if (own_n) mxFree((void *)nts);
 }
 
 #elif defined(GSMCAL_MEX_gsm_calibrate_demod_batch) || defined(GSMCAL_MEX_gsm_calibrate_sch_decode_batch)
